@@ -18,8 +18,10 @@ and frame batches (configs[1], configs[2]) are sharded over the ranks (no collec
 `cpu_baseline`: the CPU oracle (a restatement of the reference's g2o path; the reference itself cannot be built here)
             on one host core per problem, on a bounded sample of the same workload.
 --impl reference : the CPU oracle on all host cores (rank 0 only).
+--dump-outputs DIR : the results of the last timed step as .npy files (inputs are seeded: two builds compare one to one).
 """
 import argparse
+import atexit
 import ctypes as C
 import json
 import os
@@ -62,6 +64,7 @@ class ClockSampler:
         try:
             self.proc = subprocess.Popen(["nvidia-smi", f"--id={self.device}", f"--query-gpu={q}", "--format=csv,noheader,nounits",
                                           "-lms", "100"], stdout=subprocess.PIPE, stderr=subprocess.DEVNULL, text=True)
+            atexit.register(self.proc.terminate)   # an exception before stop() must not leave the sampler running
             self.t = threading.Thread(target=self._read, daemon=True)
             self.t.start()
         except Exception:
@@ -135,6 +138,25 @@ def pinned_problem(p):
         else:
             out[k] = v
     return out, keep
+
+
+DUMP_BYTES = 60 << 20   # array data written by --dump-outputs; with the .npy headers the files stay under 64 MB
+
+
+def dump_outputs(path, out):
+    """Write the result arrays of the timed path (an lld_ba_result filled by lld_ba_download) as <path>/<name>.npy so that
+    two builds can be compared output for output.  Float arrays keep their dtype; integer and flag arrays are widened
+    exactly (uint8 -> float32, int32 -> float64).  When the whole result exceeds DUMP_BYTES, every array keeps the same
+    fraction of its rows, chosen by a fixed seed and kept in order: the sample depends only on the shapes."""
+    arrs = {k: v if v.dtype.kind == "f" else v.astype(np.float32 if v.itemsize <= 2 else np.float64)
+            for k, v in out.items() if isinstance(v, np.ndarray)}
+    frac = min(1.0, DUMP_BYTES / sum(v.nbytes for v in arrs.values()))
+    os.makedirs(path, exist_ok=True)
+    for k, v in arrs.items():
+        if frac < 1.0:
+            n = len(v)
+            v = v[np.sort(np.random.default_rng(0).choice(n, int(n * frac), replace=False))]
+        np.save(os.path.join(path, k + ".npy"), v)
 
 
 def edge_counts(p):
@@ -245,7 +267,7 @@ def run_reference_arm(args):
     cores = os.cpu_count() or 1
     if args.workload == "global_ba":
         p = synth.make_global_ba(*GBA_SHAPE, synth.seed_for(5))
-        steps = max(1, min(args.steps, 2))      # ~17 s per run on one core
+        steps = args.steps      # ~17 s per run on one core
         t0 = time.perf_counter()
         its = 0
         for _ in range(steps):
@@ -395,6 +417,9 @@ def bench_global_ba(args, R, lib, d, ctx, hbm_peak, peak_src):
     launches = ctx.launch_count() - l0
     nc, nb = C.c_int64(), C.c_int64()
     d.lld_ctx_nccl_stats(ctx.handle, C.byref(nc), C.byref(nb))
+    if args.dump_outputs:
+        ctx.check(d.lld_ba_download(ctx.handle, C.byref(prob), C.byref(res), 0), "download")
+        dump_outputs(args.dump_outputs, out)
     # the landmark outputs of the other ranks are not needed for the metric: download this rank's view of the trace
     ms = R.reduce([ms], "max")[0]
     launches = int(R.reduce([launches], "sum")[0])
@@ -463,7 +488,13 @@ def main():
     ap.add_argument("--workload", default="batched_local_ba", choices=["batched_local_ba", "global_ba"])
     ap.add_argument("--windows", type=int, default=64, help="local-BA windows per GPU")
     ap.add_argument("--no-extra", action="store_true", help="skip the secondary workloads and the CPU baselines")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write the results of the last one (rank 0's batch) as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.impl == "reference" or (args.workload == "global_ba" and int(os.environ.get("WORLD_SIZE", "1")) > 1)):
+        ap.error("--dump-outputs needs --impl ours, and one GPU for --workload global_ba (its landmarks are sharded)")
     if args.impl == "reference":
         run_reference_arm(args)
         return
@@ -516,6 +547,8 @@ def main():
     clocks = sampler.stop()
     launches = ctx.launch_count() - l0
     ctx.check(d.lld_ba_download(ctx.handle, C.byref(prob), C.byref(res), 1), "download")
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, out)
     iters_per_step = int(out["n_iter_done"].sum())
     trials_per_step = int(out["trials_log"].sum())
     ms = R.reduce([ms], "max")[0]
