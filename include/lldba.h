@@ -60,7 +60,17 @@ extern "C" {
 /* Capacity limits of this implementation (the reference has none; a call outside them returns LLD_ERR_ARG /
  * LLD_ERR_UNSUPPORTED and lld_ctx_last_error() names the limit):
  *   - at most 254 observations per landmark;
- *   - a keyframe may be covisible with at most 170 free keyframes in lld_ba_global (6 * neighbours <= 1024);
+ *   - a free keyframe may have at most 169 later free neighbours (6 * (neighbours + itself) <= 1024), else LLD_ERR_UNSUPPORTED.
+ *     In lld_ba_local every later free keyframe of the window counts as a neighbour, so this is a window of at most 170 free
+ *     keyframes; in lld_ba_global a neighbour is a later free keyframe that shares a landmark, and the envelope limit below
+ *     is always reached first;
+ *   - lld_ba_global: let B be the largest distance, in free-keyframe indices (fixed keyframes are skipped), between two free
+ *     keyframes that observe one landmark.  B <= 26 solves by block cyclic reduction over super-blocks of B keyframes
+ *     (6B <= 156); B >= 27 takes the single-CTA skyline LDL^T, whose envelope must fit 220 KB of shared memory.  For a
+ *     band-shaped envelope over n_free free keyframes that is 228 B + 6 n_free <= 27952: B <= 117 at 200 free keyframes,
+ *     B <= 83 at 1500.  A wider envelope (e.g. a loop-closure landmark across the map) returns LLD_ERR_UNSUPPORTED;
+ *   - lld_ba_global: one free keyframe observing the same landmark twice is LLD_ERR_ARG (lld_ba_local accepts it and takes the
+ *     sparse path);
  *   - local windows with more than 32 free keyframes take the general (slower) sparse path;
  *   - lld_sbp_*, lld_kf_search: n_levels <= 8, at most 65535 keypoints per frame; pairs with more than 2048 keypoints or queries
  *     take the multi-kernel path instead of the single-CTA one;

@@ -688,6 +688,38 @@ static int ba_upload(LldCtx* c, const lld_ba_problem* p, bool global_mode, int l
       fill_window(w, p->ln_off, p->ln_obs_off, lc_kf, ln_order, ll_off, ll_cell, lc_pos);
     });
   }
+  // sparse mode, a landmark seen more than once by one free keyframe: per (landmark, keyframe) the list position the position
+  // tables name (the last such edge) and the positions whose W records k_fold_dup adds into it
+  std::vector<int> fold_off(1, 0), fold_dst, fold_src;
+  int n_fold_pt = 0;
+  if (!dense && dup_free.load()) {
+    auto fold_groups = [&](int n_lm, const int* off, const pvec<int>& ekf, const pvec<int>& e_pos) {
+      std::vector<std::pair<int, int>> gs;   // (free block, edge) of one landmark, sorted: edges of a block in list order
+      for (int i = 0; i < n_lm; i++) {
+        gs.clear();
+        for (int e = off[i]; e < off[i + 1]; e++)
+          if (kf_g[ekf[e]] >= 0) gs.push_back({kf_g[ekf[e]], e});
+        std::sort(gs.begin(), gs.end());
+        for (size_t a = 0; a < gs.size();) {
+          size_t b = a + 1;
+          while (b < gs.size() && gs[b].first == gs[a].first) b++;
+          if (b - a > 1) {
+            fold_dst.push_back(e_pos[gs[b - 1].second]);
+            for (size_t k = a; k + 1 < b; k++) fold_src.push_back(e_pos[gs[k].second]);
+            fold_off.push_back((int)fold_src.size());
+          }
+          a = b;
+        }
+      }
+    };
+    fold_groups(n_pt, p->pt_obs_off, pe_kf, pe_pos);
+    n_fold_pt = (int)fold_dst.size();
+    fold_groups(n_ln, p->ln_obs_off, lc_kf, lc_pos);
+  }
+  v.n_fold = (int)fold_dst.size(); v.n_fold_pt = n_fold_pt;
+  UP(tmp_i, fold_off.data(), fold_off.size()); v.fold_off = tmp_i;
+  UP(tmp_i, fold_dst.data(), fold_dst.size()); v.fold_dst = tmp_i;
+  UP(tmp_i, fold_src.data(), fold_src.size()); v.fold_src = tmp_i;
   const int n_plist = pl_off[nG], n_llist = ll_off[nG];
   UP(tmp_i, pl_off.data(), nG + 1); v.pl_off = tmp_i;
   UP(tmp_i, pl_edge.data(), n_plist); v.pl_edge = tmp_i;
@@ -1162,7 +1194,10 @@ static int ba_upload(LldCtx* c, const lld_ba_problem* p, bool global_mode, int l
       }
     }
     if (!S->use_band && !S->use_cr && S->env_smem > 220 * 1024) {
-      snprintf(c->err, sizeof(c->err), "global BA: envelope of the reduced system too wide for the on-chip solver (panel %d rows, row %d, n %d)", ph, maxlen, n);
+      snprintf(c->err, sizeof(c->err),
+               "global BA: envelope of the reduced system too wide for the on-chip solver: a landmark spans %d free keyframes "
+               "(panel %d rows, row %d, n %d) and needs %zu bytes of shared memory, the limit is %d (include/lldba.h, capacity limits)",
+               B + 1, ph, maxlen, n, S->env_smem, 220 * 1024);
       return LLD_ERR_UNSUPPORTED;
     }
   }
@@ -1715,6 +1750,7 @@ static int ba_step(LldCtx* c, int round, int stop_now, bool first = true) {
     if (S->gather_long) LLD_LAUNCH(c, k_reduce_piece_warp, cdiv(nblk * 6 + v.n_free_total, 8), 256, 0, v, nblk);
     else LLD_LAUNCH(c, k_reduce_piece, cdiv(nblk * 36 + 6 * v.n_free_total, 256), 256, 0, v, nblk);
   } else {
+    if (v.n_fold) LLD_LAUNCH(c, k_fold_dup, cdiv(v.n_fold, 128), 128, 0, v);
     const int tpb = 32 * cdiv(6 * S->max_nnb, 32);
     const int nl = v.n_chunks - v.n_chunks_pt;
     if (tpb <= 256) {

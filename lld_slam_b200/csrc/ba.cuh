@@ -84,6 +84,13 @@ struct BaView {
   const long long* pl_tab_off;  // [n_free_total] offset of block a's first entry row
   const int* ll_tab;
   const long long* ll_tab_off;
+  // sparse mode, landmarks seen more than once by one free keyframe: fold group i adds the W records at list positions
+  // fold_src[fold_off[i] .. fold_off[i+1]) into the one at fold_dst[i] (the co-edge the tables name) and zeroes them;
+  // groups [0, n_fold_pt) are point records, the rest line records (k_fold_dup)
+  int n_fold, n_fold_pt;
+  const int* fold_off;
+  const int* fold_dst;
+  const int* fold_src;
   // dense mode (every window has <= 32 free keyframes): landmarks in co-visibility-signature order, W stored per
   // landmark with its free edges sorted by keyframe; k_schur_dense keeps a window's whole S in registers
   int dense_mode;

@@ -153,6 +153,27 @@ __global__ void k_build_tab(int n_list, int nG, const int* __restrict__ l_off, c
   }
 }
 
+// sparse mode, a landmark seen more than once by one free keyframe: the position tables name ONE co-edge per (landmark,
+// keyframe) (the last one, above), so k_schur_rows would pair W_e with only that edge.  H holds one landmark-pose block per
+// (landmark, keyframe) that all those edges add into (block_solver.hpp), so the records of the other edges are added into
+// the named one and zeroed: the Schur rows and the back-substitution then see the summed block.  Runs after the
+// linearisation has rewritten every record; a group is summed by one thread in list order.
+__global__ void k_fold_dup(BaView v) {
+  const int i = blockIdx.x * blockDim.x + threadIdx.x;
+  if (i >= v.n_fold) return;
+  const bool pt = i < v.n_fold_pt;
+  const int rec = pt ? 27 : 38, nw = pt ? 18 : 24;
+  double* base = pt ? v.P_rec : v.L_rec;
+  double* d = base + (size_t)rec * v.fold_dst[i];
+  for (int k = v.fold_off[i]; k < v.fold_off[i + 1]; k++) {
+    double* s = base + (size_t)rec * v.fold_src[k];
+    for (int q = 0; q < nw; q++) {
+      d[q] += s[q];
+      s[q] = 0.0;
+    }
+  }
+}
+
 // dense mode: the W blocks of a landmark are contiguous (first slot w0[sorted position]) and sorted by keyframe, so the
 // slot of an edge is w0 + the rank of its keyframe's block among the set bits of the landmark's mask; -1 = fixed keyframe
 __global__ void k_dense_wpos(int n_e, const int* __restrict__ e_lm, const int* __restrict__ e_kf, const int* __restrict__ kf_g,
@@ -2313,17 +2334,19 @@ __global__ void __launch_bounds__(LM_TPB) k_backsub_points(BaView v) {
   {
     const bool dense = v.dense_mode != 0;
     const int* epos = dense ? v.pe_wpos : v.pe_pos;
+    // a gated-out edge has W = 0 and is skipped, unless W records were folded (k_fold_dup): then it may hold the sum
+    const bool skip_gated = v.n_fold == 0;
     // (W slot, update block) of the edge one ahead of the arithmetic: the keyframe -> block -> x chain is three loads deep
     int e = e0 + gl, pos = -1, g = 0;
     if (e < e1 && go) {
-      pos = v.pe_level[e] != 0 ? -1 : epos[e];
+      pos = (skip_gated && v.pe_level[e] != 0) ? -1 : epos[e];
       g = v.kf_g[v.pe_kf[e]];
     }
     while (e < e1 && go) {
       const int en = e + PT_G;
       int pos_n = -1, g_n = 0;
       if (en < e1) {
-        pos_n = v.pe_level[en] != 0 ? -1 : epos[en];
+        pos_n = (skip_gated && v.pe_level[en] != 0) ? -1 : epos[en];
         g_n = v.kf_g[v.pe_kf[en]];
       }
       if (pos >= 0) {

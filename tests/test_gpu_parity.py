@@ -349,7 +349,8 @@ def test_no_cpu_fallback():
 
 
 def test_global_ba_banded_envelope(gpu_ctx):
-    """a chain of 200 keyframes: reduced system 1194 x 1194 with a band envelope, on-device skyline LDL^T."""
+    """a chain of 200 keyframes: reduced system 1194 x 1194 with a band envelope (half-bandwidth B = 19 keyframes), solved
+    by block cyclic reduction over super-blocks of 19 keyframes.  The skyline and band solvers: tests/test_ba_paths.py."""
     p = synth.make_global_ba(200, 20000, 4000, 19)
     g = api.ba_global(p, 6, impl="gpu", ctx=gpu_ctx)
     o = api.ba_global(p, 6, impl="oracle")
