@@ -68,7 +68,11 @@ extern "C" {
  *     keyframes that observe one landmark.  B <= 26 solves by block cyclic reduction over super-blocks of B keyframes
  *     (6B <= 156); B >= 27 takes the single-CTA skyline LDL^T, whose envelope must fit 220 KB of shared memory.  For a
  *     band-shaped envelope over n_free free keyframes that is 228 B + 6 n_free <= 27952: B <= 117 at 200 free keyframes,
- *     B <= 83 at 1500.  A wider envelope (e.g. a loop-closure landmark across the map) returns LLD_ERR_UNSUPPORTED;
+ *     B <= 83 at 1500.  A wider envelope (e.g. a loop-closure landmark across the map) returns LLD_ERR_UNSUPPORTED,
+ *     unless lld_ctx_set_gba_sparse(ctx, 1) is on: then it is solved by block elimination over super-blocks of mb
+ *     keyframes (mb = the largest such distance that is <= 26; longer ones become edges of the super-block graph), whose
+ *     plan (blocks with fill, Z factors, solution) must fit 2 GiB of device memory (2147483648 bytes), else
+ *     LLD_ERR_UNSUPPORTED with the plan's size in the message;
  *   - lld_ba_global: one free keyframe observing the same landmark twice is LLD_ERR_ARG (lld_ba_local accepts it and takes the
  *     sparse path);
  *   - local windows with more than 32 free keyframes take the general (slower) sparse path;
@@ -169,6 +173,18 @@ int lld_ba_local(void* ctx, const lld_ba_problem* p, int its_round1, int its_rou
  * rank stops at the same step whichever rank saw the flag first. */
 int lld_ba_global(void* ctx, const lld_ba_problem* p, int n_iter, const volatile uint8_t* stop_flag,
                   lld_ba_result* out);
+
+/* Global BA after a loop closure: on = 1 lets lld_ba_global solve a reduced camera system whose envelope is too wide
+ * for the on-chip solvers (a landmark seen by keyframes at both ends of the map) by block elimination over its
+ * super-block graph; on = 0 (the default) rejects it with LLD_ERR_UNSUPPORTED.  Problems that the other solvers take are
+ * not affected.  Part of the topology-cache key: a cached structure is indexed again when the switch changes. */
+void lld_ctx_set_gba_sparse(void* ctx, int on);
+
+/* The block-elimination plan lld_ba_global would run for p with the switch on, as JSON in buf (host arithmetic only, no
+ * device needed; for tests): super-block size mb, count N, the elimination levels with their neighbour lists, the
+ * off-diagonal blocks with fill, the Z offsets and the ordered Schur contributions of every output block.  A problem
+ * another solver takes gives {"solver":"other"}; an error code comes with its message in buf. */
+int lld_gba_sparse_plan_report(const lld_ba_problem* p, char* buf, int len);
 
 /* Landmark partition used by lld_ba_global on n_ranks>1: rank r owns points [out[0], out[1]) and lines
  * [out[2], out[3]) (contiguous blocks; keyframes are replicated).  Host arithmetic only, no device needed.

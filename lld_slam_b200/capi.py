@@ -263,6 +263,10 @@ class _Lib:
             d.lld_stereo_matches.restype = C.c_int
             d.lld_ctx_set_topo_cache.argtypes = [vp, C.c_int]
             d.lld_ctx_set_topo_cache.restype = None
+            d.lld_ctx_set_gba_sparse.argtypes = [vp, C.c_int]
+            d.lld_ctx_set_gba_sparse.restype = None
+            d.lld_gba_sparse_plan_report.argtypes = [C.POINTER(BaProblem), C.c_char_p, C.c_int]
+            d.lld_gba_sparse_plan_report.restype = C.c_int
             d.lld_ctx_nccl_stats.argtypes = [vp, c_i64p, c_i64p]
             d.lld_ctx_nccl_stats.restype = None
 

@@ -22,7 +22,12 @@
 #include "ba_kernels.cuh"
 #include "ba_fused.cuh"
 #include "cr_solver.cuh"
+#include "sp_solver.cuh"
 #include "lld_ctx.h"
+
+#include <array>
+#include <map>
+#include <string>
 
 #ifdef LLD_WITH_NCCL
 #include <nccl.h>
@@ -49,6 +54,12 @@ struct BaState {
   bool use_band = false;
   bool use_cr = false;     // global BA: block cyclic reduction of the reduced camera system (cr_solver.cuh)
   CrView cr{};
+  bool use_sp = false;     // global BA across loop closures: plan-driven block elimination (sp_solver.cuh)
+  SpView sp{};
+  struct SpLevel { int p0, n_el, ntile, u0, n_blk, n_rhs; };
+  std::vector<SpLevel> sp_levels;
+  long long sp_z_total = 0, sp_n_slot = 0;
+  std::string sp_report;   // JSON of the plan (host-only runs: lld_gba_sparse_plan_report)
   bool global_mode = false;
   bool forked = false;     // dense single-rank batch small enough that concurrent passes shorten the critical path
   bool use_graph = false;  // replay one captured LM step instead of re-launching its kernels
@@ -292,7 +303,8 @@ static uint64_t hash_words(const void* data, size_t bytes, uint64_t h) {
 }
 
 // everything the index tables depend on: window / landmark / observation offsets, observing keyframes, fixed flags
-static uint64_t ba_topology_hash(BaHost& H, const lld_ba_problem* p, bool global_mode, int log_stride, const lld_ba_problem* full, int n_ranks, int rank) {
+static uint64_t ba_topology_hash(BaHost& H, const lld_ba_problem* p, bool global_mode, int log_stride, const lld_ba_problem* full, int n_ranks, int rank,
+                                 int gba_sparse) {
   const int nw = p->n_win;
   const int n_kf = p->kf_off[nw], n_pt = p->pt_off[nw], n_ln = p->ln_off[nw];
   const int n_pe = p->pt_obs_off[n_pt], n_lc = p->ln_obs_off[n_ln];
@@ -312,8 +324,8 @@ static uint64_t ba_topology_hash(BaHost& H, const lld_ba_problem* p, bool global
   std::vector<uint64_t> hs(parts.size());
   H.par_for((int)parts.size(), [&](int i) { hs[(size_t)i] = hash_words(parts[(size_t)i].d, parts[(size_t)i].bytes, 0xCBF29CE484222325ull + (uint64_t)i); });
   uint64_t h = 0x84222325CBF29CE4ull;
-  const uint64_t meta[8] = {(uint64_t)nw, (uint64_t)global_mode, (uint64_t)log_stride, (uint64_t)n_ranks, (uint64_t)rank, (uint64_t)(full != nullptr),
-                            (uint64_t)n_pe, (uint64_t)n_lc};
+  const uint64_t meta[9] = {(uint64_t)nw, (uint64_t)global_mode, (uint64_t)log_stride, (uint64_t)n_ranks, (uint64_t)rank, (uint64_t)(full != nullptr),
+                            (uint64_t)n_pe, (uint64_t)n_lc, (uint64_t)gba_sparse};
   h = hash_words(meta, sizeof(meta), h);
   h = hash_words(hs.data(), 8 * hs.size(), h);
   return h;
@@ -329,6 +341,172 @@ static void ba_set_params(BaView& v, const lld_ba_problem* p) {
   v.prm.ln_filter = p->ln_filter;
 }
 
+// Symbolic plan of the block elimination of sp_solver.cuh, from the keyframe block pattern (nb lists) alone.
+// Super-blocks of mb consecutive free keyframes, mb = the largest distance <= 26 between two covisible free keyframes
+// (6 mb <= CR_MAX_M); longer distances become edges of the super-block graph.  Levels: a maximal independent set of the
+// remaining nodes, scanned in ascending (degree, index) order, is eliminated, and the remaining neighbours of each
+// eliminated node are joined pairwise (fill).  On a chain this is odd / even cyclic reduction; a ring takes ~log2 N levels.
+static const int SP_MAX_MB = CR_MAX_M / 6;
+static const long long SP_MAX_BYTES = 2LL << 30;   // device storage of one plan (include/lldba.h, capacity limits)
+
+struct SpPlan {
+  int mb = 1, N = 0, m = 6, n_orig = 0;
+  std::vector<std::pair<int, int>> blocks;   // off-diagonal slots N, N + 1, ...: (I, J), I < J, fill included
+  std::vector<int> q_slot, el_node, el_nb_off, nb_node, nb_slot2, up_out, up_c_off, c_slot2, c_pos, c_col;
+  std::vector<long long> z_off;
+  std::vector<BaState::SpLevel> levels;
+  long long z_total = 0, bytes = 0;
+};
+
+static void sp_plan_build(int nG, const std::vector<int>& nb_off, const std::vector<int>& nb_g, SpPlan& P) {
+  int mb = 1;
+  for (int a = 0; a < nG; a++)
+    for (int q = nb_off[a]; q < nb_off[a + 1]; q++)
+      if (nb_g[q] - a <= SP_MAX_MB) mb = std::max(mb, nb_g[q] - a);
+  const int N = (nG + mb - 1) / mb, m = 6 * mb;
+  P.mb = mb; P.N = N; P.m = m;
+  std::vector<std::vector<int>> adj((size_t)N);   // sorted, both directions
+  auto link = [&](int I, int J) {
+    auto& A = adj[(size_t)I];
+    auto it = std::lower_bound(A.begin(), A.end(), J);
+    if (it == A.end() || *it != J) A.insert(it, J);
+  };
+  for (int a = 0; a < nG; a++)
+    for (int q = nb_off[a]; q < nb_off[a + 1]; q++) {
+      const int I = a / mb, J = nb_g[q] / mb;
+      if (I != J) { link(I, J); link(J, I); }
+    }
+  for (auto& A : adj) P.n_orig += (int)A.size();
+  P.n_orig /= 2;
+  // levels
+  std::vector<char> alive((size_t)N, 1), blocked((size_t)N);
+  std::vector<std::vector<int>> lv_nodes, lv_nbrs;   // per position: its remaining neighbours
+  int n_alive = N;
+  while (n_alive > 0) {
+    std::vector<std::pair<int, int>> order;
+    for (int i = 0; i < N; i++)
+      if (alive[(size_t)i]) {
+        int d = 0;
+        for (int j : adj[(size_t)i]) d += alive[(size_t)j];
+        order.push_back({d, i});
+      }
+    std::sort(order.begin(), order.end());
+    std::fill(blocked.begin(), blocked.end(), 0);
+    std::vector<int> E;
+    for (auto& o : order) {
+      const int i = o.second;
+      if (blocked[(size_t)i]) continue;
+      E.push_back(i);
+      blocked[(size_t)i] = 1;
+      for (int j : adj[(size_t)i]) blocked[(size_t)j] = 1;
+    }
+    std::sort(E.begin(), E.end());
+    for (int i : E) {
+      std::vector<int> nb;
+      for (int j : adj[(size_t)i])
+        if (alive[(size_t)j]) nb.push_back(j);
+      lv_nbrs.push_back(nb);
+    }
+    for (size_t e = 0; e < E.size(); e++) {
+      const auto& nb = lv_nbrs[lv_nbrs.size() - E.size() + e];
+      for (size_t x = 0; x < nb.size(); x++)
+        for (size_t y = x + 1; y < nb.size(); y++) { link(nb[x], nb[y]); link(nb[y], nb[x]); }
+    }
+    for (int i : E) alive[(size_t)i] = 0;
+    n_alive -= (int)E.size();
+    lv_nodes.push_back(E);
+  }
+  // slots: diagonal I, then every off-diagonal block of the filled pattern in (I, J) order
+  std::map<std::pair<int, int>, int> slot;
+  for (int I = 0; I < N; I++)
+    for (int J : adj[(size_t)I])
+      if (J > I) { slot[{I, J}] = N + (int)P.blocks.size(); P.blocks.push_back({I, J}); }
+  auto slot2 = [&](int i, int j) { return i < j ? 2 * slot[{i, j}] : 2 * slot[{j, i}] + 1; };   // U_ij, transposed when stored as (j, i)
+  P.q_slot.resize(nb_g.size());
+  for (int a = 0; a < nG; a++)
+    for (int q = nb_off[a]; q < nb_off[a + 1]; q++) {
+      const int I = a / mb, J = nb_g[q] / mb;
+      P.q_slot[(size_t)q] = I == J ? I : slot[{I, J}];
+    }
+  // positions, neighbour lists, Z offsets, update items (blocks in (j, k) order, then right-hand sides in j order; the
+  // contributions of each in ascending i)
+  P.el_nb_off.push_back(0);
+  P.up_c_off.push_back(0);
+  int pos = 0;
+  for (const auto& E : lv_nodes) {
+    BaState::SpLevel L{pos, (int)E.size(), 0, (int)P.up_out.size(), 0, 0};
+    std::map<std::pair<int, int>, std::vector<std::array<int, 3>>> blk;
+    std::map<int, std::vector<std::array<int, 3>>> rhs;
+    for (int i : E) {
+      const auto& nb = lv_nbrs[(size_t)pos];
+      P.el_node.push_back(i);
+      P.z_off.push_back(P.z_total);
+      P.z_total += (long long)m * m * (long long)nb.size();
+      for (int j : nb) { P.nb_node.push_back(j); P.nb_slot2.push_back(slot2(i, j)); }
+      P.el_nb_off.push_back((int)P.nb_node.size());
+      L.ntile = std::max(L.ntile, (m * (int)nb.size() + CR_TC - 1) / CR_TC);
+      for (size_t x = 0; x < nb.size(); x++) {
+        rhs[nb[x]].push_back({slot2(i, nb[x]), pos, (int)x});
+        for (size_t y = x; y < nb.size(); y++) blk[{nb[x], nb[y]}].push_back({slot2(i, nb[x]), pos, (int)y});
+      }
+      pos++;
+    }
+    auto put = [&](int out, const std::vector<std::array<int, 3>>& cs) {
+      P.up_out.push_back(out);
+      for (auto& cc : cs) { P.c_slot2.push_back(cc[0]); P.c_pos.push_back(cc[1]); P.c_col.push_back(cc[2]); }
+      P.up_c_off.push_back((int)P.c_slot2.size());
+    };
+    for (auto& kv : blk) put(kv.first.first == kv.first.second ? kv.first.first : slot[kv.first], kv.second);
+    for (auto& kv : rhs) put(kv.first, kv.second);
+    L.n_blk = (int)blk.size(); L.n_rhs = (int)rhs.size();
+    P.levels.push_back(L);
+  }
+  const long long mm = (long long)m * m, n_slot = N + (long long)P.blocks.size();
+  P.bytes = 8 * (n_slot * mm + N * mm + P.z_total + 3LL * N * m + (long long)P.z_off.size()) +
+            4 * (long long)(P.q_slot.size() + P.el_node.size() + P.el_nb_off.size() + P.nb_node.size() + P.nb_slot2.size() +
+                            P.up_out.size() + P.up_c_off.size() + P.c_slot2.size() + P.c_pos.size() + P.c_col.size());
+}
+
+static std::string sp_plan_json(const SpPlan& P) {
+  std::string s;
+  char tmp[96];
+  auto num = [&](long long x) { snprintf(tmp, sizeof(tmp), "%lld", x); s += tmp; };
+  auto list = [&](const int* a, int n) {
+    s += "[";
+    for (int k = 0; k < n; k++) { if (k) s += ","; num(a[k]); }
+    s += "]";
+  };
+  s += "{\"solver\":\"sparse\",\"mb\":"; num(P.mb); s += ",\"N\":"; num(P.N); s += ",\"m\":"; num(P.m);
+  s += ",\"n_orig_blocks\":"; num(P.n_orig); s += ",\"bytes\":"; num(P.bytes); s += ",\"limit\":"; num(SP_MAX_BYTES);
+  s += ",\"blocks\":[";
+  for (size_t k = 0; k < P.blocks.size(); k++) { s += k ? ",[" : "["; num(P.blocks[k].first); s += ","; num(P.blocks[k].second); s += "]"; }
+  s += "],\"levels\":[";
+  for (size_t l = 0; l < P.levels.size(); l++) {
+    const auto& L = P.levels[l];
+    s += l ? ",{" : "{";
+    s += "\"nodes\":"; list(P.el_node.data() + L.p0, L.n_el);
+    s += ",\"nbrs\":[";
+    for (int p = L.p0; p < L.p0 + L.n_el; p++) { if (p > L.p0) s += ","; list(P.nb_node.data() + P.el_nb_off[(size_t)p], P.el_nb_off[(size_t)p + 1] - P.el_nb_off[(size_t)p]); }
+    s += "],\"z_off\":[";
+    for (int p = L.p0; p < L.p0 + L.n_el; p++) { if (p > L.p0) s += ","; num(P.z_off[(size_t)p]); }
+    // update items: [output slot or node, [[i, slot(i, j), transposed, column block of k], ...]]
+    s += "],\"items\":[";
+    for (int it = L.u0; it < L.u0 + L.n_blk + L.n_rhs; it++) {
+      s += it > L.u0 ? ",[" : "[";
+      num(P.up_out[(size_t)it]); s += ",[";
+      for (int q = P.up_c_off[(size_t)it]; q < P.up_c_off[(size_t)it + 1]; q++) {
+        s += q > P.up_c_off[(size_t)it] ? ",[" : "[";
+        num(P.el_node[(size_t)P.c_pos[(size_t)q]]); s += ","; num(P.c_slot2[(size_t)q] >> 1); s += ","; num(P.c_slot2[(size_t)q] & 1);
+        s += ","; num(P.c_col[(size_t)q]); s += "]";
+      }
+      s += "]]";
+    }
+    s += "],\"n_blk\":"; num(L.n_blk); s += "}";
+  }
+  s += "]}";
+  return s;
+}
+
 // Flatten + index the problem on the host, upload, initialise device state.
 static int ba_upload(LldCtx* c, const lld_ba_problem* p, bool global_mode, int log_stride,
                      const lld_ba_problem* full = nullptr /* multi-rank: whole problem, for the rank-invariant structure */) {
@@ -340,7 +518,7 @@ static int ba_upload(LldCtx* c, const lld_ba_problem* p, bool global_mode, int l
   const bool topo_cache = c->topo_cache < 0 ? topo_env : c->topo_cache != 0;
   uint64_t th = 0;
   if (topo_cache && !c->host_only) {
-    th = ba_topology_hash(*reinterpret_cast<BaHost*>(c->ba_host), p, global_mode, log_stride, full, c->n_ranks, c->rank);
+    th = ba_topology_hash(*reinterpret_cast<BaHost*>(c->ba_host), p, global_mode, log_stride, full, c->n_ranks, c->rank, c->gba_sparse);
     if (S->topo_ok && S->topo_hash == th && S->pool_gen == c->pool_gen && S->global_mode == global_mode && S->topo_log_stride == log_stride) {
       // same structure as the problem already indexed on the device: refresh the values only
       BaView& v = S->v;
@@ -1193,7 +1371,34 @@ static int ba_upload(LldCtx* c, const lld_ba_problem* p, bool global_mode, int l
         S->use_band = false;
       }
     }
-    if (!S->use_band && !S->use_cr && S->env_smem > 220 * 1024) {
+    if (!S->use_band && !S->use_cr && S->env_smem > 220 * 1024 && c->gba_sparse) {
+      // loop closures: block elimination over the super-block graph (sp_solver.cuh)
+      SpPlan P;
+      sp_plan_build(nG, nb_off, nb_g, P);
+      if (P.bytes > SP_MAX_BYTES) {
+        snprintf(c->err, sizeof(c->err),
+                 "global BA: the block-elimination plan of the reduced system needs %lld bytes of device memory (%d super-blocks "
+                 "of %d keyframes, %zu off-diagonal blocks with fill), the limit is %lld (include/lldba.h, capacity limits)",
+                 P.bytes, P.N, P.mb, P.blocks.size(), SP_MAX_BYTES);
+        return LLD_ERR_UNSUPPORTED;
+      }
+      S->use_sp = true;
+      S->sp.N = P.N; S->sp.m = P.m; S->sp.mb = P.mb;
+      S->sp_levels = P.levels;
+      if (c->host_only) S->sp_report = sp_plan_json(P);
+      UP(tmp_i, P.q_slot.data(), P.q_slot.size()); S->sp.q_slot = tmp_i;
+      UP(tmp_i, P.el_node.data(), P.el_node.size()); S->sp.el_node = tmp_i;
+      UP(tmp_i, P.el_nb_off.data(), P.el_nb_off.size()); S->sp.el_nb_off = tmp_i;
+      { long long* tmp_z; UP(tmp_z, P.z_off.data(), P.z_off.size()); S->sp.z_off = tmp_z; }
+      UP(tmp_i, P.nb_node.data(), P.nb_node.size()); S->sp.nb_node = tmp_i;
+      UP(tmp_i, P.nb_slot2.data(), P.nb_slot2.size()); S->sp.nb_slot2 = tmp_i;
+      UP(tmp_i, P.up_out.data(), P.up_out.size()); S->sp.up_out = tmp_i;
+      UP(tmp_i, P.up_c_off.data(), P.up_c_off.size()); S->sp.up_c_off = tmp_i;
+      UP(tmp_i, P.c_slot2.data(), P.c_slot2.size()); S->sp.c_slot2 = tmp_i;
+      UP(tmp_i, P.c_pos.data(), P.c_pos.size()); S->sp.c_pos = tmp_i;
+      UP(tmp_i, P.c_col.data(), P.c_col.size()); S->sp.c_col = tmp_i;
+      S->sp_z_total = P.z_total; S->sp_n_slot = P.N + (long long)P.blocks.size();
+    } else if (!S->use_band && !S->use_cr && S->env_smem > 220 * 1024) {
       snprintf(c->err, sizeof(c->err),
                "global BA: envelope of the reduced system too wide for the on-chip solver: a landmark spans %d free keyframes "
                "(panel %d rows, row %d, n %d) and needs %zu bytes of shared memory, the limit is %d (include/lldba.h, capacity limits)",
@@ -1321,7 +1526,7 @@ static int ba_upload(LldCtx* c, const lld_ba_problem* p, bool global_mode, int l
   DEV(v.chi2_log, double, (size_t)nw * log_stride); DEV(v.lambda_log, double, (size_t)nw * log_stride);
   DEV(v.trials_log, int, (size_t)nw * log_stride); DEV(v.iter_done, int, 2 * (size_t)nw);
   DEV(v.solve_scratch, double, (size_t)scr_total);
-  DEV(v.env_A, double, (S->use_band || S->use_cr) ? 1 : (size_t)env_rowptr.back());
+  DEV(v.env_A, double, (S->use_band || S->use_cr || S->use_sp) ? 1 : (size_t)env_rowptr.back());
   if (S->use_cr) {
     CrView& cr = S->cr;
     const size_t mm = (size_t)cr.m * cr.m, N = (size_t)cr.N;
@@ -1330,6 +1535,13 @@ static int ba_upload(LldCtx* c, const lld_ba_problem* p, bool global_mode, int l
     DEV(cr.U[1], double, N * mm); DEV(cr.L, double, N * mm); DEV(cr.Z, double, N * cr.m * cr.zs);
     DEV(cr.b, double, N * cr.m); DEV(cr.zc, double, N * cr.m); DEV(cr.x, double, N * cr.m);
     DEV(cr.ok, int, 1);
+  }
+  if (S->use_sp) {
+    SpView& sp = S->sp;
+    const size_t mm = (size_t)sp.m * sp.m, N = (size_t)sp.N;
+    DEV(sp.W, double, (size_t)S->sp_n_slot * mm); DEV(sp.L, double, N * mm); DEV(sp.Z, double, std::max(S->sp_z_total, 1LL));
+    DEV(sp.b, double, N * sp.m); DEV(sp.zc, double, N * sp.m); DEV(sp.x, double, N * sp.m);
+    DEV(sp.ok, int, 1);
   }
   DEV(v.band_A, double, S->use_band ? (size_t)nG * ((v.band_B + 1) * 36 + 8) : 1);
   DEV(v.band_L, double, S->use_band ? (size_t)nG * (v.band_B + 1) * 36 : 1);
@@ -1409,6 +1621,10 @@ static int ba_upload(LldCtx* c, const lld_ba_problem* p, bool global_mode, int l
     LLD_CUDA(c, lld_raise_dyn_smem(k_cr_factor, sizeof(double) * ((size_t)S->cr.m * S->cr.m + 8 * (size_t)S->cr.m + 40)));
     LLD_CUDA(c, lld_raise_dyn_smem(k_cr_solve<15>, sizeof(double) * ((size_t)S->cr.m * S->cr.m + CR_RPT * CR_TC)));
     LLD_CUDA(c, lld_raise_dyn_smem(k_cr_solve<20>, sizeof(double) * ((size_t)S->cr.m * S->cr.m + CR_RPT * CR_TC)));
+  } else if (v.env_mode && S->use_sp) {
+    LLD_CUDA(c, lld_raise_dyn_smem(k_sp_factor, sizeof(double) * ((size_t)S->sp.m * S->sp.m + 8 * (size_t)S->sp.m + 40)));
+    LLD_CUDA(c, lld_raise_dyn_smem(k_sp_solve<15>, sizeof(double) * ((size_t)S->sp.m * S->sp.m + CR_RPT * CR_TC)));
+    LLD_CUDA(c, lld_raise_dyn_smem(k_sp_solve<20>, sizeof(double) * ((size_t)S->sp.m * S->sp.m + CR_RPT * CR_TC)));
   } else if (v.env_mode && S->use_band) LLD_CUDA(c, lld_raise_dyn_smem(k_solve_band<512>, (size_t)(int)S->band_smem) != cudaSuccess ? cudaErrorInvalidValue : lld_raise_dyn_smem(k_solve_band<1024>, (size_t)(int)S->band_smem));
   else if (v.env_mode) LLD_CUDA(c, lld_raise_dyn_smem(k_solve_env, (size_t)(int)S->env_smem));
   else if (S->max_n <= SMEM_SOLVE_MAX_N)
@@ -1541,6 +1757,34 @@ static int ba_solve_cr(LldCtx* c) {
     LLD_LAUNCH(c, k_cr_backsub, n_el * per_b, 256, 0, v, cr, s);
   }
   LLD_LAUNCH(c, k_cr_finish, 1, 1024, 0, v, cr);
+  return LLD_OK;
+}
+
+// global BA across loop closures: the plan's levels (sp_solver.cuh); every kernel returns early when the window is done or
+// an earlier factorisation failed
+static int ba_solve_sp(LldCtx* c) {
+  BaState* S = c->ba;
+  BaView& v = S->v;
+  const SpView& sp = S->sp;
+  const int N = sp.N, m = sp.m;
+  const size_t mm = (size_t)m * m;
+  LLD_CUDA(c, cudaMemsetAsync(sp.W, 0, sizeof(double) * (size_t)S->sp_n_slot * mm, c->stream));
+  const int nblk = (int)S->n_nb_total;
+  LLD_LAUNCH(c, k_sp_assemble, (nblk * 36 + N * m + 255) / 256, 256, 0, v, sp, nblk);
+  const size_t smem_f = sizeof(double) * (mm + 8 * (size_t)m + 40), smem_s = sizeof(double) * (mm + CR_RPT * CR_TC);
+  const int T = (m + CR_TILE - 1) / CR_TILE;
+  for (const auto& L : S->sp_levels) {
+    LLD_LAUNCH(c, k_sp_factor, L.n_el, 512, smem_f, v, sp, L.p0);
+    if (L.ntile == 0) continue;   // no remaining neighbours: nothing to eliminate into
+    if (m <= 15 * CR_RG) LLD_LAUNCH(c, k_sp_solve<15>, L.n_el * L.ntile, CR_TC / 2 * CR_RG, smem_s, v, sp, L.p0, L.ntile);
+    else LLD_LAUNCH(c, k_sp_solve<20>, L.n_el * L.ntile, CR_TC / 2 * CR_RG, smem_s, v, sp, L.p0, L.ntile);
+    LLD_LAUNCH(c, k_sp_update, L.n_blk * T * T + L.n_rhs, 256, 0, v, sp, L.u0, L.n_blk);
+  }
+  const int per_b = (m + 7) / 8;
+  for (auto it = S->sp_levels.rbegin(); it != S->sp_levels.rend(); ++it) LLD_LAUNCH(c, k_sp_backsub, it->n_el * per_b, 256, 0, v, sp, it->p0);
+  CrView out{};   // k_cr_finish reads the solution and the ok flag only
+  out.x = sp.x; out.ok = sp.ok;
+  LLD_LAUNCH(c, k_cr_finish, 1, 1024, 0, v, out);
   return LLD_OK;
 }
 
@@ -1768,6 +2012,9 @@ static int ba_step(LldCtx* c, int round, int stop_now, bool first = true) {
   if (S->global_mode) { int r = ba_allreduce_rows(c); if (r) return r; }
   if (v.env_mode && S->use_cr) {
     int r = ba_solve_cr(c);
+    if (r) return r;
+  } else if (v.env_mode && S->use_sp) {
+    int r = ba_solve_sp(c);
     if (r) return r;
   } else if (v.env_mode && S->use_band) {
     LLD_LAUNCH(c, k_band_assemble, v.n_free_total, 256, 0, v);
@@ -2124,6 +2371,27 @@ extern "C" int lld_ba_index_only(const lld_ba_problem* p, int global_mode) {
   static LldCtx c;  // keeps the host scratch across calls, like a real context (single-threaded helper)
   c.host_only = true;
   return ba_upload(&c, p, global_mode != 0, 8);
+}
+
+// the block-elimination plan lld_ba_global would run for p on a context with lld_ctx_set_gba_sparse(ctx, 1), as JSON
+// (host arithmetic only, no device needed: used by the CPU-side tests).  A problem that another solver takes writes
+// {"solver": "other"}; an error writes its message.
+extern "C" int lld_gba_sparse_plan_report(const lld_ba_problem* p, char* buf, int len) {
+  if (!p || !buf || len < 64) return LLD_ERR_ARG;
+  LldCtx c;
+  c.host_only = true;
+  c.gba_sparse = 1;
+  int r = ba_upload(&c, p, true, 8);
+  std::string s = r ? std::string(c.err) : c.ba->use_sp ? c.ba->sp_report : std::string("{\"solver\":\"other\"}");
+  lld_ba_state_free(c.ba);
+  lld_ba_host_free(c.ba_host);
+  c.ba = nullptr; c.ba_host = nullptr;
+  if ((int)s.size() >= len) {
+    snprintf(buf, (size_t)len, "report needs %zu bytes", s.size() + 1);
+    return LLD_ERR_ARG;
+  }
+  memcpy(buf, s.c_str(), s.size() + 1);
+  return r;
 }
 
 // landmark block partition of the multi-rank global BA (host arithmetic only; also used by the CPU-side tests)

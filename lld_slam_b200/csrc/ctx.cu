@@ -114,6 +114,12 @@ extern "C" void lld_ctx_set_topo_cache(void* ctx, int on) {
   LldCtx* c = lld_ctx_cast(ctx);
   if (c) c->topo_cache = on;
 }
+// global BA across loop closures: 1 = a reduced system too wide for the on-chip solvers is solved by block elimination
+// over its super-block graph (sp_solver.cuh), 0 = it is rejected with LLD_ERR_UNSUPPORTED
+extern "C" void lld_ctx_set_gba_sparse(void* ctx, int on) {
+  LldCtx* c = lld_ctx_cast(ctx);
+  if (c) c->gba_sparse = on != 0;
+}
 // collectives issued and bytes all-reduced (per rank) since the last lld_ba_global / lld_ba_upload on this context
 extern "C" void lld_ctx_nccl_stats(void* ctx, int64_t* calls, int64_t* bytes) {
   LldCtx* c = lld_ctx_cast(ctx);

@@ -101,6 +101,7 @@ struct LldCtx {
   cudaGraphExec_t ba_graph[2][2] = {{nullptr, nullptr}, {nullptr, nullptr}};
   int ba_graph_kernels[2][2] = {{0, 0}, {0, 0}};
   int topo_cache = -1;   // BA topology cache: -1 = default (on unless LLD_BA_TOPO_CACHE=0), 0 = off, 1 = on (lld_ctx_set_topo_cache)
+  int gba_sparse = 0;    // global BA whose envelope is too wide for the on-chip solvers: 1 = plan-driven block elimination (lld_ctx_set_gba_sparse)
   void pool_reset() { pool_next = 0; pool_gen++; }
   template <typename T>
   T* alloc(size_t n, cudaError_t* e) {
