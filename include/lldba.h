@@ -21,6 +21,7 @@
  *   lld_kf_search          <- ORBmatcher::Fuse x2, SearchByProjection(KeyFrame*,Scw,...)     src/ORBmatcher.cc:825-975, 977-1100, 290-403
  *   lld_tri_search         <- ORBmatcher::SearchForTriangulation     src/ORBmatcher.cc:657-823
  *   lld_bow_search         <- ORBmatcher::SearchByBoW x2             src/ORBmatcher.cc:159-288, 522-655
+ *   lld_init_search        <- ORBmatcher::SearchForInitialization    src/ORBmatcher.cc:405
  *   lld_line_associate     <- Tracking::AddLinesFrom                 src/Tracking.cc:996-1124
  *   lld_medoid_orb / _float<- MapPoint / MapLine::ComputeDistinctiveDescriptors              src/MapPoint.cc:242-307, src/MapLine.cc:133-201
  *
@@ -78,6 +79,9 @@ extern "C" {
  *   - local windows with more than 32 free keyframes take the general (slower) sparse path;
  *   - lld_sbp_*, lld_kf_search: n_levels <= 8, at most 65535 keypoints per frame; pairs with more than 2048 keypoints or queries
  *     take the multi-kernel path instead of the single-CTA one;
+ *   - lld_init_search: at most 65535 keypoints per frame, F2 octaves < 8; with check_orientation, F1 angles in [0, 900) and F2
+ *     angles in [0, 360) (ORB angles are in [0, 360)).  The sequential resolve keeps F2's state in shared memory when every F2
+ *     of the batch has at most 57088 keypoints (k_init_resolve_smem), else in global memory (k_init_resolve_global);
  *   - lld_line_match: descriptor widths that are a multiple of 8 up to 72 floats and at most 512 lines per side of a pair run on the
  *     tensor cores, everything else on the FP32 tile path (no failure).
  */
@@ -428,6 +432,41 @@ typedef struct lld_bow_search_problem {
 } lld_bow_search_problem;
 
 int lld_bow_search(void* ctx, const lld_bow_search_problem* p, lld_tri_search_result* out);
+
+/* ORBmatcher::SearchForInitialization(Frame& F1, Frame& F2, vector<cv::Point2f>& vbPrevMatched, vector<int>& vnMatches12,
+ * int windowSize)  src/ORBmatcher.cc:405, batched over frame pairs (Tracking::MonocularInitialization: ORBmatcher(0.9, true),
+ * windowSize = 100, vbPrevMatched carried from one call to the next).
+ * For every F1 keypoint of octave 0, in index order: the level-0 F2 keypoints of F2.GetFeaturesInArea(vbPrevMatched[i1],
+ * windowSize) (F2's 64 x 48 grid over mvKeysUn, cells x outer / y inner, insertion order) whose vMatchedDistance is above the
+ * distance are compared; best / second best with strict <; accepted at bestDist <= TH_LOW (50) and
+ * bestDist < (float)bestDist2 * nn_ratio.  An accepted match takes its F2 keypoint away from an earlier query (which becomes -1).
+ * Then the rotation-histogram filter over every accepted match, displaced ones included (ComputeThreeMaxima), and
+ * vbPrevMatched[i1] = F2.mvKeysUn[vnMatches12[i1]].pt for the matched i1. */
+typedef struct lld_init_search_problem {
+  int32_t n_pairs;
+  lld_frame_geom geom;          /* F2's grid: only min_x, max_x, min_y, max_y are read */
+  int32_t window_size;          /* windowSize */
+  float nn_ratio;               /* mfNNratio */
+  int32_t check_orientation;    /* mbCheckOrientation */
+  const int32_t* kp1_off;       /* [n_pairs+1] F1 keypoints */
+  const uint8_t* kp1_octave;    /* [n1] F1.mvKeysUn[i].octave */
+  const float* kp1_angle;       /* [n1] F1.mvKeysUn[i].angle */
+  const uint8_t* kp1_desc;      /* [n1][32] F1.mDescriptors */
+  const float* prev_matched;    /* [n1][2] vbPrevMatched on entry */
+  const int32_t* kp2_off;       /* [n_pairs+1] F2 keypoints */
+  const float* kp2_xy;          /* [n2][2] F2.mvKeysUn[i].pt */
+  const uint8_t* kp2_octave;    /* [n2] */
+  const float* kp2_angle;       /* [n2] */
+  const uint8_t* kp2_desc;      /* [n2][32] */
+} lld_init_search_problem;
+
+typedef struct lld_init_search_result {
+  int32_t* match12;       /* [n1] vnMatches12: pair-local F2 index or -1 */
+  int32_t* n_matches;     /* [n_pairs] return value */
+  float* prev_matched;    /* [n1][2] vbPrevMatched after the call; may be the problem's prev_matched array */
+} lld_init_search_result;
+
+int lld_init_search(void* ctx, const lld_init_search_problem* p, lld_init_search_result* out);
 
 /* ------------------------------------------------------------------------------------------------
  * Stereo line matching (float line descriptors)

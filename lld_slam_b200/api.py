@@ -157,6 +157,24 @@ def bow_search(p: Dict[str, Any], *, impl: str = "gpu", ctx=None):
     return out
 
 
+def init_search(p: Dict[str, Any], *, impl: str = "gpu", ctx=None):
+    """ORBmatcher::SearchForInitialization, batched over frame pairs: match12 (vnMatches12), n_matches, prev_matched
+    (vbPrevMatched after the call, [n1][2])"""
+    lib = _lib(impl)
+    geom, gk = capi.make_geom(p["geom"])
+    f = dict(p); f["geom"] = geom
+    prob, keep = capi.fill_struct(capi.InitSearchProblem, f)
+    n1 = int(p["kp1_off"][-1])
+    out = dict(match12=np.full(max(n1, 1), -2, np.int32), n_matches=np.zeros(int(p["n_pairs"]), np.int32),
+               prev_matched=np.zeros((max(n1, 1), 2), np.float32))
+    res, keep2 = capi.fill_struct(capi.InitSearchResult, out)
+    rc = lib.init_search(_handle(impl, ctx), C.byref(prob), C.byref(res))
+    _check(impl, ctx, rc, "lld_init_search")
+    out["match12"] = out["match12"][:n1]
+    out["prev_matched"] = out["prev_matched"][:n1]
+    return out
+
+
 def line_match(p: Dict[str, Any], *, impl: str = "gpu", ctx=None):
     lib = _lib(impl)
     prob, keep = capi.fill_struct(capi.LineMatchProblem, p)

@@ -3,7 +3,7 @@
 This is the Python harness over the C-ABI used by tests/ and bench.py.  The product library is
 lld_slam_b200/csrc/liblldba.so (CUDA, sm_100a); `load_library()` fails loudly when it is missing —
 there is no CPU fallback.  `load_oracle()` loads the CPU oracle (oracle/liblld_oracle.so) which
-exposes the same entry points with the `lldo_` prefix; only tests, smoke() and the bench's
+exposes the same entry points with the `lldo_` prefix (lldo_init_search from tests/hostcheck/libinit_search_oracle.so); only tests, smoke() and the bench's
 cpu_baseline / reference arm may call it.
 """
 from __future__ import annotations
@@ -17,6 +17,8 @@ import numpy as np
 _ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 LIB_PATH = os.environ.get("LLD_LIB_PATH") or os.path.join(_ROOT, "lld_slam_b200", "csrc", "liblldba.so")  # override: kernel A/B experiments
 ORACLE_PATH = os.path.join(_ROOT, "oracle", "liblld_oracle.so")
+# the oracle's SearchForInitialization (lldo_init_search) is a separate test-infrastructure library
+INIT_SEARCH_ORACLE_PATH = os.path.join(_ROOT, "tests", "hostcheck", "libinit_search_oracle.so")
 
 c_i32p = C.POINTER(C.c_int32)
 c_u8p = C.POINTER(C.c_uint8)
@@ -142,6 +144,18 @@ class BowSearchProblem(C.Structure):
     ]
 
 
+class InitSearchProblem(C.Structure):
+    _fields_ = [
+        ("n_pairs", C.c_int32), ("geom", FrameGeom), ("window_size", C.c_int32), ("nn_ratio", C.c_float), ("check_orientation", C.c_int32),
+        ("kp1_off", c_i32p), ("kp1_octave", c_u8p), ("kp1_angle", c_f32p), ("kp1_desc", c_u8p), ("prev_matched", c_f32p),
+        ("kp2_off", c_i32p), ("kp2_xy", c_f32p), ("kp2_octave", c_u8p), ("kp2_angle", c_f32p), ("kp2_desc", c_u8p),
+    ]
+
+
+class InitSearchResult(C.Structure):
+    _fields_ = [("match12", c_i32p), ("n_matches", c_i32p), ("prev_matched", c_f32p)]
+
+
 class TriSearchResult(C.Structure):
     _fields_ = [("match12", c_i32p), ("n_matches", c_i32p)]
 
@@ -239,6 +253,16 @@ class _Lib:
         self._sig("kf_search", [vp, C.POINTER(KfSearchProblem), C.POINTER(SbpResult)])
         self._sig("tri_search", [vp, C.POINTER(TriSearchProblem), C.POINTER(TriSearchResult)])
         self._sig("bow_search", [vp, C.POINTER(BowSearchProblem), C.POINTER(TriSearchResult)])
+        init_sig = [vp, C.POINTER(InitSearchProblem), C.POINTER(InitSearchResult)]
+        if self.is_oracle:
+            if not os.path.exists(INIT_SEARCH_ORACLE_PATH):
+                raise RuntimeError(f"{INIT_SEARCH_ORACLE_PATH} not found — build it first (python -c 'import __graft_entry__ as g; g.build()').")
+            self.init_dll = C.CDLL(INIT_SEARCH_ORACLE_PATH)
+            self.init_search = self.init_dll.lldo_init_search
+            self.init_search.argtypes = init_sig
+            self.init_search.restype = C.c_int
+        else:
+            self._sig("init_search", init_sig)
         self._sig("line_match", [vp, C.POINTER(LineMatchProblem), C.POINTER(LineMatchResult)])
         self._sig("descriptor_distance", [c_u8p, c_u8p])
         if not self.is_oracle:

@@ -12,21 +12,17 @@
 #include <algorithm>
 
 #include "lld_ctx.h"
+#include "orb_common.cuh"
 
 namespace {
 
-constexpr int TH_LOW = 50, HISTO_LENGTH = 30, TS_NT = 256;
+constexpr int TH_LOW = 50, TS_NT = 256;
 
 struct TriView {
   lld_tri_search_problem p;   // device pointers
   int* match12;
   int* n_matches;
 };
-
-__device__ __forceinline__ int popc256(const uint4& a0, const uint4& a1, const uint4& b0, const uint4& b1) {
-  return __popc(a0.x ^ b0.x) + __popc(a0.y ^ b0.y) + __popc(a0.z ^ b0.z) + __popc(a0.w ^ b0.w) + __popc(a1.x ^ b1.x) + __popc(a1.y ^ b1.y) +
-         __popc(a1.z ^ b1.z) + __popc(a1.w ^ b1.w);
-}
 
 __global__ void __launch_bounds__(TS_NT) k_tri_search(TriView v) {
   __shared__ int s_hist[HISTO_LENGTH];
@@ -46,7 +42,6 @@ __global__ void __launch_bounds__(TS_NT) k_tri_search(TriView v) {
   __syncthreads();
   // entries of keyframe 1's feature vector: [fv1_idx_off[f1b], fv1_idx_off[f1e])
   const int e_begin = f1b < f1e ? p.fv1_idx_off[f1b] : 0, e_end = f1b < f1e ? p.fv1_idx_off[f1e] : 0;
-  const float factor = 1.0f / HISTO_LENGTH;
   for (int e = e_begin + tid; e < e_end; e += TS_NT) {
     const int idx1 = p.fv1_idx[e];
     if (p.kp1_has_mp[a0 + idx1]) continue;
@@ -100,36 +95,19 @@ __global__ void __launch_bounds__(TS_NT) k_tri_search(TriView v) {
       v.match12[a0 + idx1] = bestIdx2;
       atomicAdd(&s_n, 1);
       if (p.check_orientation) {
-        float rot = __fsub_rn(p.kp1_angle[a0 + idx1], p.kp2_angle[b0 + bestIdx2]);
-        if (rot < 0.0f) rot = __fadd_rn(rot, 360.0f);
-        int bin = (int)roundf(__fmul_rn(rot, factor));
-        if (bin == HISTO_LENGTH) bin = 0;
+        const int bin = rot_bin(p.kp1_angle[a0 + idx1], p.kp2_angle[b0 + bestIdx2]);
         atomicAdd(&s_hist[bin], 1);
       }
     }
   }
   __syncthreads();
   if (p.check_orientation) {
-    if (tid == 0) {  // ORBmatcher::ComputeThreeMaxima
-      int max1 = 0, max2 = 0, max3 = 0, ind1 = -1, ind2 = -1, ind3 = -1;
-      for (int i = 0; i < HISTO_LENGTH; i++) {
-        const int s = s_hist[i];
-        if (s > max1) { max3 = max2; max2 = max1; max1 = s; ind3 = ind2; ind2 = ind1; ind1 = i; }
-        else if (s > max2) { max3 = max2; max2 = s; ind3 = ind2; ind2 = i; }
-        else if (s > max3) { max3 = s; ind3 = i; }
-      }
-      if ((float)max2 < 0.1f * (float)max1) { ind2 = -1; ind3 = -1; }
-      else if ((float)max3 < 0.1f * (float)max1) { ind3 = -1; }
-      s_keep[0] = ind1; s_keep[1] = ind2; s_keep[2] = ind3;
-    }
+    if (tid == 0) three_maxima(s_hist, s_keep);
     __syncthreads();
     for (int i = tid; i < n1; i += TS_NT) {
       const int m = v.match12[a0 + i];
       if (m < 0) continue;
-      float rot = __fsub_rn(p.kp1_angle[a0 + i], p.kp2_angle[b0 + m]);
-      if (rot < 0.0f) rot = __fadd_rn(rot, 360.0f);
-      int bin = (int)roundf(__fmul_rn(rot, factor));
-      if (bin == HISTO_LENGTH) bin = 0;
+      const int bin = rot_bin(p.kp1_angle[a0 + i], p.kp2_angle[b0 + m]);
       if (bin != s_keep[0] && bin != s_keep[1] && bin != s_keep[2]) {
         v.match12[a0 + i] = -1;
         atomicSub(&s_n, 1);
@@ -165,7 +143,6 @@ __global__ void __launch_bounds__(TS_NT) k_bow_search(BowView v) {
   if (tid == 0) s_n = 0;
   for (int i = tid; i < n1; i += TS_NT) v.match12[a0 + i] = -1;
   __syncthreads();
-  const float factor = 1.0f / HISTO_LENGTH;
   for (int f1 = f1b + tid; f1 < f1e; f1 += TS_NT) {
     const int node = p.fv1_node[f1];
     int l2 = f2b, h2 = f2e;
@@ -196,36 +173,19 @@ __global__ void __launch_bounds__(TS_NT) k_bow_search(BowView v) {
       v.matched2[b0 + bestIdx2] = 1;          // read again only by this thread (same node)
       atomicAdd(&s_n, 1);
       if (p.check_orientation) {
-        float rot = __fsub_rn(p.kp1_angle[a0 + idx1], p.kp2_angle[b0 + bestIdx2]);
-        if (rot < 0.0f) rot = __fadd_rn(rot, 360.0f);
-        int bin = (int)roundf(__fmul_rn(rot, factor));
-        if (bin == HISTO_LENGTH) bin = 0;
+        const int bin = rot_bin(p.kp1_angle[a0 + idx1], p.kp2_angle[b0 + bestIdx2]);
         atomicAdd(&s_hist[bin], 1);
       }
     }
   }
   __syncthreads();
   if (p.check_orientation) {
-    if (tid == 0) {  // ORBmatcher::ComputeThreeMaxima
-      int max1 = 0, max2 = 0, max3 = 0, ind1 = -1, ind2 = -1, ind3 = -1;
-      for (int i = 0; i < HISTO_LENGTH; i++) {
-        const int s = s_hist[i];
-        if (s > max1) { max3 = max2; max2 = max1; max1 = s; ind3 = ind2; ind2 = ind1; ind1 = i; }
-        else if (s > max2) { max3 = max2; max2 = s; ind3 = ind2; ind2 = i; }
-        else if (s > max3) { max3 = s; ind3 = i; }
-      }
-      if ((float)max2 < 0.1f * (float)max1) { ind2 = -1; ind3 = -1; }
-      else if ((float)max3 < 0.1f * (float)max1) { ind3 = -1; }
-      s_keep[0] = ind1; s_keep[1] = ind2; s_keep[2] = ind3;
-    }
+    if (tid == 0) three_maxima(s_hist, s_keep);
     __syncthreads();
     for (int i = tid; i < n1; i += TS_NT) {
       const int m = v.match12[a0 + i];
       if (m < 0) continue;
-      float rot = __fsub_rn(p.kp1_angle[a0 + i], p.kp2_angle[b0 + m]);
-      if (rot < 0.0f) rot = __fadd_rn(rot, 360.0f);
-      int bin = (int)roundf(__fmul_rn(rot, factor));
-      if (bin == HISTO_LENGTH) bin = 0;
+      const int bin = rot_bin(p.kp1_angle[a0 + i], p.kp2_angle[b0 + m]);
       if (bin != s_keep[0] && bin != s_keep[1] && bin != s_keep[2]) {
         v.match12[a0 + i] = -1;
         atomicSub(&s_n, 1);

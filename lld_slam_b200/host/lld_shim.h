@@ -13,6 +13,7 @@
 //   lld::LineOptimizer                      <- include/LineOptimizer.h:11-33, src/LineOptimizer.cc:28-201
 //   lld::ORBmatcher::SearchByProjection     <- src/ORBmatcher.cc:1328-1470 (frame to frame), :45-129 (frame to map points) and
 //                                              :1472-1599 (frame to keyframe, relocalisation)
+//   lld::ORBmatcher::SearchForInitialization <- src/ORBmatcher.cc:405
 //   lld::TwoFrameLineMatcher::MatchLines    <- src/TwoFrameLineMatcher.cc:26-77
 // Every entry point takes the library context as an extra first argument (the reference keeps its g2o optimizer on the
 // stack instead); Flatten* expose the flattened problem so that tests can compare it array by array with a reference
@@ -32,6 +33,7 @@
 namespace lld {
 
 struct KeyPoint { float x, y; int octave; float angle; };
+struct Point2f { float x, y; };                  // cv::Point2f
 struct KeyLine { float startPointX, startPointY, endPointX, endPointY; int octave; };
 
 struct KeyFrame {
@@ -767,6 +769,40 @@ class ORBmatcher {
     vpMatches12.assign(pKF1->mvKeysUn.size(), nullptr);                                       // :536
     for (size_t i = 0; i < pKF1->mvKeysUn.size(); i++)
       if (m12[i] >= 0) vpMatches12[i] = pKF2->mvpMapPoints[(size_t)m12[i]];                   // :597
+    return nm;
+  }
+  // int SearchForInitialization(Frame &F1, Frame &F2, vector<cv::Point2f> &vbPrevMatched, vector<int> &vnMatches12, int windowSize)
+  // src/ORBmatcher.cc:405: both frames flattened as they are (F2's grid comes from its bounds and
+  // mvKeysUn) -> lld_init_search -> vnMatches12 and vbPrevMatched
+  int SearchForInitialization(void* ctx, Frame& F1, Frame& F2, std::vector<Point2f>& vbPrevMatched, std::vector<int>& vnMatches12,
+                              int windowSize = 10) {
+    const size_t N1 = F1.mvKeysUn.size(), N2 = F2.mvKeysUn.size();
+    lld_init_search_problem p;
+    std::memset(&p, 0, sizeof(p));
+    p.n_pairs = 1;
+    p.geom.min_x = F2.mnMinX; p.geom.max_x = F2.mnMaxX; p.geom.min_y = F2.mnMinY; p.geom.max_y = F2.mnMaxY;
+    p.geom.n_levels = (int)F2.mvScaleFactors.size(); p.geom.scale_factors = F2.mvScaleFactors.data();
+    p.window_size = windowSize; p.nn_ratio = mfNNratio; p.check_orientation = mbCheckOrientation;
+    std::vector<float> ang1, prev, xy2, ang2;
+    std::vector<uint8_t> oct1, oct2;
+    for (size_t i = 0; i < N1; i++) {
+      oct1.push_back((uint8_t)F1.mvKeysUn[i].octave); ang1.push_back(F1.mvKeysUn[i].angle);
+      prev.push_back(vbPrevMatched[i].x); prev.push_back(vbPrevMatched[i].y);
+    }
+    for (size_t i = 0; i < N2; i++) {
+      xy2.push_back(F2.mvKeysUn[i].x); xy2.push_back(F2.mvKeysUn[i].y);
+      oct2.push_back((uint8_t)F2.mvKeysUn[i].octave); ang2.push_back(F2.mvKeysUn[i].angle);
+    }
+    const int32_t o1[2] = {0, (int32_t)N1}, o2[2] = {0, (int32_t)N2};
+    p.kp1_off = o1; p.kp1_octave = oct1.data(); p.kp1_angle = ang1.data(); p.kp1_desc = F1.mDescriptors.data(); p.prev_matched = prev.data();
+    p.kp2_off = o2; p.kp2_xy = xy2.data(); p.kp2_octave = oct2.data(); p.kp2_angle = ang2.data(); p.kp2_desc = F2.mDescriptors.data();
+    std::vector<int32_t> m12(N1 + 1, -1);
+    int32_t nm = 0;
+    lld_init_search_result r{m12.data(), &nm, prev.data()};
+    const int rc = lld_init_search(ctx, &p, &r);
+    if (rc) return rc;
+    vnMatches12.assign(m12.begin(), m12.begin() + N1);
+    for (size_t i = 0; i < N1; i++) { vbPrevMatched[i].x = prev[2 * i]; vbPrevMatched[i].y = prev[2 * i + 1]; }
     return nm;
   }
   // What ORBmatcher::Fuse decides for one map point (src/ORBmatcher.cc:949-968); Replace() itself is map bookkeeping and stays

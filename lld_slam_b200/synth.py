@@ -660,6 +660,65 @@ def make_bow_search_batch(n_pairs, n_kp, seed, n_nodes=150, strict_th=0, nn_rati
     return out
 
 
+def make_init_search_batch(n_pairs, n_kp, seed, window_size=100, nn_ratio=0.9, check_orientation=1, n_kp2=None, flow=20.0,
+                           unrelated_frac=0.3, flip_p=0.06, rotated_frac=0.15, dup_frac=0.05):
+    """SearchForInitialization (Tracking::MonocularInitialization): F1 = the initial frame, vbPrevMatched = its keypoints; F2 = F1
+    moved by a per-pair flow (up to `flow` px) plus 1.5 px noise, shuffled, with a share of unrelated keypoints mixed in.
+    Related descriptors differ by a few bit flips; angles follow F1 up to a small rotation except for a share of rotated
+    outliers, which the histogram filter removes.  A share of F1 keypoints repeats another one's texture nearby, so that later
+    queries take F2 keypoints away from earlier ones.  n_kp / n_kp2 may be lists (ragged pairs, 0 allowed); n_kp2 defaults to n_kp."""
+    rng = np.random.default_rng(seed)
+    g = frame_geom()
+    lvl_p = np.asarray([SCALE ** (-2.0 * l) for l in range(N_LEVELS)]); lvl_p /= lvl_p.sum()   # ORB's per-level feature share
+    acc = {k: [] for k in ("kp1_octave", "kp1_angle", "kp1_desc", "prev_matched", "kp2_xy", "kp2_octave", "kp2_angle", "kp2_desc")}
+    kp1_off, kp2_off = [0], [0]
+    for pr in range(n_pairs):
+        N1 = int(n_kp[pr]) if np.ndim(n_kp) else int(n_kp)
+        N2 = N1 if n_kp2 is None else (int(n_kp2[pr]) if np.ndim(n_kp2) else int(n_kp2))
+        xy1 = np.stack([rng.uniform(0, IMG_W, N1), rng.uniform(0, IMG_H, N1)], 1)
+        oct1 = rng.choice(N_LEVELS, N1, p=lvl_p)
+        ang1 = rng.uniform(0, 360, N1)
+        d1 = rng.integers(0, 256, (N1, 32), dtype=np.uint8)
+        # repeated texture: near-duplicate level-0 F1 keypoints a few pixels apart compete for the same F2 keypoint
+        n_dup = int(N1 * dup_frac) if N1 >= 2 else 0
+        dst, srcd = rng.choice(N1, n_dup, replace=False), rng.integers(0, N1, n_dup)
+        ok = dst != srcd
+        dst, srcd = dst[ok], srcd[ok]
+        d1[dst] = _flip_bits(d1[srcd], flip_p, rng)
+        xy1[dst] = np.clip(xy1[srcd] + rng.normal(0, 10, (len(dst), 2)), 0, [IMG_W - 1e-3, IMG_H - 1e-3])
+        oct1[dst] = 0; oct1[srcd] = 0
+        # F2: the first min(N1, N2) * (1 - unrelated_frac) keypoints follow F1, the rest are unrelated
+        n_rel = int(min(N1, N2) * (1.0 - unrelated_frac))
+        src = rng.permutation(N1)[:n_rel]
+        f = rng.uniform(-flow, flow, 2)
+        xy2 = np.concatenate([xy1[src] + f + rng.normal(0, 1.5, (n_rel, 2)),
+                              np.stack([rng.uniform(0, IMG_W, N2 - n_rel), rng.uniform(0, IMG_H, N2 - n_rel)], 1)])
+        oct2 = np.concatenate([np.where(rng.random(n_rel) < 0.9, oct1[src], rng.choice(N_LEVELS, n_rel, p=lvl_p)),
+                               rng.choice(N_LEVELS, N2 - n_rel, p=lvl_p)])
+        rot = np.where(rng.random(n_rel) < rotated_frac, rng.uniform(0, 360, n_rel), rng.normal(4, 3, n_rel))
+        ang2 = np.concatenate([np.mod(ang1[src] + rot, 360.0), rng.uniform(0, 360, N2 - n_rel)])
+        d2 = np.concatenate([_flip_bits(d1[src], flip_p, rng) if n_rel else d1[:0],
+                             rng.integers(0, 256, (N2 - n_rel, 32), dtype=np.uint8)])
+        perm = rng.permutation(N2)
+        acc["kp1_octave"].append(oct1); acc["kp1_angle"].append(ang1); acc["kp1_desc"].append(d1); acc["prev_matched"].append(xy1)
+        acc["kp2_xy"].append(xy2[perm]); acc["kp2_octave"].append(oct2[perm]); acc["kp2_angle"].append(ang2[perm])
+        acc["kp2_desc"].append(d2[perm])
+        kp1_off.append(kp1_off[-1] + N1); kp2_off.append(kp2_off[-1] + N2)
+    out = dict(n_pairs=n_pairs, geom=g, window_size=int(window_size), nn_ratio=float(nn_ratio), check_orientation=int(check_orientation),
+               kp1_off=np.asarray(kp1_off, np.int32), kp2_off=np.asarray(kp2_off, np.int32))
+    for k, v in acc.items():
+        a = np.concatenate(v)
+        if k.endswith("_octave") or k.endswith("_desc"):
+            a = a.astype(np.uint8)
+        else:
+            a = f32(a)
+            if k.endswith("_angle"):
+                a = np.mod(a, f32(360.0))
+                a[a >= 360.0] = 0.0   # float32 rounding of a tiny negative angle + 360
+        out[k] = np.ascontiguousarray(a.reshape(-1, 32) if k.endswith("_desc") else a)
+    return out
+
+
 def make_line_match_batch(n_pairs, n_lines, desc_dim, seed, tau=2.0, min_len=10, ragged=False):
     rng = np.random.default_rng(seed)
     P, N, D = n_pairs, n_lines, desc_dim
