@@ -20,7 +20,6 @@
 #include <vector>
 
 #include "ba_kernels.cuh"
-#include "ba_fused.cuh"
 #include "cr_solver.cuh"
 #include "sp_solver.cuh"
 #include "lld_ctx.h"
@@ -40,7 +39,6 @@ static const int CHUNK = 256;          // edge-list entries per chunk (k_lin_pos
 static const int SMEM_SOLVE_MAX_N = 156;  // dense LDL^T in shared memory up to this dimension (26 free KFs)
 
 void lld_ba_state_free(struct BaState* s);
-static cudaError_t ba_set_carveout(int device);
 
 struct BaState {
   BaView v{};
@@ -50,8 +48,7 @@ struct BaState {
   int max_nnb = 0;
   size_t n_nb_total = 0;
   bool gather_long = false;   // dense mode: average S-block gather list longer than a warp -> k_reduce_piece_warp
-  size_t env_smem = 0, band_smem = 0;
-  bool use_band = false;
+  size_t env_smem = 0;
   bool use_cr = false;     // global BA: block cyclic reduction of the reduced camera system (cr_solver.cuh)
   CrView cr{};
   bool use_sp = false;     // global BA across loop closures: plan-driven block elimination (sp_solver.cuh)
@@ -74,19 +71,12 @@ struct BaState {
   uint8_t* d_pt_bad = nullptr;
   uint8_t* d_ln_bad = nullptr;
   // one LM step captured as a CUDA graph per round (kernel arguments differ: round, robust flags)
-  // fused linearise -> Schur path (ba_fused.cuh): piece records and the flat edge maps it walks
   // topology cache: a repeated call with the same structure (same windows, observations lists and fixed flags — a
   // re-optimisation, or the bench's steady state) skips the host indexing stage and only refreshes the value arrays
   bool topo_ok = false;
   uint64_t topo_hash = 0, pool_gen = 0;
   int topo_log_stride = 0;
-  bool fused = false;
   bool lean = false;       // dense single-rank: steps after the first of a round run ba_step_lean
-  const FusedPiece* d_pieces = nullptr;
-  int n_pieces_pt = 0, n_pieces_ln = 0;
-  const int *d_ws_edge_p = nullptr, *d_ws_edge_l = nullptr;
-  const int *d_fx_off_p = nullptr, *d_fx_edge_p = nullptr, *d_fx_lm_p = nullptr;
-  const int *d_fx_off_l = nullptr, *d_fx_edge_l = nullptr, *d_fx_lm_l = nullptr;
   // [round][0: first step of the round (separate kernels, lambda_0), 1: later step]: the context's executable graph
   // (LldCtx::ba_graph) matches this problem
   bool graph_fresh[2][2] = {{false, false}, {false, false}};
@@ -150,8 +140,6 @@ struct BaHost {
   pvec<uint32_t> pts_mask, lns_mask;
   pvec<int> gb_off, gv_off;
   pvec<SchurItem> it_rec, it_tmp;
-  pvec<FusedPiece> pc_rec, pc_tmp;
-  pvec<int> fx_off_p, fx_edge_p, fx_lm_p, fx_off_l, fx_edge_l, fx_lm_l;
   std::vector<uint64_t> it_keys;
   pvec<long long> gb_src, gv_src;
   std::vector<BaDenseJob> jobs;
@@ -1061,9 +1049,7 @@ static int ba_upload(LldCtx* c, const lld_ba_problem* p, bool global_mode, int l
         while (e < loff[w + 1] && mask[e] == mask[b] && e - b < PIECE_CAP) e++;
         const uint32_t m = mask[b];
         const int n = __builtin_popcount(m);
-        if (n == 0) {   // seen by fixed keyframes only: a piece for the fused kernel (inverse records), no Schur tasks
-          J.pb.push_back(b); J.pe.push_back(e); J.pn.push_back(0); J.pout.push_back(J.dsize);
-        } else {
+        if (n > 0) {   // landmarks seen by fixed keyframes only have no Schur tasks
           const int pc = (int)J.pb.size();
           J.pb.push_back(b); J.pe.push_back(e); J.pn.push_back(n); J.pout.push_back(J.dsize);
           const int npair = n * (n + 1) / 2, ntask = 6 * npair + n;
@@ -1106,76 +1092,7 @@ static int ba_upload(LldCtx* c, const lld_ba_problem* p, bool global_mode, int l
         schur_item_shape(kind == 0 ? 3 : 4, R.n, R.nl, R.t0, &R.lc, &R.S, &R.nchunk);
       }
     });
-    // piece records of the fused path (opt-in, LLD_BA_FUSED=1): one per piece, ordered per kind by decreasing cost and dealt
-    // in snake order over the persistent CTAs (same balancing as the items above)
-    static const bool want_fused = getenv("LLD_BA_FUSED") && getenv("LLD_BA_FUSED")[0] == '1';
-    std::vector<int> jp(n_jobs + 1, 0);
-    if (want_fused) {
-    for (size_t jid = 0; jid < n_jobs; jid++) jp[jid + 1] = jp[jid] + (int)jobs[jid].pb.size();
-    S->n_pieces_pt = jp[std::min<size_t>((size_t)nw, n_jobs)];
-    S->n_pieces_ln = jp[n_jobs] - S->n_pieces_pt;
-    H.pc_rec.resize(std::max(jp[n_jobs], 1)); H.pc_tmp.resize(std::max(jp[n_jobs], 1));
-    par_for((int)n_jobs, [&](int jid) {
-      Job& J = jobs[jid];
-      const int kind = jid / nw, jw = jid % nw;
-      for (size_t q = 0; q < J.pb.size(); q++) {
-        FusedPiece& R = H.pc_tmp[jp[jid] + q];
-        R.l0 = J.pb[q]; R.nl = J.pe[q] - J.pb[q]; R.n = J.pn[q]; R.w = jw;
-        R.w0 = (kind == 0 ? pts_w0 : lns_w0)[J.pb[q]]; R.out = J.pout[q] + jd[jid];
-        R.lc = fused_chunk_len(kind == 0 ? 3 : 4, R.n, R.nl); R.pad0 = R.pad1 = R.pad2 = 0;
-      }
-    });
-    auto piece_order = [&](int kind) {
-      const int i0 = kind == 0 ? 0 : S->n_pieces_pt, i1 = kind == 0 ? S->n_pieces_pt : jp[n_jobs];
-      const int cntk = i1 - i0;
-      if (cntk <= 0) return;
-      const int G = std::min(cntk, (kind == 0 ? 4 : 2) * c->sm_count);
-      constexpr int NB = 2048;
-      std::vector<int> cnt(NB + 1, 0), bk((size_t)cntk);
-      for (int i = i0; i < i1; i++) {
-        const FusedPiece& R = H.pc_tmp[i];
-        const int ntask = R.n * (R.n + 1) + R.n, passes = (ntask + FU_TPB - 1) / FU_TPB;
-        const uint64_t cost = 32 + (uint64_t)R.nl * (uint64_t)(passes * (kind == 0 ? 6 : 14) * R.n + ntask);
-        const int b = NB - 1 - (int)std::min<uint64_t>(cost >> 5, NB - 1);
-        bk[(size_t)(i - i0)] = b;
-        cnt[b + 1]++;
-      }
-      for (int q = 0; q < NB; q++) cnt[q + 1] += cnt[q];
-      for (int i = i0; i < i1; i++) {
-        const int k = cnt[bk[(size_t)(i - i0)]]++;
-        const int r = k / G, j = k - r * G, len = std::min(G, cntk - r * G);
-        const int pos = (r & 1) ? len - 1 - j : j;
-        H.pc_rec[i0 + r * G + pos] = H.pc_tmp[i];
-      }
-    };
-    // edges to fixed keyframes by sorted landmark position (they feed H_ll / b_l only): offsets, edge ids, owners
-    auto fixed_lists = [&](const int* lm_off, const int* off, const pvec<int>& ekf, const pvec<int>& order, int n_lm,
-                           pvec<int>& f_off, pvec<int>& f_edge, pvec<int>& f_lm) {
-      f_off.assign((size_t)n_lm + 1, 0);
-      par_for(nw, [&](int w) {
-        for (int oi = lm_off[w]; oi < lm_off[w + 1]; oi++) {
-          const int i = order[oi];
-          int k = 0;
-          for (int e = off[i]; e < off[i + 1]; e++) k += kf_g[ekf[e]] < 0;
-          f_off[(size_t)oi + 1] = k;
-        }
-      });
-      for (int i = 0; i < n_lm; i++) f_off[(size_t)i + 1] += f_off[(size_t)i];
-      f_edge.resize(std::max(f_off[(size_t)n_lm], 1)); f_lm.resize(std::max(f_off[(size_t)n_lm], 1));
-      par_for(nw, [&](int w) {
-        for (int oi = lm_off[w]; oi < lm_off[w + 1]; oi++) {
-          const int i = order[oi];
-          int k = f_off[(size_t)oi];
-          for (int e = off[i]; e < off[i + 1]; e++)
-            if (kf_g[ekf[e]] < 0) { f_edge[(size_t)k] = e; f_lm[(size_t)k] = oi; k++; }
-        }
-      });
-    };
-    par_for(2, [&](int kind) { piece_order(kind); });
-    fixed_lists(p->pt_off, p->pt_obs_off, pe_kf, pt_order, n_pt, H.fx_off_p, H.fx_edge_p, H.fx_lm_p);
-    fixed_lists(p->ln_off, p->ln_obs_off, lc_kf, ln_order, n_ln, H.fx_off_l, H.fx_edge_l, H.fx_lm_l);
-    }
-    stage("dense: item records + pieces + fixed-edge lists");
+    stage("dense: item records");
     {
       // k_schur_tile's CTAs take items b, b + G, ... : order each kind by decreasing cost and deal the rows in snake
       // order, so that every CTA gets about the same landmark x task volume
@@ -1323,7 +1240,7 @@ static int ba_upload(LldCtx* c, const lld_ba_problem* p, bool global_mode, int l
     chS_total += 36LL * nnb + 6;
   }
   // envelope of the reduced camera system (global BA with a system too large for the dense solvers)
-  std::vector<int> env_first(1, 0), env_blk_last(1, 0), lo_off(2, 0), lo_col(1, 0), lo_src(1, 0);
+  std::vector<int> env_first(1, 0), env_blk_last(1, 0);
   std::vector<long long> env_rowptr(2, 0);
   v.env_mode = 0;
   if (global_mode && S->max_n > SMEM_SOLVE_MAX_N) {
@@ -1344,34 +1261,14 @@ static int ba_upload(LldCtx* c, const lld_ba_problem* p, bool global_mode, int l
       for (int k = fb[b]; k <= b; k++) env_blk_last[k] = std::max(env_blk_last[k], b);
     for (int k = 0; k < nG; k++) ph = std::max(ph, 6 * (env_blk_last[k] - k));
     v.env_mode = 1; v.env_panel_h = ph; v.env_maxlen = maxlen;
-    // banded sliding-window variant: block half-bandwidth and lower-block gather lists
+    // block half-bandwidth: the longest free-keyframe span of one landmark
     int B = 1;
     for (int g = 0; g < nG; g++) B = std::max(B, g - fb[g]);
-    v.band_B = B;
-    S->band_smem = sizeof(double) * ((size_t)(6 * (B + 2)) * (6 * (B + 2)) + 36 * (size_t)B + 32 + 6 * (B + 2) + 36 * (size_t)(B + 1) + 6) + 64;
-    S->use_band = S->band_smem <= 220 * 1024 && (B + 1) * 36 + 6 <= 2048;
-    lo_off.assign(nG + 1, 0);
-    for (int a = 0; a < nG; a++)
-      for (int q = nb_off[a]; q < nb_off[a + 1]; q++) lo_off[nb_g[q] + 1]++;
-    for (int g = 0; g < nG; g++) lo_off[g + 1] += lo_off[g];
-    lo_col.assign(std::max(lo_off[nG], 1), 0); lo_src.assign(std::max(lo_off[nG], 1), 0);
-    {
-      std::vector<int> cur(lo_off.begin(), lo_off.end() - 1);
-      for (int a = 0; a < nG; a++)
-        for (int q = nb_off[a]; q < nb_off[a + 1]; q++) { const int r = nb_g[q]; lo_col[cur[r]] = a; lo_src[cur[r]++] = q; }
-    }
     S->env_smem = sizeof(double) * (6 * (size_t)ph + 8 + 32 * (size_t)maxlen + (size_t)n) + 64;
-    {
-      // cyclic reduction over super-blocks of B keyframes whenever a dense super-block fits one SM's shared memory;
-      // LLD_GBA_SOLVER=band keeps the single-CTA sliding-window solver (A/B measurements)
-      const char* se = getenv("LLD_GBA_SOLVER");
-      S->use_cr = 6 * B <= CR_MAX_M && !(se && se[0] == 'b');
-      if (S->use_cr) {
-        S->cr.mb = B; S->cr.m = 6 * B; S->cr.N = (nG + B - 1) / B; S->cr.zs = 12 * B;
-        S->use_band = false;
-      }
-    }
-    if (!S->use_band && !S->use_cr && S->env_smem > 220 * 1024 && c->gba_sparse) {
+    // cyclic reduction over super-blocks of B keyframes whenever a dense super-block fits one SM's shared memory
+    S->use_cr = 6 * B <= CR_MAX_M;
+    if (S->use_cr) { S->cr.mb = B; S->cr.m = 6 * B; S->cr.N = (nG + B - 1) / B; S->cr.zs = 12 * B; }
+    if (!S->use_cr && S->env_smem > 220 * 1024 && c->gba_sparse) {
       // loop closures: block elimination over the super-block graph (sp_solver.cuh)
       SpPlan P;
       sp_plan_build(nG, nb_off, nb_g, P);
@@ -1398,7 +1295,7 @@ static int ba_upload(LldCtx* c, const lld_ba_problem* p, bool global_mode, int l
       UP(tmp_i, P.c_pos.data(), P.c_pos.size()); S->sp.c_pos = tmp_i;
       UP(tmp_i, P.c_col.data(), P.c_col.size()); S->sp.c_col = tmp_i;
       S->sp_z_total = P.z_total; S->sp_n_slot = P.N + (long long)P.blocks.size();
-    } else if (!S->use_band && !S->use_cr && S->env_smem > 220 * 1024) {
+    } else if (!S->use_cr && S->env_smem > 220 * 1024) {
       snprintf(c->err, sizeof(c->err),
                "global BA: envelope of the reduced system too wide for the on-chip solver: a landmark spans %d free keyframes "
                "(panel %d rows, row %d, n %d) and needs %zu bytes of shared memory, the limit is %d (include/lldba.h, capacity limits)",
@@ -1457,19 +1354,6 @@ static int ba_upload(LldCtx* c, const lld_ba_problem* p, bool global_mode, int l
   UP(tmp_l, gb_src.data(), gb_src.size()); v.gb_src = tmp_l;
   UP(tmp_i, gv_off.data(), gv_off.size()); v.gv_off = tmp_i;
   UP(tmp_l, gv_src.data(), gv_src.size()); v.gv_src = tmp_l;
-  int *d_ws_p = nullptr, *d_ws_l = nullptr;
-  static const bool want_fused_up = getenv("LLD_BA_FUSED") && getenv("LLD_BA_FUSED")[0] == '1';
-  if (dense && want_fused_up) {
-    FusedPiece* tmp_p; UP(tmp_p, H.pc_rec.data(), (size_t)(S->n_pieces_pt + S->n_pieces_ln)); S->d_pieces = tmp_p;
-    UP(tmp_i, H.fx_off_p.data(), H.fx_off_p.size()); S->d_fx_off_p = tmp_i;
-    UP(tmp_i, H.fx_edge_p.data(), H.fx_edge_p.size()); S->d_fx_edge_p = tmp_i;
-    UP(tmp_i, H.fx_lm_p.data(), H.fx_lm_p.size()); S->d_fx_lm_p = tmp_i;
-    UP(tmp_i, H.fx_off_l.data(), H.fx_off_l.size()); S->d_fx_off_l = tmp_i;
-    UP(tmp_i, H.fx_edge_l.data(), H.fx_edge_l.size()); S->d_fx_edge_l = tmp_i;
-    UP(tmp_i, H.fx_lm_l.data(), H.fx_lm_l.size()); S->d_fx_lm_l = tmp_i;
-    DEV(d_ws_p, int, n_pw); S->d_ws_edge_p = d_ws_p;
-    DEV(d_ws_l, int, n_lw); S->d_ws_edge_l = d_ws_l;
-  }
   {
     uint32_t* tmp_m;
     UP(tmp_m, pts_mask.data(), n_pt); v.pts_mask = tmp_m;
@@ -1479,9 +1363,6 @@ static int ba_upload(LldCtx* c, const lld_ba_problem* p, bool global_mode, int l
   UP(tmp_i, env_first.data(), env_first.size()); v.env_first = tmp_i;
   UP(tmp_i, env_blk_last.data(), env_blk_last.size()); v.env_blk_last = tmp_i;
   UP(tmp_l, env_rowptr.data(), env_rowptr.size()); v.env_rowptr = tmp_l;
-  UP(tmp_i, lo_off.data(), lo_off.size()); v.lo_off = tmp_i;
-  UP(tmp_i, lo_col.data(), lo_col.size()); v.lo_col = tmp_i;
-  UP(tmp_i, lo_src.data(), lo_src.size()); v.lo_src = tmp_i;
 
   stage("H2D enqueue");
   if (c->host_only) return LLD_OK;  // lld_ba_index_only: the host stage is complete
@@ -1526,7 +1407,7 @@ static int ba_upload(LldCtx* c, const lld_ba_problem* p, bool global_mode, int l
   DEV(v.chi2_log, double, (size_t)nw * log_stride); DEV(v.lambda_log, double, (size_t)nw * log_stride);
   DEV(v.trials_log, int, (size_t)nw * log_stride); DEV(v.iter_done, int, 2 * (size_t)nw);
   DEV(v.solve_scratch, double, (size_t)scr_total);
-  DEV(v.env_A, double, (S->use_band || S->use_cr || S->use_sp) ? 1 : (size_t)env_rowptr.back());
+  DEV(v.env_A, double, (S->use_cr || S->use_sp) ? 1 : (size_t)env_rowptr.back());
   if (S->use_cr) {
     CrView& cr = S->cr;
     const size_t mm = (size_t)cr.m * cr.m, N = (size_t)cr.N;
@@ -1543,9 +1424,6 @@ static int ba_upload(LldCtx* c, const lld_ba_problem* p, bool global_mode, int l
     DEV(sp.b, double, N * sp.m); DEV(sp.zc, double, N * sp.m); DEV(sp.x, double, N * sp.m);
     DEV(sp.ok, int, 1);
   }
-  DEV(v.band_A, double, S->use_band ? (size_t)nG * ((v.band_B + 1) * 36 + 8) : 1);
-  DEV(v.band_L, double, S->use_band ? (size_t)nG * (v.band_B + 1) * 36 : 1);
-  DEV(v.band_z, double, S->use_band ? 6 * (size_t)nG : 1);
   DEV(S->d_out_kf, double, 12 * (size_t)n_kf); DEV(S->d_out_pt, double, 3 * (size_t)n_pt);
   DEV(S->d_out_ln, double, 6 * (size_t)n_ln);
   DEV(S->d_pt_bad, uint8_t, n_pe); DEV(S->d_ln_bad, uint8_t, 2 * (size_t)n_lc);
@@ -1555,7 +1433,6 @@ static int ba_upload(LldCtx* c, const lld_ba_problem* p, bool global_mode, int l
   LLD_CUDA(c, cudaMemsetAsync(S->d_pt_bad, 0, n_pe ? n_pe : 1, c->stream));
   LLD_CUDA(c, cudaMemsetAsync(S->d_ln_bad, 0, n_lc ? 2 * (size_t)n_lc : 1, c->stream));
 
-  v.debug = getenv("LLD_BAND_DEBUG") ? 1 : 0;
   ba_set_params(v, p);
   stage("device buffers");
   c->last_h2d_bytes = S->h2d_bytes;
@@ -1565,13 +1442,7 @@ static int ba_upload(LldCtx* c, const lld_ba_problem* p, bool global_mode, int l
     const bool dense_single = v.dense_mode && !(global_mode && c->n_ranks > 1) && v.n_slices == 1 && S->max_n <= SMEM_SOLVE_MAX_N && !v.env_mode;
     S->forked = allow && dense_single;
     S->use_graph = allow && dense_single;
-    // fused linearise -> Schur steps after the first step of a round (ba_fused.cuh).  Opt-in (LLD_BA_FUSED=1): measured on the
-    // bench workload it moves 2.3x fewer DRAM bytes per step but is slower than the separate kernels (per-piece overheads and
-    // barrier-separated phases on ~37-landmark pieces; profiles/r2f_k_fused_full.txt), so the separate kernels stay the default.
-    const char* l = getenv("LLD_BA_LEAN");
-    S->lean = dense_single && !(l && l[0] == '0');
-    const char* f = getenv("LLD_BA_FUSED");
-    S->fused = dense_single && !S->gather_long && (f && f[0] == '1') && S->d_pieces != nullptr;
+    S->lean = dense_single;
   }
   // derived index arrays (stream-ordered after the uploads, before any consumer)
   {
@@ -1604,16 +1475,11 @@ static int ba_upload(LldCtx* c, const lld_ba_problem* p, bool global_mode, int l
     if (v.dense_mode) {
       if (n_pe) LLD_LAUNCH(c, k_dense_wpos, grid(n_pe), 256, 0, n_pe, v.pe_pt, v.pe_kf, v.kf_g, v.pt_win, v.w_g0, v.pt_spos, v.pts_mask, v.pts_w0, d_pe_wpos);
       if (n_lc) LLD_LAUNCH(c, k_dense_wpos, grid(n_lc), 256, 0, n_lc, v.lc_ln, v.lc_kf, v.kf_g, v.ln_win, v.w_g0, v.ln_spos, v.lns_mask, v.lns_w0, d_lc_wpos);
-      if (n_pe && d_ws_p) LLD_LAUNCH(c, k_ws_edge, grid(n_pe), 256, 0, n_pe, d_pe_wpos, d_ws_p);
-      if (n_lc && d_ws_l) LLD_LAUNCH(c, k_ws_edge, grid(n_lc), 256, 0, n_lc, d_lc_wpos, d_ws_l);
     }
     LLD_CUDA(c, cudaGetLastError());
   }
   // dynamic shared memory opt-in of the solvers (once per upload, outside any stream capture)
   if (v.dense_mode) {
-    LLD_CUDA(c, ba_set_carveout(c->device));
-    LLD_CUDA(c, lld_raise_dyn_smem(k_fused<3>, (size_t)FU_SMEM_BYTES));
-    LLD_CUDA(c, lld_raise_dyn_smem(k_fused<4>, (size_t)FU_SMEM_BYTES));
     LLD_CUDA(c, lld_raise_dyn_smem(k_schur_tile<3>, (size_t)SP_SMEM_BYTES));
     LLD_CUDA(c, lld_raise_dyn_smem(k_schur_tile<4>, (size_t)SP_SMEM_BYTES));
   }
@@ -1625,8 +1491,7 @@ static int ba_upload(LldCtx* c, const lld_ba_problem* p, bool global_mode, int l
     LLD_CUDA(c, lld_raise_dyn_smem(k_sp_factor, sizeof(double) * ((size_t)S->sp.m * S->sp.m + 8 * (size_t)S->sp.m + 40)));
     LLD_CUDA(c, lld_raise_dyn_smem(k_sp_solve<15>, sizeof(double) * ((size_t)S->sp.m * S->sp.m + CR_RPT * CR_TC)));
     LLD_CUDA(c, lld_raise_dyn_smem(k_sp_solve<20>, sizeof(double) * ((size_t)S->sp.m * S->sp.m + CR_RPT * CR_TC)));
-  } else if (v.env_mode && S->use_band) LLD_CUDA(c, lld_raise_dyn_smem(k_solve_band<512>, (size_t)(int)S->band_smem) != cudaSuccess ? cudaErrorInvalidValue : lld_raise_dyn_smem(k_solve_band<1024>, (size_t)(int)S->band_smem));
-  else if (v.env_mode) LLD_CUDA(c, lld_raise_dyn_smem(k_solve_env, (size_t)(int)S->env_smem));
+  } else if (v.env_mode) LLD_CUDA(c, lld_raise_dyn_smem(k_solve_env, (size_t)(int)S->env_smem));
   else if (S->max_n <= SMEM_SOLVE_MAX_N)
     LLD_CUDA(c, lld_raise_dyn_smem(k_solve<true>, (size_t)(int)(sizeof(double) * ((size_t)S->max_n * S->max_n + 8 * (size_t)S->max_n + 40))));
   S->topo_ok = topo_cache && th != 0;
@@ -1634,38 +1499,6 @@ static int ba_upload(LldCtx* c, const lld_ba_problem* p, bool global_mode, int l
 }
 
 static inline int cdiv(int a, int b) { return (a + b - 1) / b; }
-
-// The shared-memory carve-out is a per-SM setting that only changes on an idle SM, so kernels with different preferences
-// cannot share an SM: the point / line / pose passes that the dense LM step forks onto three streams would run one after
-// the other behind k_schur_tile (4 x 56 KB) and k_solve (> 100 KB).  LLD_BA_CARVEOUT=1 makes every kernel of the step ask
-// for the maximal shared-memory split so that they can co-reside.  Measured on B200 (cfg1, 64 windows): 20.0 ms per
-// step with the common split against 16.1 ms with the driver's per-kernel choice -- the linearisation and back-substitution
-// passes lose more from the smaller L1 than the step gains from overlap -- so the default leaves the driver's choice.
-template <typename F>
-static cudaError_t carve_max(F* f) {
-  return cudaFuncSetAttribute(reinterpret_cast<const void*>(f), cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared);
-}
-static cudaError_t ba_set_carveout(int device) {
-  static std::mutex mu;
-  static std::vector<int> done;
-  std::lock_guard<std::mutex> lk(mu);
-  if (std::find(done.begin(), done.end(), device) != done.end()) return cudaSuccess;
-  const char* e = getenv("LLD_BA_CARVEOUT");
-  if (!e || e[0] != '1') { done.push_back(device); return cudaSuccess; }
-  cudaError_t r = cudaSuccess;
-#define CARVE(k) if (r == cudaSuccess) r = carve_max(k)
-  CARVE((k_lin_points<1, false>)); CARVE((k_lin_points<4, false>)); CARVE((k_lin_points<1, true>)); CARVE((k_lin_points<4, true>));
-  CARVE((k_lin_lines<1, false>)); CARVE((k_lin_lines<2, false>)); CARVE((k_lin_lines<4, false>)); CARVE((k_lin_lines<8, false>));
-  CARVE((k_lin_lines<1, true>)); CARVE((k_lin_lines<2, true>)); CARVE((k_lin_lines<4, true>)); CARVE((k_lin_lines<8, true>));
-  CARVE(k_lin_poses); CARVE(k_pose_sum); CARVE(k_begin_fused); CARVE(k_schur_points); CARVE(k_schur_lines);
-  CARVE(k_schur_tile<3>); CARVE(k_schur_tile<4>); CARVE(k_reduce_piece); CARVE(k_reduce_piece_warp); CARVE(k_solve<true>);
-  CARVE(k_backsub_points<1>); CARVE(k_backsub_points<4>);
-  CARVE(k_backsub_lines<1>); CARVE(k_backsub_lines<2>); CARVE(k_backsub_lines<4>); CARVE(k_backsub_lines<8>);
-  CARVE(k_decide_fused); CARVE(k_decide_carry);
-#undef CARVE
-  if (r == cudaSuccess) done.push_back(device);
-  return r;
-}
 
 static int ba_init_state(LldCtx* c) {
   BaState* S = c->ba;
@@ -1795,11 +1628,6 @@ static int launch_solve(LldCtx* c, BaView& v, int max_n) {
   return LLD_OK;
 }
 
-// Dense single-rank path with the independent passes of one LM step on concurrent streams:
-//   [lin_points | lin_lines | lin_poses] -> begin -> [schur_points -> piece<3> | schur_lines -> piece<4>] -> reduce ->
-//   solve -> [backsub_points | backsub_lines] -> decide
-// (a small batch does not fill the GPU with any single pass; the critical path is what counts).  Works eagerly and
-// under stream capture (the side streams join the capture through the fork event).
 // up to this many map lines the line kernels run eight lanes per line (single windows); one lane per line above
 constexpr int LN_WIDE_MAX = 8192;
 // same for map points, four lanes per point
@@ -1829,49 +1657,6 @@ static int launch_line_kernel(LldCtx* c, cudaStream_t strm, const BaView& v, boo
     LLD_LINE_CASE(8)
   }
 #undef LLD_LINE_CASE
-  return LLD_OK;
-}
-
-static int ba_step_forked(LldCtx* c, int round, int stop_now) {
-  BaState* S = c->ba;
-  BaView& v = S->v;
-  const int gp = cdiv(std::max(v.n_pt, 1), LM_TPB), gl = cdiv(std::max(v.n_ln, 1), LM_TPB);
-  cudaStream_t s0 = c->stream, s1 = c->side[0], s2 = c->side[1];
-  auto fork = [&](cudaStream_t t) -> cudaError_t { return cudaStreamWaitEvent(t, c->ev_fork, 0); };
-  auto join = [&](int i) -> cudaError_t {
-    cudaError_t e = cudaEventRecord(c->ev_join[i], c->side[i]);
-    return e != cudaSuccess ? e : cudaStreamWaitEvent(s0, c->ev_join[i], 0);
-  };
-  LLD_CUDA(c, cudaEventRecord(c->ev_fork, s0));
-  LLD_CUDA(c, fork(s1));
-  LLD_CUDA(c, fork(s2));
-  if (v.n_pt && v.n_pt <= PT_WIDE_MAX) LLD_LAUNCH_S(c, s0, k_lin_points<4>, cdiv(v.n_pt * 4, LM_TPB), LM_TPB, 0, v);
-  else if (v.n_pt) LLD_LAUNCH_S(c, s0, k_lin_points<1>, gp, LM_TPB, 0, v);
-  { int r = launch_line_kernel(c, s1, v, true); if (r) return r; }
-  if (v.n_chunks) LLD_LAUNCH_S(c, s2, k_lin_poses, v.n_chunks, LM_TPB, 0, v);
-  LLD_CUDA(c, join(0));
-  LLD_CUDA(c, join(1));
-  LLD_LAUNCH_S(c, s0, k_begin_fused, v.n_win, FUSED_RED_TPB, 0, v);
-  const int nip = v.n_items_pt, nil = v.n_items - v.n_items_pt;
-  LLD_CUDA(c, cudaEventRecord(c->ev_fork, s0));
-  LLD_CUDA(c, fork(s1));
-  if (v.n_pt) LLD_LAUNCH_S(c, s0, k_schur_points, gp, LM_TPB, 0, v);
-  if (nip) LLD_LAUNCH_S(c, s0, k_schur_tile<3>, std::min(nip, 4 * c->sm_count), SP_TPB, SP_SMEM_BYTES, v, 0, nip);
-  if (v.n_ln) LLD_LAUNCH_S(c, s1, k_schur_lines, gl, LM_TPB, 0, v);
-  if (nil) LLD_LAUNCH_S(c, s1, k_schur_tile<4>, std::min(nil, 4 * c->sm_count), SP_TPB, SP_SMEM_BYTES, v, nip, nil);
-  LLD_CUDA(c, join(0));
-  const int nblk = (int)S->n_nb_total;
-  if (S->gather_long) LLD_LAUNCH_S(c, s0, k_reduce_piece_warp, cdiv(nblk * 6 + v.n_free_total, 8), 256, 0, v, nblk);
-  else LLD_LAUNCH_S(c, s0, k_reduce_piece, cdiv(nblk * 36 + 6 * v.n_free_total, 256), 256, 0, v, nblk);
-  { int r = launch_solve<true>(c, v, S->max_n); if (r) return r; }
-  LLD_CUDA(c, cudaEventRecord(c->ev_fork, s0));
-  LLD_CUDA(c, fork(s1));
-  if (v.n_pt && v.n_pt <= PT_WIDE_MAX) LLD_LAUNCH_S(c, s0, k_backsub_points<4>, cdiv(v.n_pt * 4, LM_TPB), LM_TPB, 0, v);
-  else if (v.n_pt) LLD_LAUNCH_S(c, s0, k_backsub_points<1>, gp, LM_TPB, 0, v);
-  { int r = launch_line_kernel(c, s1, v, false); if (r) return r; }
-  LLD_CUDA(c, join(0));
-  LLD_LAUNCH_S(c, s0, k_decide_fused, v.n_win, FUSED_RED_TPB, 0, v, round, stop_now);
-  LLD_CUDA(c, cudaGetLastError());
   return LLD_OK;
 }
 
@@ -1922,57 +1707,35 @@ static int ba_step_lean(LldCtx* c, int round, int stop_now) {
   return LLD_OK;
 }
 
-// Fused LM step (every step of a round but the first): 7 launches
-//   [k_fused<3> | k_fused<4>] -> k_reduce_fused -> k_solve -> [k_backsub_points | k_backsub_lines] -> k_decide_carry
-static int ba_step_fused(LldCtx* c, int round, int stop_now) {
-  BaState* S = c->ba;
-  BaView& v = S->v;
-  const int gp = cdiv(std::max(v.n_pt, 1), LM_TPB);
-  const bool par = S->forked && !c->prof_on;
-  cudaStream_t s0 = c->stream, s1 = par ? c->side[0] : c->stream;
-  auto fork = [&]() -> cudaError_t {
-    if (!par) return cudaSuccess;
-    cudaError_t e = cudaEventRecord(c->ev_fork, s0);
-    return e != cudaSuccess ? e : cudaStreamWaitEvent(s1, c->ev_fork, 0);
-  };
-  auto join = [&]() -> cudaError_t {
-    if (!par) return cudaSuccess;
-    cudaError_t e = cudaEventRecord(c->ev_join[0], s1);
-    return e != cudaSuccess ? e : cudaStreamWaitEvent(s0, c->ev_join[0], 0);
-  };
-  LLD_CUDA(c, fork());
-  if (S->n_pieces_pt)
-    LLD_LAUNCH_S(c, s0, k_fused<3>, std::min(S->n_pieces_pt, 4 * c->sm_count), FU_TPB, FU_SMEM_BYTES, v, S->d_pieces, S->n_pieces_pt,
-                 S->d_ws_edge_p, S->d_fx_off_p, S->d_fx_edge_p, S->d_fx_lm_p);
-  if (S->n_pieces_ln)
-    LLD_LAUNCH_S(c, s1, k_fused<4>, std::min(S->n_pieces_ln, 2 * c->sm_count), FU_TPB, FU_SMEM_BYTES, v, S->d_pieces + S->n_pieces_pt,
-                 S->n_pieces_ln, S->d_ws_edge_l, S->d_fx_off_l, S->d_fx_edge_l, S->d_fx_lm_l);
-  LLD_CUDA(c, join());
-  const int nblk = (int)S->n_nb_total;
-  LLD_LAUNCH_S(c, s0, k_reduce_fused, cdiv(nblk * 36 + 7 * v.n_free_total, 256), 256, 0, v, nblk);
-  { int r = launch_solve<true>(c, v, S->max_n); if (r) return r; }
-  LLD_CUDA(c, fork());
-  if (v.n_pt && v.n_pt <= PT_WIDE_MAX) LLD_LAUNCH_S(c, s0, k_backsub_points<4>, cdiv(v.n_pt * 4, LM_TPB), LM_TPB, 0, v);
-  else if (v.n_pt) LLD_LAUNCH_S(c, s0, k_backsub_points<1>, gp, LM_TPB, 0, v);
-  { int r = launch_line_kernel(c, s1, v, false); if (r) return r; }
-  LLD_CUDA(c, join());
-  LLD_LAUNCH_S(c, s0, k_decide_carry, v.n_win, FUSED_RED_TPB, 0, v, round, stop_now);
-  LLD_CUDA(c, cudaGetLastError());
-  return LLD_OK;
-}
-
-// one LM step of every window still running; first = first step of the round (every window at iteration 0)
+// one LM step of every window still running; first = first step of the round (every window at iteration 0).
+// A dense single-rank batch (S->forked) runs the independent passes of the step on concurrent streams:
+//   [lin_points | lin_lines | lin_poses] -> begin -> [schur_points -> schur_tile<3> | schur_lines -> schur_tile<4>] ->
+//   reduce -> solve -> [backsub_points | backsub_lines] -> decide
+// (a small batch does not fill the GPU with any single pass; the critical path is what counts).  Works eagerly and
+// under stream capture (the side streams join the capture through the fork event).  Otherwise, and in profiled runs, the
+// same launches go in the same order on one stream.
 static int ba_step(LldCtx* c, int round, int stop_now, bool first = true) {
   BaState* S = c->ba;
   BaView& v = S->v;
-  if (S->fused && !first) return ba_step_fused(c, round, stop_now);
   if (S->lean && !first) return ba_step_lean(c, round, stop_now);
-  if (S->forked && !c->prof_on) return ba_step_forked(c, round, stop_now);
   const int gp = cdiv(std::max(v.n_pt, 1), LM_TPB), gl = cdiv(std::max(v.n_ln, 1), LM_TPB);
-  if (v.n_pt && v.n_pt <= PT_WIDE_MAX) LLD_LAUNCH(c, k_lin_points<4>, cdiv(v.n_pt * 4, LM_TPB), LM_TPB, 0, v);
-  else if (v.n_pt) LLD_LAUNCH(c, k_lin_points<1>, gp, LM_TPB, 0, v);
-  { int r = launch_line_kernel(c, c->stream, v, true); if (r) return r; }
-  if (v.n_chunks) LLD_LAUNCH(c, k_lin_poses, v.n_chunks, LM_TPB, 0, v);
+  const bool par = S->forked && !c->prof_on;
+  cudaStream_t s0 = c->stream, s1 = par ? c->side[0] : c->stream, s2 = par ? c->side[1] : c->stream;
+  auto fork = [&](cudaStream_t t) -> cudaError_t { return par ? cudaStreamWaitEvent(t, c->ev_fork, 0) : cudaSuccess; };
+  auto join = [&](int i) -> cudaError_t {
+    if (!par) return cudaSuccess;
+    cudaError_t e = cudaEventRecord(c->ev_join[i], c->side[i]);
+    return e != cudaSuccess ? e : cudaStreamWaitEvent(s0, c->ev_join[i], 0);
+  };
+  if (par) LLD_CUDA(c, cudaEventRecord(c->ev_fork, s0));
+  LLD_CUDA(c, fork(s1));
+  LLD_CUDA(c, fork(s2));
+  if (v.n_pt && v.n_pt <= PT_WIDE_MAX) LLD_LAUNCH_S(c, s0, k_lin_points<4>, cdiv(v.n_pt * 4, LM_TPB), LM_TPB, 0, v);
+  else if (v.n_pt) LLD_LAUNCH_S(c, s0, k_lin_points<1>, gp, LM_TPB, 0, v);
+  { int r = launch_line_kernel(c, s1, v, true); if (r) return r; }
+  if (v.n_chunks) LLD_LAUNCH_S(c, s2, k_lin_poses, v.n_chunks, LM_TPB, 0, v);
+  LLD_CUDA(c, join(0));
+  LLD_CUDA(c, join(1));
   const bool multi = S->global_mode && c->n_ranks > 1;
   const bool fused = !multi && v.n_slices == 1;
   if (fused) {
@@ -1984,12 +1747,15 @@ static int ba_step(LldCtx* c, int round, int stop_now, bool first = true) {
     if (multi) { int r = ba_allreduce_lin(c); if (r) return r; }
     LLD_LAUNCH(c, k_begin, cdiv(v.n_win, 64), 64, 0, v);
   }
-  if (v.n_pt) LLD_LAUNCH(c, k_schur_points, gp, LM_TPB, 0, v);
-  if (v.n_ln) LLD_LAUNCH(c, k_schur_lines, gl, LM_TPB, 0, v);
+  const int nip = v.n_items_pt, nil = v.n_items - v.n_items_pt;   // dense-mode work items (none in sparse mode)
+  if (par) LLD_CUDA(c, cudaEventRecord(c->ev_fork, s0));
+  LLD_CUDA(c, fork(s1));
+  if (v.n_pt) LLD_LAUNCH_S(c, s0, k_schur_points, gp, LM_TPB, 0, v);
+  if (nip) LLD_LAUNCH_S(c, s0, k_schur_tile<3>, std::min(nip, 4 * c->sm_count), SP_TPB, SP_SMEM_BYTES, v, 0, nip);
+  if (v.n_ln) LLD_LAUNCH_S(c, s1, k_schur_lines, gl, LM_TPB, 0, v);
+  if (nil) LLD_LAUNCH_S(c, s1, k_schur_tile<4>, std::min(nil, 4 * c->sm_count), SP_TPB, SP_SMEM_BYTES, v, nip, nil);
+  LLD_CUDA(c, join(0));
   if (v.dense_mode) {
-    const int nip = v.n_items_pt, nil = v.n_items - v.n_items_pt;
-    if (nip) LLD_LAUNCH(c, k_schur_tile<3>, std::min(nip, 4 * c->sm_count), SP_TPB, SP_SMEM_BYTES, v, 0, nip);
-    if (nil) LLD_LAUNCH(c, k_schur_tile<4>, std::min(nil, 4 * c->sm_count), SP_TPB, SP_SMEM_BYTES, v, nip, nil);
     const int nblk = (int)S->n_nb_total;
     if (S->gather_long) LLD_LAUNCH(c, k_reduce_piece_warp, cdiv(nblk * 6 + v.n_free_total, 8), 256, 0, v, nblk);
     else LLD_LAUNCH(c, k_reduce_piece, cdiv(nblk * 36 + 6 * v.n_free_total, 256), 256, 0, v, nblk);
@@ -2016,17 +1782,16 @@ static int ba_step(LldCtx* c, int round, int stop_now, bool first = true) {
   } else if (v.env_mode && S->use_sp) {
     int r = ba_solve_sp(c);
     if (r) return r;
-  } else if (v.env_mode && S->use_band) {
-    LLD_LAUNCH(c, k_band_assemble, v.n_free_total, 256, 0, v);
-    if ((v.band_B + 1) * 36 + 6 <= 1024) LLD_LAUNCH(c, k_solve_band<512>, 1, 512, S->band_smem, v);   // 128 registers per thread
-    else LLD_LAUNCH(c, k_solve_band<1024>, 1, 1024, S->band_smem, v);
   } else if (v.env_mode) {
     LLD_LAUNCH(c, k_solve_env, 1, 1024, S->env_smem, v);
   } else if (S->max_n <= SMEM_SOLVE_MAX_N) { int r = launch_solve<true>(c, v, S->max_n); if (r) return r; }
   else { int r = launch_solve<false>(c, v, S->max_n); if (r) return r; }
-  if (v.n_pt && v.n_pt <= PT_WIDE_MAX) LLD_LAUNCH(c, k_backsub_points<4>, cdiv(v.n_pt * 4, LM_TPB), LM_TPB, 0, v);
-  else if (v.n_pt) LLD_LAUNCH(c, k_backsub_points<1>, gp, LM_TPB, 0, v);
-  { int r = launch_line_kernel(c, c->stream, v, false); if (r) return r; }
+  if (par) LLD_CUDA(c, cudaEventRecord(c->ev_fork, s0));
+  LLD_CUDA(c, fork(s1));
+  if (v.n_pt && v.n_pt <= PT_WIDE_MAX) LLD_LAUNCH_S(c, s0, k_backsub_points<4>, cdiv(v.n_pt * 4, LM_TPB), LM_TPB, 0, v);
+  else if (v.n_pt) LLD_LAUNCH_S(c, s0, k_backsub_points<1>, gp, LM_TPB, 0, v);
+  { int r = launch_line_kernel(c, s1, v, false); if (r) return r; }
+  LLD_CUDA(c, join(0));
   if (fused) {
     LLD_LAUNCH(c, k_decide_fused, v.n_win, FUSED_RED_TPB, 0, v, round, stop_now);
   } else {
@@ -2058,7 +1823,7 @@ static int ba_run_round(LldCtx* c, int maxit, int round, const volatile uint8_t*
   int launched = 0;
   auto one_step = [&](int stop_now) -> int {
     const bool first = launched == 0;
-    const int kind = ((S->fused || S->lean) && !first) ? 1 : 0;
+    const int kind = (S->lean && !first) ? 1 : 0;
     if (S->use_graph && !c->prof_on && !stop_now && round < 2) {
       if (!S->graph_fresh[round][kind]) {  // capture one LM step (fork / join over the side streams included)
         const int64_t l0 = c->launches;

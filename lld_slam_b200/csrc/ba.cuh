@@ -15,9 +15,9 @@ namespace lld {
 
 enum : int { PH_LIN = 0, PH_RETRY = 1, PH_DONE = 2 };
 
-// dense mode, per keyframe slot of a piece in the partial-sum scratch (dpart): b_schur part (6) + H_pp upper triangle (21)
-// + b_p (6) + number of active edges (1); k_schur_tile fills the first 6, k_fused all of them
-constexpr int SCHUR_KS = 34;
+// dense mode, per keyframe slot of a piece in the partial-sum scratch (dpart): the keyframe's b_schur part (6), written by
+// k_schur_tile
+constexpr int SCHUR_KS = 6;
 
 struct BaParams {
   int robust_pt, robust_ln;
@@ -190,15 +190,6 @@ struct BaView {
   const long long* env_rowptr;// [n+1]
   const int* env_blk_last;    // [n/6] last block row whose envelope reaches block column k
   double* env_A;
-  // banded sliding-window solver (global BA): block half-bandwidth, lower-block gather lists, column panels of L
-  int band_B;                 // max over block rows of (row - first block column)
-  const int* lo_off;          // [n_free_total+1] lower blocks (row r, col c <= r) of the reduced system
-  const int* lo_col;          // column block c
-  const int* lo_src;          // index of block (c, r) in S_blk (to be read transposed)
-  double* band_A;             // [n_free_total][(band_B+1)*36 + 8] band rows in the solver's order (k_band_assemble)
-  double* band_L;             // [n_free_total][(band_B+1)][36] column panels: block 0 = L_kk (strict lower) + D (diagonal)
-  double* band_z;             // [6 * n_free_total] forward-substituted rhs
-  int debug;                  // LLD_BAND_DEBUG: the band solver prints its phase cycle counts
   BaParams prm;
 };
 

@@ -1856,357 +1856,6 @@ __global__ void __launch_bounds__(1024) k_solve_env(BaView v) {
 }
 #undef ENV_A
 
-// ------------------------------------------------------------------------------------------------
-// Banded LDL^T with a sliding shared-memory window (global BA).  The reduced camera system of a long trajectory is
-// block-banded (half bandwidth B blocks = longest track); only block rows / columns [k, k+B] are touched while pivot
-// block k is eliminated, so the CTA keeps a circular (B+2)^2-block window in shared memory: per pivot
-//   A: thread 0 factors the 6x6 diagonal block (registers) and forward-solves its rhs,
-//   B: one thread per scalar row of the panel computes T = A_ik L_kk^-T, L = T D^-1; the spare row slot is zeroed,
-//   C: one warp per row applies the rank-6 update; column panel k of L is streamed to HBM; block row k+B+1 is
-//      gathered (transposed upper blocks) into the spare slot.
-// Three barriers per pivot, no global-memory latency on the critical path.  The backward substitution walks the stored
-// column panels with register prefetch of the next panel.
-// ------------------------------------------------------------------------------------------------
-// band row r in the solver's native order: (B+1) lower blocks (column blocks r-B .. r, each [row in block][col in
-// block]) followed by the 6 rhs values; assembled in parallel from the block rows of S (stored as upper blocks)
-__global__ void __launch_bounds__(256) k_band_assemble(BaView v) {
-  const int w = 0;
-  if (v.w_phase[w] == PH_DONE) return;
-  const int g0 = v.w_g0[w];
-  const int r = blockIdx.x, B = v.band_B, RS = (B + 1) * 36 + 8;
-  double* row = v.band_A + (size_t)r * RS;
-  for (int i = threadIdx.x; i < RS; i += blockDim.x) row[i] = 0.0;
-  __syncthreads();
-  const int q0 = v.lo_off[g0 + r], q1 = v.lo_off[g0 + r + 1];
-  for (int i = threadIdx.x; i < (q1 - q0) * 36; i += blockDim.x) {
-    const int q = q0 + i / 36, e = i % 36, rr = e / 6, cc = e - 6 * rr;
-    const int c = v.lo_col[q];
-    if (c == r && cc < rr) continue;  // diagonal block: lower triangle only
-    row[(c - (r - B)) * 36 + cc * 6 + rr] = v.S_blk[36 * (size_t)v.lo_src[q] + e];
-  }
-  if (threadIdx.x < 6) row[(B + 1) * 36 + threadIdx.x] = v.g_bs[6 * (size_t)(g0 + r) + threadIdx.x];
-}
-
-// 6x6 LDL^T of the diagonal block in window slot s by one warp (right-looking over shuffles), forward solve of its rhs;
-// writes L (strict lower) and D back, z and 1/D into zq[0..5] / zq[8..13]; returns false on a zero / non-finite pivot
-__device__ __forceinline__ bool band_factor_diag(double* Wm, int LDW, int s, const double* rw, double* zq, double* band_z_k, int lane, int li, int lj) {
-  double m = lane < 21 ? Wm[(size_t)(6 * s + li) * LDW + 6 * s + lj] : 0.0;
-  double zz = lane < 6 ? rw[6 * s + lane] : 0.0;
-  bool okk = true;
-#pragma unroll
-  for (int pv = 0; pv < 6; pv++) {
-    const double d = __shfl_sync(0xffffffffu, m, pv * (pv + 1) / 2 + pv);
-    if (!(d != 0.0) || !isfinite(d)) okk = false;
-    const double id = 1.0 / d;
-    const double tip = __shfl_sync(0xffffffffu, m, li * (li + 1) / 2 + pv);   // T(i, pv), used when li > pv
-    const double tjp = __shfl_sync(0xffffffffu, m, lj * (lj + 1) / 2 + pv);   // T(j, pv), used when lj > pv
-    if (lane < 21 && lj > pv) m -= (tip * id) * tjp;
-    if (lane < 21 && lj == pv && li > pv) m *= id;
-  }
-#pragma unroll
-  for (int pv = 0; pv < 5; pv++) {   // L z = b
-    const double zp = __shfl_sync(0xffffffffu, zz, pv);
-    const double lip = __shfl_sync(0xffffffffu, m, (lane < 6 ? lane * (lane + 1) / 2 : 0) + pv);
-    if (lane < 6 && lane > pv) zz -= lip * zp;
-  }
-  if (lane < 21) Wm[(size_t)(6 * s + li) * LDW + 6 * s + lj] = m;
-  if (lane < 21 && li == lj) zq[8 + li] = 1.0 / m;
-  if (lane < 6) {
-    zq[lane] = zz;
-    band_z_k[lane] = zz;
-  }
-  return okk;
-}
-
-// Banded LDL^T, forward elimination per pivot block k in two barrier-separated phases:
-//   B: one thread per scalar row of the panel: T = A_ik L_kk^-T (kept for the update), L = T D^-1 written back
-//   C: trailing update by 3x6 half-block items (thread = one item: 18 + 36 + 18 shared-memory loads for 108 FMAs; the
-//      item -> (row block, column block) map lives in "distance from the pivot" space and is computed once), rhs update,
-//      column panel to HBM, the prefetched block row k+B+1 enters the window — and, as soon as warp 0 has updated block
-//      (k+1, k+1), it factors it (look-ahead), so the diagonal factorisation is off the critical path.
-template <int NT>
-__global__ void __launch_bounds__(NT) k_solve_band(BaView v) {
-  extern __shared__ double bsm[];
-  const int w = 0;
-  if (v.w_phase[w] == PH_DONE) return;
-  const int g0 = v.w_g0[w], nf = v.w_g0[w + 1] - g0;
-  const int B = v.band_B, WB = B + 2, LDW = 6 * WB, PB = B + 1, RS = PB * 36 + 8;
-  const int tid = threadIdx.x, nt = blockDim.x;
-  const int lane = tid & 31, wid = tid >> 5, nw = nt >> 5;
-  double* Wm = bsm;                          // [LDW][LDW]
-  double* Tt = Wm + (size_t)LDW * LDW;       // [6][6B]: T(c, x), x = panel row (consecutive lanes -> consecutive banks)
-  double* zb = Tt + 36 * (size_t)B;          // [2][16]: z block [0,6) and 1/D [8,14) of the pivot, double-buffered
-  double* rw = zb + 32;                      // [LDW] rhs window
-  double* pan = rw + LDW;                    // [PB*36 + 6] panel buffer for the backward pass
-  __shared__ int flag;
-  __shared__ double red[32];
-  const int sel = v.w_sel[w];
-  auto fetch_row = [&](int r, double* r2) {
-#pragma unroll
-    for (int u = 0; u < 2; u++) {
-      const int i = tid + u * nt;
-      r2[u] = (r < nf && i < PB * 36 + 6) ? v.band_A[(size_t)r * RS + i] : 0.0;
-    }
-  };
-  // element roles of this thread inside a band row (loop invariant): kind 0 = matrix entry (block j, row ri, col ci), 1 = rhs
-  int el_kind[2], el_j[2], el_roff[2], el_ci[2];
-#pragma unroll
-  for (int u = 0; u < 2; u++) {
-    const int i = tid + u * nt;
-    el_kind[u] = i < PB * 36 ? 0 : (i < PB * 36 + 6 ? 1 : 2);
-    const int j = i / 36, e = i - 36 * j, ri = e / 6;
-    el_j[u] = j;
-    el_roff[u] = el_kind[u] == 0 ? ri * LDW : i - PB * 36;
-    el_ci[u] = e - 6 * ri;
-  }
-  auto commit_row = [&](int r, int s, const double* r2) {   // s = r mod WB
-    if (r >= nf) return;
-#pragma unroll
-    for (int u = 0; u < 2; u++) {
-      if (el_kind[u] == 0) {
-        int sc = s + 2 + el_j[u];   // (r - B + j) mod WB with WB = B + 2
-        if (sc >= WB) sc -= WB;
-        if (r - B + el_j[u] >= 0) Wm[6 * s * LDW + el_roff[u] + 6 * sc + el_ci[u]] = r2[u];
-      } else if (el_kind[u] == 1) {
-        rw[6 * s + el_roff[u]] = r2[u];
-      }
-    }
-  };
-  if (tid == 0) flag = 1;
-  for (int i = tid; i < LDW * LDW; i += nt) Wm[i] = 0.0;
-  __syncthreads();
-  for (int r = 0; r < nf && r <= B; r++) {
-    double t2[2];
-    fetch_row(r, t2);
-    commit_row(r, r, t2);   // r <= B < WB
-  }
-  double cur[2], nxt[2] = {0, 0};
-  fetch_row(B + 1, cur);   // enters the window at the end of pivot 0
-  // lane -> (i, j) of the 6x6 lower triangle (diagonal-block factorisation by warp 0)
-  int li = 0, lj = 0;
-  {
-    int l = lane;
-    while (li < 5 && l > li) { l -= li + 1; li++; }
-    lj = l;
-    if (lane >= 21) { li = 0; lj = 0; }
-  }
-  __syncthreads();
-  bool ok = true;
-  if (wid == 0) {   // pivot 0 has no predecessor: factor it here
-    const bool okk = band_factor_diag(Wm, LDW, 0, rw, zb, v.band_z, lane, li, lj);
-    if (!okk && lane == 0) flag = 0;
-  }
-  __syncthreads();
-  // loop-invariant roles: panel row of this thread (phase B), panel-store element, update columns of this lane
-  const int pb_d = 1 + tid / 6, pb_ri = tid - 6 * (pb_d - 1);
-  int uc_d[4], uc_rj[4];
-#pragma unroll
-  for (int q = 0; q < 4; q++) {
-    const int jj = lane + 32 * q;
-    uc_d[q] = 1 + jj / 6;
-    uc_rj[q] = jj - 6 * (uc_d[q] - 1);
-  }
-  int sk = 0;              // k mod WB
-  int s_in = (B + 1) % WB; // (k + B + 1) mod WB: slot of the incoming row
-  for (int k = 0; k < nf; k++, sk = (sk + 1 == WB ? 0 : sk + 1), s_in = (s_in + 1 == WB ? 0 : s_in + 1)) {
-    if (!flag) { ok = false; break; }
-    const int kend = min(k + B, nf - 1), nb_act = kend - k;
-    double* zq = zb + 16 * (k & 1);
-    fetch_row(k + B + 2, nxt);   // two pivots ahead of its use
-    // ---- B: panel rows
-    const int npr = 6 * nb_act;
-    for (int x = tid; x < npr; x += nt) {
-      const int d = x == tid ? pb_d : 1 + x / 6, ri = x == tid ? pb_ri : x - 6 * (1 + x / 6 - 1);
-      int sl = sk + d;
-      if (sl >= WB) sl -= WB;
-      double* row = Wm + (6 * sl + ri) * LDW + 6 * sk;
-      const double* dk = Wm + 6 * sk * LDW + 6 * sk;
-      double t6[6];
-#pragma unroll
-      for (int c = 0; c < 6; c++) {
-        double s2 = row[c];
-#pragma unroll
-        for (int q = 0; q < 6; q++)
-          if (q < c) s2 -= t6[q] * dk[c * LDW + q];
-        t6[c] = s2;
-      }
-#pragma unroll
-      for (int c = 0; c < 6; c++) {
-        row[c] = t6[c] * zq[8 + c];
-        Tt[c * 6 * B + x] = t6[c];
-      }
-    }
-    __syncthreads();
-    // ---- C: trailing update, one warp per block row di (last warp: block row 1 only, then the look-ahead): the 6x6 L block of
-    // the row lives in registers (broadcast loads), lanes walk the row's columns — T(c, column) and the six C elements
-    // of a column are consecutive over the lanes, so every shared-memory access of this phase is conflict-free
-    // (the look-ahead warp is the LAST warp: the issue arbiter favours high warp ids, and this warp is the critical path)
-    for (int di = (wid == nw - 1 ? 1 : 2 + wid); di <= nb_act; di += (wid == nw - 1 ? (1 << 20) : nw - 1)) {
-      int si = sk + di;
-      if (si >= WB) si -= WB;
-      double* rowb = Wm + (size_t)(6 * si) * LDW;
-      double L[6][6];
-#pragma unroll
-      for (int r = 0; r < 6; r++)
-#pragma unroll
-        for (int c = 0; c < 6; c++) L[r][c] = rowb[(size_t)r * LDW + 6 * sk + c];
-#pragma unroll
-      for (int q = 0; q < 4; q++) {
-        const int jj = lane + 32 * q;
-        if (jj >= 6 * di) break;
-        int sj = sk + uc_d[q];
-        if (sj >= WB) sj -= WB;
-        const int col = 6 * sj + uc_rj[q];
-        double tv[6];
-#pragma unroll
-        for (int c = 0; c < 6; c++) tv[c] = Tt[c * 6 * B + jj];
-#pragma unroll
-        for (int r = 0; r < 6; r++) {
-          double a2 = 0;
-#pragma unroll
-          for (int c = 0; c < 6; c++) a2 += L[r][c] * tv[c];
-          rowb[r * LDW + col] -= a2;
-        }
-      }
-      for (int jj = lane + 128; jj < 6 * di; jj += 32) {   // block rows wider than 128 columns (B > 21)
-        const int dj = 1 + jj / 6, rj = jj - 6 * (dj - 1);
-        int sj = sk + dj;
-        if (sj >= WB) sj -= WB;
-        const int col = 6 * sj + rj;
-        double tv[6];
-#pragma unroll
-        for (int c = 0; c < 6; c++) tv[c] = Tt[c * 6 * B + jj];
-#pragma unroll
-        for (int r = 0; r < 6; r++) {
-          double a2 = 0;
-#pragma unroll
-          for (int c = 0; c < 6; c++) a2 += L[r][c] * tv[c];
-          rowb[r * LDW + col] -= a2;
-        }
-      }
-      if (lane < 6)   // rhs rows of this block
-        rw[6 * si + lane] -= rowb[(size_t)lane * LDW + 6 * sk] * zq[0] + rowb[(size_t)lane * LDW + 6 * sk + 1] * zq[1] +
-                             rowb[(size_t)lane * LDW + 6 * sk + 2] * zq[2] + rowb[(size_t)lane * LDW + 6 * sk + 3] * zq[3] +
-                             rowb[(size_t)lane * LDW + 6 * sk + 4] * zq[4] + rowb[(size_t)lane * LDW + 6 * sk + 5] * zq[5];
-    }
-    // look-ahead: items (1,1) live on lanes 0 and 1 of warp 0 -> block (k+1, k+1) and its rhs are final
-    if (wid == nw - 1 && k + 1 < nf) {
-      __syncwarp();
-      int s1 = sk + 1;
-      if (s1 >= WB) s1 -= WB;
-      const bool okk = band_factor_diag(Wm, LDW, s1, rw, zb + 16 * ((k + 1) & 1), v.band_z + 6 * (size_t)(k + 1), lane, li, lj);
-      if (!okk && lane == 0) flag = 0;
-    }
-    // column panel k of L to HBM (backward pass) — the diagonal block of column k is no longer touched
-    if (wid != nw - 1) {
-      double* Lk = v.band_L + (size_t)k * PB * 36;
-      for (int i = tid; i < (nb_act + 1) * 36; i += nt - 32) {
-        const int d = i / 36, e = i - 36 * d, rr = e / 6, cc = e - 6 * rr;
-        int sl = sk + d;
-        if (sl >= WB) sl -= WB;
-        Lk[i] = Wm[(size_t)(6 * sl + rr) * LDW + 6 * sk + cc];
-      }
-    }
-    // the incoming block row k + B + 1 takes the window slot of block k - 1, which no item of this phase touches
-    commit_row(k + B + 1, s_in, cur);
-    cur[0] = nxt[0];
-    cur[1] = nxt[1];
-    __syncthreads();
-  }
-  if (ok) {
-    // backward substitution over the stored column panels; x window kept in rw (circular), panel k-1 prefetched
-    double pre[2] = {0, 0};
-    const int plen = PB * 36 + 6;   // panel + z_k
-    auto fetch = [&](int k, double* r2) {
-      // each thread prefetches up to 2 entries of panel k (plen <= 2 * blockDim for B <= 55)
-      for (int u = 0; u < 2; u++) {
-        const int i = tid + u * nt;
-        if (i < PB * 36) r2[u] = v.band_L[(size_t)k * PB * 36 + i];
-        else if (i < plen) r2[u] = v.band_z[6 * (size_t)k + (i - PB * 36)];
-      }
-    };
-    auto commit = [&](const double* r2) {
-      for (int u = 0; u < 2; u++) {
-        const int i = tid + u * nt;
-        if (i < plen) pan[i] = r2[u];
-      }
-    };
-    fetch(nf - 1, pre);
-    commit(pre);
-    __syncthreads();
-    for (int k = nf - 1; k >= 0; k--) {
-      const int kend = min(k + B, nf - 1);
-      if (k > 0) fetch(k - 1, pre);
-      // y_c = z_c / D_c - sum_{ib>k} sum_r L(ib,k)[r][c] x_ib[r]  : 6 warps, one per c
-      if (wid < 6) {
-        const int c = wid;
-        double acc = 0;
-        const int nterm = 6 * (kend - k);
-        for (int q = lane; q < nterm; q += 32) {
-          const int ib = k + 1 + q / 6, r = q % 6;
-          acc += pan[(size_t)(ib - k) * 36 + 6 * r + c] * rw[6 * (ib % WB) + r];
-        }
-        acc = warp_sum(acc);
-        if (lane == 0) zb[c] = pan[PB * 36 + c] / pan[6 * c + c] - acc;
-      }
-      __syncthreads();
-      if (tid == 0) {   // x_k = L_kk^-T y   (unit lower 6x6)
-        double x6[6];
-#pragma unroll
-        for (int i = 5; i >= 0; i--) {
-          double s2 = zb[i];
-#pragma unroll
-          for (int q = 0; q < 6; q++)
-            if (q > i) s2 -= pan[6 * q + i] * x6[q];
-          x6[i] = s2;
-        }
-#pragma unroll
-        for (int i = 0; i < 6; i++) {
-          rw[6 * (k % WB) + i] = x6[i];
-          v.g_x[6 * (size_t)(g0 + k) + i] = x6[i];
-        }
-      }
-      __syncthreads();
-      if (k > 0) commit(pre);
-      __syncthreads();
-    }
-  }
-  __syncthreads();
-  for (int k = v.kf_off[w] + tid; k < v.kf_off[w + 1]; k += nt) {
-    const int g = v.kf_g[k];
-    double qt[7];
-    const double* src = v.pose_qt[sel] + 7 * (size_t)k;
-    if (g >= 0 && v.g_nact[g] > 0) {
-      pose_oplus(src, v.g_x + 6 * (size_t)g, qt);
-    } else {
-#pragma unroll
-      for (int q = 0; q < 7; q++) qt[q] = src[q];
-    }
-    double Rt[12];
-    pose_to_Rt(qt, Rt);
-    double* dq = v.pose_qt[sel ^ 1] + 7 * (size_t)k;
-    double* dr = v.pose_Rt[sel ^ 1] + 12 * (size_t)k;
-#pragma unroll
-    for (int q = 0; q < 7; q++) dq[q] = qt[q];
-#pragma unroll
-    for (int q = 0; q < 12; q++) dr[q] = Rt[q];
-  }
-  const double lam = v.w_lambda[w];
-  const int n = 6 * nf;
-  double sc = 0;
-  for (int i = tid; i < n; i += nt) {
-    const int g = g0 + i / 6;
-    if (v.g_nact[g] == 0) continue;
-    const double x = v.g_x[6 * (size_t)g0 + i];
-    sc += x * (lam * x + v.g_bp[6 * (size_t)g0 + i]);
-  }
-  sc = block_sum(sc, red);
-  if (tid == 0) {
-    v.w_scale_p[w] = sc;
-    v.w_ok[w] = ok ? 1 : 0;
-  }
-}
-
 // one CTA per window: assemble the dense reduced camera system from the block rows, factor, solve, apply the
 // pose update T <- exp(x) T into the trial buffer and accumulate the pose part of computeScale().
 template <bool SMEM>
@@ -2713,6 +2362,36 @@ __global__ void __launch_bounds__(FUSED_RED_TPB) k_decide_fused(BaView v, int ro
   chi = block_sum(chi, sm);
   sc = block_sum(sc, sm);
   if (tid == 0) {
+    v.w_red_sum[4 * w + 0] = chi;
+    v.w_red_sum[4 * w + 1] = sc;
+    decide_window(v, w, round, stop_now);
+  }
+}
+
+// trial reduction + decision of the lean step: a window that starts a new outer iteration (PH_LIN) carries its chi2 over
+// from the accepted trial of the previous step — the same state, so activeRobustChi2() of
+// optimization_algorithm_levenberg.cpp:75 would return the same sum — instead of reducing it again.
+__global__ void __launch_bounds__(FUSED_RED_TPB) k_decide_carry(BaView v, int round, int stop_now) {
+  const int w = blockIdx.x;
+  if (v.w_phase[w] == PH_DONE) return;
+  __shared__ double sm[32];
+  const int tid = threadIdx.x;
+  double chi = 0, sc = 0;
+  for (int p = v.pt_off[w] + tid; p < v.pt_off[w + 1]; p += FUSED_RED_TPB) {
+    chi += v.lm_chi2[p];
+    sc += v.lm_scale[p];
+  }
+  for (int l = v.ln_off[w] + tid; l < v.ln_off[w + 1]; l += FUSED_RED_TPB) {
+    chi += v.lm_chi2[v.n_pt + l];
+    sc += v.lm_scale[v.n_pt + l];
+  }
+  chi = block_sum(chi, sm);
+  sc = block_sum(sc, sm);
+  if (tid == 0) {
+    if (v.w_phase[w] == PH_LIN) {   // solve() entry of a new outer iteration
+      v.w_inichi[w] = v.w_curchi[w];
+      v.w_trials[w] = 0;
+    }
     v.w_red_sum[4 * w + 0] = chi;
     v.w_red_sum[4 * w + 1] = sc;
     decide_window(v, w, round, stop_now);

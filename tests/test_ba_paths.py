@@ -2,10 +2,10 @@
 
 `ba.cu` picks kernels and solvers from the shape of the problem: the cyclic-reduction solve (`k_cr_solve<15>` up to a
 super-block of m = 120 scalars, `<20>` up to CR_MAX_M = 156), the single-CTA skyline LDL^T (`k_solve_env`, global BA
-whose block half-bandwidth B is 27 or more), the banded solver (`LLD_GBA_SOLVER=band`), local sparse mode (more than
-32 free keyframes in a window, or a landmark seen twice by one free keyframe), the 1024-thread Schur rows, the sliced
-reductions of windows with 32k landmarks, the lanes per line, the step schedules and the topology cache.  The windows
-of `synth.make_ba_window` reach only a few of these, so the generators below build shapes that reach the others.
+whose block half-bandwidth B is 27 or more), local sparse mode (more than 32 free keyframes in a window, or a landmark
+seen twice by one free keyframe), the 1024-thread Schur rows, the sliced reductions of windows with 32k landmarks, the
+lanes per line, the step schedules and the topology cache.  The windows of `synth.make_ba_window` reach only a few of
+these, so the generators below build shapes that reach the others.
 
 Each GPU case compares with the oracle through `check_ba` (the tolerances of test_gpu_parity.py) and proves that it ran
 the arm it is named after: kernel names from the per-launch profile (`lld_ctx_profile`), the exact host-to-device byte
@@ -205,10 +205,8 @@ def shape_claims(p):
         ph = max(6, 6 * int((last - np.arange(nG)).max()))
         maxlen = 6 * int((np.arange(nG) - fb).max()) + 6
         env_smem = 8 * (6 * ph + 8 + 32 * maxlen + 6 * nG) + 64
-        band_smem = 8 * ((6 * (B + 2)) ** 2 + 36 * B + 32 + 6 * (B + 2) + 36 * (B + 1) + 6) + 64
-        c.update(B=B, m=6 * B, N=-(-nG // B), global_nnb=global_nnb, env_smem=env_smem,
-                 band_fits=band_smem <= SMEM_LIMIT and (B + 1) * 36 + 6 <= 2048, band_512=(B + 1) * 36 + 6 <= 1024)
-        c["solver"] = ("cr" if 6 * B <= CR_MAX_M else "band" if c["band_fits"] else "env" if env_smem <= SMEM_LIMIT else "too wide")
+        c.update(B=B, m=6 * B, N=-(-nG // B), global_nnb=global_nnb, env_smem=env_smem)
+        c["solver"] = "cr" if 6 * B <= CR_MAX_M else "env" if env_smem <= SMEM_LIMIT else "too wide"
     return c
 
 
@@ -217,7 +215,6 @@ def shape_claims(p):
 # with the last super-block partial and exactly full, and a power of two
 CR_CASES = [(2, 34), (10, 85), (16, 64), (20, 50), (21, 42), (26, 130), (26, 200)]
 ENV_CASES = [dict(B=27, n_kf=101, fixed=()), dict(B=45, n_kf=151, fixed=(40, 41, 90))]
-BAND_CASES = [19, 24]
 
 
 def cr_problem(B, n_free, robust=False):
@@ -300,19 +297,6 @@ def test_env_shapes(case):
     c = shape_claims(env_problem(**case))
     assert c["B"] == case["B"] and c["solver"] == "env", c
     assert c["n_free"][0] == case["n_kf"] - 1 - len(case["fixed"])
-
-
-@pytest.mark.parametrize("B", BAND_CASES)
-def test_band_shapes(B):
-    c = shape_claims(cr_problem(B, 60))
-    assert c["B"] == B and c["band_fits"] and c["band_512"]
-
-
-def test_band_solver_fits_up_to_B24_only():
-    """LLD_GBA_SOLVER=band needs B <= 24; its 1024-thread instance needs (B + 1) * 36 + 6 > 1024, i.e. B >= 28"""
-    fits = [B for B in range(1, 60) if 8 * ((6 * (B + 2)) ** 2 + 36 * B + 32 + 6 * (B + 2) + 36 * (B + 1) + 6) + 64 <= SMEM_LIMIT]
-    assert max(fits) == 24
-    assert min(B for B in range(1, 60) if (B + 1) * 36 + 6 > 1024) == 28
 
 
 def test_envelope_limit_shapes():
@@ -485,7 +469,7 @@ def test_global_cr(ctx, B, n_free):
     _, names = checked(p, ctx, "global", (8,), f"CR B={B} n_free={n_free}")
     want = "k_cr_solve<15>" if 6 * B <= 120 else "k_cr_solve<20>"
     assert {"k_cr_factor", "k_cr_assemble", "k_cr_update", want} <= names, names
-    assert not names & {"k_solve_env", "k_solve_band<512>", "k_cr_solve<15>", "k_cr_solve<20>"} - {want}, names
+    assert not names & {"k_solve_env", "k_cr_solve<15>", "k_cr_solve<20>"} - {want}, names
 
 
 @pytest.mark.gpu
@@ -493,7 +477,7 @@ def test_global_cr(ctx, B, n_free):
 def test_global_skyline(ctx, case):
     p = env_problem(**case)
     _, names = checked(p, ctx, "global", (8,), f"skyline B={case['B']}")
-    assert "k_solve_env" in names and not any(n.startswith("k_cr_") or n.startswith("k_solve_band") for n in names), names
+    assert "k_solve_env" in names and not any(n.startswith("k_cr_") for n in names), names
 
 
 @pytest.mark.gpu
@@ -503,16 +487,6 @@ def test_global_robust_flag(ctx, kind, robust):
     p = cr_problem(16, 64, robust=robust) if kind == "cr" else env_problem(**ENV_CASES[0], robust=robust)
     _, names = checked(p, ctx, "global", (8,), f"{kind} robust={robust}")
     assert ("k_cr_factor" if kind == "cr" else "k_solve_env") in names
-
-
-@pytest.mark.gpu
-@pytest.mark.parametrize("B", BAND_CASES)
-def test_global_band_solver(ctx, monkeypatch, B):
-    """LLD_GBA_SOLVER=band is read at upload (the module context indexes every call again)"""
-    monkeypatch.setenv("LLD_GBA_SOLVER", "band")
-    p = cr_problem(B, 60)
-    _, names = checked(p, ctx, "global", (8,), f"band B={B}")
-    assert {"k_band_assemble", "k_solve_band<512>"} <= names and not any(n.startswith("k_cr_") for n in names), names
 
 
 @pytest.mark.gpu
@@ -618,11 +592,11 @@ def test_local_lanes_per_line(tmp_path, lanes):
 
 
 @pytest.mark.gpu
-@pytest.mark.parametrize("env", [{"LLD_BA_GRAPH": "0"}, {"LLD_BA_LEAN": "0"}], ids=["eager", "not-lean"])
+@pytest.mark.parametrize("env", [{"LLD_BA_GRAPH": "0"}], ids=["eager"])
 def test_local_step_schedules(ctx, monkeypatch, env):
-    """graph replay against eager launches: the same kernels in the same order of sums, bit-identical.  Without the lean
-    steps other kernels run (k_decide_fused instead of k_decide_carry): oracle tolerances.  Both batches are dense and
-    single-rank, so the default runs graph replay on forked streams and lean steps (test_ragged_and_target_are_dense_single)."""
+    """graph replay against eager launches: the same kernels in the same order of sums, bit-identical.  Both batches are
+    dense and single-rank, so the default runs graph replay on forked streams and lean steps
+    (test_ragged_and_target_are_dense_single)."""
     for name in ("ragged", "target"):
         p = globals()[f"{name}_batch"]()
         ref = run(p, ctx, "local")
@@ -630,11 +604,8 @@ def test_local_step_schedules(ctx, monkeypatch, env):
             for k, v in env.items():
                 m.setenv(k, v)
             g, names = checked(p, ctx, "local", what=f"{name} {env}")
-        if "LLD_BA_GRAPH" in env:
-            assert_identical(g, ref, f"{name} eager vs graph")
-            assert "k_decide_carry" in names
-        else:
-            assert "k_decide_carry" not in names and "k_decide_fused" in names, names
+        assert_identical(g, ref, f"{name} eager vs graph")
+        assert "k_decide_carry" in names
 
 
 @pytest.mark.gpu

@@ -282,7 +282,7 @@ def sctx(built):
 
 def assert_sparse_arm(names):
     assert SP_KERNELS <= names, names
-    assert not names & {"k_cr_factor", "k_cr_solve<15>", "k_cr_solve<20>", "k_cr_update", "k_solve_env", "k_solve_band<512>"}, names
+    assert not names & {"k_cr_factor", "k_cr_solve<15>", "k_cr_solve<20>", "k_cr_update", "k_solve_env"}, names
 
 
 @pytest.mark.gpu

@@ -77,27 +77,6 @@ def test_local_ba_batch_ragged(gpu_ctx):
     check_ba(g, o, "ragged")
 
 
-def test_fused_step_parity(gpu_ctx):
-    """the opt-in fused linearise -> Schur step (ba_fused.cuh, LLD_BA_FUSED=1; the switch is read once per process, hence
-    the subprocess): same ragged batch + the target shape, same checks against the oracle"""
-    import subprocess, sys, os
-    code = (
-        "import sys, numpy as np; sys.path.insert(0, 'tests')\n"
-        "from lld_slam_b200 import api, capi, synth\n"
-        "from test_gpu_parity import check_ba\n"
-        "ctx = capi.Context(0)\n"
-        "rng = np.random.default_rng(5)\n"
-        "wins = [synth.make_ba_window(8, 500, 100, rng, n_fixed_extra=2), synth.make_ba_window(5, 300, 0, rng),\n"
-        "        synth.make_ba_window(12, 50, 200, rng), synth.make_ba_window(20, 800, 150, rng, n_fixed_extra=1),\n"
-        "        synth.make_ba_window(3, 40, 10, rng)]\n"
-        "for p in (synth.batch_ba(wins, 'local'), synth.make_local_ba_batch(1, 10, 5000, 1000, 77)):\n"
-        "    check_ba(api.ba_local(p, 5, 15, impl='gpu', ctx=ctx), api.ba_local(p, 5, 15, impl='oracle'), 'fused')\n"
-        "print('fused-ok')\n")
-    root = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-    r = subprocess.run([sys.executable, "-c", code], cwd=root, env=dict(os.environ, LLD_BA_FUSED="1"), capture_output=True, text=True, timeout=600)
-    assert r.returncode == 0 and "fused-ok" in r.stdout, r.stdout[-2000:] + r.stderr[-2000:]
-
-
 def test_local_ba_batch_pipelined(gpu_ctx, monkeypatch):
     """large batches are cut into sub-batches that two worker contexts pipeline (host indexing of one overlaps the LM steps
     of the other); forced here on a ragged batch: every window must still match the oracle."""
