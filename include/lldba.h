@@ -22,6 +22,7 @@
  *   lld_tri_search         <- ORBmatcher::SearchForTriangulation     src/ORBmatcher.cc:657-823
  *   lld_bow_search         <- ORBmatcher::SearchByBoW x2             src/ORBmatcher.cc:159-288, 522-655
  *   lld_init_search        <- ORBmatcher::SearchForInitialization    src/ORBmatcher.cc:405
+ *   lld_sim3_opt           <- Optimizer::OptimizeSim3                src/Optimizer.cc:1656-1858
  *   lld_line_associate     <- Tracking::AddLinesFrom                 src/Tracking.cc:996-1124
  *   lld_medoid_orb / _float<- MapPoint / MapLine::ComputeDistinctiveDescriptors              src/MapPoint.cc:242-307, src/MapLine.cc:133-201
  *
@@ -82,6 +83,8 @@ extern "C" {
  *   - lld_init_search: at most 65535 keypoints per frame, F2 octaves < 8; with check_orientation, F1 angles in [0, 900) and F2
  *     angles in [0, 360) (ORB angles are in [0, 360)).  The sequential resolve keeps F2's state in shared memory when every F2
  *     of the batch has at most 57088 keypoints (k_init_resolve_smem), else in global memory (k_init_resolve_global);
+ *   - lld_sim3_opt: no limit on the correspondences of a problem.  When every problem of the batch has at most 4266 (48 bytes each
+ *     within 200 KB) the edge records are staged in shared memory (k_sim3_opt_smem), else read from global memory (k_sim3_opt_global);
  *   - lld_line_match: descriptor widths that are a multiple of 8 up to 72 floats and at most 512 lines per side of a pair run on the
  *     tensor cores, everything else on the FP32 tile path (no failure).
  */
@@ -467,6 +470,54 @@ typedef struct lld_init_search_result {
 } lld_init_search_result;
 
 int lld_init_search(void* ctx, const lld_init_search_problem* p, lld_init_search_result* out);
+
+/* ------------------------------------------------------------------------------------------------
+ * Loop-candidate Sim3 optimisation: Optimizer::OptimizeSim3(pKF1, pKF2, vpMatches1, g2oS12, th2, bFixScale)
+ * src/Optimizer.cc:1656-1858, batched over loop candidates (LoopClosing::ComputeSim3 calls it with th2 = 10 and mbFixScale).
+ * One VertexSim3Expmap (estimate g2oS12, _fix_scale, K1 / K2) and, per correspondence i in vpMatches1 order, the fixed
+ * camera-frame points P1c = R1w X1w + t1w, P2c = R2w X2w + t2w and two edges in this order:
+ *   e12 = obs1 - cam_map1(project(S12.map(P2c))),  e21 = obs2 - cam_map2(project(S12.inverse().map(P1c))),
+ * information invSigma2 I2 of the keypoint's own keyframe, Huber delta = sqrtf(th2).  The edges are differentiated
+ * numerically as g2o does (central differences at 1e-9; with a fixed scale the scale column is 0).  Levenberg-Marquardt
+ * with a dense 7x7 LDL^T: optimize(its_first); a correspondence whose e12 or e21 chi2 (of the last evaluated error, also
+ * when that LM trial was rejected) exceeds th2 is dropped (inlier = 0); fewer than 10 left: n_in = 0 and S12 = the input
+ * (the drops stay); else optimize(its_more_outliers if any was dropped, its_more_clean otherwise) from the state reached,
+ * the same test again, n_in = the correspondences that pass it.  Correspondences the reference skips (no map point in
+ * pKF1, a bad point, i2 < 0) are not passed; the caller leaves their vpMatches1 entries as they are.
+ * ---------------------------------------------------------------------------------------------- */
+typedef struct lld_sim3_problem {
+  int32_t n_problems;
+  const double* S12;          /* [n][8] g2o::Sim3: qx qy qz qw, tx ty tz, s */
+  const double* cam;          /* [n][8] fx1 fy1 cx1 cy1 fx2 fy2 cx2 cy2: pKF1->mK, pKF2->mK (float values, widened) */
+  const int32_t* fix_scale;   /* [n] bFixScale: 0 or 1 */
+  const float* th2;           /* [n] th2 > 0 */
+  const int32_t* off;         /* [n+1] CSR over correspondences, off[0] = 0 */
+  const float* p1c;           /* [m][3] P1c, computed in float as the reference does (cv::Mat) */
+  const float* p2c;           /* [m][3] P2c */
+  const float* obs1;          /* [m][2] pKF1->mvKeysUn[i].pt */
+  const float* obs2;          /* [m][2] pKF2->mvKeysUn[i2].pt */
+  const float* info1;         /* [m] pKF1->mvInvLevelSigma2[octave of kpUn1] */
+  const float* info2;         /* [m] pKF2->mvInvLevelSigma2[octave of kpUn2] */
+  int32_t its_first;          /* 5 */
+  int32_t its_more_outliers;  /* 10 */
+  int32_t its_more_clean;     /* 5 */
+} lld_sim3_problem;
+
+typedef struct lld_sim3_result {
+  double* S12;          /* [n][8] g2oS12 after the call */
+  uint8_t* inlier;      /* [m] 1 = vpMatches1[i] kept, 0 = cleared */
+  int32_t* n_in;        /* [n] return value */
+  /* LM trace, [n][log_stride] (log_stride >= its_first + max(its_more_*) + 2 when a log is given): round 1 at entry 0, round 2
+   * at entry its_first + 1; in each round entry 0 = robust chi2 at the start, entry k = chi2 / lambda / trials after LM
+   * iteration k; the rest is 0.  n_iter_done[n][2] = iterations run per round (0 for a round that did not run). */
+  int32_t log_stride;
+  double* chi2_log;     /* may be NULL */
+  double* lambda_log;   /* may be NULL */
+  int32_t* trials_log;  /* may be NULL */
+  int32_t* n_iter_done; /* may be NULL */
+} lld_sim3_result;
+
+int lld_sim3_opt(void* ctx, const lld_sim3_problem* p, lld_sim3_result* out);
 
 /* ------------------------------------------------------------------------------------------------
  * Stereo line matching (float line descriptors)

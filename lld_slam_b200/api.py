@@ -175,6 +175,25 @@ def init_search(p: Dict[str, Any], *, impl: str = "gpu", ctx=None):
     return out
 
 
+def sim3_opt(p: Dict[str, Any], *, impl: str = "gpu", ctx=None):
+    """Optimizer::OptimizeSim3, batched over loop candidates: S12 (g2oS12 after the call, [n][8] q t s), inlier (vpMatches1 kept,
+    [m]), n_in (return value) and the LM trace of both rounds (include/lldba.h)"""
+    lib = _lib(impl)
+    prob, keep = capi.fill_struct(capi.Sim3Problem, p)
+    n, m = int(p["n_problems"]), int(p["off"][-1])
+    stride = int(p["its_first"]) + max(int(p["its_more_outliers"]), int(p["its_more_clean"])) + 2
+    out = dict(S12=np.zeros((max(n, 1), 8)), inlier=np.full(max(m, 1), 2, np.uint8), n_in=np.full(max(n, 1), -1, np.int32),
+               log_stride=stride, chi2_log=np.zeros((max(n, 1), stride)), lambda_log=np.zeros((max(n, 1), stride)),
+               trials_log=np.zeros((max(n, 1), stride), np.int32), n_iter_done=np.zeros((max(n, 1), 2), np.int32))
+    res, keep2 = capi.fill_struct(capi.Sim3Result, out)
+    rc = lib.sim3_opt(_handle(impl, ctx), C.byref(prob), C.byref(res))
+    _check(impl, ctx, rc, "lld_sim3_opt")
+    for k in ("S12", "n_in", "chi2_log", "lambda_log", "trials_log", "n_iter_done"):
+        out[k] = out[k][:n]
+    out["inlier"] = out["inlier"][:m]
+    return out
+
+
 def line_match(p: Dict[str, Any], *, impl: str = "gpu", ctx=None):
     lib = _lib(impl)
     prob, keep = capi.fill_struct(capi.LineMatchProblem, p)

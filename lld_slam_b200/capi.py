@@ -3,7 +3,8 @@
 This is the Python harness over the C-ABI used by tests/ and bench.py.  The product library is
 lld_slam_b200/csrc/liblldba.so (CUDA, sm_100a); `load_library()` fails loudly when it is missing —
 there is no CPU fallback.  `load_oracle()` loads the CPU oracle (oracle/liblld_oracle.so) which
-exposes the same entry points with the `lldo_` prefix (lldo_init_search from tests/hostcheck/libinit_search_oracle.so); only tests, smoke() and the bench's
+exposes the same entry points with the `lldo_` prefix (lldo_init_search from tests/hostcheck/libinit_search_oracle.so, lldo_sim3_opt from
+tests/hostcheck/libsim3_oracle.so); only tests, smoke() and the bench's
 cpu_baseline / reference arm may call it.
 """
 from __future__ import annotations
@@ -19,6 +20,7 @@ LIB_PATH = os.environ.get("LLD_LIB_PATH") or os.path.join(_ROOT, "lld_slam_b200"
 ORACLE_PATH = os.path.join(_ROOT, "oracle", "liblld_oracle.so")
 # the oracle's SearchForInitialization (lldo_init_search) is a separate test-infrastructure library
 INIT_SEARCH_ORACLE_PATH = os.path.join(_ROOT, "tests", "hostcheck", "libinit_search_oracle.so")
+SIM3_ORACLE_PATH = os.path.join(_ROOT, "tests", "hostcheck", "libsim3_oracle.so")
 
 c_i32p = C.POINTER(C.c_int32)
 c_u8p = C.POINTER(C.c_uint8)
@@ -156,6 +158,21 @@ class InitSearchResult(C.Structure):
     _fields_ = [("match12", c_i32p), ("n_matches", c_i32p), ("prev_matched", c_f32p)]
 
 
+class Sim3Problem(C.Structure):
+    _fields_ = [
+        ("n_problems", C.c_int32), ("S12", c_f64p), ("cam", c_f64p), ("fix_scale", c_i32p), ("th2", c_f32p), ("off", c_i32p),
+        ("p1c", c_f32p), ("p2c", c_f32p), ("obs1", c_f32p), ("obs2", c_f32p), ("info1", c_f32p), ("info2", c_f32p),
+        ("its_first", C.c_int32), ("its_more_outliers", C.c_int32), ("its_more_clean", C.c_int32),
+    ]
+
+
+class Sim3Result(C.Structure):
+    _fields_ = [
+        ("S12", c_f64p), ("inlier", c_u8p), ("n_in", c_i32p), ("log_stride", C.c_int32),
+        ("chi2_log", c_f64p), ("lambda_log", c_f64p), ("trials_log", c_i32p), ("n_iter_done", c_i32p),
+    ]
+
+
 class TriSearchResult(C.Structure):
     _fields_ = [("match12", c_i32p), ("n_matches", c_i32p)]
 
@@ -263,6 +280,16 @@ class _Lib:
             self.init_search.restype = C.c_int
         else:
             self._sig("init_search", init_sig)
+        sim3_sig = [vp, C.POINTER(Sim3Problem), C.POINTER(Sim3Result)]
+        if self.is_oracle:
+            if not os.path.exists(SIM3_ORACLE_PATH):
+                raise RuntimeError(f"{SIM3_ORACLE_PATH} not found — build it first (python -c 'import __graft_entry__ as g; g.build()').")
+            self.sim3_dll = C.CDLL(SIM3_ORACLE_PATH)
+            self.sim3_opt = self.sim3_dll.lldo_sim3_opt
+            self.sim3_opt.argtypes = sim3_sig
+            self.sim3_opt.restype = C.c_int
+        else:
+            self._sig("sim3_opt", sim3_sig)
         self._sig("line_match", [vp, C.POINTER(LineMatchProblem), C.POINTER(LineMatchResult)])
         self._sig("descriptor_distance", [c_u8p, c_u8p])
         if not self.is_oracle:

@@ -343,6 +343,126 @@ LLD_HD bool line_depth_positive(const double* X0c, const double* ldc, double f, 
   return ok;
 }
 
+// ---- Sim3 (g2o::Sim3 of ORB-SLAM2's vendored g2o, types/sim3.h) -----------------------------------
+// State S[8] = q (x y z w), t[3], s.  Every expression follows the source's evaluation order (Eigen evaluates the
+// 3x3 products coefficient-wise, k = 0..2 left to right), so that the host build of this header, the CPU oracle and
+// the kernel agree to the bit wherever no transcendental function is involved.
+LLD_HD void sim3_map(const double* S, const double* x, double* o) {  // s * (r * x) + t
+  double rx[3];
+  quat_rot(S, x, rx);
+  o[0] = S[7] * rx[0] + S[4];
+  o[1] = S[7] * rx[1] + S[5];
+  o[2] = S[7] * rx[2] + S[6];
+}
+LLD_HD void sim3_mul(const double* A, const double* B, double* O) {  // (r_A r_B, s_A (r_A t_B) + t_A, s_A s_B)
+  double q[4], rt[3];
+  quat_mul(A, B, q);
+  quat_rot(A, B + 4, rt);
+  O[0] = q[0]; O[1] = q[1]; O[2] = q[2]; O[3] = q[3];
+  O[4] = A[7] * rt[0] + A[4];
+  O[5] = A[7] * rt[1] + A[5];
+  O[6] = A[7] * rt[2] + A[6];
+  O[7] = A[7] * B[7];
+}
+LLD_HD void sim3_inverse(const double* S, double* O) {  // (r^-1, r^-1 ((-1/s) t), 1/s), r^-1 = conjugate
+  const double qc[4] = {-S[0], -S[1], -S[2], S[3]};
+  const double c = -1. / S[7];
+  const double v[3] = {c * S[4], c * S[5], c * S[6]};
+  double rt[3];
+  quat_rot(qc, v, rt);
+  O[0] = qc[0]; O[1] = qc[1]; O[2] = qc[2]; O[3] = qc[3];
+  O[4] = rt[0]; O[5] = rt[1]; O[6] = rt[2];
+  O[7] = 1. / S[7];
+}
+// Sim3(const Vector7d& update): omega = u[0:3], upsilon = u[3:6], sigma = u[6]
+LLD_HD void sim3_exp(const double* u, double* S) {
+  const double w0 = u[0], w1 = u[1], w2 = u[2], sigma = u[6];
+  const double theta = sqrt(w0 * w0 + w1 * w1 + w2 * w2);
+  const double O[9] = {0, -w2, w1, w2, 0, -w0, -w1, w0, 0};
+  double O2[9];
+#pragma unroll
+  for (int i = 0; i < 3; i++)
+#pragma unroll
+    for (int j = 0; j < 3; j++) O2[3 * i + j] = O[3 * i] * O[j] + O[3 * i + 1] * O[3 + j] + O[3 * i + 2] * O[6 + j];
+  const double s = exp(sigma);
+  const double eps = 0.00001;
+  double A, B, C, ra = 1.0, rb = 1.0;  // R = I + ra * Omega + rb * Omega^2
+  bool small = false;                     // theta < eps: R = I + Omega + Omega^2 (sic)
+  if (fabs(sigma) < eps) {
+    C = 1;
+    if (theta < eps) {
+      A = 1. / 2.;
+      B = 1. / 6.;
+      small = true;
+    } else {
+      const double theta2 = theta * theta;
+      A = (1 - cos(theta)) / (theta2);
+      B = (theta - sin(theta)) / (theta2 * theta);
+      ra = sin(theta) / theta; rb = (1 - cos(theta)) / (theta * theta);
+    }
+  } else {
+    C = (s - 1) / sigma;
+    if (theta < eps) {
+      const double sigma2 = sigma * sigma;
+      A = ((sigma - 1) * s + 1) / sigma2;
+      B = ((0.5 * sigma2 - sigma + 1) * s) / (sigma2 * sigma);
+      small = true;
+    } else {
+      ra = sin(theta) / theta; rb = (1 - cos(theta)) / (theta * theta);
+      const double a = s * sin(theta);
+      const double b = s * cos(theta);
+      const double theta2 = theta * theta;
+      const double sigma2 = sigma * sigma;
+      const double c = theta2 + sigma2;
+      A = (a * sigma + (1 - b) * theta) / (theta * c);
+      B = (C - ((b - 1) * sigma + a * theta) / (c)) * 1. / (theta2);
+    }
+  }
+  double R[9], W[9];
+#pragma unroll
+  for (int i = 0; i < 9; i++) {
+    const double id = (i == 0 || i == 4 || i == 8) ? 1.0 : 0.0;
+    R[i] = small ? id + O[i] + O2[i] : id + ra * O[i] + rb * O2[i];
+    W[i] = A * O[i] + B * O2[i] + C * id;
+  }
+  quat_from_R(R, S);
+  S[4] = W[0] * u[3] + W[1] * u[4] + W[2] * u[5];
+  S[5] = W[3] * u[3] + W[4] * u[4] + W[5] * u[5];
+  S[6] = W[6] * u[3] + W[7] * u[4] + W[8] * u[5];
+  S[7] = s;
+}
+// VertexSim3Expmap::oplusImpl: with _fix_scale the caller's update[6] is set to 0, then estimate = Sim3(update) * estimate
+LLD_HD void sim3_oplus(const double* S, double* u, bool fix_scale, double* out) {
+  if (fix_scale) u[6] = 0;
+  double E[8];
+  sim3_exp(u, E);
+  sim3_mul(E, S, out);
+}
+// EdgeSim3ProjectXYZ / EdgeInverseSim3ProjectXYZ::computeError: obs - cam_map(project(S.map(P))), where S is the
+// estimate (e12, P = P2c, K1) or its inverse (e21, P = P1c, K2); K = fx fy cx cy
+LLD_HD void sim3_edge_error(const double* S, const double* P, const double* K, const double* obs, double* err) {
+  double x[3];
+  sim3_map(S, P, x);
+  const double p0 = x[0] / x[2], p1 = x[1] / x[2];
+  err[0] = obs[0] - (p0 * K[0] + K[2]);
+  err[1] = obs[1] - (p1 * K[1] + K[3]);
+}
+// The 14 states of g2o's numeric Jacobian (BaseBinaryEdge::linearizeOplus, delta = 1e-9): Sk[2d] = oplus(S, +delta e_d),
+// Sk[2d+1] = oplus(S, -delta e_d); each with its inverse for the e21 edge.  Writes 8 doubles per state.
+LLD_HD void sim3_perturbed(const double* S, int k, bool fix_scale, double* Sk, double* Skinv) {
+  const double delta = 1e-9;
+  double add[7] = {0, 0, 0, 0, 0, 0, 0};
+  add[k >> 1] = (k & 1) ? -delta : delta;
+  sim3_oplus(S, add, fix_scale, Sk);
+  sim3_inverse(Sk, Skinv);
+}
+// One column of the 2x7 numeric Jacobian from the errors at the +delta / -delta states: scalar * (e+ - e-)
+LLD_HD void sim3_jac_col(const double* ep, const double* em, double* J, int d) {
+  const double scalar = 1.0 / (2 * 1e-9);
+  J[d] = scalar * (ep[0] - em[0]);
+  J[7 + d] = scalar * (ep[1] - em[1]);
+}
+
 // ---- tiny dense helpers --------------------------------------------------------------------------
 // symmetric 3x3 / 4x4 inverse via cofactors / blockwise (general inverse, like MatrixXd::inverse()).
 LLD_HD void inv3_sym(const double* A /*full 9*/, double* I) {

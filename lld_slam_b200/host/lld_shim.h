@@ -14,6 +14,7 @@
 //   lld::ORBmatcher::SearchByProjection     <- src/ORBmatcher.cc:1328-1470 (frame to frame), :45-129 (frame to map points) and
 //                                              :1472-1599 (frame to keyframe, relocalisation)
 //   lld::ORBmatcher::SearchForInitialization <- src/ORBmatcher.cc:405
+//   lld::Optimizer::OptimizeSim3            <- src/Optimizer.cc:1656-1858
 //   lld::TwoFrameLineMatcher::MatchLines    <- src/TwoFrameLineMatcher.cc:26-77
 // Every entry point takes the library context as an extra first argument (the reference keeps its g2o optimizer on the
 // stack instead); Flatten* expose the flattened problem so that tests can compare it array by array with a reference
@@ -34,6 +35,7 @@ namespace lld {
 
 struct KeyPoint { float x, y; int octave; float angle; };
 struct Point2f { float x, y; };                  // cv::Point2f
+struct Sim3 { double q[4], t[3], s; };           // g2o::Sim3: rotation (x y z w), translation, scale; map(x) = s (q x) + t
 struct KeyLine { float startPointX, startPointY, endPointX, endPointY; int octave; };
 
 struct KeyFrame {
@@ -77,6 +79,10 @@ struct MapPoint {
   uint8_t mDescriptor[32] = {0};                     // GetDescriptor()
   float mNormalVector[3] = {0, 0, 1};                // GetNormal()
   bool IsInKeyFrame(KeyFrame* pKF) const { return observations.count(pKF) != 0; }
+  int GetIndexInKeyFrame(KeyFrame* pKF) const {                 // src/MapPoint.cc
+    auto it = observations.find(pKF);
+    return it == observations.end() ? -1 : (int)it->second;
+  }
   float mfMinDistance = 0, mfMaxDistance = 0;        // scale-invariance range (src/MapPoint.cc:373-383)
   float GetMinDistanceInvariance() const { return 0.8f * mfMinDistance; }
   float GetMaxDistanceInvariance() const { return 1.2f * mfMaxDistance; }
@@ -535,6 +541,62 @@ class Optimizer {
     for (size_t j = 0; j < lidx.size(); j++) F->mvbOutlierLines[lidx[j]] = lo_[j] != 0;
     for (int c = 0; c < 12; c++) F->mTcw[c] = (float)oT[c];
     return n_inl;
+  }
+
+  // int static OptimizeSim3(KeyFrame* pKF1, KeyFrame* pKF2, vector<MapPoint*>& vpMatches1, g2o::Sim3& g2oS12, const float th2,
+  //                         const bool bFixScale)   include/Optimizer.h, src/Optimizer.cc:1656-1858
+  // Correspondences without a map point in pKF1, with a bad point or with a point not in pKF2 are skipped and their vpMatches1
+  // entries left as they are; P1c / P2c in float (cv::Mat: R * X + t accumulates in double and rounds once) -> lld_sim3_opt ->
+  // vpMatches1[i] cleared for the dropped correspondences, g2oS12 written unless fewer than 10 correspondences survived.
+  static int OptimizeSim3(void* ctx, KeyFrame* pKF1, KeyFrame* pKF2, std::vector<MapPoint*>& vpMatches1, Sim3& g2oS12, const float th2,
+                          const bool bFixScale) {
+    const std::vector<MapPoint*>& vpMapPoints1 = pKF1->mvpMapPoints;   // GetMapPointMatches()
+    std::vector<float> p1c, p2c, obs1, obs2, info1, info2;
+    std::vector<size_t> vnIndexEdge;
+    auto cam_frame = [](const KeyFrame* k, const float* X, std::vector<float>& out) {
+      const float* T = k->Tcw;
+      for (int r = 0; r < 3; r++)
+        out.push_back((float)((double)T[3 * r] * X[0] + (double)T[3 * r + 1] * X[1] + (double)T[3 * r + 2] * X[2] + (double)T[9 + r]));
+    };
+    for (size_t i = 0; i < vpMatches1.size(); i++) {
+      if (!vpMatches1[i]) continue;
+      MapPoint* pMP1 = vpMapPoints1[i];
+      MapPoint* pMP2 = vpMatches1[i];
+      const int i2 = pMP2->GetIndexInKeyFrame(pKF2);
+      if (!pMP1 || pMP1->isBad() || pMP2->isBad() || i2 < 0) continue;
+      cam_frame(pKF1, pMP1->pos, p1c);
+      cam_frame(pKF2, pMP2->pos, p2c);
+      const KeyPoint& k1 = pKF1->mvKeysUn[i];
+      const KeyPoint& k2 = pKF2->mvKeysUn[(size_t)i2];
+      obs1.push_back(k1.x); obs1.push_back(k1.y);
+      obs2.push_back(k2.x); obs2.push_back(k2.y);
+      info1.push_back(pKF1->mvInvLevelSigma2[k1.octave]);
+      info2.push_back(pKF2->mvInvLevelSigma2[k2.octave]);
+      vnIndexEdge.push_back(i);
+    }
+    const int m = (int)vnIndexEdge.size();
+    double S[8] = {g2oS12.q[0], g2oS12.q[1], g2oS12.q[2], g2oS12.q[3], g2oS12.t[0], g2oS12.t[1], g2oS12.t[2], g2oS12.s};
+    const double cam[8] = {pKF1->fx, pKF1->fy, pKF1->cx, pKF1->cy, pKF2->fx, pKF2->fy, pKF2->cx, pKF2->cy};
+    const int32_t fix = bFixScale ? 1 : 0, off[2] = {0, m};
+    lld_sim3_problem p;
+    std::memset(&p, 0, sizeof(p));
+    p.n_problems = 1; p.S12 = S; p.cam = cam; p.fix_scale = &fix; p.th2 = &th2; p.off = off;
+    p.p1c = p1c.data(); p.p2c = p2c.data(); p.obs1 = obs1.data(); p.obs2 = obs2.data(); p.info1 = info1.data(); p.info2 = info2.data();
+    p.its_first = 5; p.its_more_outliers = 10; p.its_more_clean = 5;
+    double oS[8];
+    std::vector<uint8_t> inl((size_t)m + 1);
+    int32_t n_in = 0;
+    lld_sim3_result r;
+    std::memset(&r, 0, sizeof(r));
+    r.S12 = oS; r.inlier = inl.data(); r.n_in = &n_in;
+    const int rc = lld_sim3_opt(ctx, &p, &r);
+    if (rc) return rc;
+    for (int j = 0; j < m; j++)
+      if (!inl[j]) vpMatches1[vnIndexEdge[j]] = nullptr;
+    for (int k = 0; k < 4; k++) g2oS12.q[k] = oS[k];   // the early return hands the input back: g2oS12 keeps its value
+    for (int k = 0; k < 3; k++) g2oS12.t[k] = oS[4 + k];
+    g2oS12.s = oS[7];
+    return n_in;
   }
 };
 

@@ -719,6 +719,74 @@ def make_init_search_batch(n_pairs, n_kp, seed, window_size=100, nn_ratio=0.9, c
     return out
 
 
+def _quat_xyzw(R):
+    """unit quaternion (x y z w, w >= 0) of a rotation matrix"""
+    w = np.sqrt(max(0.0, 1.0 + R[0, 0] + R[1, 1] + R[2, 2])) / 2.0
+    x = np.copysign(np.sqrt(max(0.0, 1.0 + R[0, 0] - R[1, 1] - R[2, 2])) / 2.0, R[2, 1] - R[1, 2])
+    y = np.copysign(np.sqrt(max(0.0, 1.0 - R[0, 0] + R[1, 1] - R[2, 2])) / 2.0, R[0, 2] - R[2, 0])
+    z = np.copysign(np.sqrt(max(0.0, 1.0 - R[0, 0] - R[1, 1] + R[2, 2])) / 2.0, R[1, 0] - R[0, 1])
+    q = np.array([x, y, z, w])
+    return q / np.linalg.norm(q)
+
+
+def make_sim3_batch(n_problems, n_corr, seed, fix_scale=1, outlier_frac=0.1, th2=10.0, rot_deg=3.0, trans_m=0.3, scale_pct=3.0):
+    """Optimizer::OptimizeSim3 as LoopClosing::ComputeSim3 calls it (th2 = 10, 5 / 10 / 5 iterations): per loop candidate two
+    KITTI-camera keyframes related by a Sim3 S12 (P1c = s R P2c + t; s = 1 with fix_scale, s in [0.5, 2] otherwise), points 4-40 m
+    in front of keyframe 1 and visible from both, keypoints at ORB octaves 0-7 with 1.2^octave px noise, a share of gross outliers
+    (one of the two keypoints replaced by an unrelated one), and an initial S12 off by a few degrees, decimetres and (free
+    scale) percent.  n_corr may be a list (ragged problems, 0 allowed)."""
+    rng = np.random.default_rng(seed)
+    lvl_p = np.asarray([SCALE ** (-2.0 * l) for l in range(N_LEVELS)]); lvl_p /= lvl_p.sum()
+    isig = inv_level_sigma2()
+    K = np.array([FX, FY, CX, CY], np.float32).astype(np.float64)
+    acc = {k: [] for k in ("p1c", "p2c", "obs1", "obs2", "info1", "info2")}
+    S12, cams, off = [], [], [0]
+    for pb in range(n_problems):
+        m = int(n_corr[pb]) if np.ndim(n_corr) else int(n_corr)
+        R = _rodrigues(rng.normal(0, 1, 3) * np.deg2rad(4.0) / np.sqrt(3))
+        t = np.array([rng.uniform(-1, 1), rng.uniform(-0.2, 0.2), rng.uniform(-2, 2)])
+        s = 1.0 if fix_scale else float(np.exp(rng.uniform(np.log(0.5), np.log(2.0))))
+        # points in keyframe 1: inside its image, visible from keyframe 2
+        X1 = np.zeros((0, 3))
+        while len(X1) < m:
+            z = rng.uniform(4.0, 40.0, 2 * m + 8)
+            u, v = rng.uniform(20, IMG_W - 20, z.size), rng.uniform(20, IMG_H - 20, z.size)
+            X = np.stack([(u - CX) / FX * z, (v - CY) / FY * z, z], 1)
+            X2 = ((X - t) @ R) / s                         # S12^-1
+            u2 = FX * X2[:, 0] / X2[:, 2] + CX; v2 = FY * X2[:, 1] / X2[:, 2] + CY
+            ok = (X2[:, 2] > 1.0) & (u2 > 0) & (u2 < IMG_W) & (v2 > 0) & (v2 < IMG_H)
+            X1 = np.concatenate([X1, X[ok]])[:m]
+        X2 = ((X1 - t) @ R) / s
+        oct1, oct2 = rng.choice(N_LEVELS, m, p=lvl_p), rng.choice(N_LEVELS, m, p=lvl_p)
+        def obs(X, o):
+            return np.stack([FX * X[:, 0] / X[:, 2] + CX, FY * X[:, 1] / X[:, 2] + CY], 1) + rng.normal(0, 1, (len(X), 2)) * (SCALE ** o)[:, None]
+        o1, o2 = obs(X1, oct1), obs(X2, oct2)
+        bad = rng.random(m) < outlier_frac
+        side = rng.random(m) < 0.5
+        junk = np.stack([rng.uniform(0, IMG_W, m), rng.uniform(0, IMG_H, m)], 1)
+        o1[bad & side] = junk[bad & side]; o2[bad & ~side] = junk[bad & ~side]
+        # map point positions carry their own small errors (5 mm at 10 m, growing with depth)
+        P1 = X1 + rng.normal(0, 1, X1.shape) * 0.0005 * X1[:, 2:3]
+        P2 = X2 + rng.normal(0, 1, X2.shape) * 0.0005 * X2[:, 2:3]
+        acc["p1c"].append(P1); acc["p2c"].append(P2); acc["obs1"].append(o1); acc["obs2"].append(o2)
+        acc["info1"].append(isig[oct1]); acc["info2"].append(isig[oct2])
+        # initial estimate: the truth off by a few degrees, decimetres and percent
+        dR = _rodrigues(rng.normal(0, 1, 3) * np.deg2rad(rot_deg) / np.sqrt(3))
+        s0 = s if fix_scale else s * (1.0 + rng.uniform(-1, 1) * scale_pct / 100.0)
+        S12.append(np.concatenate([_quat_xyzw(dR @ R), t + rng.normal(0, 1, 3) * trans_m / np.sqrt(3), [s0]]))
+        cams.append(np.concatenate([K, K]))
+        off.append(off[-1] + m)
+    out = dict(n_problems=n_problems, S12=np.ascontiguousarray(np.asarray(S12, np.float64).reshape(-1, 8)),
+               cam=np.ascontiguousarray(np.asarray(cams, np.float64).reshape(-1, 8)),
+               fix_scale=np.full(n_problems, int(fix_scale), np.int32), th2=np.full(n_problems, th2, np.float32),
+               off=np.asarray(off, np.int32), its_first=5, its_more_outliers=10, its_more_clean=5)
+    for k, v in acc.items():
+        w = 3 if k[0] == "p" else (2 if k[0] == "o" else 1)
+        a = np.concatenate(v) if v else np.zeros((0, w))
+        out[k] = np.ascontiguousarray(f32(a).reshape(-1, w) if w > 1 else f32(a).reshape(-1))
+    return out
+
+
 def make_line_match_batch(n_pairs, n_lines, desc_dim, seed, tau=2.0, min_len=10, ragged=False):
     rng = np.random.default_rng(seed)
     P, N, D = n_pairs, n_lines, desc_dim

@@ -1,6 +1,6 @@
 #!/usr/bin/env python
 """Timing of the SURVEY §8(f) kernels (ComputeStereoMatches, relocalisation / map-point SearchByProjection, temporal line
-association, distinctive descriptors, SearchForInitialization): device compute time from the library's own CUDA events (host buffers in, results
+association, distinctive descriptors, SearchForInitialization, OptimizeSim3): device compute time from the library's own CUDA events (host buffers in, results
 out through the public call), wall clock of the same call, and the CPU oracle on the same or a smaller sample.
 Prints one JSON object; results are compared with the oracle where the sample is the same.
 Usage: aux_kernels.py [section ...]   (default: every section)"""
@@ -140,4 +140,44 @@ if want("search_for_initialization"):
                      "candidate_listing": part(["k_init_count", "k_init_scan", "k_init_fill"]),
                      "resolve": part(["k_init_resolve_smem", "k_init_resolve_global"]), "histogram_and_output": part(["k_init_finalize"])},
         "gpu": torch.cuda.get_device_name(0), "nvidia_smi_name_power_limit": smi.strip()}
+# ---- OptimizeSim3 (LoopClosing::ComputeSim3: th2 = 10, 5 / 10 / 5 iterations), both scale modes
+if want("optimize_sim3"):
+    import subprocess
+    import ctypes as C
+    import torch
+    d = ctx.lib.dll
+    d.lld_ctx_profile.argtypes = [C.c_void_p, C.c_int]; d.lld_ctx_profile.restype = None
+    d.lld_ctx_profile_report.argtypes = [C.c_void_p, C.c_char_p, C.c_int]; d.lld_ctx_profile_report.restype = C.c_int
+    res = {}
+    for fix in (1, 0):
+        ps = synth.make_sim3_batch(4096, 300, 131 + fix, fix_scale=fix)
+        g, ms, wall = timed(lambda: api.sim3_opt(ps, impl="gpu", ctx=ctx))
+        d.lld_ctx_profile(ctx.handle, 1)                     # separate, profiled run: per-launch CUDA events
+        api.sim3_opt(ps, impl="gpu", ctx=ctx)
+        buf = C.create_string_buffer(1 << 16)
+        ctx.check(d.lld_ctx_profile_report(ctx.handle, buf, len(buf)), "lld_ctx_profile_report")
+        d.lld_ctx_profile(ctx.handle, 0)
+        prof = json.loads(buf.value.decode())
+        p1 = synth.make_sim3_batch(1, 300, 131 + fix, fix_scale=fix)   # the batch-of-one call the shim makes per candidate
+        one = []
+        api.sim3_opt(p1, impl="gpu", ctx=ctx)
+        for _ in range(50):
+            t0 = time.perf_counter(); api.sim3_opt(p1, impl="gpu", ctx=ctx); one.append((time.perf_counter() - t0) * 1e3)
+        one_dev = ctx.last_timing()[1]
+        p16 = synth.make_sim3_batch(16, 300, 131 + fix, fix_scale=fix)  # the first 16 problems of the batch above
+        o, tc = cpu(lambda: api.sim3_opt(p16, impl="oracle"))
+        same = (np.array_equal(g["inlier"][:int(p16["off"][-1])], o["inlier"]) and np.array_equal(g["n_in"][:16], o["n_in"])
+                and np.array_equal(g["n_iter_done"][:16], o["n_iter_done"]))
+        rel = float((np.abs(g["chi2_log"][:16] - o["chi2_log"]) / np.maximum(np.abs(o["chi2_log"]), 1e-300)).max())
+        res["fixed_scale" if fix else "free_scale"] = {
+            "problems": 4096, "correspondences": 300, "device_ms": ms, "call_ms_from_host_buffers": wall,
+            "problems_per_s_device": 4096 / ms * 1e3, "kernel_profile_ms": {k: v["ms"] for k, v in prof.items()},
+            "batch_of_one_call_ms_median": float(np.median(one)), "batch_of_one_device_ms": one_dev,
+            "cpu_oracle_ms_per_problem": tc / 16, "mean_inliers": float(g["n_in"].mean()),
+            "oracle_sample_16": {"inlier_n_in_iterations_identical": bool(same), "chi2_log_max_rel": rel}}
+    smi = subprocess.run(["nvidia-smi", "--query-gpu=name,power.limit", "--format=csv,noheader"], stdout=subprocess.PIPE, text=True).stdout
+    res["gpu"] = torch.cuda.get_device_name(0)
+    res["nvidia_smi_name_power_limit"] = smi.strip()
+    res["cpu"] = next((l.split(":", 1)[1].strip() for l in open("/proc/cpuinfo") if l.startswith("model name")), "")
+    out["optimize_sim3"] = res
 print(json.dumps(out))
