@@ -556,7 +556,7 @@ typedef struct lld_stereo_problem {
   const int32_t* left_off;     /* [n_frames+1] */
   const int32_t* right_off;    /* [n_frames+1]; at most 65535 right keypoints per frame */
   const float* left_xy;        /* [n_left][2]  mvKeys[i].pt (level-0 pixel coordinates) */
-  const uint8_t* left_octave;  /* [n_left]     mvKeys[i].octave */
+  const uint8_t* left_octave;  /* [n_left]     mvKeys[i].octave, < n_levels (both sides) */
   const uint8_t* left_desc;    /* [n_left][32] mDescriptors */
   const float* right_xy;       /* mvKeysRight, mDescriptorsRight */
   const uint8_t* right_octave;
@@ -606,11 +606,12 @@ typedef struct lld_line_assoc_problem {
   const double* ml_x1x2;         /* [n_ml][6] GetMainPoints3D */
   const float* ml_desc;          /* [n_ml][desc_dim] descs[i] / mLastFrame.mDescriptorsLines.row(i) */
   const int32_t* cand_off;       /* [n_ml+1] */
-  const int32_t* cand_idx;       /* sub_inds: frame-local indices of current left lines, in SubselectWithGrid order */
+  const int32_t* cand_idx;       /* sub_inds: frame-local indices of current left lines, in SubselectWithGrid order;
+                                    in [0, the frame's current lines) */
   const int32_t* cur_off;        /* [n_frames+1] current frame left lines */
   const float* cur_left;         /* [n_cur][4] mvLinesLeft start / end point */
   const int32_t* cur_octave;     /* [n_cur] mvLinesLeft[si].octave */
-  const int32_t* cur_line_match; /* [n_cur] line_matches[si]: frame-local right line or -1 */
+  const int32_t* cur_line_match; /* [n_cur] line_matches[si]: frame-local right line (< the frame's right lines) or -1 */
   const uint8_t* cur_taken;      /* [n_cur] mvpMapLines[si] != NULL on entry */
   const float* cur_desc;         /* [n_cur][desc_dim] mDescriptorsLines */
   const int32_t* right_off;      /* [n_frames+1] */

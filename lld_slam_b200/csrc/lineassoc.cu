@@ -102,6 +102,9 @@ __global__ void __launch_bounds__(32) k_line_associate(AssocView v) {
             ss += df * df;
           }
           cd = sqrt(ss);
+          // the reference accepts only cd < md, md starting at 1e10; dropping the rest here also keeps a NaN distance (from a
+          // NaN in a descriptor) out of the argmin, whose comparisons would otherwise leave the lanes with different winners
+          if (!(cd < 1e10)) { cd = 1e300; si = -1; }
         } else {
           si = -1;
         }
@@ -136,11 +139,22 @@ __global__ void __launch_bounds__(32) k_line_associate(AssocView v) {
 extern "C" int lld_line_associate(void* ctx, const lld_line_assoc_problem* p, lld_line_assoc_result* out) {
   LldCtx* c = lld_ctx_cast(ctx);
   if (!c || !p || !out) return LLD_ERR_ARG;
-  LLD_ARG(c, p->n_frames >= 1 && p->desc_dim >= 1);
-  LLD_CUDA(c, cudaSetDevice(c->device));
   c->launches = 0;
-  c->pool_reset();
+  LLD_ARG(c, p->n_frames >= 1 && p->desc_dim >= 1);
   const int F = p->n_frames, n_ml = p->ml_off[F], n_cur = p->cur_off[F], n_r = p->right_off[F], n_cand = p->cand_off[n_ml], D = p->desc_dim;
+  // candidates index the frame's current lines (taken bitset, cur_line_match); a stereo match indexes its right lines
+  for (int f = 0; f < F; f++) {
+    const int nc = p->cur_off[f + 1] - p->cur_off[f], nr = p->right_off[f + 1] - p->right_off[f];
+    for (int q = p->cand_off[p->ml_off[f]]; q < p->cand_off[p->ml_off[f + 1]]; q++) LLD_ARG(c, p->cand_idx[q] >= 0 && p->cand_idx[q] < nc);
+    if (!p->monocular)
+      for (int i = p->cur_off[f]; i < p->cur_off[f + 1]; i++) LLD_ARG(c, p->cur_line_match[i] < nr);
+  }
+  int max_cur = 1;
+  for (int f = 0; f < F; f++) max_cur = std::max(max_cur, p->cur_off[f + 1] - p->cur_off[f]);
+  const size_t smem = 4 * (size_t)((max_cur + 31) / 32);
+  LLD_ARG(c, smem <= 48 * 1024);
+  LLD_CUDA(c, cudaSetDevice(c->device));
+  c->pool_reset();
   cudaError_t e = cudaSuccess;
   auto up = [&](const void* src, size_t bytes) -> void* {
     if (e != cudaSuccess) return nullptr;
@@ -172,10 +186,6 @@ extern "C" int lld_line_associate(void* ctx, const lld_line_assoc_problem* p, ll
   if (e == cudaSuccess) v.cur_assoc = c->alloc<int>((size_t)std::max(n_cur, 1), &e);
   if (e == cudaSuccess) v.n_added = c->alloc<int>((size_t)F, &e);
   LLD_CUDA(c, e);
-  int max_cur = 1;
-  for (int f = 0; f < F; f++) max_cur = std::max(max_cur, p->cur_off[f + 1] - p->cur_off[f]);
-  const size_t smem = 4 * (size_t)((max_cur + 31) / 32);
-  LLD_ARG(c, smem <= 48 * 1024);
   LLD_CUDA(c, cudaEventRecord(c->ev[1], c->stream));
   LLD_LAUNCH(c, k_line_associate, F, 32, smem, v);
   LLD_CUDA(c, cudaGetLastError());

@@ -274,14 +274,17 @@ __global__ void __launch_bounds__(ST_NT) k_stereo(StereoView v) {
 extern "C" int lld_stereo_matches(void* ctx, const lld_stereo_problem* p, lld_stereo_result* out) {
   LldCtx* c = lld_ctx_cast(ctx);
   if (!c || !p || !out) return LLD_ERR_ARG;
-  LLD_ARG(c, p->n_frames >= 1 && p->n_levels >= 1 && p->n_levels <= 8);
-  LLD_CUDA(c, cudaSetDevice(c->device));
   c->launches = 0;
-  c->pool_reset();
+  LLD_ARG(c, p->n_frames >= 1 && p->n_levels >= 1 && p->n_levels <= 8);
   const int F = p->n_frames, n_l = p->left_off[F], n_r = p->right_off[F];
   int max_r = 0;
   for (int f = 0; f < F; f++) max_r = std::max(max_r, p->right_off[f + 1] - p->right_off[f]);
   LLD_ARG(c, max_r <= 65535);
+  // octaves index scale / rows / cols / stride and pyr_off on the device
+  for (int i = 0; i < n_l; i++) LLD_ARG(c, p->left_octave[i] < p->n_levels);
+  for (int i = 0; i < n_r; i++) LLD_ARG(c, p->right_octave[i] < p->n_levels);
+  LLD_CUDA(c, cudaSetDevice(c->device));
+  c->pool_reset();
   StereoView v{};
   v.n_frames = F; v.n_levels = p->n_levels; v.mb = p->mb; v.mbf = p->mbf;
   for (int l = 0; l < p->n_levels; l++) {

@@ -842,10 +842,11 @@ def make_stereo_frame(seed, n_kp=400, rows=240, cols=376, n_levels=4, sf=1.2):
     with random octaves and ORB-like descriptors (right = left with a few flipped bits; a share are outliers)."""
     import cv2
     rng = np.random.default_rng(seed)
-    base = rng.integers(0, 256, (rows // 4 + 2, (cols + 64) // 4 + 2), dtype=np.uint8)
-    wide = cv2.resize(base, (cols + 64, rows), interpolation=cv2.INTER_CUBIC)
-    left = np.ascontiguousarray(wide[:, 32:32 + cols])
     disp_of_row = 4 + (np.arange(rows) // 40) * 3            # 4, 7, 10, ... pixels
+    extra = max(64, 32 + int(disp_of_row.max()))              # source columns beyond the frame: 64 up to 376 rows
+    base = rng.integers(0, 256, (rows // 4 + 2, (cols + extra) // 4 + 2), dtype=np.uint8)
+    wide = cv2.resize(base, (cols + extra, rows), interpolation=cv2.INTER_CUBIC)
+    left = np.ascontiguousarray(wide[:, 32:32 + cols])
     right = np.empty_like(left)
     for y in range(rows):
         d = int(disp_of_row[y])
@@ -878,20 +879,25 @@ def make_stereo_frame(seed, n_kp=400, rows=240, cols=376, n_levels=4, sf=1.2):
                 mbf=np.float32(0.54 * 45.0))
 
 
-def batch_stereo(frames):
-    """frames from make_stereo_frame (same pyramid geometry) -> lld_stereo_problem field dict"""
+def batch_stereo(frames, pad=0):
+    """frames from make_stereo_frame (same pyramid geometry) -> lld_stereo_problem field dict.  pad > 0 lays every level out
+    as a region inside a wider buffer, row stride cols + pad, as ORBextractor's bordered pyramid (pad = 2 * EDGE_THRESHOLD =
+    38): pad // 2 columns of noise left of the image, the rest right of it."""
     f0 = frames[0]
     n_levels = len(f0["pyrL"])
     rows = np.array([a.shape[0] for a in f0["pyrL"]], np.int32)
     cols = np.array([a.shape[1] for a in f0["pyrL"]], np.int32)
-    stride = cols.copy()
+    stride = cols + np.int32(pad)
+    rng = np.random.default_rng(12345)
     offs, blobs, pos = [], [], 0
     for f in frames:
         for side in ("pyrL", "pyrR"):
             for l in range(n_levels):
-                a = np.ascontiguousarray(f[side][l])
+                a = np.asarray(f[side][l])
                 assert a.shape == (rows[l], cols[l])
-                offs.append(pos); blobs.append(a.reshape(-1)); pos += a.size
+                buf = rng.integers(0, 256, (rows[l], stride[l]), dtype=np.uint8)
+                buf[:, pad // 2:pad // 2 + cols[l]] = a
+                offs.append(pos + pad // 2); blobs.append(buf.reshape(-1)); pos += buf.size
     pyr = np.concatenate(blobs)
     return dict(
         n_frames=len(frames), left_off=_csr([len(f["kpL"]) for f in frames]), right_off=_csr([len(f["kpR"]) for f in frames]),
