@@ -23,6 +23,7 @@
  *   lld_bow_search         <- ORBmatcher::SearchByBoW x2             src/ORBmatcher.cc:159-288, 522-655
  *   lld_init_search        <- ORBmatcher::SearchForInitialization    src/ORBmatcher.cc:405
  *   lld_sim3_opt           <- Optimizer::OptimizeSim3                src/Optimizer.cc:1656-1858
+ *   lld_sim3_ransac        <- Sim3Solver::iterate / ComputeSim3 / CheckInliers (ORB-SLAM2 src/Sim3Solver.cc)
  *   lld_line_associate     <- Tracking::AddLinesFrom                 src/Tracking.cc:996-1124
  *   lld_medoid_orb / _float<- MapPoint / MapLine::ComputeDistinctiveDescriptors              src/MapPoint.cc:242-307, src/MapLine.cc:133-201
  *
@@ -85,6 +86,8 @@ extern "C" {
  *     of the batch has at most 57088 keypoints (k_init_resolve_smem), else in global memory (k_init_resolve_global);
  *   - lld_sim3_opt: no limit on the correspondences of a problem.  When every problem of the batch has at most 4266 (48 bytes each
  *     within 200 KB) the edge records are staged in shared memory (k_sim3_opt_smem), else read from global memory (k_sim3_opt_global);
+ *   - lld_sim3_ransac: no limit on the correspondences or minimal sets of a problem (correspondence data is read from global
+ *     memory; one CTA per problem evaluates 8 minimal sets at a time, k_sim3_ransac);
  *   - lld_line_match: descriptor widths that are a multiple of 8 up to 72 floats and at most 512 lines per side of a pair run on the
  *     tensor cores, everything else on the FP32 tile path (no failure).
  */
@@ -518,6 +521,79 @@ typedef struct lld_sim3_result {
 } lld_sim3_result;
 
 int lld_sim3_opt(void* ctx, const lld_sim3_problem* p, lld_sim3_result* out);
+
+/* ------------------------------------------------------------------------------------------------
+ * Loop-candidate Sim3 RANSAC: Sim3Solver (ORB-SLAM2 src/Sim3Solver.cc, inherited unchanged by LLD-SLAM), batched over loop
+ * candidates (LoopClosing::ComputeSim3 calls SetRansacParameters(0.99, 20, 300) and iterate(5, ...) per candidate per round).
+ * Correspondences are the ones the constructor keeps (vpMatched12[i1] and pKF1's map point i1 both present and good, and both
+ * points' GetIndexInKeyFrame >= 0), in vpMatched12 order; x1c / x2c are their camera-frame points mvX3Dc1 / mvX3Dc2 as the
+ * caller computed them, sigma2_1 / sigma2_2 the mvLevelSigma2 of their keypoints' octaves.  The library forms everything else
+ * as the reference does:
+ *   - thresholds mvnMaxError = 9.210 * sigma2 stored in a size_t, i.e. truncated to an integer (9 at octave 0);
+ *   - mvP1im1 / mvP2im2: the points' own camera coordinates projected with K1 / K2 (float invz, no depth test);
+ *   - ComputeSim3 (Horn 1987) in CV_32F: centroids (cv::reduce, then / 3), M = Pr2 Pr1^T, the symmetric 4x4 N, the eigenvector
+ *     of its largest eigenvalue as the quaternion (w first), ang = atan2(|v|, w) and v = 2 ang v / |v| in double,
+ *     cv::Rodrigues, s = Pr1 . (R Pr2) / sum (R Pr2)^2 (nom, den in double; s = 1 with fix_scale), t = O1 - s R O2,
+ *     T12 = [sR | t], T21 = [(1/s) R^T | -(1/s) R^T t];
+ *   - CheckInliers: x2c projected with T12 / K1 against mvP1im1 and x1c with T21 / K2 against mvP2im2, err = dist . dist
+ *     (float); inlier iff err1 < maxErr1 && err2 < maxErr2 (a NaN from a degenerate minimal set is an outlier).
+ * Products of small CV_32F matrices follow cv::gemm: a 3-long product without transposition sums float products in float,
+ * M = Pr2 Pr1^T sums in double; both round once to float.  The eigen solver is a cyclic Jacobi in double on the float N, not
+ * OpenCV's: its eigenvector may differ in the last bits, and the sign of the eigenvector cancels in the atan2 form.
+ *
+ * iterate(nIterations): with N = off[p+1] - off[p] < min_inliers nothing is drawn, no_more = 1.  Otherwise minimal sets are
+ * evaluated in order while its_done < max_its and fewer than n_iterations were evaluated in this call: a set whose inlier
+ * count reaches best_inliers (>=) becomes the best; if its count also exceeds min_inliers (strictly: 20 is not enough, 21 is)
+ * the call stops with found = 1 and that estimate.  Afterwards (no success) no_more = its_done >= max_its; a success on the
+ * last allowed set returns no_more = 0 and the next call evaluates nothing and sets it.  its_done and best_inliers are the
+ * solver's mnIterations and mnBestInliers: the caller passes them back in the next round (a candidate whose OptimizeSim3
+ * failed is iterated again and a new set must reach the carried best).
+ *
+ * Random draws: the reference draws each set with DUtils::Random::RandomInt(0, size - 1) on rand() by swap-with-back from a
+ * fresh copy of 0..N-1.  rand() is one stream for the whole process (relocalisation's PnPsolver draws from it on another
+ * thread), so the global sequence is not a contract.  The contract is: given the same minimal sets, this computes what
+ * iterate() computes.  The caller draws the sets: problem p receives exactly
+ *   B = N < min_inliers ? 0 : min(n_iterations, max(0, max_its - its_done))
+ * sets (hyp_off[p+1] - hyp_off[p] == B).  Drawing a whole round up front consumes draws from rand() after an early success,
+ * which the reference would not consume.
+ * ---------------------------------------------------------------------------------------------- */
+typedef struct lld_sim3_ransac_problem {
+  int32_t n_problems;
+  const float* cam;            /* [n][8] fx1 fy1 cx1 cy1 fx2 fy2 cx2 cy2: pKF1->mK, pKF2->mK */
+  const int32_t* fix_scale;    /* [n] mbFixScale: 0 or 1 */
+  const int32_t* off;          /* [n+1] CSR over correspondences, off[0] = 0 */
+  const float* x1c;            /* [m][3] mvX3Dc1 */
+  const float* x2c;            /* [m][3] mvX3Dc2 */
+  const float* sigma2_1;       /* [m] pKF1->mvLevelSigma2[octave] */
+  const float* sigma2_2;       /* [m] pKF2->mvLevelSigma2[octave] */
+  int32_t min_inliers;         /* mRansacMinInliers (20) */
+  const int32_t* max_its;      /* [n] mRansacMaxIts after SetRansacParameters (lld_sim3_ransac_max_its), >= 1 */
+  const int32_t* its_done;     /* [n] mnIterations before the call */
+  const int32_t* best_inliers; /* [n] mnBestInliers before the call */
+  int32_t n_iterations;        /* iterate(nIterations): 5 in LoopClosing::ComputeSim3 */
+  const int32_t* hyp_off;      /* [n+1] CSR over minimal sets, hyp_off[0] = 0, B sets per problem (above) */
+  const int32_t* hyp_idx;      /* [h][3] problem-local correspondence indices of each set, in draw order, distinct */
+} lld_sim3_ransac_problem;
+
+typedef struct lld_sim3_ransac_result {
+  uint8_t* found;          /* [n] iterate() returned an estimate */
+  uint8_t* no_more;        /* [n] bNoMore */
+  int32_t* n_inliers;      /* [n] nInliers (0 unless found) */
+  float* T12;              /* [n][13] GetEstimatedRotation (R, row-major, unscaled), GetEstimatedTranslation, GetEstimatedScale;
+                              written where found, zero elsewhere */
+  uint8_t* inlier;         /* [m] vbInliers in CSR order (all 0 unless found) */
+  int32_t* its_done;       /* [n] mnIterations after the call (may alias the input) */
+  int32_t* best_inliers;   /* [n] mnBestInliers after the call (may alias the input) */
+  int32_t* hyp_inliers;    /* [h] mnInliersi of each set, -1 where the set was not evaluated; may be NULL */
+} lld_sim3_ransac_result;
+
+/* SetRansacParameters(probability, minInliers, maxIterations) for N = n_corr correspondences, host arithmetic:
+ * epsilon = (float)minInliers / N; nIterations = minInliers == N ? 1 : ceil(log(1 - p) / log(1 - pow(epsilon, 3)));
+ * returns max(1, min(nIterations, maxIterations)).  Defined for n_corr >= min_inliers; below, iterate() draws nothing and the
+ * function returns 1. */
+int32_t lld_sim3_ransac_max_its(int32_t n_corr, double probability, int32_t min_inliers, int32_t max_iterations);
+
+int lld_sim3_ransac(void* ctx, const lld_sim3_ransac_problem* p, lld_sim3_ransac_result* out);
 
 /* ------------------------------------------------------------------------------------------------
  * Stereo line matching (float line descriptors)

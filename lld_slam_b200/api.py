@@ -194,6 +194,33 @@ def sim3_opt(p: Dict[str, Any], *, impl: str = "gpu", ctx=None):
     return out
 
 
+def sim3_ransac(p: Dict[str, Any], *, impl: str = "gpu", ctx=None):
+    """Sim3Solver::iterate batched over loop candidates (include/lldba.h): found, no_more, n_inliers, T12 ([n][13]: R, t, s),
+    inlier ([m], vbInliers in CSR order), its_done / best_inliers after the call and hyp_inliers (per minimal set, -1 where
+    not evaluated)"""
+    lib = _lib(impl)
+    prob, keep = capi.fill_struct(capi.Sim3RansacProblem, p)
+    n, m, h = int(p["n_problems"]), int(p["off"][-1]), int(p["hyp_off"][-1])
+    out = dict(found=np.zeros(max(n, 1), np.uint8), no_more=np.zeros(max(n, 1), np.uint8), n_inliers=np.zeros(max(n, 1), np.int32),
+               T12=np.zeros((max(n, 1), 13), np.float32), inlier=np.zeros(max(m, 1), np.uint8),
+               its_done=np.zeros(max(n, 1), np.int32), best_inliers=np.zeros(max(n, 1), np.int32),
+               hyp_inliers=np.full(max(h, 1), -2, np.int32))
+    res, keep2 = capi.fill_struct(capi.Sim3RansacResult, out)
+    rc = lib.sim3_ransac(_handle(impl, ctx), C.byref(prob), C.byref(res))
+    _check(impl, ctx, rc, "lld_sim3_ransac")
+    for k in ("found", "no_more", "n_inliers", "T12", "its_done", "best_inliers"):
+        out[k] = out[k][:n]
+    out["inlier"] = out["inlier"][:m]
+    out["hyp_inliers"] = out["hyp_inliers"][:h]
+    return out
+
+
+def sim3_ransac_max_its(n_corr: int, probability: float = 0.99, min_inliers: int = 20, max_iterations: int = 300) -> int:
+    """Sim3Solver::SetRansacParameters: the RANSAC iteration limit mRansacMaxIts for n_corr correspondences (host arithmetic of
+    the library)"""
+    return int(capi.load_library().sim3_ransac_max_its(int(n_corr), float(probability), int(min_inliers), int(max_iterations)))
+
+
 def line_match(p: Dict[str, Any], *, impl: str = "gpu", ctx=None):
     lib = _lib(impl)
     prob, keep = capi.fill_struct(capi.LineMatchProblem, p)

@@ -4,7 +4,7 @@ This is the Python harness over the C-ABI used by tests/ and bench.py.  The prod
 lld_slam_b200/csrc/liblldba.so (CUDA, sm_100a); `load_library()` fails loudly when it is missing —
 there is no CPU fallback.  `load_oracle()` loads the CPU oracle (oracle/liblld_oracle.so) which
 exposes the same entry points with the `lldo_` prefix (lldo_init_search from tests/hostcheck/libinit_search_oracle.so, lldo_sim3_opt from
-tests/hostcheck/libsim3_oracle.so); only tests, smoke() and the bench's
+tests/hostcheck/libsim3_oracle.so, lldo_sim3_ransac from tests/hostcheck/libsim3_ransac_oracle.so); only tests, smoke() and the bench's
 cpu_baseline / reference arm may call it.
 """
 from __future__ import annotations
@@ -21,6 +21,7 @@ ORACLE_PATH = os.path.join(_ROOT, "oracle", "liblld_oracle.so")
 # the oracle's SearchForInitialization (lldo_init_search) is a separate test-infrastructure library
 INIT_SEARCH_ORACLE_PATH = os.path.join(_ROOT, "tests", "hostcheck", "libinit_search_oracle.so")
 SIM3_ORACLE_PATH = os.path.join(_ROOT, "tests", "hostcheck", "libsim3_oracle.so")
+SIM3_RANSAC_ORACLE_PATH = os.path.join(_ROOT, "tests", "hostcheck", "libsim3_ransac_oracle.so")
 
 c_i32p = C.POINTER(C.c_int32)
 c_u8p = C.POINTER(C.c_uint8)
@@ -173,6 +174,21 @@ class Sim3Result(C.Structure):
     ]
 
 
+class Sim3RansacProblem(C.Structure):
+    _fields_ = [
+        ("n_problems", C.c_int32), ("cam", c_f32p), ("fix_scale", c_i32p), ("off", c_i32p), ("x1c", c_f32p), ("x2c", c_f32p),
+        ("sigma2_1", c_f32p), ("sigma2_2", c_f32p), ("min_inliers", C.c_int32), ("max_its", c_i32p), ("its_done", c_i32p),
+        ("best_inliers", c_i32p), ("n_iterations", C.c_int32), ("hyp_off", c_i32p), ("hyp_idx", c_i32p),
+    ]
+
+
+class Sim3RansacResult(C.Structure):
+    _fields_ = [
+        ("found", c_u8p), ("no_more", c_u8p), ("n_inliers", c_i32p), ("T12", c_f32p), ("inlier", c_u8p), ("its_done", c_i32p),
+        ("best_inliers", c_i32p), ("hyp_inliers", c_i32p),
+    ]
+
+
 class TriSearchResult(C.Structure):
     _fields_ = [("match12", c_i32p), ("n_matches", c_i32p)]
 
@@ -290,6 +306,18 @@ class _Lib:
             self.sim3_opt.restype = C.c_int
         else:
             self._sig("sim3_opt", sim3_sig)
+        ransac_sig = [vp, C.POINTER(Sim3RansacProblem), C.POINTER(Sim3RansacResult)]
+        if self.is_oracle:
+            if not os.path.exists(SIM3_RANSAC_ORACLE_PATH):
+                raise RuntimeError(f"{SIM3_RANSAC_ORACLE_PATH} not found — build it first (python -c 'import __graft_entry__ as g; g.build()').")
+            self.sim3_ransac_dll = C.CDLL(SIM3_RANSAC_ORACLE_PATH)
+            self.sim3_ransac = self.sim3_ransac_dll.lldo_sim3_ransac
+            self.sim3_ransac.argtypes = ransac_sig
+            self.sim3_ransac.restype = C.c_int
+        else:
+            self._sig("sim3_ransac", ransac_sig)
+            self._sig("sim3_ransac_max_its", [C.c_int32, C.c_double, C.c_int32, C.c_int32])
+            self.sim3_ransac_max_its.restype = C.c_int32
         self._sig("line_match", [vp, C.POINTER(LineMatchProblem), C.POINTER(LineMatchResult)])
         self._sig("descriptor_distance", [c_u8p, c_u8p])
         if not self.is_oracle:

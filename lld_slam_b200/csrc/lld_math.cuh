@@ -463,6 +463,203 @@ LLD_HD void sim3_jac_col(const double* ep, const double* em, double* J, int d) {
   J[7 + d] = scalar * (ep[1] - em[1]);
 }
 
+// ---- Sim3Solver (ORB-SLAM2 src/Sim3Solver.cc): Horn's closed form and the inlier test in CV_32F -----------------------
+// Small CV_32F products follow cv::gemm: a 3-long product without transposition sums float products in float (k = 0..2)
+// and then rounds s0 * alpha + c * beta, formed in double, once to float.
+LLD_HD float cv_gemm3(float a0, float a1, float a2, float b0, float b1, float b2) {
+  const float p0 = a0 * b0, p1 = a1 * b1, p2 = a2 * b2;
+  return (p0 + p1) + p2;
+}
+// Largest eigenpair of a symmetric 4x4 (cv::eigen's row 0): cyclic Jacobi in double on the float matrix, eigenvector rounded
+// to float.  Ties go to the lowest index; a zero matrix gives e0.
+LLD_HD void sym4_top_eigvec(const float* Nf, float* q) {
+  double A[4][4], V[4][4];
+#pragma unroll
+  for (int i = 0; i < 4; i++)
+#pragma unroll
+    for (int j = 0; j < 4; j++) {
+      A[i][j] = (double)Nf[4 * i + j];
+      V[i][j] = i == j ? 1.0 : 0.0;
+    }
+  for (int sweep = 0; sweep < 32; sweep++) {
+    double off = 0.0, dia = 0.0;
+#pragma unroll
+    for (int i = 0; i < 4; i++) {
+      dia += fabs(A[i][i]);
+#pragma unroll
+      for (int j = i + 1; j < 4; j++) off += fabs(A[i][j]);
+    }
+    if (!(off > 1e-15 * dia)) break;
+#pragma unroll
+    for (int p = 0; p < 3; p++)
+#pragma unroll
+      for (int r = p + 1; r < 4; r++) {
+        const double apr = A[p][r];
+        if (apr == 0.0) continue;
+        const double th = (A[r][r] - A[p][p]) / (2.0 * apr);
+        const double t = (th >= 0.0 ? 1.0 : -1.0) / (fabs(th) + sqrt(th * th + 1.0));
+        const double c = 1.0 / sqrt(t * t + 1.0), s = t * c;
+#pragma unroll
+        for (int k = 0; k < 4; k++) {
+          const double akp = A[k][p], akr = A[k][r];
+          A[k][p] = c * akp - s * akr;
+          A[k][r] = s * akp + c * akr;
+        }
+#pragma unroll
+        for (int k = 0; k < 4; k++) {
+          const double apk = A[p][k], ark = A[r][k];
+          A[p][k] = c * apk - s * ark;
+          A[r][k] = s * apk + c * ark;
+        }
+#pragma unroll
+        for (int k = 0; k < 4; k++) {
+          const double vkp = V[k][p], vkr = V[k][r];
+          V[k][p] = c * vkp - s * vkr;
+          V[k][r] = s * vkp + c * vkr;
+        }
+      }
+  }
+  int im = 0;
+  double best = A[0][0];
+#pragma unroll
+  for (int i = 1; i < 4; i++)
+    if (A[i][i] > best) { best = A[i][i]; im = i; }
+#pragma unroll
+  for (int i = 0; i < 4; i++) {
+    double v = V[i][0];
+#pragma unroll
+    for (int j = 1; j < 4; j++) v = im == j ? V[i][j] : v;
+    q[i] = (float)v;
+  }
+}
+// cv::Rodrigues of a float rotation vector into a float 3x3 (computed in double)
+LLD_HD void cv_rodrigues(const float* rv, float* R) {
+  double r[3] = {(double)rv[0], (double)rv[1], (double)rv[2]};
+  const double theta = sqrt(r[0] * r[0] + r[1] * r[1] + r[2] * r[2]);
+  if (theta < 2.220446049250313e-16) {
+#pragma unroll
+    for (int i = 0; i < 9; i++) R[i] = (i == 0 || i == 4 || i == 8) ? 1.f : 0.f;
+    return;
+  }
+  const double c = cos(theta), s = sin(theta), c1 = 1. - c;
+  const double it = 1. / theta;
+  r[0] *= it; r[1] *= it; r[2] *= it;
+  const double rx[9] = {0, -r[2], r[1], r[2], 0, -r[0], -r[1], r[0], 0};
+#pragma unroll
+  for (int i = 0; i < 3; i++)
+#pragma unroll
+    for (int j = 0; j < 3; j++) R[3 * i + j] = (float)((c * (i == j ? 1.0 : 0.0) + c1 * (r[i] * r[j])) + s * rx[3 * i + j]);
+}
+// Sim3Solver::ComputeSim3 on one minimal set.  P1, P2: the three points, point-major ([k][3] = column k of P3Dc1i / P3Dc2i).
+// Writes the unscaled rotation R (row-major), t and s as GetEstimatedRotation / Translation / Scale return them.
+LLD_HD void sim3r_horn(const float* P1, const float* P2, bool fix_scale, float* R, float* t, float* s_out) {
+  float O1[3], O2[3], Pr1[3][3], Pr2[3][3];   // Pr[coordinate][point]
+#pragma unroll
+  for (int r = 0; r < 3; r++) {
+    O1[r] = ((P1[r] + P1[3 + r]) + P1[6 + r]) * (1.0f / 3.0f);   // cv::reduce(SUM), C / P.cols
+    O2[r] = ((P2[r] + P2[3 + r]) + P2[6 + r]) * (1.0f / 3.0f);
+#pragma unroll
+    for (int k = 0; k < 3; k++) {
+      Pr1[r][k] = P1[3 * k + r] - O1[r];
+      Pr2[r][k] = P2[3 * k + r] - O2[r];
+    }
+  }
+  float M[3][3];   // Pr2 * Pr1^T
+#pragma unroll
+  for (int i = 0; i < 3; i++)
+#pragma unroll
+    for (int j = 0; j < 3; j++)
+      M[i][j] = (float)(((double)Pr2[i][0] * (double)Pr1[j][0] + (double)Pr2[i][1] * (double)Pr1[j][1]) +
+                        (double)Pr2[i][2] * (double)Pr1[j][2]);
+  const float N11 = (M[0][0] + M[1][1]) + M[2][2], N12 = M[1][2] - M[2][1], N13 = M[2][0] - M[0][2], N14 = M[0][1] - M[1][0];
+  const float N22 = (M[0][0] - M[1][1]) - M[2][2], N23 = M[0][1] + M[1][0], N24 = M[2][0] + M[0][2];
+  const float N33 = (-M[0][0] + M[1][1]) - M[2][2], N34 = M[1][2] + M[2][1], N44 = (-M[0][0] - M[1][1]) + M[2][2];
+  const float N[16] = {N11, N12, N13, N14, N12, N22, N23, N24, N13, N23, N33, N34, N14, N24, N34, N44};
+  float q[4];
+  sym4_top_eigvec(N, q);
+  // cv::norm of the float 1x3 (double, in OpenCV's lane order), ang = atan2(|v|, w), v = 2 ang v / |v|
+  const double nrm = sqrt(((double)q[1] * (double)q[1] + (double)q[3] * (double)q[3]) + (double)q[2] * (double)q[2]);
+  const double ang = atan2(nrm, (double)q[0]);
+  const double al = (2 * ang) * (1. / nrm);
+  const float rv[3] = {(float)(al * (double)q[1]), (float)(al * (double)q[2]), (float)(al * (double)q[3])};
+  cv_rodrigues(rv, R);
+  float s = 1.0f;
+  if (!fix_scale) {
+    float P3[3][3];   // R * Pr2
+#pragma unroll
+    for (int r = 0; r < 3; r++)
+#pragma unroll
+      for (int k = 0; k < 3; k++) P3[r][k] = cv_gemm3(R[3 * r], R[3 * r + 1], R[3 * r + 2], Pr2[0][k], Pr2[1][k], Pr2[2][k]);
+    double nom = 0, den = 0;
+#pragma unroll
+    for (int r = 0; r < 3; r++)
+#pragma unroll
+      for (int k = 0; k < 3; k++) {
+        nom += (double)Pr1[r][k] * (double)P3[r][k];
+        den += (double)(P3[r][k] * P3[r][k]);
+      }
+    s = (float)(nom / den);
+  }
+#pragma unroll
+  for (int r = 0; r < 3; r++)   // t = O1 - s R O2: gemm(R, O2, -s, O1, 1)
+    t[r] = (float)((double)cv_gemm3(R[3 * r], R[3 * r + 1], R[3 * r + 2], O2[0], O2[1], O2[2]) * -(double)s + (double)O1[r]);
+  *s_out = s;
+}
+// T12 = [sR | t], T21 = [(1/s) R^T | -(1/s) R^T t] of one estimate (R, t, s)
+struct Sim3Pair {
+  float A12[9], b12[3], A21[9], b21[3];
+};
+LLD_HD void sim3r_pair(const float* R, const float* t, float s, Sim3Pair* T) {
+  const double is = 1.0 / (double)s;
+#pragma unroll
+  for (int i = 0; i < 3; i++)
+#pragma unroll
+    for (int j = 0; j < 3; j++) {
+      T->A12[3 * i + j] = s * R[3 * i + j];
+      T->A21[3 * i + j] = (float)(is * (double)R[3 * j + i]);
+    }
+#pragma unroll
+  for (int r = 0; r < 3; r++) {
+    T->b12[r] = t[r];
+    T->b21[r] = -cv_gemm3(T->A21[3 * r], T->A21[3 * r + 1], T->A21[3 * r + 2], t[0], t[1], t[2]);
+  }
+}
+// Sim3Solver::Project of one point (Rcw * X + tcw, float invz, no depth test); K = fx fy cx cy
+LLD_HD void sim3r_project(const float* A, const float* b, const float* X, const float* K, float* uv) {
+  float Y[3];
+#pragma unroll
+  for (int r = 0; r < 3; r++) Y[r] = (float)((double)cv_gemm3(A[3 * r], A[3 * r + 1], A[3 * r + 2], X[0], X[1], X[2]) + (double)b[r]);
+  const float invz = 1 / Y[2];
+  const float x = Y[0] * invz, y = Y[1] * invz;
+  uv[0] = K[0] * x + K[2];
+  uv[1] = K[1] * y + K[3];
+}
+// Sim3Solver::FromCameraToImage of one point
+LLD_HD void sim3r_own(const float* X, const float* K, float* uv) {
+  const float invz = 1 / X[2];
+  const float x = X[0] * invz, y = X[1] * invz;
+  uv[0] = K[0] * x + K[2];
+  uv[1] = K[1] * y + K[3];
+}
+// dist.dot(dist) of a float 2-vector (double accumulation, stored in a float)
+LLD_HD float sim3r_err(const float* a, const float* b) {
+  const float d0 = a[0] - b[0], d1 = a[1] - b[1];
+  return (float)((double)d0 * (double)d0 + (double)d1 * (double)d1);
+}
+// mvnMaxError = 9.210 * sigma2 stored in a size_t
+LLD_HD float sim3r_max_err(float sigma2) { return (float)(unsigned long long)(9.210 * (double)sigma2); }
+// CheckInliers for one correspondence; K = K1 (4), K2 (4).  err1 / err2 out for the tests.
+LLD_HD bool sim3r_inlier(const Sim3Pair& T, const float* x1, const float* x2, float sig1, float sig2, const float* K, float* e) {
+  float own1[2], own2[2], p21[2], p12[2];
+  sim3r_own(x1, K, own1);
+  sim3r_own(x2, K + 4, own2);
+  sim3r_project(T.A12, T.b12, x2, K, p21);
+  sim3r_project(T.A21, T.b21, x1, K + 4, p12);
+  e[0] = sim3r_err(own1, p21);
+  e[1] = sim3r_err(p12, own2);
+  return e[0] < sim3r_max_err(sig1) && e[1] < sim3r_max_err(sig2);
+}
+
 // ---- tiny dense helpers --------------------------------------------------------------------------
 // symmetric 3x3 / 4x4 inverse via cofactors / blockwise (general inverse, like MatrixXd::inverse()).
 LLD_HD void inv3_sym(const double* A /*full 9*/, double* I) {

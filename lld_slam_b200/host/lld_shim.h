@@ -15,6 +15,7 @@
 //                                              :1472-1599 (frame to keyframe, relocalisation)
 //   lld::ORBmatcher::SearchForInitialization <- src/ORBmatcher.cc:405
 //   lld::Optimizer::OptimizeSim3            <- src/Optimizer.cc:1656-1858
+//   lld::Sim3Solver                         <- ORB-SLAM2 src/Sim3Solver.cc (constructor, SetRansacParameters, iterate, getters)
 //   lld::TwoFrameLineMatcher::MatchLines    <- src/TwoFrameLineMatcher.cc:26-77
 // Every entry point takes the library context as an extra first argument (the reference keeps its g2o optimizer on the
 // stack instead); Flatten* expose the flattened problem so that tests can compare it array by array with a reference
@@ -23,7 +24,9 @@
 #include <algorithm>
 #include <cmath>
 #include <cstdint>
+#include <cstdlib>
 #include <cstring>
+#include <functional>
 #include <map>
 #include <set>
 #include <utility>
@@ -598,6 +601,192 @@ class Optimizer {
     g2oS12.s = oS[7];
     return n_in;
   }
+};
+
+// g2o::Sim3(R, t, s) as LoopClosing builds it from the Sim3Solver getters (Converter::toMatrix3d / toVector3d): the rotation
+// through Eigen's Quaterniond(Matrix3d), in its branch order
+inline Sim3 ToSim3(const float R[9], const float t[3], float s) {
+  double m[9];
+  for (int i = 0; i < 9; i++) m[i] = R[i];
+  Sim3 S;
+  double q[4];
+  double tr = m[0] + m[4] + m[8];
+  if (tr > 0.0) {
+    tr = std::sqrt(tr + 1.0);
+    q[3] = 0.5 * tr;
+    tr = 0.5 / tr;
+    q[0] = (m[7] - m[5]) * tr; q[1] = (m[2] - m[6]) * tr; q[2] = (m[3] - m[1]) * tr;
+  } else {
+    int i = 0;
+    if (m[4] > m[0]) i = 1;
+    if (m[8] > m[4 * i]) i = 2;
+    const int j = (i + 1) % 3, k = (j + 1) % 3;
+    tr = std::sqrt(m[4 * i] - m[4 * j] - m[4 * k] + 1.0);
+    q[i] = 0.5 * tr;
+    tr = 0.5 / tr;
+    q[3] = (m[3 * k + j] - m[3 * j + k]) * tr;
+    q[j] = (m[3 * j + i] + m[3 * i + j]) * tr;
+    q[k] = (m[3 * k + i] + m[3 * i + k]) * tr;
+  }
+  for (int c = 0; c < 4; c++) S.q[c] = q[c];
+  for (int c = 0; c < 3; c++) S.t[c] = t[c];
+  S.s = s;
+  return S;
+}
+
+// Sim3Solver (ORB-SLAM2 include/Sim3Solver.h, src/Sim3Solver.cc) over lld_sim3_ransac.  The constructor keeps the
+// correspondences the reference keeps and computes mvX3Dc1 / mvX3Dc2 in float; SetRansacParameters is
+// lld_sim3_ransac_max_its; iterate() draws its minimal sets on the host through RandomInt (the DUtils formula on rand() by
+// default) and evaluates them on the device.  IterateBatch runs one ComputeSim3 round for many candidates in one call: each
+// solver's whole round is drawn up front, so draws after an early success are consumed from the stream where the reference
+// would not consume them (include/lldba.h).  The getters are valid after iterate() returned true.
+class Sim3Solver {
+ public:
+  static int DefaultRandomInt(int min, int max) {   // DUtils::Random::RandomInt
+    const int d = max - min + 1;
+    return int(((double)rand() / ((double)RAND_MAX + 1.0)) * d) + min;
+  }
+  std::function<int(int, int)> RandomInt = DefaultRandomInt;
+
+  Sim3Solver(KeyFrame* pKF1, KeyFrame* pKF2, const std::vector<MapPoint*>& vpMatched12, const bool bFixScale = true)
+      : mbFixScale(bFixScale), mN1((int)vpMatched12.size()) {
+    const std::vector<MapPoint*>& vpKeyFrameMP1 = pKF1->mvpMapPoints;   // GetMapPointMatches()
+    auto cam_frame = [](const KeyFrame* k, const float* X, std::vector<float>& out) {   // Rcw * X + tcw, cv::gemm in float
+      const float* T = k->Tcw;
+      for (int r = 0; r < 3; r++) {
+        float s0 = T[3 * r] * X[0];
+        s0 = s0 + T[3 * r + 1] * X[1];
+        s0 = s0 + T[3 * r + 2] * X[2];
+        out.push_back((float)((double)s0 + (double)T[9 + r]));
+      }
+    };
+    for (int i1 = 0; i1 < mN1; i1++) {
+      if (!vpMatched12[(size_t)i1]) continue;
+      MapPoint* pMP1 = vpKeyFrameMP1[(size_t)i1];
+      MapPoint* pMP2 = vpMatched12[(size_t)i1];
+      if (!pMP1) continue;
+      if (pMP1->isBad() || pMP2->isBad()) continue;
+      const int indexKF1 = pMP1->GetIndexInKeyFrame(pKF1);
+      const int indexKF2 = pMP2->GetIndexInKeyFrame(pKF2);
+      if (indexKF1 < 0 || indexKF2 < 0) continue;
+      const KeyPoint& kp1 = pKF1->mvKeysUn[(size_t)indexKF1];
+      const KeyPoint& kp2 = pKF2->mvKeysUn[(size_t)indexKF2];
+      mSigma2_1.push_back(pKF1->mvLevelSigma2[(size_t)kp1.octave]);
+      mSigma2_2.push_back(pKF2->mvLevelSigma2[(size_t)kp2.octave]);
+      cam_frame(pKF1, pMP1->pos, mvX3Dc1);
+      cam_frame(pKF2, pMP2->pos, mvX3Dc2);
+      mvnIndices1.push_back(i1);
+    }
+    const float K[8] = {pKF1->fx, pKF1->fy, pKF1->cx, pKF1->cy, pKF2->fx, pKF2->fy, pKF2->cx, pKF2->cy};
+    std::memcpy(mK, K, sizeof(mK));
+    N = (int)mvnIndices1.size();
+    SetRansacParameters();
+  }
+
+  void SetRansacParameters(double probability = 0.99, int minInliers = 6, int maxIterations = 300) {
+    mRansacMinInliers = minInliers;
+    mRansacMaxIts = lld_sim3_ransac_max_its(N, probability, minInliers, maxIterations);
+    mnIterations = 0;
+  }
+
+  // cv::Mat iterate(int nIterations, bool& bNoMore, vector<bool>& vbInliers, int& nInliers): true where the reference returns
+  // an estimate.  A failed library call returns false with LastError() != 0.
+  bool iterate(void* ctx, int nIterations, bool& bNoMore, std::vector<bool>& vbInliers, int& nInliers) {
+    std::vector<Sim3Solver*> one{this};
+    mLastError = IterateBatch(ctx, one, nIterations);
+    bNoMore = mbNoMore;
+    vbInliers = mvbInliers;
+    nInliers = mnInliers;
+    return mbFound;
+  }
+
+  // One ComputeSim3 round (iterate(nIterations) for every solver) in one lld_sim3_ransac call; each solver's outputs are read
+  // with Found() / NoMore() / Inliers() / NumInliers().  Returns the library's status.
+  static int IterateBatch(void* ctx, const std::vector<Sim3Solver*>& solvers, int nIterations) {
+    const int n = (int)solvers.size();
+    std::vector<float> cam, x1, x2, s1, s2;
+    std::vector<int32_t> fix, off{0}, max_its, its, best, hoff{0}, hidx;
+    for (Sim3Solver* S : solvers) {
+      cam.insert(cam.end(), S->mK, S->mK + 8);
+      fix.push_back(S->mbFixScale);
+      x1.insert(x1.end(), S->mvX3Dc1.begin(), S->mvX3Dc1.end());
+      x2.insert(x2.end(), S->mvX3Dc2.begin(), S->mvX3Dc2.end());
+      s1.insert(s1.end(), S->mSigma2_1.begin(), S->mSigma2_1.end());
+      s2.insert(s2.end(), S->mSigma2_2.begin(), S->mSigma2_2.end());
+      off.push_back(off.back() + S->N);
+      max_its.push_back(S->mRansacMaxIts);
+      its.push_back(S->mnIterations);
+      best.push_back(S->mnBestInliers);
+      if (S->mRansacMinInliers != solvers[0]->mRansacMinInliers) return LLD_ERR_ARG;
+      const int B = S->N < S->mRansacMinInliers ? 0 : std::min(nIterations, std::max(0, S->mRansacMaxIts - S->mnIterations));
+      for (int h = 0; h < B; h++) {   // the minimal set of iterate(): swap-with-back from a fresh copy of mvAllIndices
+        std::vector<int> vAvailableIndices(S->N);
+        for (int i = 0; i < S->N; i++) vAvailableIndices[(size_t)i] = i;
+        for (int i = 0; i < 3; ++i) {
+          const int randi = S->RandomInt(0, (int)vAvailableIndices.size() - 1);
+          hidx.push_back(vAvailableIndices[(size_t)randi]);
+          vAvailableIndices[(size_t)randi] = vAvailableIndices.back();
+          vAvailableIndices.pop_back();
+        }
+      }
+      hoff.push_back(hoff.back() + B);
+    }
+    if (n == 0) return 0;
+    lld_sim3_ransac_problem p;
+    std::memset(&p, 0, sizeof(p));
+    p.n_problems = n; p.cam = cam.data(); p.fix_scale = fix.data(); p.off = off.data(); p.x1c = x1.data(); p.x2c = x2.data();
+    p.sigma2_1 = s1.data(); p.sigma2_2 = s2.data(); p.min_inliers = solvers[0]->mRansacMinInliers; p.max_its = max_its.data();
+    p.its_done = its.data(); p.best_inliers = best.data(); p.n_iterations = nIterations; p.hyp_off = hoff.data(); p.hyp_idx = hidx.data();
+    std::vector<uint8_t> found((size_t)n), no_more((size_t)n), inl((size_t)off.back() + 1);
+    std::vector<int32_t> n_in((size_t)n);
+    std::vector<float> T12(13 * (size_t)n);
+    lld_sim3_ransac_result r;
+    std::memset(&r, 0, sizeof(r));
+    r.found = found.data(); r.no_more = no_more.data(); r.n_inliers = n_in.data(); r.T12 = T12.data(); r.inlier = inl.data();
+    r.its_done = its.data(); r.best_inliers = best.data();
+    const int rc = lld_sim3_ransac(ctx, &p, &r);
+    if (rc) return rc;
+    for (int k = 0; k < n; k++) {
+      Sim3Solver* S = solvers[(size_t)k];
+      S->mnIterations = its[(size_t)k];
+      S->mnBestInliers = best[(size_t)k];
+      S->mbFound = found[(size_t)k] != 0;
+      S->mbNoMore = no_more[(size_t)k] != 0;
+      S->mnInliers = n_in[(size_t)k];
+      S->mvbInliers.assign((size_t)S->mN1, false);
+      for (int i = 0; i < S->N; i++)
+        if (inl[(size_t)off[(size_t)k] + i]) S->mvbInliers[(size_t)S->mvnIndices1[(size_t)i]] = true;
+      if (S->mbFound) {
+        std::memcpy(S->mBestRotation, &T12[13 * (size_t)k], 9 * sizeof(float));
+        std::memcpy(S->mBestTranslation, &T12[13 * (size_t)k + 9], 3 * sizeof(float));
+        S->mBestScale = T12[13 * (size_t)k + 12];
+      }
+    }
+    return 0;
+  }
+
+  bool Found() const { return mbFound; }
+  bool NoMore() const { return mbNoMore; }
+  const std::vector<bool>& Inliers() const { return mvbInliers; }
+  int NumInliers() const { return mnInliers; }
+  int LastError() const { return mLastError; }
+  int NumCorrespondences() const { return N; }
+  int MaxIterations() const { return mRansacMaxIts; }
+  void GetEstimatedRotation(float R[9]) const { std::memcpy(R, mBestRotation, sizeof(mBestRotation)); }
+  void GetEstimatedTranslation(float t[3]) const { std::memcpy(t, mBestTranslation, sizeof(mBestTranslation)); }
+  float GetEstimatedScale() const { return mBestScale; }
+
+ private:
+  bool mbFixScale;
+  int mN1, N = 0;
+  float mK[8];
+  std::vector<float> mvX3Dc1, mvX3Dc2, mSigma2_1, mSigma2_2;
+  std::vector<int> mvnIndices1;
+  int mRansacMinInliers = 6, mRansacMaxIts = 300, mnIterations = 0, mnBestInliers = 0;
+  bool mbFound = false, mbNoMore = false;
+  std::vector<bool> mvbInliers;
+  int mnInliers = 0, mLastError = 0;
+  float mBestRotation[9] = {0}, mBestTranslation[3] = {0}, mBestScale = 1.f;
 };
 
 class ORBmatcher {

@@ -6,6 +6,8 @@ src/Converter.cc:37-47,110-116 does.  Camera and thresholds: Examples/Stereo/KIT
 """
 from __future__ import annotations
 
+import math
+
 import numpy as np
 
 # Examples/Stereo/KITTI04-12_LBD.yaml:8-25
@@ -785,6 +787,98 @@ def make_sim3_batch(n_problems, n_corr, seed, fix_scale=1, outlier_frac=0.1, th2
         a = np.concatenate(v) if v else np.zeros((0, w))
         out[k] = np.ascontiguousarray(f32(a).reshape(-1, w) if w > 1 else f32(a).reshape(-1))
     return out
+
+
+def level_sigma2():
+    """mvLevelSigma2 of the ORB pyramid (src/ORBextractor.cc): scale factors accumulated in float, squared in float"""
+    sf = [np.float32(1.0)]
+    for _ in range(1, N_LEVELS):
+        sf.append(np.float32(sf[-1] * np.float32(SCALE)))
+    sf = f32(sf)
+    return f32(sf * sf)
+
+
+RAND_MAX = 2147483647   # glibc
+
+
+def random_int(r, lo, hi):
+    """DUtils::Random::RandomInt(min, max) on one rand() value r"""
+    return int((float(r) / (float(RAND_MAX) + 1.0)) * (hi - lo + 1)) + lo
+
+
+def rand_stream(seed):
+    """a stream of rand()-like values in [0, RAND_MAX]"""
+    rng = np.random.default_rng(seed)
+    while True:
+        for r in rng.integers(0, RAND_MAX + 1, 4096):
+            yield int(r)
+
+
+def draw_minimal_set(n, stream):
+    """Sim3Solver::iterate's draw: three indices by swap-with-back from a fresh copy of 0..n-1"""
+    avail = list(range(n))
+    out = []
+    for _ in range(3):
+        k = random_int(next(stream), 0, len(avail) - 1)
+        out.append(avail[k])
+        avail[k] = avail[-1]
+        avail.pop()
+    return out
+
+
+def sim3_ransac_budget(p):
+    """minimal sets lld_sim3_ransac expects per problem: N < min_inliers ? 0 : min(n_iterations, max(0, max_its - its_done))"""
+    N = np.diff(p["off"])
+    return np.where(N < p["min_inliers"], 0, np.minimum(p["n_iterations"], np.maximum(0, p["max_its"] - p["its_done"]))).astype(np.int32)
+
+
+def draw_sim3_ransac_sets(p, stream):
+    """fills hyp_off / hyp_idx of p with each problem's budget of minimal sets, drawn in problem order from stream"""
+    B = sim3_ransac_budget(p)
+    N = np.diff(p["off"])
+    idx = [draw_minimal_set(int(N[i]), stream) for i in range(len(B)) for _ in range(int(B[i]))]
+    p["hyp_off"] = np.concatenate([[0], np.cumsum(B)]).astype(np.int32)
+    p["hyp_idx"] = np.ascontiguousarray(np.asarray(idx, np.int32).reshape(-1, 3))
+    return p
+
+
+def sim3_ransac_max_its_py(n, probability=0.99, min_inliers=20, max_iterations=300):
+    """SetRansacParameters in Python (glibc log / pow / ceil through math)"""
+    if n < min_inliers:
+        return 1
+    if min_inliers == n:
+        it = 1
+    else:
+        eps = float(np.float32(np.float32(min_inliers) / np.float32(n)))
+        it = math.ceil(math.log(1 - probability) / math.log(1 - math.pow(eps, 3)))
+    return max(1, min(it, max_iterations))
+
+
+def make_sim3_ransac_batch(n_problems, n_corr, seed, fix_scale=1, outlier_range=(0.05, 0.9), n_iterations=300, min_inliers=20):
+    """Sim3Solver as LoopClosing::ComputeSim3 uses it (SetRansacParameters(0.99, 20, 300)): the keyframe-pair geometry of
+    make_sim3_batch (camera-frame points, octaves recovered from its information values), outliers as 3-D mismatches (x2c
+    swapped among a share of the correspondences drawn per problem from outlier_range), fresh solvers (its_done = best = 0) and
+    each problem's budget of minimal sets drawn with DUtils' RandomInt from a seeded stream.  n_corr may be a list."""
+    base = make_sim3_batch(n_problems, n_corr, seed, fix_scale=fix_scale, outlier_frac=0.0)
+    rng = np.random.default_rng(seed + 7919)
+    isig, sig = inv_level_sigma2(), level_sigma2()
+    oct1 = np.searchsorted(-isig, -base["info1"])
+    oct2 = np.searchsorted(-isig, -base["info2"])
+    assert np.array_equal(isig[oct1], base["info1"]) and np.array_equal(isig[oct2], base["info2"])
+    x1c, x2c = base["p1c"].copy(), base["p2c"].copy()
+    off = base["off"]
+    for pb in range(n_problems):
+        a, z = int(off[pb]), int(off[pb + 1])
+        bad = np.where(rng.random(z - a) < rng.uniform(*outlier_range))[0] + a
+        if len(bad) >= 2:
+            x2c[bad] = x2c[np.roll(bad, 1)]
+    N = np.diff(off)
+    p = dict(n_problems=n_problems, cam=np.ascontiguousarray(f32(base["cam"])), fix_scale=base["fix_scale"].copy(), off=off.copy(),
+             x1c=np.ascontiguousarray(x1c), x2c=np.ascontiguousarray(x2c), sigma2_1=np.ascontiguousarray(sig[oct1]),
+             sigma2_2=np.ascontiguousarray(sig[oct2]), min_inliers=min_inliers,
+             max_its=np.asarray([sim3_ransac_max_its_py(int(k), 0.99, min_inliers, 300) for k in N], np.int32),
+             its_done=np.zeros(n_problems, np.int32), best_inliers=np.zeros(n_problems, np.int32), n_iterations=n_iterations)
+    return draw_sim3_ransac_sets(p, rand_stream(seed))
 
 
 def make_line_match_batch(n_pairs, n_lines, desc_dim, seed, tau=2.0, min_len=10, ragged=False):

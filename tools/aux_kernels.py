@@ -1,6 +1,6 @@
 #!/usr/bin/env python
 """Timing of the SURVEY §8(f) kernels (ComputeStereoMatches, relocalisation / map-point SearchByProjection, temporal line
-association, distinctive descriptors, SearchForInitialization, OptimizeSim3): device compute time from the library's own CUDA events (host buffers in, results
+association, distinctive descriptors, SearchForInitialization, OptimizeSim3, Sim3Solver): device compute time from the library's own CUDA events (host buffers in, results
 out through the public call), wall clock of the same call, and the CPU oracle on the same or a smaller sample.
 Prints one JSON object; results are compared with the oracle where the sample is the same.
 Usage: aux_kernels.py [section ...]   (default: every section)"""
@@ -180,4 +180,57 @@ if want("optimize_sim3"):
     res["nvidia_smi_name_power_limit"] = smi.strip()
     res["cpu"] = next((l.split(":", 1)[1].strip() for l in open("/proc/cpuinfo") if l.startswith("model name")), "")
     out["optimize_sim3"] = res
+# ---- Sim3Solver (LoopClosing::ComputeSim3: SetRansacParameters(0.99, 20, 300), iterate(5) per round), both scale modes
+if want("sim3_ransac"):
+    import subprocess
+    import ctypes as C
+    import torch
+    from test_sim3_ransac import run_rounds
+    d = ctx.lib.dll
+    d.lld_ctx_profile.argtypes = [C.c_void_p, C.c_int]; d.lld_ctx_profile.restype = None
+    d.lld_ctx_profile_report.argtypes = [C.c_void_p, C.c_char_p, C.c_int]; d.lld_ctx_profile_report.restype = C.c_int
+    res = {}
+    for fix in (1, 0):
+        ps = synth.make_sim3_ransac_batch(4096, 300, 701 + fix, fix_scale=fix)
+        g, ms, wall = timed(lambda: api.sim3_ransac(ps, impl="gpu", ctx=ctx))
+        d.lld_ctx_profile(ctx.handle, 1)                     # separate, profiled run: per-launch CUDA events
+        api.sim3_ransac(ps, impl="gpu", ctx=ctx)
+        buf = C.create_string_buffer(1 << 16)
+        ctx.check(d.lld_ctx_profile_report(ctx.handle, buf, len(buf)), "lld_ctx_profile_report")
+        d.lld_ctx_profile(ctx.handle, 0)
+        prof = json.loads(buf.value.decode())
+        # ComputeSim3 rounds of 5 over the same candidates (each round one call; draws on the host are not timed)
+        dev, calls = [], []
+        def gpu_round(q):
+            t0 = time.perf_counter(); o = api.sim3_ransac(q, impl="gpu", ctx=ctx); calls.append((time.perf_counter() - t0) * 1e3)
+            dev.append(ctx.last_timing()[1]); return o
+        run_rounds(ps, gpu_round, seed=fix)
+        # the batch-of-one round (5 sets) a caller without batching makes per candidate
+        p1 = synth.make_sim3_ransac_batch(1, 300, 711 + fix, fix_scale=fix, outlier_range=(0.9, 0.9), n_iterations=5)
+        one = []
+        api.sim3_ransac(p1, impl="gpu", ctx=ctx)
+        for _ in range(50):
+            t0 = time.perf_counter(); api.sim3_ransac(p1, impl="gpu", ctx=ctx); one.append((time.perf_counter() - t0) * 1e3)
+        one_dev = ctx.last_timing()[1]
+        o1, t1 = cpu(lambda: [api.sim3_ransac(p1, impl="oracle") for _ in range(50)])
+        sub = synth.make_sim3_ransac_batch(64, 300, 701 + fix, fix_scale=fix)   # the first 64 problems of the batch above
+        o, tc = cpu(lambda: api.sim3_ransac(sub, impl="oracle"))
+        h = int(sub["hyp_off"][-1])
+        same = all(np.array_equal(g[k][:len(o[k])], o[k]) for k in ("found", "no_more", "n_inliers", "its_done", "inlier"))
+        res["fixed_scale" if fix else "free_scale"] = {
+            "problems": 4096, "correspondences": 300, "minimal_sets_in_call": int(ps["hyp_off"][-1]),
+            "sets_evaluated": int((g["hyp_inliers"] >= 0).sum()), "found": int(g["found"].sum()),
+            "full_budget_one_call": {"device_ms": ms, "call_ms_from_host_buffers": wall, "problems_per_s_device": 4096 / ms * 1e3,
+                                     "kernel_profile_ms": {k: v["ms"] for k, v in prof.items()}},
+            "rounds_of_5": {"rounds": len(dev), "device_ms_total": float(np.sum(dev)), "call_ms_total": float(np.sum(calls)),
+                            "first_round_call_ms": calls[0], "last_round_call_ms": calls[-1]},
+            "batch_of_one_round_of_5": {"call_ms_median": float(np.median(one)), "device_ms": one_dev,
+                                        "cpu_oracle_ms": t1 / 50},
+            "cpu_oracle_ms_per_problem_full_budget": tc / 64, "cpu_oracle_sets_evaluated_sample": int((o["hyp_inliers"] >= 0).sum()),
+            "oracle_sample_64_identical": bool(same)}
+    smi = subprocess.run(["nvidia-smi", "--query-gpu=name,power.limit", "--format=csv,noheader"], stdout=subprocess.PIPE, text=True).stdout
+    res["gpu"] = torch.cuda.get_device_name(0)
+    res["nvidia_smi_name_power_limit"] = smi.strip()
+    res["cpu"] = next((l.split(":", 1)[1].strip() for l in open("/proc/cpuinfo") if l.startswith("model name")), "")
+    out["sim3_ransac"] = res
 print(json.dumps(out))
