@@ -10,6 +10,7 @@ cpu_baseline / reference arm may call it.
 from __future__ import annotations
 
 import ctypes as C
+import json
 import os
 from typing import Any, Dict
 
@@ -286,36 +287,10 @@ class _Lib:
         self._sig("kf_search", [vp, C.POINTER(KfSearchProblem), C.POINTER(SbpResult)])
         self._sig("tri_search", [vp, C.POINTER(TriSearchProblem), C.POINTER(TriSearchResult)])
         self._sig("bow_search", [vp, C.POINTER(BowSearchProblem), C.POINTER(TriSearchResult)])
-        init_sig = [vp, C.POINTER(InitSearchProblem), C.POINTER(InitSearchResult)]
-        if self.is_oracle:
-            if not os.path.exists(INIT_SEARCH_ORACLE_PATH):
-                raise RuntimeError(f"{INIT_SEARCH_ORACLE_PATH} not found — build it first (python -c 'import __graft_entry__ as g; g.build()').")
-            self.init_dll = C.CDLL(INIT_SEARCH_ORACLE_PATH)
-            self.init_search = self.init_dll.lldo_init_search
-            self.init_search.argtypes = init_sig
-            self.init_search.restype = C.c_int
-        else:
-            self._sig("init_search", init_sig)
-        sim3_sig = [vp, C.POINTER(Sim3Problem), C.POINTER(Sim3Result)]
-        if self.is_oracle:
-            if not os.path.exists(SIM3_ORACLE_PATH):
-                raise RuntimeError(f"{SIM3_ORACLE_PATH} not found — build it first (python -c 'import __graft_entry__ as g; g.build()').")
-            self.sim3_dll = C.CDLL(SIM3_ORACLE_PATH)
-            self.sim3_opt = self.sim3_dll.lldo_sim3_opt
-            self.sim3_opt.argtypes = sim3_sig
-            self.sim3_opt.restype = C.c_int
-        else:
-            self._sig("sim3_opt", sim3_sig)
-        ransac_sig = [vp, C.POINTER(Sim3RansacProblem), C.POINTER(Sim3RansacResult)]
-        if self.is_oracle:
-            if not os.path.exists(SIM3_RANSAC_ORACLE_PATH):
-                raise RuntimeError(f"{SIM3_RANSAC_ORACLE_PATH} not found — build it first (python -c 'import __graft_entry__ as g; g.build()').")
-            self.sim3_ransac_dll = C.CDLL(SIM3_RANSAC_ORACLE_PATH)
-            self.sim3_ransac = self.sim3_ransac_dll.lldo_sim3_ransac
-            self.sim3_ransac.argtypes = ransac_sig
-            self.sim3_ransac.restype = C.c_int
-        else:
-            self._sig("sim3_ransac", ransac_sig)
+        self._sig("init_search", [vp, C.POINTER(InitSearchProblem), C.POINTER(InitSearchResult)], INIT_SEARCH_ORACLE_PATH)
+        self._sig("sim3_opt", [vp, C.POINTER(Sim3Problem), C.POINTER(Sim3Result)], SIM3_ORACLE_PATH)
+        self._sig("sim3_ransac", [vp, C.POINTER(Sim3RansacProblem), C.POINTER(Sim3RansacResult)], SIM3_RANSAC_ORACLE_PATH)
+        if not self.is_oracle:
             self._sig("sim3_ransac_max_its", [C.c_int32, C.c_double, C.c_int32, C.c_int32])
             self.sim3_ransac_max_its.restype = C.c_int32
         self._sig("line_match", [vp, C.POINTER(LineMatchProblem), C.POINTER(LineMatchResult)])
@@ -332,6 +307,12 @@ class _Lib:
             d.lld_ctx_launch_count.restype = C.c_int64
             d.lld_ctx_last_timing.argtypes = [vp, c_f32p, c_f32p, c_f32p]
             d.lld_ctx_last_timing.restype = None
+            d.lld_ctx_last_bytes.argtypes = [vp, c_i64p, c_i64p]
+            d.lld_ctx_last_bytes.restype = None
+            d.lld_ctx_profile.argtypes = [vp, C.c_int]
+            d.lld_ctx_profile.restype = None
+            d.lld_ctx_profile_report.argtypes = [vp, C.c_char_p, C.c_int]
+            d.lld_ctx_profile_report.restype = C.c_int
             d.lld_comm_unique_id.argtypes = [c_u8p]
             d.lld_comm_unique_id.restype = C.c_int
             d.lld_comm_init.argtypes = [vp, C.c_int, C.c_int, c_u8p]
@@ -349,8 +330,13 @@ class _Lib:
             d.lld_ctx_nccl_stats.argtypes = [vp, c_i64p, c_i64p]
             d.lld_ctx_nccl_stats.restype = None
 
-    def _sig(self, name, argtypes):
-        f = getattr(self.dll, self.prefix + name)
+    def _sig(self, name, argtypes, oracle_path=None):
+        dll = self.dll
+        if self.is_oracle and oracle_path:  # an oracle restatement built as its own library under tests/hostcheck
+            if not os.path.exists(oracle_path):
+                raise RuntimeError(f"{oracle_path} not found — build it first (python -c 'import __graft_entry__ as g; g.build()').")
+            dll = C.CDLL(oracle_path)
+        f = getattr(dll, self.prefix + name)
         f.argtypes = argtypes
         f.restype = C.c_int
         setattr(self, name, f)
@@ -393,6 +379,18 @@ class Context:
         a, b, c = C.c_float(), C.c_float(), C.c_float()
         self.lib.dll.lld_ctx_last_timing(self.handle, C.byref(a), C.byref(b), C.byref(c))
         return a.value, b.value, c.value
+
+    def profile(self, fn):
+        """Run fn() with one CUDA-event pair around every kernel launch: (fn(), {kernel: {"ms": total, "n": launches}})."""
+        d = self.lib.dll
+        d.lld_ctx_profile(self.handle, 1)
+        try:
+            out = fn()
+            buf = C.create_string_buffer(1 << 16)
+            self.check(d.lld_ctx_profile_report(self.handle, buf, len(buf)), "lld_ctx_profile_report")
+        finally:
+            d.lld_ctx_profile(self.handle, 0)
+        return out, json.loads(buf.value.decode())
 
     def close(self):
         if self.handle:

@@ -236,42 +236,28 @@ static unsigned long long up_trace_hash(const void* p, size_t bytes) {
   return h;
 }
 
+// lld_up with the host stage's extras: no device work for lld_ba_index_only, and the uploaded bytes counted in *bytes
 template <typename T>
-int up(LldCtx* c, T** dst, const T* src, size_t n, size_t* bytes) {
+int up(LldCtx* c, T*& dst, const std::remove_const_t<T>* src, size_t n, size_t* bytes) {
   if (c->host_only) {  // lld_ba_index_only: time / test the host stage without a device
-    *dst = nullptr;
+    dst = nullptr;
     return LLD_OK;
   }
-  cudaError_t e = cudaSuccess;
-  T* d = c->alloc<T>(n ? n : 1, &e);
-  if (e != cudaSuccess) {
-    snprintf(c->err, sizeof(c->err), "cudaMalloc(%zu bytes): %s", n * sizeof(T), cudaGetErrorString(e));
-    return LLD_ERR_CUDA;
-  }
-  if (n && src) {
-    e = cudaMemcpyAsync(d, src, n * sizeof(T), cudaMemcpyHostToDevice, c->stream);
-    if (e != cudaSuccess) {
-      snprintf(c->err, sizeof(c->err), "cudaMemcpyAsync H2D: %s", cudaGetErrorString(e));
-      return LLD_ERR_CUDA;
-    }
-    if (bytes) *bytes += n * sizeof(T);
-  }
-  *dst = d;
-  return LLD_OK;
+  const int r = lld_up(c, dst, src, n);
+  if (r == LLD_OK && n && src && bytes) *bytes += n * sizeof(T);
+  return r;
 }
 #define UP(dst, src, n)                                                     \
   do {                                                                      \
     if (getenv("LLD_UP_TRACE")) fprintf(stderr, "[up] %-28s %10.3f MB  fnv %016llx\n", #src, (double)(n) * sizeof(*(dst)) / 1e6, \
                                         up_trace_hash((src), (size_t)(n) * sizeof(*(dst))));                \
-    int _r = up(c, &(dst), (src), (size_t)(n), &S->h2d_bytes);              \
+    int _r = up(c, (dst), (src), (size_t)(n), &S->h2d_bytes);               \
     if (_r != LLD_OK) return _r;                                            \
   } while (0)
-#define DEV(dst, T, n)                                                      \
+#define DEV(dst, n)                                                         \
   do {                                                                      \
-    T* _p = nullptr;                                                        \
-    int _r = up<T>(c, &_p, nullptr, (size_t)(n), nullptr);                  \
+    int _r = up(c, (dst), nullptr, (size_t)(n), nullptr);                   \
     if (_r != LLD_OK) return _r;                                            \
-    (dst) = _p;                                                             \
   } while (0)
 
 }  // namespace
@@ -1317,13 +1303,13 @@ static int ba_upload(LldCtx* c, const lld_ba_problem* p, bool global_mode, int l
   UP(tmp_i, kf_win.data(), n_kf); v.kf_win = tmp_i;
   // owner arrays (landmark -> window, edge -> landmark) and W slots are derived on the device from the offsets / masks
   int *d_pt_win, *d_ln_win, *d_pe_pt, *d_lc_ln, *d_pe_wpos, *d_lc_wpos;
-  DEV(d_pt_win, int, n_pt); v.pt_win = d_pt_win;
-  DEV(d_ln_win, int, n_ln); v.ln_win = d_ln_win;
+  DEV(d_pt_win, n_pt); v.pt_win = d_pt_win;
+  DEV(d_ln_win, n_ln); v.ln_win = d_ln_win;
   UP(tmp_i, kf_g.data(), n_kf); v.kf_g = tmp_i;
   UP(tmp_i, g_kf.data(), nG); v.g_kf = tmp_i;
   UP(tmp_i, w_g0.data(), nw + 1); v.w_g0 = tmp_i;
-  DEV(d_pe_pt, int, n_pe); v.pe_pt = d_pe_pt;
-  DEV(d_lc_ln, int, n_lc); v.lc_ln = d_lc_ln;
+  DEV(d_pe_pt, n_pe); v.pe_pt = d_pe_pt;
+  DEV(d_lc_ln, n_lc); v.lc_ln = d_lc_ln;
   UP(tmp_i, pe_pos.data(), dense ? 0 : n_pe); v.pe_pos = tmp_i;   // list positions are only read outside dense mode
   UP(tmp_i, lc_pos.data(), dense ? 0 : n_lc); v.lc_pos = tmp_i;
   UP(tmp_i, ch_g.data(), n_ch); v.ch_g = tmp_i;
@@ -1337,8 +1323,8 @@ static int ba_upload(LldCtx* c, const lld_ba_problem* p, bool global_mode, int l
   UP(tmp_i, nb_off.data(), nG + 1); v.nb_off = tmp_i;
   UP(tmp_i, nb_g.data(), nb_g.size()); v.nb_g = tmp_i;
   int *d_pl_tab = nullptr, *d_ll_tab = nullptr;
-  DEV(d_pl_tab, int, std::max(pl_tab_total, 1LL)); v.pl_tab = d_pl_tab;
-  DEV(d_ll_tab, int, std::max(ll_tab_total, 1LL)); v.ll_tab = d_ll_tab;
+  DEV(d_pl_tab, std::max(pl_tab_total, 1LL)); v.pl_tab = d_pl_tab;
+  DEV(d_ll_tab, std::max(ll_tab_total, 1LL)); v.ll_tab = d_ll_tab;
   long long* tmp_l;
   UP(tmp_l, pl_tab_off.data(), nG); v.pl_tab_off = tmp_l;
   UP(tmp_l, ll_tab_off.data(), nG); v.ll_tab_off = tmp_l;
@@ -1347,8 +1333,8 @@ static int ba_upload(LldCtx* c, const lld_ba_problem* p, bool global_mode, int l
   UP(tmp_i, ln_spos.data(), n_ln); v.ln_spos = tmp_i;
   UP(tmp_i, pts_w0.data(), n_pt + 1); v.pts_w0 = tmp_i;
   UP(tmp_i, lns_w0.data(), n_ln + 1); v.lns_w0 = tmp_i;
-  DEV(d_pe_wpos, int, n_pe); v.pe_wpos = d_pe_wpos;
-  DEV(d_lc_wpos, int, n_lc); v.lc_wpos = d_lc_wpos;
+  DEV(d_pe_wpos, n_pe); v.pe_wpos = d_pe_wpos;
+  DEV(d_lc_wpos, n_lc); v.lc_wpos = d_lc_wpos;
   { SchurItem* tmp_r; UP(tmp_r, H.it_rec.data(), (size_t)n_items_all); v.it_rec = tmp_r; }
   UP(tmp_i, gb_off.data(), gb_off.size()); v.gb_off = tmp_i;
   UP(tmp_l, gb_src.data(), gb_src.size()); v.gb_src = tmp_l;
@@ -1368,65 +1354,65 @@ static int ba_upload(LldCtx* c, const lld_ba_problem* p, bool global_mode, int l
   if (c->host_only) return LLD_OK;  // lld_ba_index_only: the host stage is complete
   // ---- device-only buffers ----
   for (int b = 0; b < 2; b++) {
-    DEV(v.pose_qt[b], double, 7 * (size_t)n_kf);
-    DEV(v.pose_Rt[b], double, 12 * (size_t)n_kf);
-    DEV(v.pt_xyz[b], double, 3 * (size_t)n_pt);
-    DEV(v.ln_st[b], double, 5 * (size_t)n_ln);
+    DEV(v.pose_qt[b], 7 * (size_t)n_kf);
+    DEV(v.pose_Rt[b], 12 * (size_t)n_kf);
+    DEV(v.pt_xyz[b], 3 * (size_t)n_pt);
+    DEV(v.ln_st[b], 5 * (size_t)n_ln);
   }
-  DEV(v.pe_level, uint8_t, n_pe); DEV(v.lc_level, uint8_t, 2 * (size_t)n_lc); DEV(v.ln_removed, uint8_t, n_ln);
-  DEV(v.pe_chi2, double, n_pe); DEV(v.lc_chi2, double, 2 * (size_t)n_lc);
-  DEV(v.pt_H, double, 9 * (size_t)n_pt); DEV(v.ln_H, double, 14 * (size_t)n_ln);
-  DEV(v.P_rec, double, dense ? 1 : 27 * (size_t)n_plist); DEV(v.L_rec, double, dense ? 1 : 38 * (size_t)n_llist);
-  DEV(v.pe_Wl, double, 18 * n_pw); DEV(v.lc_Wl, double, 24 * n_lw);
-  DEV(v.pts_D, double, dense ? 10 * (size_t)n_pt : 1); DEV(v.lns_D, double, dense ? 14 * (size_t)n_ln : 1);
-  DEV(v.dpart, double, (size_t)dpart_total);
-  DEV(v.ch_pose, double, 28 * (size_t)n_ch);
+  DEV(v.pe_level, n_pe); DEV(v.lc_level, 2 * (size_t)n_lc); DEV(v.ln_removed, n_ln);
+  DEV(v.pe_chi2, n_pe); DEV(v.lc_chi2, 2 * (size_t)n_lc);
+  DEV(v.pt_H, 9 * (size_t)n_pt); DEV(v.ln_H, 14 * (size_t)n_ln);
+  DEV(v.P_rec, dense ? 1 : 27 * (size_t)n_plist); DEV(v.L_rec, dense ? 1 : 38 * (size_t)n_llist);
+  DEV(v.pe_Wl, 18 * n_pw); DEV(v.lc_Wl, 24 * n_lw);
+  DEV(v.pts_D, dense ? 10 * (size_t)n_pt : 1); DEV(v.lns_D, dense ? 14 * (size_t)n_ln : 1);
+  DEV(v.dpart, (size_t)dpart_total);
+  DEV(v.ch_pose, 28 * (size_t)n_ch);
   // [g_bp | w_red_sum | g_Hpp] and [S_blk | g_bs] are contiguous: the multi-rank global BA all-reduces each group in one call
-  DEV(v.g_bp, double, 6 * (size_t)nG + 4 * (size_t)nw + 21 * (size_t)nG);
+  DEV(v.g_bp, 6 * (size_t)nG + 4 * (size_t)nw + 21 * (size_t)nG);
   v.w_red_sum = v.g_bp + 6 * (size_t)nG; v.g_Hpp = v.w_red_sum + 4 * (size_t)nw;
-  DEV(v.g_nact, int, nG);
-  DEV(v.lm_chi2lin, double, n_pt + n_ln); DEV(v.lm_maxdiag, double, n_pt + n_ln); DEV(v.lm_active, uint8_t, n_pt + n_ln);
-  DEV(v.ch_S, double, (size_t)chS_total);
-  DEV(v.S_blk, double, 36 * nb_g.size() + 6 * (size_t)nG);
-  v.g_bs = v.S_blk + 36 * nb_g.size(); DEV(v.g_x, double, 6 * (size_t)nG);
-  DEV(v.pt_D, double, 9 * (size_t)n_pt); DEV(v.ln_D, double, 14 * (size_t)n_ln);
-  DEV(v.pt_xl, double, 3 * (size_t)n_pt); DEV(v.ln_xl, double, 4 * (size_t)n_ln);
-  DEV(v.lm_chi2, double, n_pt + n_ln); DEV(v.lm_scale, double, n_pt + n_ln);
-  DEV(v.w_phase, int, nw); DEV(v.w_sel, int, nw); DEV(v.w_iter, int, nw); DEV(v.w_trials, int, nw);
-  DEV(v.w_maxit, int, nw); DEV(v.w_nbad, int, nw); DEV(v.w_ok, int, nw); DEV(v.w_nlog, int, nw);
-  DEV(v.w_lambda, double, nw); DEV(v.w_ni, double, nw); DEV(v.w_curchi, double, nw); DEV(v.w_inichi, double, nw);
-  DEV(v.w_scale_p, double, nw); DEV(v.w_red_max, double, nw);
+  DEV(v.g_nact, nG);
+  DEV(v.lm_chi2lin, n_pt + n_ln); DEV(v.lm_maxdiag, n_pt + n_ln); DEV(v.lm_active, n_pt + n_ln);
+  DEV(v.ch_S, (size_t)chS_total);
+  DEV(v.S_blk, 36 * nb_g.size() + 6 * (size_t)nG);
+  v.g_bs = v.S_blk + 36 * nb_g.size(); DEV(v.g_x, 6 * (size_t)nG);
+  DEV(v.pt_D, 9 * (size_t)n_pt); DEV(v.ln_D, 14 * (size_t)n_ln);
+  DEV(v.pt_xl, 3 * (size_t)n_pt); DEV(v.ln_xl, 4 * (size_t)n_ln);
+  DEV(v.lm_chi2, n_pt + n_ln); DEV(v.lm_scale, n_pt + n_ln);
+  DEV(v.w_phase, nw); DEV(v.w_sel, nw); DEV(v.w_iter, nw); DEV(v.w_trials, nw);
+  DEV(v.w_maxit, nw); DEV(v.w_nbad, nw); DEV(v.w_ok, nw); DEV(v.w_nlog, nw);
+  DEV(v.w_lambda, nw); DEV(v.w_ni, nw); DEV(v.w_curchi, nw); DEV(v.w_inichi, nw);
+  DEV(v.w_scale_p, nw); DEV(v.w_red_max, nw);
   {
     int max_lm = 0;
     for (int w = 0; w < nw; w++) max_lm = std::max(max_lm, (p->pt_off[w + 1] - p->pt_off[w]) + (p->ln_off[w + 1] - p->ln_off[w]));
     v.n_slices = std::max(1, std::min(128, max_lm / 16384));
   }
-  DEV(v.w_part, double, 4 * (size_t)nw * v.n_slices);
-  DEV(v.n_active_win, int, 2);   // [0] windows still running, [1] multi-rank stop agreement word
+  DEV(v.w_part, 4 * (size_t)nw * v.n_slices);
+  DEV(v.n_active_win, 2);   // [0] windows still running, [1] multi-rank stop agreement word
   v.log_stride = log_stride;
-  DEV(v.chi2_log, double, (size_t)nw * log_stride); DEV(v.lambda_log, double, (size_t)nw * log_stride);
-  DEV(v.trials_log, int, (size_t)nw * log_stride); DEV(v.iter_done, int, 2 * (size_t)nw);
-  DEV(v.solve_scratch, double, (size_t)scr_total);
-  DEV(v.env_A, double, (S->use_cr || S->use_sp) ? 1 : (size_t)env_rowptr.back());
+  DEV(v.chi2_log, (size_t)nw * log_stride); DEV(v.lambda_log, (size_t)nw * log_stride);
+  DEV(v.trials_log, (size_t)nw * log_stride); DEV(v.iter_done, 2 * (size_t)nw);
+  DEV(v.solve_scratch, (size_t)scr_total);
+  DEV(v.env_A, (S->use_cr || S->use_sp) ? 1 : (size_t)env_rowptr.back());
   if (S->use_cr) {
     CrView& cr = S->cr;
     const size_t mm = (size_t)cr.m * cr.m, N = (size_t)cr.N;
     // D and U[0] are zero-filled together before every assembly: one allocation
-    DEV(cr.D, double, 2 * N * mm); cr.U[0] = cr.D + N * mm;
-    DEV(cr.U[1], double, N * mm); DEV(cr.L, double, N * mm); DEV(cr.Z, double, N * cr.m * cr.zs);
-    DEV(cr.b, double, N * cr.m); DEV(cr.zc, double, N * cr.m); DEV(cr.x, double, N * cr.m);
-    DEV(cr.ok, int, 1);
+    DEV(cr.D, 2 * N * mm); cr.U[0] = cr.D + N * mm;
+    DEV(cr.U[1], N * mm); DEV(cr.L, N * mm); DEV(cr.Z, N * cr.m * cr.zs);
+    DEV(cr.b, N * cr.m); DEV(cr.zc, N * cr.m); DEV(cr.x, N * cr.m);
+    DEV(cr.ok, 1);
   }
   if (S->use_sp) {
     SpView& sp = S->sp;
     const size_t mm = (size_t)sp.m * sp.m, N = (size_t)sp.N;
-    DEV(sp.W, double, (size_t)S->sp_n_slot * mm); DEV(sp.L, double, N * mm); DEV(sp.Z, double, std::max(S->sp_z_total, 1LL));
-    DEV(sp.b, double, N * sp.m); DEV(sp.zc, double, N * sp.m); DEV(sp.x, double, N * sp.m);
-    DEV(sp.ok, int, 1);
+    DEV(sp.W, (size_t)S->sp_n_slot * mm); DEV(sp.L, N * mm); DEV(sp.Z, std::max(S->sp_z_total, 1LL));
+    DEV(sp.b, N * sp.m); DEV(sp.zc, N * sp.m); DEV(sp.x, N * sp.m);
+    DEV(sp.ok, 1);
   }
-  DEV(S->d_out_kf, double, 12 * (size_t)n_kf); DEV(S->d_out_pt, double, 3 * (size_t)n_pt);
-  DEV(S->d_out_ln, double, 6 * (size_t)n_ln);
-  DEV(S->d_pt_bad, uint8_t, n_pe); DEV(S->d_ln_bad, uint8_t, 2 * (size_t)n_lc);
+  DEV(S->d_out_kf, 12 * (size_t)n_kf); DEV(S->d_out_pt, 3 * (size_t)n_pt);
+  DEV(S->d_out_ln, 6 * (size_t)n_ln);
+  DEV(S->d_pt_bad, n_pe); DEV(S->d_ln_bad, 2 * (size_t)n_lc);
   LLD_CUDA(c, cudaMemsetAsync(v.chi2_log, 0, sizeof(double) * (size_t)nw * log_stride, c->stream));
   LLD_CUDA(c, cudaMemsetAsync(v.lambda_log, 0, sizeof(double) * (size_t)nw * log_stride, c->stream));
   LLD_CUDA(c, cudaMemsetAsync(v.trials_log, 0, sizeof(int) * (size_t)nw * log_stride, c->stream));
@@ -1908,28 +1894,20 @@ static int ba_download(LldCtx* c, const lld_ba_problem* p, lld_ba_result* out, b
   LLD_LAUNCH(c, k_export, cdiv(n, 256), 256, 0, v, S->d_out_kf, S->d_out_pt, S->d_out_ln, S->d_ln_in);
   LLD_CUDA(c, cudaGetLastError());
   LLD_CUDA(c, cudaEventRecord(c->ev[2], c->stream));
-  auto D2H = [&](void* dst, const void* src, size_t bytes) -> cudaError_t {
-    if (!dst || !bytes) return cudaSuccess;
-    return cudaMemcpyAsync(dst, src, bytes, cudaMemcpyDeviceToHost, c->stream);
-  };
-  LLD_CUDA(c, D2H(out->kf_Tcw, S->d_out_kf, sizeof(double) * 12 * (size_t)v.n_kf));
-  LLD_CUDA(c, D2H(out->pt_xyz, S->d_out_pt, sizeof(double) * 3 * (size_t)v.n_pt));
-  LLD_CUDA(c, D2H(out->ln_x0_dir, S->d_out_ln, sizeof(double) * 6 * (size_t)v.n_ln));
-  LLD_CUDA(c, D2H(out->pt_obs_bad, S->d_pt_bad, (size_t)v.n_pe));
-  LLD_CUDA(c, D2H(out->ln_obs_bad, S->d_ln_bad, 2 * (size_t)v.n_lc));
-  LLD_CUDA(c, D2H(out->ln_removed, v.ln_removed, (size_t)v.n_ln));
+  LLD_DOWN(c, out->kf_Tcw, S->d_out_kf, 12 * (size_t)v.n_kf);
+  LLD_DOWN(c, out->pt_xyz, S->d_out_pt, 3 * (size_t)v.n_pt);
+  LLD_DOWN(c, out->ln_x0_dir, S->d_out_ln, 6 * (size_t)v.n_ln);
+  LLD_DOWN(c, out->pt_obs_bad, S->d_pt_bad, v.n_pe);
+  LLD_DOWN(c, out->ln_obs_bad, S->d_ln_bad, 2 * (size_t)v.n_lc);
+  LLD_DOWN(c, out->ln_removed, v.ln_removed, v.n_ln);
   const int ls = std::min(out->log_stride, v.log_stride);
   if (out->log_stride == v.log_stride) {
-    LLD_CUDA(c, D2H(out->chi2_log, v.chi2_log, sizeof(double) * (size_t)v.n_win * ls));
-    LLD_CUDA(c, D2H(out->lambda_log, v.lambda_log, sizeof(double) * (size_t)v.n_win * ls));
-    LLD_CUDA(c, D2H(out->trials_log, v.trials_log, sizeof(int) * (size_t)v.n_win * ls));
+    LLD_DOWN(c, out->chi2_log, v.chi2_log, (size_t)v.n_win * ls);
+    LLD_DOWN(c, out->lambda_log, v.lambda_log, (size_t)v.n_win * ls);
+    LLD_DOWN(c, out->trials_log, v.trials_log, (size_t)v.n_win * ls);
   }
-  LLD_CUDA(c, D2H(out->n_iter_done, v.iter_done, sizeof(int) * 2 * (size_t)v.n_win));
-  LLD_CUDA(c, cudaEventRecord(c->ev[3], c->stream));
-  LLD_CUDA(c, cudaStreamSynchronize(c->stream));
-  cudaEventElapsedTime(&c->ms_h2d, c->ev[0], c->ev[1]);
-  cudaEventElapsedTime(&c->ms_compute, c->ev[1], c->ev[2]);
-  cudaEventElapsedTime(&c->ms_d2h, c->ev[2], c->ev[3]);
+  LLD_DOWN(c, out->n_iter_done, v.iter_done, 2 * (size_t)v.n_win);
+  if (int r = lld_call_end(c)) return r;
   c->last_d2h_bytes = sizeof(double) * (12 * (size_t)v.n_kf + 3 * (size_t)v.n_pt + 6 * (size_t)v.n_ln) + (size_t)v.n_pe +
                       2 * (size_t)v.n_lc + (size_t)v.n_ln + (sizeof(double) * 2 + sizeof(int)) * (size_t)v.n_win * ls +
                       sizeof(int) * 2 * (size_t)v.n_win;

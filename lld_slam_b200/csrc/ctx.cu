@@ -38,6 +38,23 @@ cudaError_t lld_raise_dyn_smem(const void* func, int bytes) {
   return r;
 }
 
+int lld_call_begin(LldCtx* c, bool full) {
+  LLD_CUDA(c, cudaSetDevice(c->device));
+  if (full) c->launches = 0;
+  c->pool_reset();
+  LLD_CUDA(c, cudaEventRecord(c->ev[0], c->stream));
+  return LLD_OK;
+}
+
+int lld_call_end(LldCtx* c) {
+  LLD_CUDA(c, cudaEventRecord(c->ev[3], c->stream));
+  LLD_CUDA(c, cudaStreamSynchronize(c->stream));
+  cudaEventElapsedTime(&c->ms_h2d, c->ev[0], c->ev[1]);
+  cudaEventElapsedTime(&c->ms_compute, c->ev[1], c->ev[2]);
+  cudaEventElapsedTime(&c->ms_d2h, c->ev[2], c->ev[3]);
+  return LLD_OK;
+}
+
 extern "C" const char* lld_version(void) { return "lldba 0.1 (sm_100a)"; }
 
 extern "C" int lld_ctx_create(int device, void** out) {

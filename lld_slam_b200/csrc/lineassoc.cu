@@ -139,7 +139,7 @@ __global__ void __launch_bounds__(32) k_line_associate(AssocView v) {
 extern "C" int lld_line_associate(void* ctx, const lld_line_assoc_problem* p, lld_line_assoc_result* out) {
   LldCtx* c = lld_ctx_cast(ctx);
   if (!c || !p || !out) return LLD_ERR_ARG;
-  c->launches = 0;
+  c->launches = 0;   // a rejected call reports no launches
   LLD_ARG(c, p->n_frames >= 1 && p->desc_dim >= 1);
   const int F = p->n_frames, n_ml = p->ml_off[F], n_cur = p->cur_off[F], n_r = p->right_off[F], n_cand = p->cand_off[n_ml], D = p->desc_dim;
   // candidates index the frame's current lines (taken bitset, cur_line_match); a stereo match indexes its right lines
@@ -153,49 +153,33 @@ extern "C" int lld_line_associate(void* ctx, const lld_line_assoc_problem* p, ll
   for (int f = 0; f < F; f++) max_cur = std::max(max_cur, p->cur_off[f + 1] - p->cur_off[f]);
   const size_t smem = 4 * (size_t)((max_cur + 31) / 32);
   LLD_ARG(c, smem <= 48 * 1024);
-  LLD_CUDA(c, cudaSetDevice(c->device));
-  c->pool_reset();
-  cudaError_t e = cudaSuccess;
-  auto up = [&](const void* src, size_t bytes) -> void* {
-    if (e != cudaSuccess) return nullptr;
-    uint8_t* d = c->alloc<uint8_t>(bytes ? bytes : 1, &e);
-    if (e == cudaSuccess && bytes) e = cudaMemcpyAsync(d, src, bytes, cudaMemcpyHostToDevice, c->stream);
-    return d;
-  };
+  if (int r = lld_call_begin(c, true)) return r;
   AssocView v{};
   v.p = *p;
-  LLD_CUDA(c, cudaEventRecord(c->ev[0], c->stream));
-  v.p.ml_off = (const int32_t*)up(p->ml_off, 4 * (size_t)(F + 1));
-  v.p.ml_valid = (const uint8_t*)up(p->ml_valid, (size_t)n_ml);
-  v.p.ml_x0_dir = (const double*)up(p->ml_x0_dir, 48 * (size_t)n_ml);
-  v.p.ml_x1x2 = (const double*)up(p->ml_x1x2, 48 * (size_t)n_ml);
-  v.p.ml_desc = (const float*)up(p->ml_desc, 4 * (size_t)D * n_ml);
-  v.p.cand_off = (const int32_t*)up(p->cand_off, 4 * (size_t)(n_ml + 1));
-  v.p.cand_idx = (const int32_t*)up(p->cand_idx, 4 * (size_t)n_cand);
-  v.p.cur_off = (const int32_t*)up(p->cur_off, 4 * (size_t)(F + 1));
-  v.p.cur_left = (const float*)up(p->cur_left, 16 * (size_t)n_cur);
-  v.p.cur_octave = (const int32_t*)up(p->cur_octave, 4 * (size_t)n_cur);
-  v.p.cur_line_match = (const int32_t*)up(p->cur_line_match, 4 * (size_t)n_cur);
-  v.p.cur_taken = (const uint8_t*)up(p->cur_taken, (size_t)n_cur);
-  v.p.cur_desc = (const float*)up(p->cur_desc, 4 * (size_t)D * n_cur);
-  v.p.right_off = (const int32_t*)up(p->right_off, 4 * (size_t)(F + 1));
-  v.p.cur_right = (const float*)up(p->cur_right, 16 * (size_t)n_r);
-  v.p.T_curr = (const double*)up(p->T_curr, 128 * (size_t)F);
-  v.p.T_right = (const double*)up(p->T_right, 128 * (size_t)F);
-  v.cur_assoc = (int*)up(nullptr, 0);
-  if (e == cudaSuccess) v.cur_assoc = c->alloc<int>((size_t)std::max(n_cur, 1), &e);
-  if (e == cudaSuccess) v.n_added = c->alloc<int>((size_t)F, &e);
-  LLD_CUDA(c, e);
+  LLD_UP(c, v.p.ml_off, p->ml_off, F + 1);
+  LLD_UP(c, v.p.ml_valid, p->ml_valid, n_ml);
+  LLD_UP(c, v.p.ml_x0_dir, p->ml_x0_dir, 6 * (size_t)n_ml);
+  LLD_UP(c, v.p.ml_x1x2, p->ml_x1x2, 6 * (size_t)n_ml);
+  LLD_UP(c, v.p.ml_desc, p->ml_desc, (size_t)D * n_ml);
+  LLD_UP(c, v.p.cand_off, p->cand_off, n_ml + 1);
+  LLD_UP(c, v.p.cand_idx, p->cand_idx, n_cand);
+  LLD_UP(c, v.p.cur_off, p->cur_off, F + 1);
+  LLD_UP(c, v.p.cur_left, p->cur_left, 4 * (size_t)n_cur);
+  LLD_UP(c, v.p.cur_octave, p->cur_octave, n_cur);
+  LLD_UP(c, v.p.cur_line_match, p->cur_line_match, n_cur);
+  LLD_UP(c, v.p.cur_taken, p->cur_taken, n_cur);
+  LLD_UP(c, v.p.cur_desc, p->cur_desc, (size_t)D * n_cur);
+  LLD_UP(c, v.p.right_off, p->right_off, F + 1);
+  LLD_UP(c, v.p.cur_right, p->cur_right, 4 * (size_t)n_r);
+  LLD_UP(c, v.p.T_curr, p->T_curr, 16 * (size_t)F);
+  LLD_UP(c, v.p.T_right, p->T_right, 16 * (size_t)F);
+  LLD_DEV(c, v.cur_assoc, n_cur);
+  LLD_DEV(c, v.n_added, F);
   LLD_CUDA(c, cudaEventRecord(c->ev[1], c->stream));
   LLD_LAUNCH(c, k_line_associate, F, 32, smem, v);
   LLD_CUDA(c, cudaGetLastError());
   LLD_CUDA(c, cudaEventRecord(c->ev[2], c->stream));
-  if (n_cur) LLD_CUDA(c, cudaMemcpyAsync(out->cur_assoc, v.cur_assoc, 4 * (size_t)n_cur, cudaMemcpyDeviceToHost, c->stream));
-  if (out->n_added) LLD_CUDA(c, cudaMemcpyAsync(out->n_added, v.n_added, 4 * (size_t)F, cudaMemcpyDeviceToHost, c->stream));
-  LLD_CUDA(c, cudaEventRecord(c->ev[3], c->stream));
-  LLD_CUDA(c, cudaStreamSynchronize(c->stream));
-  cudaEventElapsedTime(&c->ms_h2d, c->ev[0], c->ev[1]);
-  cudaEventElapsedTime(&c->ms_compute, c->ev[1], c->ev[2]);
-  cudaEventElapsedTime(&c->ms_d2h, c->ev[2], c->ev[3]);
-  return LLD_OK;
+  LLD_DOWN(c, out->cur_assoc, v.cur_assoc, n_cur);
+  LLD_DOWN(c, out->n_added, v.n_added, F);
+  return lld_call_end(c);
 }

@@ -985,32 +985,6 @@ __global__ void __launch_bounds__(256) k_line_exact2(LineTc2View t, int swap_gri
   if (live && sub == 0) v.mdist[a0 + j] = bi >= 0 ? sqrtf(s2) : INFINITY;
 }
 
-template <typename T>
-int upm(LldCtx* c, T** dst, const T* src, size_t n) {
-  cudaError_t e = cudaSuccess;
-  T* d = c->alloc<T>(n ? n : 1, &e);
-  if (e != cudaSuccess) {
-    snprintf(c->err, sizeof(c->err), "cudaMalloc: %s", cudaGetErrorString(e));
-    return LLD_ERR_CUDA;
-  }
-  if (n && src) {
-    e = cudaMemcpyAsync(d, src, n * sizeof(T), cudaMemcpyHostToDevice, c->stream);
-    if (e != cudaSuccess) {
-      snprintf(c->err, sizeof(c->err), "cudaMemcpyAsync H2D: %s", cudaGetErrorString(e));
-      return LLD_ERR_CUDA;
-    }
-  }
-  *dst = d;
-  return LLD_OK;
-}
-#define UPM(dst, T, src, n)                                \
-  do {                                                     \
-    T* _p = nullptr;                                       \
-    int _r = upm<T>(c, &_p, (const T*)(src), (size_t)(n)); \
-    if (_r) return _r;                                     \
-    (dst) = _p;                                            \
-  } while (0)
-
 inline int cdiv(int a, int b) { return (a + b - 1) / b; }
 
 }  // namespace
@@ -1018,9 +992,7 @@ inline int cdiv(int a, int b) { return (a + b - 1) / b; }
 extern "C" int lld_line_match(void* ctx, const lld_line_match_problem* p, lld_line_match_result* out) {
   LldCtx* c = lld_ctx_cast(ctx);
   if (!c || !p || !out) return LLD_ERR_ARG;
-  LLD_CUDA(c, cudaSetDevice(c->device));
-  c->launches = 0;
-  c->pool_reset();
+  if (int r = lld_call_begin(c, true)) return r;
   LLD_ARG(c, p->n_pairs >= 1 && p->desc_dim >= 1 && p->desc_dim <= 512);
   LineMatchView v;
   const int P = p->n_pairs;
@@ -1049,33 +1021,32 @@ extern "C" int lld_line_match(void* ctx, const lld_line_match_problem* p, lld_li
     for (int r = 0; r < cdiv(na, LT); r++)
       for (int cc = 0; cc < cdiv(nb, LT); cc++) { tp.push_back(i); tr.push_back(r); tc.push_back(cc); }
   }
-  LLD_CUDA(c, cudaEventRecord(c->ev[0], c->stream));
-  UPM(v.left_off, int, p->left_off, P + 1);
-  UPM(v.right_off, int, p->right_off, P + 1);
-  UPM(v.left_seg, float, p->left_seg, 4 * (size_t)n_left);
-  UPM(v.left_oct, int, p->left_octave, n_left);
-  UPM(v.right_seg, float, p->right_seg, 4 * (size_t)n_right);
-  UPM(v.right_oct, int, p->right_octave, n_right);
-  UPM(v.left_desc, float, p->left_desc, (size_t)n_left * v.D);
-  UPM(v.right_desc, float, p->right_desc, (size_t)n_right * v.D);
-  UPM(v.mat_off, long long, mat_off.data(), P);
+  LLD_UP(c, v.left_off, p->left_off, P + 1);
+  LLD_UP(c, v.right_off, p->right_off, P + 1);
+  LLD_UP(c, v.left_seg, p->left_seg, 4 * (size_t)n_left);
+  LLD_UP(c, v.left_oct, p->left_octave, n_left);
+  LLD_UP(c, v.right_seg, p->right_seg, 4 * (size_t)n_right);
+  LLD_UP(c, v.right_oct, p->right_octave, n_right);
+  LLD_UP(c, v.left_desc, p->left_desc, (size_t)n_left * v.D);
+  LLD_UP(c, v.right_desc, p->right_desc, (size_t)n_right * v.D);
+  LLD_UP(c, v.mat_off, mat_off.data(), P);
   long long* d_taken_off;
-  UPM(d_taken_off, long long, taken_off.data(), P);
+  LLD_UP(c, d_taken_off, taken_off.data(), P);
   int *d_tp, *d_tr, *d_tc;
-  UPM(d_tp, int, tp.data(), tp.size());
-  UPM(d_tr, int, tr.data(), tr.size());
-  UPM(d_tc, int, tc.data(), tc.size());
-  UPM(v.left_leq, double, nullptr, 3 * (size_t)n_left);
-  UPM(v.right_leq, double, nullptr, 3 * (size_t)n_right);
-  UPM(v.left_len, double, nullptr, n_left);
-  UPM(v.right_len, double, nullptr, n_right);
-  UPM(v.left_un, double, nullptr, 3 * (size_t)n_left);
-  UPM(v.right_un, double, nullptr, 3 * (size_t)n_right);
-  UPM(v.dist, float, nullptr, (size_t)tot);
-  UPM(v.match, int, nullptr, n_left);
-  UPM(v.mdist, float, nullptr, n_left);
+  LLD_UP(c, d_tp, tp.data(), tp.size());
+  LLD_UP(c, d_tr, tr.data(), tr.size());
+  LLD_UP(c, d_tc, tc.data(), tc.size());
+  LLD_DEV(c, v.left_leq, 3 * (size_t)n_left);
+  LLD_DEV(c, v.right_leq, 3 * (size_t)n_right);
+  LLD_DEV(c, v.left_len, n_left);
+  LLD_DEV(c, v.right_len, n_right);
+  LLD_DEV(c, v.left_un, 3 * (size_t)n_left);
+  LLD_DEV(c, v.right_un, 3 * (size_t)n_right);
+  LLD_DEV(c, v.dist, (size_t)tot);
+  LLD_DEV(c, v.match, n_left);
+  LLD_DEV(c, v.mdist, n_left);
   int* d_taken;
-  UPM(d_taken, int, nullptr, (size_t)ttot);
+  LLD_DEV(c, d_taken, (size_t)ttot);
   LLD_CUDA(c, cudaEventRecord(c->ev[1], c->stream));
   const int nmax = std::max(std::max(n_left, n_right), 1);
   int* d_tc_err = nullptr;
@@ -1084,16 +1055,16 @@ extern "C" int lld_line_match(void* ctx, const lld_line_match_problem* p, lld_li
     LineTc2View t;
     t.v = v;
     t.nl_chunk = v.D <= 64 ? 256 : 128;
-    UPM(t.rc.lrec, float4, nullptr, n_left);
-    UPM(t.rc.rrec, float4, nullptr, n_right);
-    UPM(t.rc.rh, float, nullptr, n_right);
-    UPM(t.rc.loct, int8_t, nullptr, n_left);
-    UPM(t.rc.roct, int8_t, nullptr, n_right);
-    UPM(t.rc.lgeo, float4, nullptr, 7 * (size_t)n_left);
-    UPM(t.rc.rleq, float4, nullptr, n_right);
-    UPM(t.cand, uint2, nullptr, (size_t)n_left * T2_CAP);
-    UPM(t.cand_cnt, uint16_t, nullptr, n_left);
-    UPM(t.err_flag, int, nullptr, 8);
+    LLD_DEV(c, t.rc.lrec, n_left);
+    LLD_DEV(c, t.rc.rrec, n_right);
+    LLD_DEV(c, t.rc.rh, n_right);
+    LLD_DEV(c, t.rc.loct, n_left);
+    LLD_DEV(c, t.rc.roct, n_right);
+    LLD_DEV(c, t.rc.lgeo, 7 * (size_t)n_left);
+    LLD_DEV(c, t.rc.rleq, n_right);
+    LLD_DEV(c, t.cand, (size_t)n_left * T2_CAP);
+    LLD_DEV(c, t.cand_cnt, n_left);
+    LLD_DEV(c, t.err_flag, 8);
     d_tc_err = t.err_flag;
     LLD_CUDA(c, cudaMemsetAsync(t.err_flag, 0, 8 * sizeof(int), c->stream));
     LLD_CUDA(c, cudaMemsetAsync(t.cand_cnt, 0, sizeof(uint16_t) * (size_t)n_left, c->stream));   // pairs without right lines
@@ -1129,16 +1100,10 @@ extern "C" int lld_line_match(void* ctx, const lld_line_match_problem* p, lld_li
   LLD_CUDA(c, cudaEventRecord(c->ev[2], c->stream));
   int* h_err = reinterpret_cast<int*>(c->pinned);
   for (int i = 0; i < 8; i++) h_err[i] = 0;
-  if (d_tc_err) LLD_CUDA(c, cudaMemcpyAsync(h_err, d_tc_err, 8 * sizeof(int), cudaMemcpyDeviceToHost, c->stream));
-  if (n_left) {
-    LLD_CUDA(c, cudaMemcpyAsync(out->match, v.match, sizeof(int) * (size_t)n_left, cudaMemcpyDeviceToHost, c->stream));
-    if (out->dist) LLD_CUDA(c, cudaMemcpyAsync(out->dist, v.mdist, sizeof(float) * (size_t)n_left, cudaMemcpyDeviceToHost, c->stream));
-  }
-  LLD_CUDA(c, cudaEventRecord(c->ev[3], c->stream));
-  LLD_CUDA(c, cudaStreamSynchronize(c->stream));
-  cudaEventElapsedTime(&c->ms_h2d, c->ev[0], c->ev[1]);
-  cudaEventElapsedTime(&c->ms_compute, c->ev[1], c->ev[2]);
-  cudaEventElapsedTime(&c->ms_d2h, c->ev[2], c->ev[3]);
+  if (d_tc_err) LLD_DOWN(c, h_err, d_tc_err, 8);
+  LLD_DOWN(c, out->match, v.match, n_left);
+  LLD_DOWN(c, out->dist, v.mdist, n_left);
+  if (int r = lld_call_end(c)) return r;
   if (getenv("LLD_LINE_STATS") && d_tc_err)
     fprintf(stderr, "[lld_line_match] rows with an overflowed list %d, listed candidates %d, decided in FP64 %d, FP32/FP64 disagreements %d, largest FP32 error / bound %.3g\n",
             h_err[1], h_err[2], h_err[4], h_err[5], (double)*reinterpret_cast<float*>(h_err + 6));

@@ -6,6 +6,7 @@
 #include <string.h>
 
 #include <mutex>
+#include <type_traits>
 #include <vector>
 
 #include "../../include/lldba.h"
@@ -150,5 +151,56 @@ struct LldCtx {
     (ctx)->launches++;                                                          \
   } while (0)
 #define LLD_LAUNCH(ctx, kernel, grid, block, smem, ...) LLD_LAUNCH_S(ctx, (ctx)->stream, kernel, grid, block, smem, __VA_ARGS__)
+
+// ---- one C-ABI call: ev[0] .. ev[1] upload, ev[1] .. ev[2] compute, ev[2] .. ev[3] download (lld_ctx_last_timing) ----
+// Each entry point records ev[1] and ev[2] itself, at its own phase boundaries.
+
+// Opens a call: current device, launch count (full: the resident-mode uploads keep it), a fresh device pool, ev[0].
+int lld_call_begin(LldCtx* c, bool full);
+// Closes a call: ev[3], waits for the stream and fills ms_h2d / ms_compute / ms_d2h.
+int lld_call_end(LldCtx* c);
+
+// Takes the next pool buffer, max(n, 1) elements of T, and copies n elements from src into it when n && src (no source:
+// device-only scratch).  T comes from the destination alone, so a const T* field of a copied problem struct takes it as is.
+template <typename T>
+inline int lld_up(LldCtx* c, T*& dst, const std::remove_const_t<T>* src, size_t n) {
+  cudaError_t e = cudaSuccess;
+  std::remove_const_t<T>* d = c->alloc<std::remove_const_t<T>>(n ? n : 1, &e);
+  if (e != cudaSuccess) {
+    snprintf(c->err, sizeof(c->err), "cudaMalloc(%zu bytes): %s", n * sizeof(T), cudaGetErrorString(e));
+    return LLD_ERR_CUDA;
+  }
+  if (n && src) {
+    e = cudaMemcpyAsync(d, src, n * sizeof(T), cudaMemcpyHostToDevice, c->stream);
+    if (e != cudaSuccess) {
+      snprintf(c->err, sizeof(c->err), "cudaMemcpyAsync H2D: %s", cudaGetErrorString(e));
+      return LLD_ERR_CUDA;
+    }
+  }
+  dst = d;
+  return LLD_OK;
+}
+// Copies n elements device-to-host when n && dst (an output the caller did not ask for is skipped).
+template <typename T>
+inline int lld_down(LldCtx* c, T* dst, const T* src, size_t n) {
+  if (!n || !dst) return LLD_OK;
+  cudaError_t e = cudaMemcpyAsync(dst, src, n * sizeof(T), cudaMemcpyDeviceToHost, c->stream);
+  if (e != cudaSuccess) {
+    snprintf(c->err, sizeof(c->err), "cudaMemcpyAsync D2H: %s", cudaGetErrorString(e));
+    return LLD_ERR_CUDA;
+  }
+  return LLD_OK;
+}
+#define LLD_UP(ctx, dst, src, n)                               \
+  do {                                                         \
+    int _r = lld_up((ctx), (dst), (src), (size_t)(n));         \
+    if (_r) return _r;                                         \
+  } while (0)
+#define LLD_DEV(ctx, dst, n) LLD_UP(ctx, dst, nullptr, n)
+#define LLD_DOWN(ctx, dst, src, n)                             \
+  do {                                                         \
+    int _r = lld_down((ctx), (dst), (src), (size_t)(n));       \
+    if (_r) return _r;                                         \
+  } while (0)
 
 static inline LldCtx* lld_ctx_cast(void* p) { return reinterpret_cast<LldCtx*>(p); }

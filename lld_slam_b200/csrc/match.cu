@@ -1144,32 +1144,6 @@ __global__ void __launch_bounds__(256) k_init_finalize(MatchView v, InitView w) 
 
 inline int cdiv(int a, int b) { return (a + b - 1) / b; }
 
-template <typename T>
-int up(LldCtx* c, T** dst, const T* src, size_t n) {
-  cudaError_t e = cudaSuccess;
-  T* d = c->alloc<T>(n ? n : 1, &e);
-  if (e != cudaSuccess) {
-    snprintf(c->err, sizeof(c->err), "cudaMalloc: %s", cudaGetErrorString(e));
-    return LLD_ERR_CUDA;
-  }
-  if (n && src) {
-    e = cudaMemcpyAsync(d, src, n * sizeof(T), cudaMemcpyHostToDevice, c->stream);
-    if (e != cudaSuccess) {
-      snprintf(c->err, sizeof(c->err), "cudaMemcpyAsync H2D: %s", cudaGetErrorString(e));
-      return LLD_ERR_CUDA;
-    }
-  }
-  *dst = d;
-  return LLD_OK;
-}
-#define UPC(dst, T, src, n)                              \
-  do {                                                   \
-    T* _p = nullptr;                                     \
-    int _r = up<T>(c, &_p, (const T*)(src), (size_t)(n)); \
-    if (_r) return _r;                                   \
-    (dst) = _p;                                          \
-  } while (0)
-
 struct MatchState {
   MatchView v{};
 };
@@ -1208,7 +1182,7 @@ static int match_run(LldCtx* c, MatchView& v, int* passes_out) {
     while (true) {
       LLD_LAUNCH(c, k_match_resolve, cdiv(v.n_q, 128), 128, 0, v, pass);
       if (pass > 0) {
-        LLD_CUDA(c, cudaMemcpyAsync(h_changed, v.changed, sizeof(int), cudaMemcpyDeviceToHost, c->stream));
+        LLD_DOWN(c, h_changed, v.changed, 1);
         LLD_CUDA(c, cudaStreamSynchronize(c->stream));
         if (!*h_changed) break;
       }
@@ -1228,20 +1202,20 @@ static int match_run(LldCtx* c, MatchView& v, int* passes_out) {
 }
 
 static int match_alloc_common(LldCtx* c, MatchView& v) {
-  UPC(v.cell_count, int, nullptr, (size_t)v.n_pairs * (N_CELLS + 1));
-  UPC(v.cell_fill, int, nullptr, (size_t)v.n_pairs * N_CELLS);
-  UPC(v.kp_cell, int, nullptr, v.n_cur);
-  UPC(v.s_rec, uint4, nullptr, 3 * (size_t)v.n_cur);
-  UPC(v.owner, int, nullptr, v.n_cur);
-  UPC(v.q_best, int, nullptr, v.n_q);
-  UPC(v.q_dist, int, nullptr, v.n_q);
-  UPC(v.changed, int, nullptr, 1);
-  UPC(v.q_pair, int, nullptr, v.n_q);
-  UPC(v.pair_mode, int, nullptr, v.n_pairs);
-  UPC(v.q_top, unsigned long long, nullptr, 4 * (size_t)v.n_q);
-  UPC(v.q_ncand, int, nullptr, v.n_q);
-  UPC(v.match, int, nullptr, v.n_cur);
-  UPC(v.n_matches, int, nullptr, v.n_pairs);
+  LLD_DEV(c, v.cell_count, (size_t)v.n_pairs * (N_CELLS + 1));
+  LLD_DEV(c, v.cell_fill, (size_t)v.n_pairs * N_CELLS);
+  LLD_DEV(c, v.kp_cell, v.n_cur);
+  LLD_DEV(c, v.s_rec, 3 * (size_t)v.n_cur);
+  LLD_DEV(c, v.owner, v.n_cur);
+  LLD_DEV(c, v.q_best, v.n_q);
+  LLD_DEV(c, v.q_dist, v.n_q);
+  LLD_DEV(c, v.changed, 1);
+  LLD_DEV(c, v.q_pair, v.n_q);
+  LLD_DEV(c, v.pair_mode, v.n_pairs);
+  LLD_DEV(c, v.q_top, 4 * (size_t)v.n_q);
+  LLD_DEV(c, v.q_ncand, v.n_q);
+  LLD_DEV(c, v.match, v.n_cur);
+  LLD_DEV(c, v.n_matches, v.n_pairs);
   LLD_CUDA(c, cudaMemsetAsync(v.changed, 0, sizeof(int), c->stream));
   return LLD_OK;
 }
@@ -1269,16 +1243,12 @@ static void set_geom(MatchView& v, const lld_frame_geom& g) {
 static int match_download(LldCtx* c, MatchView& v, lld_sbp_result* out) {
   LLD_CUDA(c, cudaEventRecord(c->ev[2], c->stream));
   int* h_flag = reinterpret_cast<int*>(c->pinned);
-  LLD_CUDA(c, cudaMemcpyAsync(h_flag, v.changed, sizeof(int), cudaMemcpyDeviceToHost, c->stream));
-  if (out->match && v.n_cur) LLD_CUDA(c, cudaMemcpyAsync(out->match, v.match, sizeof(int) * (size_t)v.n_cur, cudaMemcpyDeviceToHost, c->stream));
-  if (out->n_matches) LLD_CUDA(c, cudaMemcpyAsync(out->n_matches, v.n_matches, sizeof(int) * (size_t)v.n_pairs, cudaMemcpyDeviceToHost, c->stream));
-  if (out->best_idx && v.n_q) LLD_CUDA(c, cudaMemcpyAsync(out->best_idx, v.q_best, sizeof(int) * (size_t)v.n_q, cudaMemcpyDeviceToHost, c->stream));
-  if (out->best_dist && v.n_q) LLD_CUDA(c, cudaMemcpyAsync(out->best_dist, v.q_dist, sizeof(int) * (size_t)v.n_q, cudaMemcpyDeviceToHost, c->stream));
-  LLD_CUDA(c, cudaEventRecord(c->ev[3], c->stream));
-  LLD_CUDA(c, cudaStreamSynchronize(c->stream));
-  cudaEventElapsedTime(&c->ms_h2d, c->ev[0], c->ev[1]);
-  cudaEventElapsedTime(&c->ms_compute, c->ev[1], c->ev[2]);
-  cudaEventElapsedTime(&c->ms_d2h, c->ev[2], c->ev[3]);
+  LLD_DOWN(c, h_flag, v.changed, 1);
+  LLD_DOWN(c, out->match, v.match, v.n_cur);
+  LLD_DOWN(c, out->n_matches, v.n_matches, v.n_pairs);
+  LLD_DOWN(c, out->best_idx, v.q_best, v.n_q);
+  LLD_DOWN(c, out->best_dist, v.q_dist, v.n_q);
+  if (int r = lld_call_end(c)) return r;
   if (*h_flag & 2) {
     snprintf(c->err, sizeof(c->err), "claim resolution did not converge in 64 passes");
     return LLD_ERR_CUDA;
@@ -1302,7 +1272,6 @@ static bool resident_valid(LldCtx* c) {
 }
 
 static int sbp_frame_upload(LldCtx* c, const lld_sbp_frame_problem* p, MatchView& v) {
-  c->pool_reset();
   v = MatchView();
   v.n_pairs = p->n_pairs;
   LLD_ARG(c, p->n_pairs >= 1);
@@ -1315,28 +1284,27 @@ static int sbp_frame_upload(LldCtx* c, const lld_sbp_frame_problem* p, MatchView
   set_geom(v, p->geom);
   v.th = p->th; v.nn_ratio = 0; v.mono = p->mono; v.check_ori = p->check_orientation;
   v.th_high = p->th_high > 0 ? p->th_high : TH_HIGH; v.allow_neg_z = p->allow_negative_depth != 0;
-  UPC(v.scale, float, p->geom.scale_factors, p->geom.n_levels);
-  UPC(v.cur_off, int, p->cur_off, p->n_pairs + 1);
-  UPC(v.cur_xy, float, p->cur_xy, 2 * (size_t)v.n_cur);
-  UPC(v.cur_octave, uint8_t, p->cur_octave, v.n_cur);
-  UPC(v.cur_angle, float, p->cur_angle, v.n_cur);
-  UPC(v.cur_uright, float, p->cur_uright, v.n_cur);
-  UPC(v.cur_desc, uint8_t, p->cur_desc, 32 * (size_t)v.n_cur);
-  UPC(v.cur_claimed, uint8_t, p->cur_claimed, v.n_cur);
-  UPC(v.cur_Tcw, float, p->cur_Tcw, 12 * (size_t)p->n_pairs);
-  UPC(v.last_Tcw, float, p->last_Tcw, 12 * (size_t)p->n_pairs);
-  UPC(v.q_off, int, p->last_off, p->n_pairs + 1);
-  UPC(v.q_valid, uint8_t, p->last_valid, v.n_q);
-  UPC(v.q_xw, float, p->last_xw, 3 * (size_t)v.n_q);
-  UPC(v.q_octave, uint8_t, p->last_octave, v.n_q);
-  UPC(v.q_angle, float, p->last_angle, v.n_q);
-  UPC(v.q_desc, uint8_t, p->last_desc, 32 * (size_t)v.n_q);
-  UPC(v.q_has_obs, uint8_t, p->last_has_obs, v.n_q);
+  LLD_UP(c, v.scale, p->geom.scale_factors, p->geom.n_levels);
+  LLD_UP(c, v.cur_off, p->cur_off, p->n_pairs + 1);
+  LLD_UP(c, v.cur_xy, p->cur_xy, 2 * (size_t)v.n_cur);
+  LLD_UP(c, v.cur_octave, p->cur_octave, v.n_cur);
+  LLD_UP(c, v.cur_angle, p->cur_angle, v.n_cur);
+  LLD_UP(c, v.cur_uright, p->cur_uright, v.n_cur);
+  LLD_UP(c, v.cur_desc, p->cur_desc, 32 * (size_t)v.n_cur);
+  LLD_UP(c, v.cur_claimed, p->cur_claimed, v.n_cur);
+  LLD_UP(c, v.cur_Tcw, p->cur_Tcw, 12 * (size_t)p->n_pairs);
+  LLD_UP(c, v.last_Tcw, p->last_Tcw, 12 * (size_t)p->n_pairs);
+  LLD_UP(c, v.q_off, p->last_off, p->n_pairs + 1);
+  LLD_UP(c, v.q_valid, p->last_valid, v.n_q);
+  LLD_UP(c, v.q_xw, p->last_xw, 3 * (size_t)v.n_q);
+  LLD_UP(c, v.q_octave, p->last_octave, v.n_q);
+  LLD_UP(c, v.q_angle, p->last_angle, v.n_q);
+  LLD_UP(c, v.q_desc, p->last_desc, 32 * (size_t)v.n_q);
+  LLD_UP(c, v.q_has_obs, p->last_has_obs, v.n_q);
   return match_alloc_common(c, v);
 }
 
 static int sbp_mp_upload(LldCtx* c, const lld_sbp_mp_problem* p, MatchView& v) {
-  c->pool_reset();
   v = MatchView();
   v.n_pairs = p->n_pairs;
   LLD_ARG(c, p->n_pairs >= 1);
@@ -1349,27 +1317,26 @@ static int sbp_mp_upload(LldCtx* c, const lld_sbp_mp_problem* p, MatchView& v) {
   set_geom(v, p->geom);
   v.th = p->th; v.nn_ratio = p->nn_ratio; v.mono = 0; v.check_ori = 0;
   v.th_high = TH_HIGH; v.allow_neg_z = 0;
-  UPC(v.scale, float, p->geom.scale_factors, p->geom.n_levels);
-  UPC(v.cur_off, int, p->cur_off, p->n_pairs + 1);
-  UPC(v.cur_xy, float, p->cur_xy, 2 * (size_t)v.n_cur);
-  UPC(v.cur_octave, uint8_t, p->cur_octave, v.n_cur);
-  UPC(v.cur_uright, float, p->cur_uright, v.n_cur);
-  UPC(v.cur_desc, uint8_t, p->cur_desc, 32 * (size_t)v.n_cur);
-  UPC(v.cur_claimed, uint8_t, p->cur_claimed, v.n_cur);
+  LLD_UP(c, v.scale, p->geom.scale_factors, p->geom.n_levels);
+  LLD_UP(c, v.cur_off, p->cur_off, p->n_pairs + 1);
+  LLD_UP(c, v.cur_xy, p->cur_xy, 2 * (size_t)v.n_cur);
+  LLD_UP(c, v.cur_octave, p->cur_octave, v.n_cur);
+  LLD_UP(c, v.cur_uright, p->cur_uright, v.n_cur);
+  LLD_UP(c, v.cur_desc, p->cur_desc, 32 * (size_t)v.n_cur);
+  LLD_UP(c, v.cur_claimed, p->cur_claimed, v.n_cur);
   v.cur_angle = nullptr;
-  UPC(v.q_off, int, p->mp_off, p->n_pairs + 1);
-  UPC(v.q_valid, uint8_t, p->mp_valid, v.n_q);
-  UPC(v.q_xw, float, p->mp_proj, 3 * (size_t)v.n_q);
-  UPC(v.q_level, int, p->mp_level, v.n_q);
-  UPC(v.q_viewcos, float, p->mp_viewcos, v.n_q);
-  UPC(v.q_desc, uint8_t, p->mp_desc, 32 * (size_t)v.n_q);
-  UPC(v.q_has_obs, uint8_t, p->mp_has_obs, v.n_q);
+  LLD_UP(c, v.q_off, p->mp_off, p->n_pairs + 1);
+  LLD_UP(c, v.q_valid, p->mp_valid, v.n_q);
+  LLD_UP(c, v.q_xw, p->mp_proj, 3 * (size_t)v.n_q);
+  LLD_UP(c, v.q_level, p->mp_level, v.n_q);
+  LLD_UP(c, v.q_viewcos, p->mp_viewcos, v.n_q);
+  LLD_UP(c, v.q_desc, p->mp_desc, 32 * (size_t)v.n_q);
+  LLD_UP(c, v.q_has_obs, p->mp_has_obs, v.n_q);
   return match_alloc_common(c, v);
 }
 
 // keyframe searches (Fuse, Fuse with Sim3, SearchByProjection with Sim3): variant 2
 static int kf_search_upload(LldCtx* c, const lld_kf_search_problem* p, MatchView& v) {
-  c->pool_reset();
   v = MatchView();
   v.n_pairs = p->n_pairs;
   LLD_ARG(c, p->n_pairs >= 1);
@@ -1384,23 +1351,23 @@ static int kf_search_upload(LldCtx* c, const lld_kf_search_problem* p, MatchView
   v.th_high = p->th_low; v.allow_neg_z = 0;
   v.chi2_gate = p->chi2_gate != 0;
   for (int i = 0; i < 8; i++) v.inv_sigma2[i] = p->inv_level_sigma2[i];
-  UPC(v.scale, float, p->geom.scale_factors, p->geom.n_levels);
-  UPC(v.cur_off, int, p->kp_off, p->n_pairs + 1);
-  UPC(v.cur_xy, float, p->kp_xy, 2 * (size_t)v.n_cur);
-  UPC(v.cur_octave, uint8_t, p->kp_octave, v.n_cur);
-  UPC(v.cur_uright, float, p->kp_uright, v.n_cur);
-  UPC(v.cur_desc, uint8_t, p->kp_desc, 32 * (size_t)v.n_cur);
-  UPC(v.cur_claimed, uint8_t, p->kp_claimed, v.n_cur);
+  LLD_UP(c, v.scale, p->geom.scale_factors, p->geom.n_levels);
+  LLD_UP(c, v.cur_off, p->kp_off, p->n_pairs + 1);
+  LLD_UP(c, v.cur_xy, p->kp_xy, 2 * (size_t)v.n_cur);
+  LLD_UP(c, v.cur_octave, p->kp_octave, v.n_cur);
+  LLD_UP(c, v.cur_uright, p->kp_uright, v.n_cur);
+  LLD_UP(c, v.cur_desc, p->kp_desc, 32 * (size_t)v.n_cur);
+  LLD_UP(c, v.cur_claimed, p->kp_claimed, v.n_cur);
   v.cur_angle = nullptr;
-  UPC(v.q_off, int, p->mp_off, p->n_pairs + 1);
-  UPC(v.q_valid, uint8_t, p->mp_valid, v.n_q);
-  UPC(v.q_xw, float, p->mp_proj, 3 * (size_t)v.n_q);
-  UPC(v.q_level, int, p->mp_level, v.n_q);
+  LLD_UP(c, v.q_off, p->mp_off, p->n_pairs + 1);
+  LLD_UP(c, v.q_valid, p->mp_valid, v.n_q);
+  LLD_UP(c, v.q_xw, p->mp_proj, 3 * (size_t)v.n_q);
+  LLD_UP(c, v.q_level, p->mp_level, v.n_q);
   v.q_viewcos = nullptr;
-  UPC(v.q_desc, uint8_t, p->mp_desc, 32 * (size_t)v.n_q);
+  LLD_UP(c, v.q_desc, p->mp_desc, 32 * (size_t)v.n_q);
   // every accepted point claims its keypoint (vpMatched[bestIdx] = pMP) or none does (Fuse)
   uint8_t* has = nullptr;
-  UPC(has, uint8_t, nullptr, v.n_q);
+  LLD_DEV(c, has, v.n_q);
   LLD_CUDA(c, cudaMemsetAsync(has, p->sequential_claims ? 1 : 0, v.n_q ? v.n_q : 1, c->stream));
   v.q_has_obs = has;
   return match_alloc_common(c, v);
@@ -1409,10 +1376,8 @@ static int kf_search_upload(LldCtx* c, const lld_kf_search_problem* p, MatchView
 extern "C" int lld_kf_search(void* ctx, const lld_kf_search_problem* p, lld_sbp_result* out) {
   LldCtx* c = lld_ctx_cast(ctx);
   if (!c || !p || !out) return LLD_ERR_ARG;
-  LLD_CUDA(c, cudaSetDevice(c->device));
-  c->launches = 0;
+  if (int r = lld_call_begin(c, true)) return r;
   MatchView v;
-  LLD_CUDA(c, cudaEventRecord(c->ev[0], c->stream));
   int r = kf_search_upload(c, p, v);
   if (r) return r;
   LLD_CUDA(c, cudaEventRecord(c->ev[1], c->stream));
@@ -1448,32 +1413,29 @@ extern "C" int lld_init_search(void* ctx, const lld_init_search_problem* p, lld_
     for (int i = 0; i < n1; i++) LLD_ARG(c, p->kp1_angle[i] >= 0.f && p->kp1_angle[i] < 900.f);
     for (int i = 0; i < n2; i++) LLD_ARG(c, p->kp2_angle[i] >= 0.f && p->kp2_angle[i] < 360.f);
   }
-  LLD_CUDA(c, cudaSetDevice(c->device));
-  c->launches = 0;
-  c->pool_reset();
-  LLD_CUDA(c, cudaEventRecord(c->ev[0], c->stream));
+  if (int r = lld_call_begin(c, true)) return r;
   MatchView v{};
   v.n_pairs = P;
   v.n_cur = n2;
   set_geom(v, p->geom);
-  UPC(v.cur_off, int, p->kp2_off, P + 1);
-  UPC(v.cur_xy, float, p->kp2_xy, 2 * (size_t)n2);
-  UPC(v.cur_octave, uint8_t, p->kp2_octave, n2);
-  UPC(v.cur_desc, uint8_t, p->kp2_desc, 32 * (size_t)n2);
+  LLD_UP(c, v.cur_off, p->kp2_off, P + 1);
+  LLD_UP(c, v.cur_xy, p->kp2_xy, 2 * (size_t)n2);
+  LLD_UP(c, v.cur_octave, p->kp2_octave, n2);
+  LLD_UP(c, v.cur_desc, p->kp2_desc, 32 * (size_t)n2);
   float* uright = nullptr;   // the grid record's stereo and claim fields are not used by this search
   uint8_t* claimed = nullptr;
-  UPC(uright, float, nullptr, n2);
-  UPC(claimed, uint8_t, nullptr, n2);
+  LLD_DEV(c, uright, n2);
+  LLD_DEV(c, claimed, n2);
   LLD_CUDA(c, cudaMemsetAsync(uright, 0, sizeof(float) * (size_t)std::max(n2, 1), c->stream));
   LLD_CUDA(c, cudaMemsetAsync(claimed, 0, (size_t)std::max(n2, 1), c->stream));
   v.cur_uright = uright;
   v.cur_claimed = claimed;
-  UPC(v.cell_count, int, nullptr, (size_t)P * (N_CELLS + 1));
-  UPC(v.cell_fill, int, nullptr, (size_t)P * N_CELLS);
-  UPC(v.kp_cell, int, nullptr, n2);
-  UPC(v.s_rec, uint4, nullptr, 3 * (size_t)n2);
-  UPC(v.owner, int, nullptr, n2);
-  UPC(v.match, int, nullptr, n2);
+  LLD_DEV(c, v.cell_count, (size_t)P * (N_CELLS + 1));
+  LLD_DEV(c, v.cell_fill, (size_t)P * N_CELLS);
+  LLD_DEV(c, v.kp_cell, n2);
+  LLD_DEV(c, v.s_rec, 3 * (size_t)n2);
+  LLD_DEV(c, v.owner, n2);
+  LLD_DEV(c, v.match, n2);
   InitView w{};
   w.n_pairs = P;
   w.n1 = n1;
@@ -1481,19 +1443,19 @@ extern "C" int lld_init_search(void* ctx, const lld_init_search_problem* p, lld_
   w.nn_ratio = p->nn_ratio;
   w.keep_max = init_keep_max(p->nn_ratio);
   w.check_ori = p->check_orientation != 0;
-  UPC(w.kp1_off, int, p->kp1_off, P + 1);
-  UPC(w.kp1_octave, uint8_t, p->kp1_octave, n1);
-  UPC(w.kp1_angle, float, p->kp1_angle, n1);
-  UPC(w.kp1_desc, uint8_t, p->kp1_desc, 32 * (size_t)n1);
-  UPC(w.prev, float, p->prev_matched, 2 * (size_t)n1);
-  UPC(w.kp2_angle, float, p->kp2_angle, n2);
-  UPC(w.cnt, int, nullptr, n1);
-  UPC(w.pair_total, int, nullptr, P);
-  UPC(w.m12, int, nullptr, n1);
-  UPC(w.b2, int, nullptr, n1);
-  UPC(w.n_matches, int, nullptr, P);
+  LLD_UP(c, w.kp1_off, p->kp1_off, P + 1);
+  LLD_UP(c, w.kp1_octave, p->kp1_octave, n1);
+  LLD_UP(c, w.kp1_angle, p->kp1_angle, n1);
+  LLD_UP(c, w.kp1_desc, p->kp1_desc, 32 * (size_t)n1);
+  LLD_UP(c, w.prev, p->prev_matched, 2 * (size_t)n1);
+  LLD_UP(c, w.kp2_angle, p->kp2_angle, n2);
+  LLD_DEV(c, w.cnt, n1);
+  LLD_DEV(c, w.pair_total, P);
+  LLD_DEV(c, w.m12, n1);
+  LLD_DEV(c, w.b2, n1);
+  LLD_DEV(c, w.n_matches, P);
   int* pair_base = nullptr;
-  UPC(pair_base, int, nullptr, P);
+  LLD_DEV(c, pair_base, P);
   w.pair_base = pair_base;
   LLD_CUDA(c, cudaEventRecord(c->ev[1], c->stream));
 
@@ -1505,7 +1467,7 @@ extern "C" int lld_init_search(void* ctx, const lld_init_search_problem* p, lld_
   LLD_LAUNCH(c, k_init_scan, P, 1024, 0, w);
   // the candidate buffer is sized from the counts: one read-back of the pair totals
   std::vector<int> total((size_t)P), base((size_t)P);
-  LLD_CUDA(c, cudaMemcpyAsync(total.data(), w.pair_total, sizeof(int) * (size_t)P, cudaMemcpyDeviceToHost, c->stream));
+  LLD_DOWN(c, total.data(), w.pair_total, P);
   LLD_CUDA(c, cudaStreamSynchronize(c->stream));
   long long sum = 0;
   for (int i = 0; i < P; i++) {
@@ -1517,7 +1479,7 @@ extern "C" int lld_init_search(void* ctx, const lld_init_search_problem* p, lld_
     }
   }
   LLD_CUDA(c, cudaMemcpyAsync(pair_base, base.data(), sizeof(int) * (size_t)P, cudaMemcpyHostToDevice, c->stream));
-  UPC(w.keys, unsigned long long, nullptr, (size_t)sum);
+  LLD_DEV(c, w.keys, (size_t)sum);
   if (n1) LLD_LAUNCH(c, k_init_fill, cdiv(n1, 128), 128, 0, v, w);
   if (max2 <= INIT_SMEM_MAX_KP) {
     const int smem = 4 * std::max(max2, 1);
@@ -1529,26 +1491,17 @@ extern "C" int lld_init_search(void* ctx, const lld_init_search_problem* p, lld_
   LLD_LAUNCH(c, k_init_finalize, P, 256, 0, v, w);
   LLD_CUDA(c, cudaGetLastError());
   LLD_CUDA(c, cudaEventRecord(c->ev[2], c->stream));
-  if (n1) {
-    LLD_CUDA(c, cudaMemcpyAsync(out->match12, w.m12, sizeof(int) * (size_t)n1, cudaMemcpyDeviceToHost, c->stream));
-    LLD_CUDA(c, cudaMemcpyAsync(out->prev_matched, w.prev, 2 * sizeof(float) * (size_t)n1, cudaMemcpyDeviceToHost, c->stream));
-  }
-  LLD_CUDA(c, cudaMemcpyAsync(out->n_matches, w.n_matches, sizeof(int) * (size_t)P, cudaMemcpyDeviceToHost, c->stream));
-  LLD_CUDA(c, cudaEventRecord(c->ev[3], c->stream));
-  LLD_CUDA(c, cudaStreamSynchronize(c->stream));
-  cudaEventElapsedTime(&c->ms_h2d, c->ev[0], c->ev[1]);
-  cudaEventElapsedTime(&c->ms_compute, c->ev[1], c->ev[2]);
-  cudaEventElapsedTime(&c->ms_d2h, c->ev[2], c->ev[3]);
-  return LLD_OK;
+  LLD_DOWN(c, out->match12, w.m12, n1);
+  LLD_DOWN(c, out->prev_matched, w.prev, 2 * (size_t)n1);
+  LLD_DOWN(c, out->n_matches, w.n_matches, P);
+  return lld_call_end(c);
 }
 
 extern "C" int lld_sbp_frame(void* ctx, const lld_sbp_frame_problem* p, lld_sbp_result* out) {
   LldCtx* c = lld_ctx_cast(ctx);
   if (!c || !p || !out) return LLD_ERR_ARG;
-  LLD_CUDA(c, cudaSetDevice(c->device));
-  c->launches = 0;
+  if (int r = lld_call_begin(c, true)) return r;
   MatchView v;
-  LLD_CUDA(c, cudaEventRecord(c->ev[0], c->stream));
   int r = sbp_frame_upload(c, p, v);
   if (r) return r;
   LLD_CUDA(c, cudaEventRecord(c->ev[1], c->stream));
@@ -1560,10 +1513,8 @@ extern "C" int lld_sbp_frame(void* ctx, const lld_sbp_frame_problem* p, lld_sbp_
 extern "C" int lld_sbp_mappoints(void* ctx, const lld_sbp_mp_problem* p, lld_sbp_result* out) {
   LldCtx* c = lld_ctx_cast(ctx);
   if (!c || !p || !out) return LLD_ERR_ARG;
-  LLD_CUDA(c, cudaSetDevice(c->device));
-  c->launches = 0;
+  if (int r = lld_call_begin(c, true)) return r;
   MatchView v;
-  LLD_CUDA(c, cudaEventRecord(c->ev[0], c->stream));
   int r = sbp_mp_upload(c, p, v);
   if (r) return r;
   LLD_CUDA(c, cudaEventRecord(c->ev[1], c->stream));
@@ -1576,7 +1527,7 @@ extern "C" int lld_sbp_mappoints(void* ctx, const lld_sbp_mp_problem* p, lld_sbp
 extern "C" int lld_sbp_frame_upload(void* ctx, const lld_sbp_frame_problem* p) {
   LldCtx* c = lld_ctx_cast(ctx);
   if (!c || !p) return LLD_ERR_ARG;
-  LLD_CUDA(c, cudaSetDevice(c->device));
+  if (int r = lld_call_begin(c, false)) return r;
   int r = sbp_frame_upload(c, p, *resident_view(c, true));
   c->resident_gen[0] = r ? 0 : c->pool_gen;
   if (r) return r;

@@ -124,38 +124,27 @@ __global__ void __launch_bounds__(256) k_medoid_float(int n_lm, const int* __res
 
 static int medoid_common(LldCtx* c, int n_lm, const int32_t* off, const void* desc, size_t row_bytes, int D, int32_t* best) {
   LLD_ARG(c, n_lm >= 1 && off && best);
-  LLD_CUDA(c, cudaSetDevice(c->device));
-  c->launches = 0;
-  c->pool_reset();
+  if (int r = lld_call_begin(c, true)) return r;
   const int n = off[n_lm];
   for (int l = 0; l < n_lm; l++)
     if (off[l + 1] - off[l] > 32 * MD_MAXC) {
       snprintf(c->err, sizeof(c->err), "medoid descriptor: a landmark has %d observations, at most %d are supported", off[l + 1] - off[l], 32 * MD_MAXC);
       return LLD_ERR_UNSUPPORTED;
     }
-  cudaError_t e = cudaSuccess;
-  int* d_off = c->alloc<int>((size_t)n_lm + 1, &e);
-  LLD_CUDA(c, e);
-  uint8_t* d_desc = c->alloc<uint8_t>(row_bytes * (size_t)std::max(n, 1), &e);
-  LLD_CUDA(c, e);
-  int* d_best = c->alloc<int>((size_t)n_lm, &e);
-  LLD_CUDA(c, e);
-  LLD_CUDA(c, cudaEventRecord(c->ev[0], c->stream));
-  LLD_CUDA(c, cudaMemcpyAsync(d_off, off, 4 * ((size_t)n_lm + 1), cudaMemcpyHostToDevice, c->stream));
-  if (n) LLD_CUDA(c, cudaMemcpyAsync(d_desc, desc, row_bytes * (size_t)n, cudaMemcpyHostToDevice, c->stream));
+  const int* d_off;
+  const uint8_t* d_desc;
+  int* d_best;
+  LLD_UP(c, d_off, off, n_lm + 1);
+  LLD_UP(c, d_desc, static_cast<const uint8_t*>(desc), row_bytes * (size_t)n);
+  LLD_DEV(c, d_best, n_lm);
   LLD_CUDA(c, cudaEventRecord(c->ev[1], c->stream));
   const int grid = (n_lm + 7) / 8;
   if (D == 0) LLD_LAUNCH(c, k_medoid_orb, grid, 256, 0, n_lm, d_off, d_desc, d_best);
   else LLD_LAUNCH(c, k_medoid_float, grid, 256, 0, n_lm, d_off, D, reinterpret_cast<const float*>(d_desc), d_best);
   LLD_CUDA(c, cudaGetLastError());
   LLD_CUDA(c, cudaEventRecord(c->ev[2], c->stream));
-  LLD_CUDA(c, cudaMemcpyAsync(best, d_best, 4 * (size_t)n_lm, cudaMemcpyDeviceToHost, c->stream));
-  LLD_CUDA(c, cudaEventRecord(c->ev[3], c->stream));
-  LLD_CUDA(c, cudaStreamSynchronize(c->stream));
-  cudaEventElapsedTime(&c->ms_h2d, c->ev[0], c->ev[1]);
-  cudaEventElapsedTime(&c->ms_compute, c->ev[1], c->ev[2]);
-  cudaEventElapsedTime(&c->ms_d2h, c->ev[2], c->ev[3]);
-  return LLD_OK;
+  LLD_DOWN(c, best, d_best, n_lm);
+  return lld_call_end(c);
 }
 
 extern "C" int lld_medoid_orb(void* ctx, int32_t n_lm, const int32_t* off, const uint8_t* desc, int32_t* best) {

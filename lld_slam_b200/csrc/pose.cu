@@ -427,32 +427,6 @@ __global__ void __launch_bounds__(PTPB) k_pose_opt(PoseView v, int stage_smem) {
   }
 }
 
-template <typename T>
-int upl(LldCtx* c, T** dst, const T* src, size_t n) {
-  cudaError_t e = cudaSuccess;
-  T* d = c->alloc<T>(n ? n : 1, &e);
-  if (e != cudaSuccess) {
-    snprintf(c->err, sizeof(c->err), "cudaMalloc: %s", cudaGetErrorString(e));
-    return LLD_ERR_CUDA;
-  }
-  if (n && src) {
-    e = cudaMemcpyAsync(d, src, n * sizeof(T), cudaMemcpyHostToDevice, c->stream);
-    if (e != cudaSuccess) {
-      snprintf(c->err, sizeof(c->err), "cudaMemcpyAsync H2D: %s", cudaGetErrorString(e));
-      return LLD_ERR_CUDA;
-    }
-  }
-  *dst = d;
-  return LLD_OK;
-}
-#define UPP(dst, T, src, n)                                \
-  do {                                                     \
-    T* _p = nullptr;                                       \
-    int _r = upl<T>(c, &_p, (const T*)(src), (size_t)(n)); \
-    if (_r) return _r;                                     \
-    (dst) = _p;                                            \
-  } while (0)
-
 // resident-mode view (bench), owned by the context; invalid once another entry point of the context recycles the device pool
 struct PoseResident { PoseView v; size_t smem = 0; };
 PoseResident* pose_resident(LldCtx* c, bool create) {
@@ -469,40 +443,39 @@ bool pose_resident_valid(LldCtx* c) {
 }
 
 int pose_upload(LldCtx* c, const lld_pose_problem* p, PoseView& v, size_t* smem_out) {
-  c->pool_reset();
   v = PoseView();
   const int F = p->n_frames;
   LLD_ARG(c, F >= 1);
   const int np = p->pt_off[F], nl = p->ln_off[F];
   v.n_frames = F;
-  UPP(v.Tcw, double, p->Tcw, 12 * (size_t)F);
-  UPP(v.intr, double, p->intr, 5 * (size_t)F);
-  UPP(v.line_cam, double, p->line_cam, 4 * (size_t)F);
-  UPP(v.pt_off, int, p->pt_off, F + 1);
-  UPP(v.pt_xw, float, p->pt_xw, 3 * (size_t)np);
-  UPP(v.pt_uvr, float, p->pt_uvr, 3 * (size_t)np);
-  UPP(v.pt_info, float, p->pt_info, np);
-  UPP(v.ln_off, int, p->ln_off, F + 1);
-  UPP(v.ln_x0_dir, double, p->ln_x0_dir, 6 * (size_t)nl);
-  UPP(v.ln_left, float, p->ln_left, 4 * (size_t)nl);
-  UPP(v.ln_right, float, p->ln_right, 4 * (size_t)nl);
-  UPP(v.ln_info, double, p->ln_info, 2 * (size_t)nl);
-  UPP(v.ln_stereo, uint8_t, p->ln_stereo, nl);
-  UPP(v.ln_gate_stereo, uint8_t, p->ln_gate_stereo, 2 * (size_t)nl);
+  LLD_UP(c, v.Tcw, p->Tcw, 12 * (size_t)F);
+  LLD_UP(c, v.intr, p->intr, 5 * (size_t)F);
+  LLD_UP(c, v.line_cam, p->line_cam, 4 * (size_t)F);
+  LLD_UP(c, v.pt_off, p->pt_off, F + 1);
+  LLD_UP(c, v.pt_xw, p->pt_xw, 3 * (size_t)np);
+  LLD_UP(c, v.pt_uvr, p->pt_uvr, 3 * (size_t)np);
+  LLD_UP(c, v.pt_info, p->pt_info, np);
+  LLD_UP(c, v.ln_off, p->ln_off, F + 1);
+  LLD_UP(c, v.ln_x0_dir, p->ln_x0_dir, 6 * (size_t)nl);
+  LLD_UP(c, v.ln_left, p->ln_left, 4 * (size_t)nl);
+  LLD_UP(c, v.ln_right, p->ln_right, 4 * (size_t)nl);
+  LLD_UP(c, v.ln_info, p->ln_info, 2 * (size_t)nl);
+  LLD_UP(c, v.ln_stereo, p->ln_stereo, nl);
+  LLD_UP(c, v.ln_gate_stereo, p->ln_gate_stereo, 2 * (size_t)nl);
   v.delta_mono = p->delta_mono; v.delta_stereo = p->delta_stereo;
   v.delta_ln_mono = p->delta_ln_mono; v.delta_ln_stereo = p->delta_ln_stereo;
   v.chi2_mono = p->chi2_mono; v.chi2_stereo = p->chi2_stereo;
   v.gate_ln_mono = p->gate_ln_mono; v.gate_ln_stereo = p->gate_ln_stereo;
   v.n_rounds = p->n_rounds; v.its = p->its;
-  UPP(v.pt_chi2, double, nullptr, np);
-  UPP(v.ln_chi2, double, nullptr, 2 * (size_t)nl);
-  UPP(v.pt_level, uint8_t, nullptr, np);
-  UPP(v.ln_level, uint8_t, nullptr, 2 * (size_t)nl);
-  UPP(v.out_Tcw, double, nullptr, 12 * (size_t)F);
-  UPP(v.pt_outlier, uint8_t, nullptr, np);
-  UPP(v.ln_outlier, uint8_t, nullptr, nl);
-  UPP(v.n_inliers, int, nullptr, F);
-  UPP(v.chi2_final, double, nullptr, F);
+  LLD_DEV(c, v.pt_chi2, np);
+  LLD_DEV(c, v.ln_chi2, 2 * (size_t)nl);
+  LLD_DEV(c, v.pt_level, np);
+  LLD_DEV(c, v.ln_level, 2 * (size_t)nl);
+  LLD_DEV(c, v.out_Tcw, 12 * (size_t)F);
+  LLD_DEV(c, v.pt_outlier, np);
+  LLD_DEV(c, v.ln_outlier, nl);
+  LLD_DEV(c, v.n_inliers, F);
+  LLD_DEV(c, v.chi2_final, F);
   // shared-memory staging size = largest frame
   size_t mx = 0;
   for (int f = 0; f < F; f++) {
@@ -528,18 +501,12 @@ int pose_download(LldCtx* c, PoseView& v, const lld_pose_problem* p, lld_pose_re
   const int F = v.n_frames;
   const int np = p->pt_off[F], nl = p->ln_off[F];
   LLD_CUDA(c, cudaEventRecord(c->ev[2], c->stream));
-  LLD_CUDA(c, cudaMemcpyAsync(out->Tcw, v.out_Tcw, sizeof(double) * 12 * (size_t)F, cudaMemcpyDeviceToHost, c->stream));
-  if (np) LLD_CUDA(c, cudaMemcpyAsync(out->pt_outlier, v.pt_outlier, (size_t)np, cudaMemcpyDeviceToHost, c->stream));
-  if (nl) LLD_CUDA(c, cudaMemcpyAsync(out->ln_outlier, v.ln_outlier, (size_t)nl, cudaMemcpyDeviceToHost, c->stream));
-  LLD_CUDA(c, cudaMemcpyAsync(out->n_inliers, v.n_inliers, sizeof(int) * (size_t)F, cudaMemcpyDeviceToHost, c->stream));
-  if (out->chi2_final)
-    LLD_CUDA(c, cudaMemcpyAsync(out->chi2_final, v.chi2_final, sizeof(double) * (size_t)F, cudaMemcpyDeviceToHost, c->stream));
-  LLD_CUDA(c, cudaEventRecord(c->ev[3], c->stream));
-  LLD_CUDA(c, cudaStreamSynchronize(c->stream));
-  cudaEventElapsedTime(&c->ms_h2d, c->ev[0], c->ev[1]);
-  cudaEventElapsedTime(&c->ms_compute, c->ev[1], c->ev[2]);
-  cudaEventElapsedTime(&c->ms_d2h, c->ev[2], c->ev[3]);
-  return LLD_OK;
+  LLD_DOWN(c, out->Tcw, v.out_Tcw, 12 * (size_t)F);
+  LLD_DOWN(c, out->pt_outlier, v.pt_outlier, (size_t)np);
+  LLD_DOWN(c, out->ln_outlier, v.ln_outlier, (size_t)nl);
+  LLD_DOWN(c, out->n_inliers, v.n_inliers, (size_t)F);
+  LLD_DOWN(c, out->chi2_final, v.chi2_final, (size_t)F);
+  return lld_call_end(c);
 }
 
 }  // namespace
@@ -547,11 +514,9 @@ int pose_download(LldCtx* c, PoseView& v, const lld_pose_problem* p, lld_pose_re
 extern "C" int lld_pose_opt(void* ctx, const lld_pose_problem* p, lld_pose_result* out) {
   LldCtx* c = lld_ctx_cast(ctx);
   if (!c || !p || !out) return LLD_ERR_ARG;
-  LLD_CUDA(c, cudaSetDevice(c->device));
-  c->launches = 0;
+  if (int r = lld_call_begin(c, true)) return r;
   PoseView v;
   size_t smem = 0;
-  LLD_CUDA(c, cudaEventRecord(c->ev[0], c->stream));
   int r = pose_upload(c, p, v, &smem);
   if (r) return r;
   LLD_CUDA(c, cudaEventRecord(c->ev[1], c->stream));
@@ -564,7 +529,7 @@ extern "C" int lld_pose_opt(void* ctx, const lld_pose_problem* p, lld_pose_resul
 extern "C" int lld_pose_upload(void* ctx, const lld_pose_problem* p) {
   LldCtx* c = lld_ctx_cast(ctx);
   if (!c || !p) return LLD_ERR_ARG;
-  LLD_CUDA(c, cudaSetDevice(c->device));
+  if (int r = lld_call_begin(c, false)) return r;
   PoseResident* R = pose_resident(c, true);
   int r = pose_upload(c, p, R->v, &R->smem);
   c->resident_gen[1] = r ? 0 : c->pool_gen;

@@ -354,39 +354,6 @@ __device__ void sim3_body(const Sim3View& v) {
 __global__ void __launch_bounds__(STPB) k_sim3_opt_smem(Sim3View v) { sim3_body<true>(v); }
 __global__ void __launch_bounds__(STPB) k_sim3_opt_global(Sim3View v) { sim3_body<false>(v); }
 
-template <typename T>
-int upl(LldCtx* c, T** dst, const T* src, size_t n) {
-  cudaError_t e = cudaSuccess;
-  T* d = c->alloc<T>(n ? n : 1, &e);
-  if (e != cudaSuccess) {
-    snprintf(c->err, sizeof(c->err), "cudaMalloc: %s", cudaGetErrorString(e));
-    return LLD_ERR_CUDA;
-  }
-  if (n && src) {
-    e = cudaMemcpyAsync(d, src, n * sizeof(T), cudaMemcpyHostToDevice, c->stream);
-    if (e != cudaSuccess) {
-      snprintf(c->err, sizeof(c->err), "cudaMemcpyAsync H2D: %s", cudaGetErrorString(e));
-      return LLD_ERR_CUDA;
-    }
-  }
-  *dst = d;
-  return LLD_OK;
-}
-#define UPS(dst, T, src, n)                                \
-  do {                                                     \
-    T* _p = nullptr;                                       \
-    int _r = upl<T>(c, &_p, (const T*)(src), (size_t)(n)); \
-    if (_r) return _r;                                     \
-    (dst) = _p;                                            \
-  } while (0)
-
-template <typename T>
-int down(LldCtx* c, T* dst, const T* src, size_t n) {
-  if (!n || !dst) return LLD_OK;
-  LLD_CUDA(c, cudaMemcpyAsync(dst, src, n * sizeof(T), cudaMemcpyDeviceToHost, c->stream));
-  return LLD_OK;
-}
-
 }  // namespace
 
 extern "C" int lld_sim3_opt(void* ctx, const lld_sim3_problem* p, lld_sim3_result* out) {
@@ -408,33 +375,30 @@ extern "C" int lld_sim3_opt(void* ctx, const lld_sim3_problem* p, lld_sim3_resul
   const int its2 = std::max(p->its_more_outliers, p->its_more_clean);
   LLD_ARG(c, !logs || out->log_stride >= p->its_first + its2 + 2);
   const int m = p->off[n];
-  LLD_CUDA(c, cudaSetDevice(c->device));
-  c->launches = 0;
-  c->pool_reset();
-  LLD_CUDA(c, cudaEventRecord(c->ev[0], c->stream));
+  if (int r = lld_call_begin(c, true)) return r;
   Sim3View v{};
   v.n = n;
-  UPS(v.S12, double, p->S12, 8 * (size_t)n);
-  UPS(v.cam, double, p->cam, 8 * (size_t)n);
-  UPS(v.fix_scale, int, p->fix_scale, n);
-  UPS(v.th2, float, p->th2, n);
-  UPS(v.off, int, p->off, n + 1);
-  UPS(v.p1c, float, p->p1c, 3 * (size_t)m);
-  UPS(v.p2c, float, p->p2c, 3 * (size_t)m);
-  UPS(v.obs1, float, p->obs1, 2 * (size_t)m);
-  UPS(v.obs2, float, p->obs2, 2 * (size_t)m);
-  UPS(v.info1, float, p->info1, m);
-  UPS(v.info2, float, p->info2, m);
+  LLD_UP(c, v.S12, p->S12, 8 * (size_t)n);
+  LLD_UP(c, v.cam, p->cam, 8 * (size_t)n);
+  LLD_UP(c, v.fix_scale, p->fix_scale, n);
+  LLD_UP(c, v.th2, p->th2, n);
+  LLD_UP(c, v.off, p->off, n + 1);
+  LLD_UP(c, v.p1c, p->p1c, 3 * (size_t)m);
+  LLD_UP(c, v.p2c, p->p2c, 3 * (size_t)m);
+  LLD_UP(c, v.obs1, p->obs1, 2 * (size_t)m);
+  LLD_UP(c, v.obs2, p->obs2, 2 * (size_t)m);
+  LLD_UP(c, v.info1, p->info1, m);
+  LLD_UP(c, v.info2, p->info2, m);
   v.its1 = p->its_first; v.its_bad = p->its_more_outliers; v.its_clean = p->its_more_clean;
-  UPS(v.chi2, double, nullptr, 2 * (size_t)m);
-  UPS(v.out_S12, double, nullptr, 8 * (size_t)n);
-  UPS(v.inlier, uint8_t, nullptr, m);
-  UPS(v.n_in, int, nullptr, n);
+  LLD_DEV(c, v.chi2, 2 * (size_t)m);
+  LLD_DEV(c, v.out_S12, 8 * (size_t)n);
+  LLD_DEV(c, v.inlier, m);
+  LLD_DEV(c, v.n_in, n);
   v.log_stride = out->log_stride;
-  if (out->chi2_log) UPS(v.chi2_log, double, nullptr, (size_t)n * out->log_stride);
-  if (out->lambda_log) UPS(v.lambda_log, double, nullptr, (size_t)n * out->log_stride);
-  if (out->trials_log) UPS(v.trials_log, int, nullptr, (size_t)n * out->log_stride);
-  if (out->n_iter_done) UPS(v.n_iter_done, int, nullptr, 2 * (size_t)n);
+  if (out->chi2_log) LLD_DEV(c, v.chi2_log, (size_t)n * out->log_stride);
+  if (out->lambda_log) LLD_DEV(c, v.lambda_log, (size_t)n * out->log_stride);
+  if (out->trials_log) LLD_DEV(c, v.trials_log, (size_t)n * out->log_stride);
+  if (out->n_iter_done) LLD_DEV(c, v.n_iter_done, 2 * (size_t)n);
   LLD_CUDA(c, cudaEventRecord(c->ev[1], c->stream));
   const size_t smem = EDGE_BYTES * max_m;
   if (smem <= SMEM_LIMIT) {
@@ -445,18 +409,12 @@ extern "C" int lld_sim3_opt(void* ctx, const lld_sim3_problem* p, lld_sim3_resul
   }
   LLD_CUDA(c, cudaGetLastError());
   LLD_CUDA(c, cudaEventRecord(c->ev[2], c->stream));
-  int r;
-  if ((r = down(c, out->S12, v.out_S12, 8 * (size_t)n))) return r;
-  if ((r = down(c, out->inlier, v.inlier, (size_t)m))) return r;
-  if ((r = down(c, out->n_in, v.n_in, (size_t)n))) return r;
-  if ((r = down(c, out->chi2_log, v.chi2_log, (size_t)n * out->log_stride))) return r;
-  if ((r = down(c, out->lambda_log, v.lambda_log, (size_t)n * out->log_stride))) return r;
-  if ((r = down(c, out->trials_log, v.trials_log, (size_t)n * out->log_stride))) return r;
-  if ((r = down(c, out->n_iter_done, v.n_iter_done, 2 * (size_t)n))) return r;
-  LLD_CUDA(c, cudaEventRecord(c->ev[3], c->stream));
-  LLD_CUDA(c, cudaStreamSynchronize(c->stream));
-  cudaEventElapsedTime(&c->ms_h2d, c->ev[0], c->ev[1]);
-  cudaEventElapsedTime(&c->ms_compute, c->ev[1], c->ev[2]);
-  cudaEventElapsedTime(&c->ms_d2h, c->ev[2], c->ev[3]);
-  return LLD_OK;
+  LLD_DOWN(c, out->S12, v.out_S12, 8 * (size_t)n);
+  LLD_DOWN(c, out->inlier, v.inlier, (size_t)m);
+  LLD_DOWN(c, out->n_in, v.n_in, (size_t)n);
+  LLD_DOWN(c, out->chi2_log, v.chi2_log, (size_t)n * out->log_stride);
+  LLD_DOWN(c, out->lambda_log, v.lambda_log, (size_t)n * out->log_stride);
+  LLD_DOWN(c, out->trials_log, v.trials_log, (size_t)n * out->log_stride);
+  LLD_DOWN(c, out->n_iter_done, v.n_iter_done, 2 * (size_t)n);
+  return lld_call_end(c);
 }

@@ -148,39 +148,6 @@ __global__ void __launch_bounds__(RTPB) k_sim3_ransac(RansacView v) {
   if (tid == 0) v.n_inliers[pb] = found ? s_cnt[0] : 0;
 }
 
-template <typename T>
-int upl(LldCtx* c, T** dst, const T* src, size_t n) {
-  cudaError_t e = cudaSuccess;
-  T* d = c->alloc<T>(n ? n : 1, &e);
-  if (e != cudaSuccess) {
-    snprintf(c->err, sizeof(c->err), "cudaMalloc: %s", cudaGetErrorString(e));
-    return LLD_ERR_CUDA;
-  }
-  if (n && src) {
-    e = cudaMemcpyAsync(d, src, n * sizeof(T), cudaMemcpyHostToDevice, c->stream);
-    if (e != cudaSuccess) {
-      snprintf(c->err, sizeof(c->err), "cudaMemcpyAsync H2D: %s", cudaGetErrorString(e));
-      return LLD_ERR_CUDA;
-    }
-  }
-  *dst = d;
-  return LLD_OK;
-}
-#define UPR(dst, T, src, n)                                \
-  do {                                                     \
-    T* _p = nullptr;                                       \
-    int _r = upl<T>(c, &_p, (const T*)(src), (size_t)(n)); \
-    if (_r) return _r;                                     \
-    (dst) = _p;                                            \
-  } while (0)
-
-template <typename T>
-int down(LldCtx* c, T* dst, const T* src, size_t n) {
-  if (!n || !dst) return LLD_OK;
-  LLD_CUDA(c, cudaMemcpyAsync(dst, src, n * sizeof(T), cudaMemcpyDeviceToHost, c->stream));
-  return LLD_OK;
-}
-
 }  // namespace
 
 extern "C" int32_t lld_sim3_ransac_max_its(int32_t n_corr, double probability, int32_t min_inliers, int32_t max_iterations) {
@@ -230,50 +197,41 @@ extern "C" int lld_sim3_ransac(void* ctx, const lld_sim3_ransac_problem* p, lld_
     }
   }
   const int m = p->off[n], h = p->hyp_off[n];
-  LLD_CUDA(c, cudaSetDevice(c->device));
-  c->launches = 0;
-  c->pool_reset();
-  LLD_CUDA(c, cudaEventRecord(c->ev[0], c->stream));
+  if (int r = lld_call_begin(c, true)) return r;
   RansacView v{};
-  UPR(v.cam, float, p->cam, 8 * (size_t)n);
-  UPR(v.fix_scale, int, p->fix_scale, n);
-  UPR(v.off, int, p->off, n + 1);
-  UPR(v.x1c, float, p->x1c, 3 * (size_t)m);
-  UPR(v.x2c, float, p->x2c, 3 * (size_t)m);
-  UPR(v.sig1, float, p->sigma2_1, m);
-  UPR(v.sig2, float, p->sigma2_2, m);
+  LLD_UP(c, v.cam, p->cam, 8 * (size_t)n);
+  LLD_UP(c, v.fix_scale, p->fix_scale, n);
+  LLD_UP(c, v.off, p->off, n + 1);
+  LLD_UP(c, v.x1c, p->x1c, 3 * (size_t)m);
+  LLD_UP(c, v.x2c, p->x2c, 3 * (size_t)m);
+  LLD_UP(c, v.sig1, p->sigma2_1, m);
+  LLD_UP(c, v.sig2, p->sigma2_2, m);
   v.min_inliers = p->min_inliers;
-  UPR(v.max_its, int, p->max_its, n);
-  UPR(v.its_in, int, p->its_done, n);
-  UPR(v.best_in, int, p->best_inliers, n);
+  LLD_UP(c, v.max_its, p->max_its, n);
+  LLD_UP(c, v.its_in, p->its_done, n);
+  LLD_UP(c, v.best_in, p->best_inliers, n);
   v.n_iterations = p->n_iterations;
-  UPR(v.hyp_off, int, p->hyp_off, n + 1);
-  UPR(v.hyp_idx, int, p->hyp_idx, 3 * (size_t)h);
-  UPR(v.found, uint8_t, nullptr, n);
-  UPR(v.no_more, uint8_t, nullptr, n);
-  UPR(v.n_inliers, int, nullptr, n);
-  UPR(v.T12, float, nullptr, 13 * (size_t)n);
-  UPR(v.inlier, uint8_t, nullptr, m);
-  UPR(v.its_out, int, nullptr, n);
-  UPR(v.best_out, int, nullptr, n);
-  if (out->hyp_inliers) UPR(v.hyp_inliers, int, nullptr, h);
+  LLD_UP(c, v.hyp_off, p->hyp_off, n + 1);
+  LLD_UP(c, v.hyp_idx, p->hyp_idx, 3 * (size_t)h);
+  LLD_DEV(c, v.found, n);
+  LLD_DEV(c, v.no_more, n);
+  LLD_DEV(c, v.n_inliers, n);
+  LLD_DEV(c, v.T12, 13 * (size_t)n);
+  LLD_DEV(c, v.inlier, m);
+  LLD_DEV(c, v.its_out, n);
+  LLD_DEV(c, v.best_out, n);
+  if (out->hyp_inliers) LLD_DEV(c, v.hyp_inliers, h);
   LLD_CUDA(c, cudaEventRecord(c->ev[1], c->stream));
   LLD_LAUNCH(c, k_sim3_ransac, n, RTPB, 0, v);
   LLD_CUDA(c, cudaGetLastError());
   LLD_CUDA(c, cudaEventRecord(c->ev[2], c->stream));
-  int r;
-  if ((r = down(c, out->found, v.found, (size_t)n))) return r;
-  if ((r = down(c, out->no_more, v.no_more, (size_t)n))) return r;
-  if ((r = down(c, out->n_inliers, v.n_inliers, (size_t)n))) return r;
-  if ((r = down(c, out->T12, v.T12, 13 * (size_t)n))) return r;
-  if ((r = down(c, out->inlier, v.inlier, (size_t)m))) return r;
-  if ((r = down(c, out->its_done, v.its_out, (size_t)n))) return r;
-  if ((r = down(c, out->best_inliers, v.best_out, (size_t)n))) return r;
-  if ((r = down(c, out->hyp_inliers, v.hyp_inliers, (size_t)h))) return r;
-  LLD_CUDA(c, cudaEventRecord(c->ev[3], c->stream));
-  LLD_CUDA(c, cudaStreamSynchronize(c->stream));
-  cudaEventElapsedTime(&c->ms_h2d, c->ev[0], c->ev[1]);
-  cudaEventElapsedTime(&c->ms_compute, c->ev[1], c->ev[2]);
-  cudaEventElapsedTime(&c->ms_d2h, c->ev[2], c->ev[3]);
-  return LLD_OK;
+  LLD_DOWN(c, out->found, v.found, (size_t)n);
+  LLD_DOWN(c, out->no_more, v.no_more, (size_t)n);
+  LLD_DOWN(c, out->n_inliers, v.n_inliers, (size_t)n);
+  LLD_DOWN(c, out->T12, v.T12, 13 * (size_t)n);
+  LLD_DOWN(c, out->inlier, v.inlier, (size_t)m);
+  LLD_DOWN(c, out->its_done, v.its_out, (size_t)n);
+  LLD_DOWN(c, out->best_inliers, v.best_out, (size_t)n);
+  LLD_DOWN(c, out->hyp_inliers, v.hyp_inliers, (size_t)h);
+  return lld_call_end(c);
 }

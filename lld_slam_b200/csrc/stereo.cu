@@ -274,7 +274,7 @@ __global__ void __launch_bounds__(ST_NT) k_stereo(StereoView v) {
 extern "C" int lld_stereo_matches(void* ctx, const lld_stereo_problem* p, lld_stereo_result* out) {
   LldCtx* c = lld_ctx_cast(ctx);
   if (!c || !p || !out) return LLD_ERR_ARG;
-  c->launches = 0;
+  c->launches = 0;   // a rejected call reports no launches
   LLD_ARG(c, p->n_frames >= 1 && p->n_levels >= 1 && p->n_levels <= 8);
   const int F = p->n_frames, n_l = p->left_off[F], n_r = p->right_off[F];
   int max_r = 0;
@@ -283,8 +283,7 @@ extern "C" int lld_stereo_matches(void* ctx, const lld_stereo_problem* p, lld_st
   // octaves index scale / rows / cols / stride and pyr_off on the device
   for (int i = 0; i < n_l; i++) LLD_ARG(c, p->left_octave[i] < p->n_levels);
   for (int i = 0; i < n_r; i++) LLD_ARG(c, p->right_octave[i] < p->n_levels);
-  LLD_CUDA(c, cudaSetDevice(c->device));
-  c->pool_reset();
+  if (int r = lld_call_begin(c, true)) return r;
   StereoView v{};
   v.n_frames = F; v.n_levels = p->n_levels; v.mb = p->mb; v.mbf = p->mbf;
   for (int l = 0; l < p->n_levels; l++) {
@@ -295,52 +294,35 @@ extern "C" int lld_stereo_matches(void* ctx, const lld_stereo_problem* p, lld_st
   float smax = 1.f;
   for (int l = 0; l < p->n_levels; l++) smax = std::max(smax, p->scale_factors[l]);
   v.list_cap = std::max(1, max_r) * (2 * (int)std::ceil(2.0f * smax) + 3);
-  cudaError_t e = cudaSuccess;
-  auto up = [&](const void* src, size_t bytes) -> void* {
-    if (e != cudaSuccess) return nullptr;
-    uint8_t* d = c->alloc<uint8_t>(bytes ? bytes : 1, &e);
-    if (e == cudaSuccess && bytes) e = cudaMemcpyAsync(d, src, bytes, cudaMemcpyHostToDevice, c->stream);
-    return d;
-  };
-  auto dev = [&](size_t bytes) -> void* {
-    if (e != cudaSuccess) return nullptr;
-    return c->alloc<uint8_t>(bytes ? bytes : 1, &e);
-  };
-  LLD_CUDA(c, cudaEventRecord(c->ev[0], c->stream));
-  v.l_off = (const int*)up(p->left_off, 4 * (size_t)(F + 1));
-  v.r_off = (const int*)up(p->right_off, 4 * (size_t)(F + 1));
-  v.l_xy = (const float*)up(p->left_xy, 8 * (size_t)n_l);
-  v.l_oct = (const uint8_t*)up(p->left_octave, (size_t)n_l);
-  v.l_desc = (const uint8_t*)up(p->left_desc, 32 * (size_t)n_l);
-  v.r_xy = (const float*)up(p->right_xy, 8 * (size_t)n_r);
-  v.r_oct = (const uint8_t*)up(p->right_octave, (size_t)n_r);
-  v.r_desc = (const uint8_t*)up(p->right_desc, 32 * (size_t)n_r);
-  v.pyr = (const uint8_t*)up(p->pyr, (size_t)p->pyr_bytes);
-  v.pyr_off = (const long long*)up(p->pyr_off, 8 * (size_t)F * 2 * p->n_levels);
-  v.row_start = (int*)dev(4 * (size_t)F * (v.rows[0] + 1));
-  v.row_list = (unsigned short*)dev(2 * (size_t)F * v.list_cap);
-  v.best_r = (int*)dev(4 * (size_t)n_l);
-  v.sad = (int*)dev(4 * (size_t)n_l);
-  v.uright = (float*)dev(4 * (size_t)n_l);
-  v.depth = (float*)dev(4 * (size_t)n_l);
-  v.n_matched = (int*)dev(4 * (size_t)F);
-  v.overflow = (int*)dev(4);
-  LLD_CUDA(c, e);
+  LLD_UP(c, v.l_off, p->left_off, F + 1);
+  LLD_UP(c, v.r_off, p->right_off, F + 1);
+  LLD_UP(c, v.l_xy, p->left_xy, 2 * (size_t)n_l);
+  LLD_UP(c, v.l_oct, p->left_octave, n_l);
+  LLD_UP(c, v.l_desc, p->left_desc, 32 * (size_t)n_l);
+  LLD_UP(c, v.r_xy, p->right_xy, 2 * (size_t)n_r);
+  LLD_UP(c, v.r_oct, p->right_octave, n_r);
+  LLD_UP(c, v.r_desc, p->right_desc, 32 * (size_t)n_r);
+  LLD_UP(c, v.pyr, p->pyr, (size_t)p->pyr_bytes);
+  LLD_UP(c, v.pyr_off, reinterpret_cast<const long long*>(p->pyr_off), (size_t)F * 2 * p->n_levels);
+  LLD_DEV(c, v.row_start, (size_t)F * (v.rows[0] + 1));
+  LLD_DEV(c, v.row_list, (size_t)F * v.list_cap);
+  LLD_DEV(c, v.best_r, n_l);
+  LLD_DEV(c, v.sad, n_l);
+  LLD_DEV(c, v.uright, n_l);
+  LLD_DEV(c, v.depth, n_l);
+  LLD_DEV(c, v.n_matched, F);
+  LLD_DEV(c, v.overflow, 1);
   LLD_CUDA(c, cudaMemsetAsync(v.overflow, 0, 4, c->stream));
   LLD_CUDA(c, cudaEventRecord(c->ev[1], c->stream));
   LLD_LAUNCH(c, k_stereo, F, ST_NT, 0, v);
   LLD_CUDA(c, cudaGetLastError());
   LLD_CUDA(c, cudaEventRecord(c->ev[2], c->stream));
   int* h_over = reinterpret_cast<int*>(c->pinned);
-  LLD_CUDA(c, cudaMemcpyAsync(out->uright, v.uright, 4 * (size_t)n_l, cudaMemcpyDeviceToHost, c->stream));
-  LLD_CUDA(c, cudaMemcpyAsync(out->depth, v.depth, 4 * (size_t)n_l, cudaMemcpyDeviceToHost, c->stream));
-  if (out->n_matched) LLD_CUDA(c, cudaMemcpyAsync(out->n_matched, v.n_matched, 4 * (size_t)F, cudaMemcpyDeviceToHost, c->stream));
-  LLD_CUDA(c, cudaMemcpyAsync(h_over, v.overflow, 4, cudaMemcpyDeviceToHost, c->stream));
-  LLD_CUDA(c, cudaEventRecord(c->ev[3], c->stream));
-  LLD_CUDA(c, cudaStreamSynchronize(c->stream));
-  cudaEventElapsedTime(&c->ms_h2d, c->ev[0], c->ev[1]);
-  cudaEventElapsedTime(&c->ms_compute, c->ev[1], c->ev[2]);
-  cudaEventElapsedTime(&c->ms_d2h, c->ev[2], c->ev[3]);
+  LLD_DOWN(c, out->uright, v.uright, n_l);
+  LLD_DOWN(c, out->depth, v.depth, n_l);
+  LLD_DOWN(c, out->n_matched, v.n_matched, F);
+  LLD_DOWN(c, h_over, v.overflow, 1);
+  if (int r = lld_call_end(c)) return r;
   if (*h_over) {
     snprintf(c->err, sizeof(c->err), "stereo matching: row-band list capacity exceeded");
     return LLD_ERR_UNSUPPORTED;

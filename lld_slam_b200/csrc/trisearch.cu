@@ -202,113 +202,81 @@ extern "C" int lld_bow_search(void* ctx, const lld_bow_search_problem* p, lld_tr
   LldCtx* c = lld_ctx_cast(ctx);
   if (!c || !p || !out) return LLD_ERR_ARG;
   LLD_ARG(c, p->n_pairs >= 1);
-  LLD_CUDA(c, cudaSetDevice(c->device));
-  c->launches = 0;
-  c->pool_reset();
+  if (int r = lld_call_begin(c, true)) return r;
   const int P = p->n_pairs, n1 = p->kp1_off[P], n2 = p->kp2_off[P];
   const int nn1 = p->fv1_node_off[P], nn2 = p->fv2_node_off[P];
   const int ne1 = nn1 ? p->fv1_idx_off[nn1] : 0, ne2 = nn2 ? p->fv2_idx_off[nn2] : 0;
-  cudaError_t e = cudaSuccess;
-  auto up = [&](const void* src, size_t bytes) -> void* {
-    if (e != cudaSuccess) return nullptr;
-    uint8_t* d = c->alloc<uint8_t>(bytes ? bytes : 1, &e);
-    if (e == cudaSuccess && bytes) e = cudaMemcpyAsync(d, src, bytes, cudaMemcpyHostToDevice, c->stream);
-    return d;
-  };
   BowView v{};
   v.p = *p;
-  LLD_CUDA(c, cudaEventRecord(c->ev[0], c->stream));
-  v.p.kp1_off = (const int32_t*)up(p->kp1_off, 4 * (size_t)(P + 1));
-  v.p.kp1_angle = (const float*)up(p->kp1_angle, 4 * (size_t)n1);
-  v.p.kp1_valid = (const uint8_t*)up(p->kp1_valid, (size_t)n1);
-  v.p.kp1_desc = (const uint8_t*)up(p->kp1_desc, 32 * (size_t)n1);
-  v.p.kp2_off = (const int32_t*)up(p->kp2_off, 4 * (size_t)(P + 1));
-  v.p.kp2_angle = (const float*)up(p->kp2_angle, 4 * (size_t)n2);
-  v.p.kp2_valid = (const uint8_t*)up(p->kp2_valid, (size_t)n2);
-  v.p.kp2_desc = (const uint8_t*)up(p->kp2_desc, 32 * (size_t)n2);
-  v.p.fv1_node_off = (const int32_t*)up(p->fv1_node_off, 4 * (size_t)(P + 1));
-  v.p.fv1_node = (const int32_t*)up(p->fv1_node, 4 * (size_t)nn1);
-  v.p.fv1_idx_off = (const int32_t*)up(p->fv1_idx_off, 4 * (size_t)(nn1 + 1));
-  v.p.fv1_idx = (const int32_t*)up(p->fv1_idx, 4 * (size_t)ne1);
-  v.p.fv2_node_off = (const int32_t*)up(p->fv2_node_off, 4 * (size_t)(P + 1));
-  v.p.fv2_node = (const int32_t*)up(p->fv2_node, 4 * (size_t)nn2);
-  v.p.fv2_idx_off = (const int32_t*)up(p->fv2_idx_off, 4 * (size_t)(nn2 + 1));
-  v.p.fv2_idx = (const int32_t*)up(p->fv2_idx, 4 * (size_t)ne2);
-  if (e == cudaSuccess) v.match12 = c->alloc<int>((size_t)std::max(n1, 1), &e);
-  if (e == cudaSuccess) v.n_matches = c->alloc<int>((size_t)P, &e);
-  if (e == cudaSuccess) v.matched2 = c->alloc<uint8_t>((size_t)std::max(n2, 1), &e);
-  LLD_CUDA(c, e);
+  LLD_UP(c, v.p.kp1_off, p->kp1_off, P + 1);
+  LLD_UP(c, v.p.kp1_angle, p->kp1_angle, n1);
+  LLD_UP(c, v.p.kp1_valid, p->kp1_valid, n1);
+  LLD_UP(c, v.p.kp1_desc, p->kp1_desc, 32 * (size_t)n1);
+  LLD_UP(c, v.p.kp2_off, p->kp2_off, P + 1);
+  LLD_UP(c, v.p.kp2_angle, p->kp2_angle, n2);
+  LLD_UP(c, v.p.kp2_valid, p->kp2_valid, n2);
+  LLD_UP(c, v.p.kp2_desc, p->kp2_desc, 32 * (size_t)n2);
+  LLD_UP(c, v.p.fv1_node_off, p->fv1_node_off, P + 1);
+  LLD_UP(c, v.p.fv1_node, p->fv1_node, nn1);
+  LLD_UP(c, v.p.fv1_idx_off, p->fv1_idx_off, nn1 + 1);
+  LLD_UP(c, v.p.fv1_idx, p->fv1_idx, ne1);
+  LLD_UP(c, v.p.fv2_node_off, p->fv2_node_off, P + 1);
+  LLD_UP(c, v.p.fv2_node, p->fv2_node, nn2);
+  LLD_UP(c, v.p.fv2_idx_off, p->fv2_idx_off, nn2 + 1);
+  LLD_UP(c, v.p.fv2_idx, p->fv2_idx, ne2);
+  LLD_DEV(c, v.match12, n1);
+  LLD_DEV(c, v.n_matches, P);
+  LLD_DEV(c, v.matched2, n2);
   LLD_CUDA(c, cudaMemsetAsync(v.matched2, 0, (size_t)std::max(n2, 1), c->stream));
   LLD_CUDA(c, cudaEventRecord(c->ev[1], c->stream));
   LLD_LAUNCH(c, k_bow_search, P, TS_NT, 0, v);
   LLD_CUDA(c, cudaGetLastError());
   LLD_CUDA(c, cudaEventRecord(c->ev[2], c->stream));
-  if (n1) LLD_CUDA(c, cudaMemcpyAsync(out->match12, v.match12, 4 * (size_t)n1, cudaMemcpyDeviceToHost, c->stream));
-  LLD_CUDA(c, cudaMemcpyAsync(out->n_matches, v.n_matches, 4 * (size_t)P, cudaMemcpyDeviceToHost, c->stream));
-  LLD_CUDA(c, cudaEventRecord(c->ev[3], c->stream));
-  LLD_CUDA(c, cudaStreamSynchronize(c->stream));
-  cudaEventElapsedTime(&c->ms_h2d, c->ev[0], c->ev[1]);
-  cudaEventElapsedTime(&c->ms_compute, c->ev[1], c->ev[2]);
-  cudaEventElapsedTime(&c->ms_d2h, c->ev[2], c->ev[3]);
-  return LLD_OK;
+  LLD_DOWN(c, out->match12, v.match12, n1);
+  LLD_DOWN(c, out->n_matches, v.n_matches, P);
+  return lld_call_end(c);
 }
 
 extern "C" int lld_tri_search(void* ctx, const lld_tri_search_problem* p, lld_tri_search_result* out) {
   LldCtx* c = lld_ctx_cast(ctx);
   if (!c || !p || !out) return LLD_ERR_ARG;
   LLD_ARG(c, p->n_pairs >= 1 && p->n_levels >= 1 && p->n_levels <= 8);
-  LLD_CUDA(c, cudaSetDevice(c->device));
-  c->launches = 0;
-  c->pool_reset();
+  if (int r = lld_call_begin(c, true)) return r;
   const int P = p->n_pairs, n1 = p->kp1_off[P], n2 = p->kp2_off[P];
   const int nn1 = p->fv1_node_off[P], nn2 = p->fv2_node_off[P];
   const int ne1 = nn1 ? p->fv1_idx_off[nn1] : 0, ne2 = nn2 ? p->fv2_idx_off[nn2] : 0;
-  cudaError_t e = cudaSuccess;
-  auto up = [&](const void* src, size_t bytes) -> void* {
-    if (e != cudaSuccess) return nullptr;
-    uint8_t* d = c->alloc<uint8_t>(bytes ? bytes : 1, &e);
-    if (e == cudaSuccess && bytes) e = cudaMemcpyAsync(d, src, bytes, cudaMemcpyHostToDevice, c->stream);
-    return d;
-  };
   TriView v{};
   v.p = *p;
-  LLD_CUDA(c, cudaEventRecord(c->ev[0], c->stream));
-  v.p.F12 = (const float*)up(p->F12, 36 * (size_t)P);
-  v.p.epipole = (const float*)up(p->epipole, 8 * (size_t)P);
-  v.p.kp1_off = (const int32_t*)up(p->kp1_off, 4 * (size_t)(P + 1));
-  v.p.kp1_xy = (const float*)up(p->kp1_xy, 8 * (size_t)n1);
-  v.p.kp1_angle = (const float*)up(p->kp1_angle, 4 * (size_t)n1);
-  v.p.kp1_uright = (const float*)up(p->kp1_uright, 4 * (size_t)n1);
-  v.p.kp1_has_mp = (const uint8_t*)up(p->kp1_has_mp, (size_t)n1);
-  v.p.kp1_desc = (const uint8_t*)up(p->kp1_desc, 32 * (size_t)n1);
-  v.p.kp2_off = (const int32_t*)up(p->kp2_off, 4 * (size_t)(P + 1));
-  v.p.kp2_xy = (const float*)up(p->kp2_xy, 8 * (size_t)n2);
-  v.p.kp2_octave = (const uint8_t*)up(p->kp2_octave, (size_t)n2);
-  v.p.kp2_angle = (const float*)up(p->kp2_angle, 4 * (size_t)n2);
-  v.p.kp2_uright = (const float*)up(p->kp2_uright, 4 * (size_t)n2);
-  v.p.kp2_has_mp = (const uint8_t*)up(p->kp2_has_mp, (size_t)n2);
-  v.p.kp2_desc = (const uint8_t*)up(p->kp2_desc, 32 * (size_t)n2);
-  v.p.fv1_node_off = (const int32_t*)up(p->fv1_node_off, 4 * (size_t)(P + 1));
-  v.p.fv1_node = (const int32_t*)up(p->fv1_node, 4 * (size_t)nn1);
-  v.p.fv1_idx_off = (const int32_t*)up(p->fv1_idx_off, 4 * (size_t)(nn1 + 1));
-  v.p.fv1_idx = (const int32_t*)up(p->fv1_idx, 4 * (size_t)ne1);
-  v.p.fv2_node_off = (const int32_t*)up(p->fv2_node_off, 4 * (size_t)(P + 1));
-  v.p.fv2_node = (const int32_t*)up(p->fv2_node, 4 * (size_t)nn2);
-  v.p.fv2_idx_off = (const int32_t*)up(p->fv2_idx_off, 4 * (size_t)(nn2 + 1));
-  v.p.fv2_idx = (const int32_t*)up(p->fv2_idx, 4 * (size_t)ne2);
-  if (e == cudaSuccess) v.match12 = c->alloc<int>((size_t)std::max(n1, 1), &e);
-  if (e == cudaSuccess) v.n_matches = c->alloc<int>((size_t)P, &e);
-  LLD_CUDA(c, e);
+  LLD_UP(c, v.p.F12, p->F12, 9 * (size_t)P);
+  LLD_UP(c, v.p.epipole, p->epipole, 2 * (size_t)P);
+  LLD_UP(c, v.p.kp1_off, p->kp1_off, P + 1);
+  LLD_UP(c, v.p.kp1_xy, p->kp1_xy, 2 * (size_t)n1);
+  LLD_UP(c, v.p.kp1_angle, p->kp1_angle, n1);
+  LLD_UP(c, v.p.kp1_uright, p->kp1_uright, n1);
+  LLD_UP(c, v.p.kp1_has_mp, p->kp1_has_mp, n1);
+  LLD_UP(c, v.p.kp1_desc, p->kp1_desc, 32 * (size_t)n1);
+  LLD_UP(c, v.p.kp2_off, p->kp2_off, P + 1);
+  LLD_UP(c, v.p.kp2_xy, p->kp2_xy, 2 * (size_t)n2);
+  LLD_UP(c, v.p.kp2_octave, p->kp2_octave, n2);
+  LLD_UP(c, v.p.kp2_angle, p->kp2_angle, n2);
+  LLD_UP(c, v.p.kp2_uright, p->kp2_uright, n2);
+  LLD_UP(c, v.p.kp2_has_mp, p->kp2_has_mp, n2);
+  LLD_UP(c, v.p.kp2_desc, p->kp2_desc, 32 * (size_t)n2);
+  LLD_UP(c, v.p.fv1_node_off, p->fv1_node_off, P + 1);
+  LLD_UP(c, v.p.fv1_node, p->fv1_node, nn1);
+  LLD_UP(c, v.p.fv1_idx_off, p->fv1_idx_off, nn1 + 1);
+  LLD_UP(c, v.p.fv1_idx, p->fv1_idx, ne1);
+  LLD_UP(c, v.p.fv2_node_off, p->fv2_node_off, P + 1);
+  LLD_UP(c, v.p.fv2_node, p->fv2_node, nn2);
+  LLD_UP(c, v.p.fv2_idx_off, p->fv2_idx_off, nn2 + 1);
+  LLD_UP(c, v.p.fv2_idx, p->fv2_idx, ne2);
+  LLD_DEV(c, v.match12, n1);
+  LLD_DEV(c, v.n_matches, P);
   LLD_CUDA(c, cudaEventRecord(c->ev[1], c->stream));
   LLD_LAUNCH(c, k_tri_search, P, TS_NT, 0, v);
   LLD_CUDA(c, cudaGetLastError());
   LLD_CUDA(c, cudaEventRecord(c->ev[2], c->stream));
-  if (n1) LLD_CUDA(c, cudaMemcpyAsync(out->match12, v.match12, 4 * (size_t)n1, cudaMemcpyDeviceToHost, c->stream));
-  LLD_CUDA(c, cudaMemcpyAsync(out->n_matches, v.n_matches, 4 * (size_t)P, cudaMemcpyDeviceToHost, c->stream));
-  LLD_CUDA(c, cudaEventRecord(c->ev[3], c->stream));
-  LLD_CUDA(c, cudaStreamSynchronize(c->stream));
-  cudaEventElapsedTime(&c->ms_h2d, c->ev[0], c->ev[1]);
-  cudaEventElapsedTime(&c->ms_compute, c->ev[1], c->ev[2]);
-  cudaEventElapsedTime(&c->ms_d2h, c->ev[2], c->ev[3]);
-  return LLD_OK;
+  LLD_DOWN(c, out->match12, v.match12, n1);
+  LLD_DOWN(c, out->n_matches, v.n_matches, P);
+  return lld_call_end(c);
 }

@@ -366,19 +366,9 @@ def test_ragged_and_target_are_dense_single():
 # ------------------------------------------------------------------------------------------------------------------
 # GPU harness
 # ------------------------------------------------------------------------------------------------------------------
-def _bind(lib):
-    d = lib.dll
-    vp = C.c_void_p
-    d.lld_ctx_profile.argtypes = [vp, C.c_int]; d.lld_ctx_profile.restype = None
-    d.lld_ctx_profile_report.argtypes = [vp, C.c_char_p, C.c_int]; d.lld_ctx_profile_report.restype = C.c_int
-    d.lld_ctx_last_bytes.argtypes = [vp, C.POINTER(C.c_int64), C.POINTER(C.c_int64)]; d.lld_ctx_last_bytes.restype = None
-    d.lld_ctx_set_topo_cache.argtypes = [vp, C.c_int]; d.lld_ctx_set_topo_cache.restype = None
-    return d
-
-
 def _context(topo_cache):
     c = capi.Context(0)
-    _bind(c.lib).lld_ctx_set_topo_cache(c.handle, topo_cache)
+    c.lib.dll.lld_ctx_set_topo_cache(c.handle, topo_cache)
     return c
 
 
@@ -423,15 +413,8 @@ def oracle(p, mode, its=(5, 15)):
 
 
 def profiled(p, c, mode, its=(5, 15)):
-    d = c.lib.dll
-    d.lld_ctx_profile(c.handle, 1)
-    try:
-        out = run(p, c, mode, its)
-        buf = C.create_string_buffer(1 << 16)
-        c.check(d.lld_ctx_profile_report(c.handle, buf, len(buf)), "lld_ctx_profile_report")
-    finally:
-        d.lld_ctx_profile(c.handle, 0)
-    return out, set(json.loads(buf.value.decode()))
+    out, prof = c.profile(lambda: run(p, c, mode, its))
+    return out, set(prof)
 
 
 def assert_identical(a, b, what=""):

@@ -16,7 +16,7 @@ import numpy as np
 import pytest
 
 from lld_slam_b200 import capi, synth
-from test_ba_paths import (ERR_UNSUPPORTED, SMEM_LIMIT, _bind, _free_sets, add_points, assert_identical, checked, cr_problem,
+from test_ba_paths import (ERR_UNSUPPORTED, SMEM_LIMIT, _free_sets, add_points, assert_identical, checked, cr_problem,
                            expect_error, free_kfs, h2d_bytes, new_values, oracle, profiled, run, shape_claims,
                            too_wide_problem, value_bytes)
 from test_gpu_parity import check_ba
@@ -266,8 +266,7 @@ SP_KERNELS = {"k_sp_assemble", "k_sp_factor", "k_sp_solve<15>", "k_sp_update", "
 
 def _context(topo_cache, sparse):
     c = capi.Context(0)
-    d = _bind(c.lib)
-    d.lld_ctx_set_topo_cache(c.handle, topo_cache)
+    c.lib.dll.lld_ctx_set_topo_cache(c.handle, topo_cache)
     c.lib.dll.lld_ctx_set_gba_sparse(c.handle, sparse)
     return c
 

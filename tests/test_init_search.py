@@ -4,7 +4,6 @@ the histogram counting displaced matches, the bin-30 wrap, windows clipped or ou
 tiny pairs, F1 keypoints above level 0), and the GPU is bit-exact against the oracle on match12, n_matches and prev_matched,
 on both resolve arms (F2 state in shared memory / in global memory, told apart by the per-launch profile)."""
 import ctypes as C
-import json
 import math
 import os
 import subprocess
@@ -391,17 +390,8 @@ def test_shim_search_for_initialization_on_host(built, tmp_path):
 # GPU
 # ------------------------------------------------------------------------------------------------------------------
 def _profiled(p, ctx):
-    d = ctx.lib.dll
-    d.lld_ctx_profile.argtypes = [C.c_void_p, C.c_int]; d.lld_ctx_profile.restype = None
-    d.lld_ctx_profile_report.argtypes = [C.c_void_p, C.c_char_p, C.c_int]; d.lld_ctx_profile_report.restype = C.c_int
-    d.lld_ctx_profile(ctx.handle, 1)
-    try:
-        out = api.init_search(p, impl="gpu", ctx=ctx)
-        buf = C.create_string_buffer(1 << 16)
-        ctx.check(d.lld_ctx_profile_report(ctx.handle, buf, len(buf)), "lld_ctx_profile_report")
-    finally:
-        d.lld_ctx_profile(ctx.handle, 0)
-    return out, set(json.loads(buf.value.decode()))
+    out, prof = ctx.profile(lambda: api.init_search(p, impl="gpu", ctx=ctx))
+    return out, set(prof)
 
 
 def _check_gpu(p, ctx, arm):

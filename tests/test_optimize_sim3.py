@@ -4,7 +4,6 @@ early return) pins the CPU oracle; hand-built problems pin one rule each; the ho
 Sim3 pieces; the shim writes back what the reference writes; on the GPU the batched kernel matches the oracle on both staging
 arms (edge records in shared memory / in global memory, told apart by the per-launch profile)."""
 import ctypes as C
-import json
 import math
 import os
 import subprocess
@@ -656,17 +655,8 @@ def test_shim_optimize_sim3_on_host(built, tmp_path):
 # GPU
 # ------------------------------------------------------------------------------------------------------------------
 def _profiled(p, ctx):
-    d = ctx.lib.dll
-    d.lld_ctx_profile.argtypes = [C.c_void_p, C.c_int]; d.lld_ctx_profile.restype = None
-    d.lld_ctx_profile_report.argtypes = [C.c_void_p, C.c_char_p, C.c_int]; d.lld_ctx_profile_report.restype = C.c_int
-    d.lld_ctx_profile(ctx.handle, 1)
-    try:
-        out = api.sim3_opt(p, impl="gpu", ctx=ctx)
-        buf = C.create_string_buffer(1 << 16)
-        ctx.check(d.lld_ctx_profile_report(ctx.handle, buf, len(buf)), "lld_ctx_profile_report")
-    finally:
-        d.lld_ctx_profile(ctx.handle, 0)
-    return out, set(json.loads(buf.value.decode()))
+    out, prof = ctx.profile(lambda: api.sim3_opt(p, impl="gpu", ctx=ctx))
+    return out, set(prof)
 
 
 def _rel_log(g, o, pb, its1):

@@ -3,7 +3,6 @@ itself (cv2.reduce, cv2.gemm, cv2.eigen, cv2.norm, cv2.Rodrigues on float32 arra
 pin one rule each; the host build of the device math equals the oracle's pieces; on the GPU the batched kernel matches the
 oracle with the full budget in one call and as ComputeSim3 rounds of 5, and its winners feed lld_sim3_opt."""
 import ctypes as C
-import json
 import math
 import os
 import sys
@@ -437,17 +436,8 @@ def _same(g, o, p, strict, py=None):
 
 
 def _profiled(p, ctx):
-    d = ctx.lib.dll
-    d.lld_ctx_profile.argtypes = [C.c_void_p, C.c_int]; d.lld_ctx_profile.restype = None
-    d.lld_ctx_profile_report.argtypes = [C.c_void_p, C.c_char_p, C.c_int]; d.lld_ctx_profile_report.restype = C.c_int
-    d.lld_ctx_profile(ctx.handle, 1)
-    try:
-        out = api.sim3_ransac(p, impl="gpu", ctx=ctx)
-        buf = C.create_string_buffer(1 << 16)
-        ctx.check(d.lld_ctx_profile_report(ctx.handle, buf, len(buf)), "lld_ctx_profile_report")
-    finally:
-        d.lld_ctx_profile(ctx.handle, 0)
-    return out, set(json.loads(buf.value.decode()))
+    out, prof = ctx.profile(lambda: api.sim3_ransac(p, impl="gpu", ctx=ctx))
+    return out, set(prof)
 
 
 def run_rounds(p, run, n_iterations=5, seed=0):

@@ -111,7 +111,6 @@ if want("medoid"):
 # ---- SearchForInitialization (Tracking::MonocularInitialization: ORBmatcher(0.9, true), windowSize = 100)
 if want("search_for_initialization"):
     import subprocess
-    import ctypes as C
     import torch
     pi = synth.make_init_search_batch(256, 2000, 71)
     g, ms, wall = timed(lambda: api.init_search(pi, impl="gpu", ctx=ctx))
@@ -120,15 +119,7 @@ if want("search_for_initialization"):
     n8 = int(p8["kp1_off"][-1])
     exact = (np.array_equal(g["match12"][:n8], o["match12"]) and np.array_equal(g["n_matches"][:8], o["n_matches"])
              and np.array_equal(g["prev_matched"][:n8].view(np.uint32), o["prev_matched"].view(np.uint32)))
-    d = ctx.lib.dll
-    d.lld_ctx_profile.argtypes = [C.c_void_p, C.c_int]; d.lld_ctx_profile.restype = None
-    d.lld_ctx_profile_report.argtypes = [C.c_void_p, C.c_char_p, C.c_int]; d.lld_ctx_profile_report.restype = C.c_int
-    d.lld_ctx_profile(ctx.handle, 1)                         # separate, profiled run: per-launch CUDA events
-    api.init_search(pi, impl="gpu", ctx=ctx)
-    buf = C.create_string_buffer(1 << 16)
-    ctx.check(d.lld_ctx_profile_report(ctx.handle, buf, len(buf)), "lld_ctx_profile_report")
-    d.lld_ctx_profile(ctx.handle, 0)
-    prof = json.loads(buf.value.decode())
+    _, prof = ctx.profile(lambda: api.init_search(pi, impl="gpu", ctx=ctx))   # separate, profiled run: per-launch CUDA events
     part = lambda names: sum(prof[k]["ms"] for k in names if k in prof)   # noqa: E731
     smi = subprocess.run(["nvidia-smi", "--query-gpu=name,power.limit", "--format=csv,noheader"], stdout=subprocess.PIPE, text=True).stdout
     out["search_for_initialization"] = {
@@ -143,21 +134,12 @@ if want("search_for_initialization"):
 # ---- OptimizeSim3 (LoopClosing::ComputeSim3: th2 = 10, 5 / 10 / 5 iterations), both scale modes
 if want("optimize_sim3"):
     import subprocess
-    import ctypes as C
     import torch
-    d = ctx.lib.dll
-    d.lld_ctx_profile.argtypes = [C.c_void_p, C.c_int]; d.lld_ctx_profile.restype = None
-    d.lld_ctx_profile_report.argtypes = [C.c_void_p, C.c_char_p, C.c_int]; d.lld_ctx_profile_report.restype = C.c_int
     res = {}
     for fix in (1, 0):
         ps = synth.make_sim3_batch(4096, 300, 131 + fix, fix_scale=fix)
         g, ms, wall = timed(lambda: api.sim3_opt(ps, impl="gpu", ctx=ctx))
-        d.lld_ctx_profile(ctx.handle, 1)                     # separate, profiled run: per-launch CUDA events
-        api.sim3_opt(ps, impl="gpu", ctx=ctx)
-        buf = C.create_string_buffer(1 << 16)
-        ctx.check(d.lld_ctx_profile_report(ctx.handle, buf, len(buf)), "lld_ctx_profile_report")
-        d.lld_ctx_profile(ctx.handle, 0)
-        prof = json.loads(buf.value.decode())
+        _, prof = ctx.profile(lambda: api.sim3_opt(ps, impl="gpu", ctx=ctx))   # separate, profiled run: per-launch CUDA events
         p1 = synth.make_sim3_batch(1, 300, 131 + fix, fix_scale=fix)   # the batch-of-one call the shim makes per candidate
         one = []
         api.sim3_opt(p1, impl="gpu", ctx=ctx)
@@ -183,22 +165,13 @@ if want("optimize_sim3"):
 # ---- Sim3Solver (LoopClosing::ComputeSim3: SetRansacParameters(0.99, 20, 300), iterate(5) per round), both scale modes
 if want("sim3_ransac"):
     import subprocess
-    import ctypes as C
     import torch
     from test_sim3_ransac import run_rounds
-    d = ctx.lib.dll
-    d.lld_ctx_profile.argtypes = [C.c_void_p, C.c_int]; d.lld_ctx_profile.restype = None
-    d.lld_ctx_profile_report.argtypes = [C.c_void_p, C.c_char_p, C.c_int]; d.lld_ctx_profile_report.restype = C.c_int
     res = {}
     for fix in (1, 0):
         ps = synth.make_sim3_ransac_batch(4096, 300, 701 + fix, fix_scale=fix)
         g, ms, wall = timed(lambda: api.sim3_ransac(ps, impl="gpu", ctx=ctx))
-        d.lld_ctx_profile(ctx.handle, 1)                     # separate, profiled run: per-launch CUDA events
-        api.sim3_ransac(ps, impl="gpu", ctx=ctx)
-        buf = C.create_string_buffer(1 << 16)
-        ctx.check(d.lld_ctx_profile_report(ctx.handle, buf, len(buf)), "lld_ctx_profile_report")
-        d.lld_ctx_profile(ctx.handle, 0)
-        prof = json.loads(buf.value.decode())
+        _, prof = ctx.profile(lambda: api.sim3_ransac(ps, impl="gpu", ctx=ctx))   # separate, profiled run: per-launch CUDA events
         # ComputeSim3 rounds of 5 over the same candidates (each round one call; draws on the host are not timed)
         dev, calls = [], []
         def gpu_round(q):

@@ -38,8 +38,6 @@ def measure(p, iters, reps, sparse):
     ctx = capi.Context(0)
     d = ctx.lib.dll
     d.lld_ctx_set_gba_sparse(ctx.handle, 1 if sparse else 0)
-    d.lld_ctx_profile.argtypes = [C.c_void_p, C.c_int]; d.lld_ctx_profile.restype = None
-    d.lld_ctx_profile_report.argtypes = [C.c_void_p, C.c_char_p, C.c_int]; d.lld_ctx_profile_report.restype = C.c_int
     api.ba_global(p, iters, impl="gpu", ctx=ctx)   # warm-up (indexes the structure; later calls hit the topology cache)
     e2e, res = [], []
     for _ in range(reps):
@@ -47,12 +45,7 @@ def measure(p, iters, reps, sparse):
         g = api.ba_global(p, iters, impl="gpu", ctx=ctx)
         e2e.append(1e3 * (time.perf_counter() - t))
         res.append(ctx.last_timing()[1])
-    d.lld_ctx_profile(ctx.handle, 1)
-    api.ba_global(p, iters, impl="gpu", ctx=ctx)
-    buf = C.create_string_buffer(1 << 16)
-    ctx.check(d.lld_ctx_profile_report(ctx.handle, buf, len(buf)), "lld_ctx_profile_report")
-    d.lld_ctx_profile(ctx.handle, 0)
-    prof = json.loads(buf.value.decode())
+    _, prof = ctx.profile(lambda: api.ba_global(p, iters, impl="gpu", ctx=ctx))
     ctx.close()
     total = sum(v["ms"] for v in prof.values())
     solver = {k: v for k, v in prof.items() if k.startswith("k_sp_") or k.startswith("k_cr_")}
