@@ -24,6 +24,7 @@
  *   lld_init_search        <- ORBmatcher::SearchForInitialization    src/ORBmatcher.cc:405
  *   lld_sim3_opt           <- Optimizer::OptimizeSim3                src/Optimizer.cc:1656-1858
  *   lld_sim3_ransac        <- Sim3Solver::iterate / ComputeSim3 / CheckInliers (ORB-SLAM2 src/Sim3Solver.cc)
+ *   lld_pnp_ransac         <- PnPsolver::iterate / Refine / CheckInliers / compute_pose (ORB-SLAM2 src/PnPsolver.cc)
  *   lld_line_associate     <- Tracking::AddLinesFrom                 src/Tracking.cc:996-1124
  *   lld_medoid_orb / _float<- MapPoint / MapLine::ComputeDistinctiveDescriptors              src/MapPoint.cc:242-307, src/MapLine.cc:133-201
  *
@@ -88,6 +89,8 @@ extern "C" {
  *     within 200 KB) the edge records are staged in shared memory (k_sim3_opt_smem), else read from global memory (k_sim3_opt_global);
  *   - lld_sim3_ransac: no limit on the correspondences or minimal sets of a problem (correspondence data is read from global
  *     memory; one CTA per problem evaluates 8 minimal sets at a time, k_sim3_ransac);
+ *   - lld_pnp_ransac: no limit on the correspondences or minimal sets of a problem (one CTA per problem, one warp per minimal
+ *     set, 8 at a time, Refine over the whole CTA; correspondence data is read from global memory, k_pnp_ransac);
  *   - lld_line_match: descriptor widths that are a multiple of 8 up to 72 floats and at most 512 lines per side of a pair run on the
  *     tensor cores, everything else on the FP32 tile path (no failure).
  */
@@ -594,6 +597,83 @@ typedef struct lld_sim3_ransac_result {
 int32_t lld_sim3_ransac_max_its(int32_t n_corr, double probability, int32_t min_inliers, int32_t max_iterations);
 
 int lld_sim3_ransac(void* ctx, const lld_sim3_ransac_problem* p, lld_sim3_ransac_result* out);
+
+/* ------------------------------------------------------------------------------------------------
+ * Relocalisation EPnP RANSAC: PnPsolver (ORB-SLAM2 src/PnPsolver.cc, inherited unchanged by LLD-SLAM), batched over
+ * relocalisation candidates (Tracking::Relocalization calls SetRansacParameters(0.99, 10, 300, 4, 0.5, 5.991) and
+ * iterate(5, ...) per candidate per round).  The reference source is not at hand: the rules below are transcribed from
+ * ORB-SLAM2's PnPsolver.cc as recalled, and they are the contract.
+ *   - Constructor PnPsolver(F, vpMapPointMatches): every i whose map point is present and not bad, in index order; p2d =
+ *     F.mvKeysUn[i].pt, p3dw = GetWorldPos() (float), sigma2 = F.mvLevelSigma2[octave]; fu fv uc vc = F.fx fy cx cy.
+ *   - max_err[i] = mvMaxError[i] = sigma2 * th2 in float, formed by the caller.
+ *   - iterate(nIterations): with N < min_inliers nothing is drawn and no_more = 1.  Otherwise minimal sets of 4 are evaluated
+ *     while (its_done < max_its || evaluated in this call < n_iterations) (an ||, where Sim3Solver has &&).  Per set: EPnP,
+ *     CheckInliers; if its count reaches min_inliers (>=): when it beats best_inliers (strictly) its mask, count and pose become
+ *     the best, and then Refine runs on the best mask (possibly carried from an earlier set or call): EPnP over every best
+ *     inlier, CheckInliers; it succeeds iff the refined count exceeds min_inliers (strictly), and the call returns the refined
+ *     pose, count and mask with found = 1, no_more = 0.  After the loop no_more = 1 and, if best_inliers >= min_inliers, the call
+ *     returns the best pose, count and mask (found = 1).  A call that does not succeed always ends with no_more = 1.
+ *   - CheckInliers: Xc, Yc, invZc = 1 / (...) computed in double (double R, t times the float point) and stored to float;
+ *     ue = uc + fu * Xc * invZc in double; distX = u - ue stored to float; error2 = distX^2 + distY^2 in float; inlier iff
+ *     error2 < max_err (a NaN is an outlier; there is no depth test).
+ *   - EPnP (compute_pose) is Lepetit's epnp.cpp: control points (centroid, principal axes of PW0^T PW0 scaled by sqrt(d / n)),
+ *     barycentric coordinates through CC^-1 (the SVD pseudo-inverse), M^T M, the eigenvectors of its four smallest eigenvalues, L_6x10 and rho,
+ *     find_betas_approx_1 / 2 / 3 (L columns {0,1,3,6} / {0,1,2} / {0,1,2,3,4}, least squares through the SVD, their sign and
+ *     sqrt rules; as in OpenCV's back-substitution, the SVD solves and CC^-1 skip singular values at or below
+ *     2 DBL_EPSILON times their sum, so coplanar world points drop the vanishing control axis; for
+ *     them the third left singular vector of ABt, which OpenCV draws from its RNG, is the cross product of the other two), each followed by 5 Gauss-Newton steps (unpivoted Householder QR of the 6x4 system; a singular system adds
+ *     nothing), compute_R_and_t (ccs from ut rows 11 - i, pcs, the sign flip on the first point's depth, R = U V^T of the SVD
+ *     of ABt with row 2 negated when det < 0, the mean of the sqrt reprojection distances).  Solution 1 is kept, replaced by 2
+ *     if its error is smaller, then by 3 if smaller than the kept one.  The SVDs and the eigen decomposition are cyclic
+ *     Jacobi in double (two-sided on the symmetric PW0^T PW0 and M^T M, one-sided on CC, ABt and the L systems), not OpenCV's:
+ *     singular vectors differ in sign and, in a repeated null space (four points), in basis, which the betas absorb.
+ *     Every sum over correspondences runs serially in correspondence order.
+ * Random draws: as lld_sim3_ransac, the caller draws the sets (DUtils::Random::RandomInt on rand(), swap-with-back from a fresh
+ * 0..N-1); given the same sets this computes what iterate() computes.  Problem p receives exactly
+ *   B = N < min_inliers ? 0 : max(n_iterations, max_its - its_done)
+ * sets.  The state the reference keeps between calls (mnIterations, mnBestInliers, mvbBestInliers, mBestTcw) is passed in and
+ * out.  The minimal set size is 4 (SetRansacParameters' minSet only enters the min_inliers floor).
+ * ---------------------------------------------------------------------------------------------- */
+typedef struct lld_pnp_ransac_problem {
+  int32_t n_problems;
+  const float* cam;            /* [n][4] fx fy cx cy (widened to double as fu fv uc vc) */
+  const int32_t* min_inliers;  /* [n] mRansacMinInliers after SetRansacParameters (lld_pnp_ransac_params), >= 4 */
+  const int32_t* max_its;      /* [n] mRansacMaxIts after SetRansacParameters, >= 1 */
+  const int32_t* its_done;     /* [n] mnIterations before the call */
+  const int32_t* best_inliers; /* [n] mnBestInliers before the call */
+  const int32_t* off;          /* [n+1] CSR over correspondences, off[0] = 0 */
+  const float* p2d;            /* [m][2] mvP2D */
+  const float* p3dw;           /* [m][3] mvP3Dw */
+  const float* max_err;        /* [m] mvMaxError = mvSigma2 * th2 (float) */
+  const uint8_t* best_mask;    /* [m] mvbBestInliers before the call (read where best_inliers >= min_inliers) */
+  const float* best_Tcw;       /* [n][12] mBestTcw before the call: R row-major, t */
+  int32_t n_iterations;        /* iterate(nIterations): 5 in Tracking::Relocalization */
+  const int32_t* hyp_off;      /* [n+1] CSR over minimal sets, hyp_off[0] = 0, B sets per problem (above) */
+  const int32_t* hyp_idx;      /* [h][4] problem-local correspondence indices of each set, in draw order, distinct */
+} lld_pnp_ransac_problem;
+
+typedef struct lld_pnp_ransac_result {
+  uint8_t* found;          /* [n] iterate() returned a pose */
+  uint8_t* no_more;        /* [n] bNoMore */
+  int32_t* n_inliers;      /* [n] nInliers (0 unless found) */
+  float* Tcw;              /* [n][12] the returned pose, R row-major then t (float); zero where not found */
+  uint8_t* inlier;         /* [m] vbInliers in CSR order (all 0 unless found) */
+  int32_t* its_done;       /* [n] mnIterations after the call (may alias the input) */
+  int32_t* best_inliers;   /* [n] mnBestInliers after the call (may alias the input) */
+  uint8_t* best_mask;      /* [m] mvbBestInliers after the call (may alias the input) */
+  float* best_Tcw;         /* [n][12] mBestTcw after the call (may alias the input) */
+  int32_t* hyp_inliers;    /* [h] mnInliersi of each set, -1 where the set was not evaluated; may be NULL */
+} lld_pnp_ransac_result;
+
+/* SetRansacParameters(probability, minInliers, maxIterations, minSet, epsilon, th2) for N = n_corr, host arithmetic:
+ * nMinInliers = (int)(N * epsilon) (float product), raised to minInliers, then to minSet; epsilon raised to
+ * (float)nMinInliers / N; nIterations = nMinInliers == N ? 1 : ceil(log(1 - p) / log(1 - pow(epsilon, 3))); out[0] = nMinInliers,
+ * out[1] = max(1, min(nIterations, maxIterations)) (1 where the logarithm is undefined, N < nMinInliers).  Returns LLD_ERR_ARG
+ * for n_corr < 0 or a NULL out. */
+int lld_pnp_ransac_params(int32_t n_corr, double probability, int32_t min_inliers, int32_t max_iterations, int32_t min_set,
+                          float epsilon, int32_t out[2]);
+
+int lld_pnp_ransac(void* ctx, const lld_pnp_ransac_problem* p, lld_pnp_ransac_result* out);
 
 /* ------------------------------------------------------------------------------------------------
  * Stereo line matching (float line descriptors)

@@ -221,6 +221,41 @@ def sim3_ransac_max_its(n_corr: int, probability: float = 0.99, min_inliers: int
     return int(capi.load_library().sim3_ransac_max_its(int(n_corr), float(probability), int(min_inliers), int(max_iterations)))
 
 
+def pnp_ransac(p: Dict[str, Any], *, impl: str = "gpu", ctx=None):
+    """PnPsolver::iterate batched over relocalisation candidates (include/lldba.h): found, no_more, n_inliers, Tcw ([n][12]:
+    R row-major, t), inlier ([m], vbInliers in CSR order), the solver state after the call (its_done, best_inliers, best_mask,
+    best_Tcw) and hyp_inliers (per minimal set, -1 where not evaluated)"""
+    lib = _lib(impl)
+    prob, keep = capi.fill_struct(capi.PnpRansacProblem, p)
+    n, m, h = int(p["n_problems"]), int(p["off"][-1]), int(p["hyp_off"][-1])
+    out = dict(found=np.full(max(n, 1), 2, np.uint8), no_more=np.full(max(n, 1), 2, np.uint8),
+               n_inliers=np.full(max(n, 1), -2, np.int32), Tcw=np.full((max(n, 1), 12), np.nan, np.float32),
+               inlier=np.full(max(m, 1), 2, np.uint8), its_done=np.full(max(n, 1), -2, np.int32),
+               best_inliers=np.full(max(n, 1), -2, np.int32), best_mask=np.full(max(m, 1), 2, np.uint8),
+               best_Tcw=np.full((max(n, 1), 12), np.nan, np.float32), hyp_inliers=np.full(max(h, 1), -2, np.int32))
+    res, keep2 = capi.fill_struct(capi.PnpRansacResult, out)
+    rc = lib.pnp_ransac(_handle(impl, ctx), C.byref(prob), C.byref(res))
+    _check(impl, ctx, rc, "lld_pnp_ransac")
+    for k in ("found", "no_more", "n_inliers", "Tcw", "its_done", "best_inliers", "best_Tcw"):
+        out[k] = out[k][:n]
+    for k in ("inlier", "best_mask"):
+        out[k] = out[k][:m]
+    out["hyp_inliers"] = out["hyp_inliers"][:h]
+    return out
+
+
+def pnp_ransac_params(n_corr: int, probability: float = 0.99, min_inliers: int = 8, max_iterations: int = 300, min_set: int = 4,
+                      epsilon: float = 0.4):
+    """PnPsolver::SetRansacParameters (the reference's defaults): (mRansacMinInliers, mRansacMaxIts) for n_corr
+    correspondences, host arithmetic of the library"""
+    out = np.zeros(2, np.int32)
+    rc = capi.load_library().pnp_ransac_params(int(n_corr), float(probability), int(min_inliers), int(max_iterations), int(min_set),
+                                               float(epsilon), out.ctypes.data_as(capi.c_i32p))
+    if rc != 0:
+        raise RuntimeError(f"lld_pnp_ransac_params failed with {rc}")
+    return int(out[0]), int(out[1])
+
+
 def line_match(p: Dict[str, Any], *, impl: str = "gpu", ctx=None):
     lib = _lib(impl)
     prob, keep = capi.fill_struct(capi.LineMatchProblem, p)

@@ -4,7 +4,8 @@ This is the Python harness over the C-ABI used by tests/ and bench.py.  The prod
 lld_slam_b200/csrc/liblldba.so (CUDA, sm_100a); `load_library()` fails loudly when it is missing —
 there is no CPU fallback.  `load_oracle()` loads the CPU oracle (oracle/liblld_oracle.so) which
 exposes the same entry points with the `lldo_` prefix (lldo_init_search from tests/hostcheck/libinit_search_oracle.so, lldo_sim3_opt from
-tests/hostcheck/libsim3_oracle.so, lldo_sim3_ransac from tests/hostcheck/libsim3_ransac_oracle.so); only tests, smoke() and the bench's
+tests/hostcheck/libsim3_oracle.so, lldo_sim3_ransac from tests/hostcheck/libsim3_ransac_oracle.so, lldo_pnp_ransac from
+tests/hostcheck/libpnp_ransac_oracle.so); only tests, smoke() and the bench's
 cpu_baseline / reference arm may call it.
 """
 from __future__ import annotations
@@ -23,6 +24,7 @@ ORACLE_PATH = os.path.join(_ROOT, "oracle", "liblld_oracle.so")
 INIT_SEARCH_ORACLE_PATH = os.path.join(_ROOT, "tests", "hostcheck", "libinit_search_oracle.so")
 SIM3_ORACLE_PATH = os.path.join(_ROOT, "tests", "hostcheck", "libsim3_oracle.so")
 SIM3_RANSAC_ORACLE_PATH = os.path.join(_ROOT, "tests", "hostcheck", "libsim3_ransac_oracle.so")
+PNP_RANSAC_ORACLE_PATH = os.path.join(_ROOT, "tests", "hostcheck", "libpnp_ransac_oracle.so")
 
 c_i32p = C.POINTER(C.c_int32)
 c_u8p = C.POINTER(C.c_uint8)
@@ -190,6 +192,21 @@ class Sim3RansacResult(C.Structure):
     ]
 
 
+class PnpRansacProblem(C.Structure):
+    _fields_ = [
+        ("n_problems", C.c_int32), ("cam", c_f32p), ("min_inliers", c_i32p), ("max_its", c_i32p), ("its_done", c_i32p),
+        ("best_inliers", c_i32p), ("off", c_i32p), ("p2d", c_f32p), ("p3dw", c_f32p), ("max_err", c_f32p), ("best_mask", c_u8p),
+        ("best_Tcw", c_f32p), ("n_iterations", C.c_int32), ("hyp_off", c_i32p), ("hyp_idx", c_i32p),
+    ]
+
+
+class PnpRansacResult(C.Structure):
+    _fields_ = [
+        ("found", c_u8p), ("no_more", c_u8p), ("n_inliers", c_i32p), ("Tcw", c_f32p), ("inlier", c_u8p), ("its_done", c_i32p),
+        ("best_inliers", c_i32p), ("best_mask", c_u8p), ("best_Tcw", c_f32p), ("hyp_inliers", c_i32p),
+    ]
+
+
 class TriSearchResult(C.Structure):
     _fields_ = [("match12", c_i32p), ("n_matches", c_i32p)]
 
@@ -293,6 +310,9 @@ class _Lib:
         if not self.is_oracle:
             self._sig("sim3_ransac_max_its", [C.c_int32, C.c_double, C.c_int32, C.c_int32])
             self.sim3_ransac_max_its.restype = C.c_int32
+        self._sig("pnp_ransac", [vp, C.POINTER(PnpRansacProblem), C.POINTER(PnpRansacResult)], PNP_RANSAC_ORACLE_PATH)
+        if not self.is_oracle:
+            self._sig("pnp_ransac_params", [C.c_int32, C.c_double, C.c_int32, C.c_int32, C.c_int32, C.c_float, c_i32p])
         self._sig("line_match", [vp, C.POINTER(LineMatchProblem), C.POINTER(LineMatchResult)])
         self._sig("descriptor_distance", [c_u8p, c_u8p])
         if not self.is_oracle:

@@ -660,6 +660,533 @@ LLD_HD bool sim3r_inlier(const Sim3Pair& T, const float* x1, const float* x2, fl
   return e[0] < sim3r_max_err(sig1) && e[1] < sim3r_max_err(sig2);
 }
 
+// ---- PnPsolver (ORB-SLAM2 src/PnPsolver.cc: EPnP of Lepetit et al., epnp.cpp) -------------------------------------
+// One EPnP runs on a group of threads described by a Par: the serial host build (PnpSerial), one warp (a minimal set) or
+// one CTA (Refine over the best inliers).  Every sum over correspondences is formed by one thread, serially in
+// correspondence order, so all three give the same bits; the group splits only over independent outputs (matrix entries,
+// Jacobi rotation rows) and joins with Par::sync().  Shared state lives in a PnpWork the group can all read.
+struct PnpSerial {
+  LLD_HD int rank() const { return 0; }
+  LLD_HD int size() const { return 1; }
+  LLD_HD void sync() const {}
+};
+#if defined(__CUDACC__)
+struct PnpWarp {
+  int lane;
+  __device__ int rank() const { return lane; }
+  __device__ int size() const { return 32; }
+  __device__ void sync() const { __syncwarp(); }
+};
+struct PnpCta {
+  __device__ int rank() const { return (int)threadIdx.x; }
+  __device__ int size() const { return (int)blockDim.x; }
+  __device__ void sync() const { __syncthreads(); }
+};
+#endif
+
+struct PnpCam {
+  double fu, fv, uc, vc;
+};
+
+struct PnpWork {
+  double c0[3];         // cws[0]: centroid of the world points
+  double cws[4][3];     // control points
+  double cci[9];        // CC^-1 (cvInvert(CC, CV_SVD))
+  double a[144];        // the symmetric matrix under Jacobi (PW0^T PW0 in a[0..8], M^T M)
+  double v[144];        // its eigenvectors (columns)
+  int ord[12];          // eigen indices by decreasing eigenvalue
+  double ccs[3][12];    // camera control points of the three beta solutions (sign resolved)
+  double pw0[3], pc0[3][3];
+  double abt[3][9];
+  double R[3][9], t[3][3], err[3];
+};
+
+// cyclic Jacobi on the symmetric n x n A (row-major, overwritten; the diagonal ends as the eigenvalues), eigenvectors in the
+// columns of V, ord = eigen indices by decreasing eigenvalue (first index on ties).  The group splits each rotation over rows.
+template <class P>
+LLD_HD void pnp_sym_jacobi(const P& par, double* A, double* V, int n, int* ord) {
+  for (int k = par.rank(); k < n * n; k += par.size()) V[k] = (k / n == k % n) ? 1.0 : 0.0;
+  par.sync();
+  for (int sweep = 0; sweep < 32; sweep++) {
+    double off = 0, dia = 0;
+    for (int i = 0; i < n; i++) {
+      dia += fabs(A[i * n + i]);
+      for (int j = i + 1; j < n; j++) off += fabs(A[i * n + j]);
+    }
+    if (!(off > 1e-15 * dia)) break;
+    for (int p = 0; p < n - 1; p++)
+      for (int q = p + 1; q < n; q++) {
+        const double apq = A[p * n + q];
+        if (apq == 0.0) continue;
+        const double theta = (A[q * n + q] - A[p * n + p]) / (2.0 * apq);
+        const double tt = (theta >= 0.0 ? 1.0 : -1.0) / (fabs(theta) + sqrt(theta * theta + 1.0));
+        const double c = 1.0 / sqrt(tt * tt + 1.0), s = tt * c;
+        par.sync();
+        for (int k = par.rank(); k < n; k += par.size()) {
+          const double x = A[k * n + p], y = A[k * n + q];
+          A[k * n + p] = c * x - s * y;
+          A[k * n + q] = s * x + c * y;
+          const double vx = V[k * n + p], vy = V[k * n + q];
+          V[k * n + p] = c * vx - s * vy;
+          V[k * n + q] = s * vx + c * vy;
+        }
+        par.sync();
+        for (int k = par.rank(); k < n; k += par.size()) {
+          const double x = A[p * n + k], y = A[q * n + k];
+          A[p * n + k] = c * x - s * y;
+          A[q * n + k] = s * x + c * y;
+        }
+        par.sync();
+      }
+  }
+  if (par.rank() == 0) {
+    for (int i = 0; i < n; i++) ord[i] = i;
+    for (int i = 1; i < n; i++) {   // insertion sort by decreasing eigenvalue, stable
+      const int x = ord[i];
+      int j = i;
+      for (; j > 0 && A[x * n + x] > A[ord[j - 1] * n + ord[j - 1]]; j--) ord[j] = ord[j - 1];
+      ord[j] = x;
+    }
+  }
+  par.sync();
+}
+
+// one-sided (Hestenes) Jacobi SVD of the m x k A (row-major, m <= 6, k <= 5): A is overwritten by U diag(sig), V (k x k)
+// holds the right singular vectors in its columns, ord the column indices by decreasing singular value.
+LLD_HD void pnp_svd_jacobi(double* A, int m, int k, double* V, double* sig, int* ord) {
+  for (int i = 0; i < k * k; i++) V[i] = (i / k == i % k) ? 1.0 : 0.0;
+  for (int sweep = 0; sweep < 32; sweep++) {
+    bool rotated = false;
+    for (int p = 0; p < k - 1; p++)
+      for (int q = p + 1; q < k; q++) {
+        double al = 0, be = 0, ga = 0;
+        for (int r = 0; r < m; r++) {
+          al += A[r * k + p] * A[r * k + p];
+          be += A[r * k + q] * A[r * k + q];
+          ga += A[r * k + p] * A[r * k + q];
+        }
+        if (!(fabs(ga) > 1e-15 * sqrt(al * be))) continue;
+        const double zeta = (be - al) / (2.0 * ga);
+        const double tt = (zeta >= 0.0 ? 1.0 : -1.0) / (fabs(zeta) + sqrt(1.0 + zeta * zeta));
+        const double c = 1.0 / sqrt(1.0 + tt * tt), s = c * tt;
+        for (int r = 0; r < m; r++) {
+          const double x = A[r * k + p], y = A[r * k + q];
+          A[r * k + p] = c * x - s * y;
+          A[r * k + q] = s * x + c * y;
+        }
+        for (int r = 0; r < k; r++) {
+          const double x = V[r * k + p], y = V[r * k + q];
+          V[r * k + p] = c * x - s * y;
+          V[r * k + q] = s * x + c * y;
+        }
+        rotated = true;
+      }
+    if (!rotated) break;
+  }
+  for (int j = 0; j < k; j++) {
+    double s2 = 0;
+    for (int r = 0; r < m; r++) s2 += A[r * k + j] * A[r * k + j];
+    sig[j] = sqrt(s2);
+  }
+  for (int i = 0; i < k; i++) ord[i] = i;
+  for (int i = 1; i < k; i++) {   // insertion sort by decreasing sig, stable
+    const int x = ord[i];
+    int j = i;
+    for (; j > 0 && sig[x] > sig[ord[j - 1]]; j--) ord[j] = ord[j - 1];
+    ord[j] = x;
+  }
+}
+
+// least-squares solve of the m x k system A x = b through the SVD (cvSolve(..., CV_SVD)); A is destroyed
+LLD_HD void pnp_svd_solve(double* A, int m, int k, const double* b, double* x) {
+  double V[25], sig[5];
+  int ord[5];
+  pnp_svd_jacobi(A, m, k, V, sig, ord);
+  for (int i = 0; i < k; i++) x[i] = 0.0;
+  double thr = 0;   // OpenCV's back-substitution skips singular values <= 2 DBL_EPSILON sum(sig)
+  for (int jj = 0; jj < k; jj++) thr += sig[ord[jj]];
+  thr *= 2 * 2.220446049250313e-16;
+  for (int jj = 0; jj < k; jj++) {
+    const int j = ord[jj];
+    if (fabs(sig[j]) <= thr) continue;
+    double ub = 0;
+    for (int r = 0; r < m; r++) ub += (A[r * k + j] / sig[j]) * b[r];
+    const double w = ub / sig[j];
+    for (int i = 0; i < k; i++) x[i] += V[i * k + j] * w;
+  }
+}
+
+// Lepetit's qr_solve on the 6 x 4 Gauss-Newton system (unpivoted Householder); a singular A leaves x at 0
+LLD_HD void pnp_qr_solve_6x4(double* A, double* b, double* x) {
+  const int nr = 6, nc = 4;
+  double A1[4], A2[4];
+  for (int k = 0; k < nc; k++) x[k] = 0.0;
+  for (int k = 0; k < nc; k++) {
+    double eta = fabs(A[k * nc + k]);
+    for (int i = k + 1; i < nr; i++) {
+      const double elt = fabs(A[i * nc + k]);
+      if (eta < elt) eta = elt;
+    }
+    if (eta == 0) return;
+    double sum = 0.0;
+    for (int i = k; i < nr; i++) {
+      A[i * nc + k] /= eta;
+      sum += A[i * nc + k] * A[i * nc + k];
+    }
+    double sigma = sqrt(sum);
+    if (A[k * nc + k] < 0) sigma = -sigma;
+    A[k * nc + k] += sigma;
+    A1[k] = sigma * A[k * nc + k];
+    A2[k] = -eta * sigma;
+    for (int j = k + 1; j < nc; j++) {
+      double s = 0;
+      for (int i = k; i < nr; i++) s += A[i * nc + k] * A[i * nc + j];
+      const double tau = s / A1[k];
+      for (int i = k; i < nr; i++) A[i * nc + j] -= tau * A[i * nc + k];
+    }
+  }
+  for (int j = 0; j < nc; j++) {
+    double tau = 0;
+    for (int i = j; i < nr; i++) tau += A[i * nc + j] * b[i];
+    tau /= A1[j];
+    for (int i = j; i < nr; i++) b[i] -= tau * A[i * nc + j];
+  }
+  x[nc - 1] = b[nc - 1] / A2[nc - 1];
+  for (int i = nc - 2; i >= 0; i--) {
+    double s = 0;
+    for (int j = i + 1; j < nc; j++) s += A[i * nc + j] * x[j];
+    x[i] = (b[i] - s) / A2[i];
+  }
+}
+
+LLD_HD double pnp_dot(const double* a, const double* b) { return a[0] * b[0] + a[1] * b[1] + a[2] * b[2]; }
+
+// compute_barycentric_coordinates for one world point
+LLD_HD void pnp_alphas(const PnpWork& w, const float* X, double* al) {
+  const double p0 = X[0], p1 = X[1], p2 = X[2];
+  for (int j = 0; j < 3; j++)
+    al[1 + j] = w.cci[3 * j] * (p0 - w.cws[0][0]) + w.cci[3 * j + 1] * (p1 - w.cws[0][1]) + w.cci[3 * j + 2] * (p2 - w.cws[0][2]);
+  al[0] = 1.0 - al[1] - al[2] - al[3];
+}
+
+// compute_pcs for one point: camera coordinate j under the control points ccs
+LLD_HD double pnp_pc(const double* al, const double* ccs, int j) {
+  return al[0] * ccs[j] + al[1] * ccs[3 + j] + al[2] * ccs[6 + j] + al[3] * ccs[9 + j];
+}
+
+// compute_L_6x10 on the eigenvectors of the four smallest eigenvalues, compute_rho
+LLD_HD void pnp_L_rho(const PnpWork& w, double* L, double* rho) {
+  double v[4][12];
+  for (int i = 0; i < 4; i++)
+    for (int k = 0; k < 12; k++) v[i][k] = w.v[k * 12 + w.ord[11 - i]];   // ut row 11 - i
+  double dv[4][6][3];
+  for (int i = 0; i < 4; i++) {
+    int a = 0, b = 1;
+    for (int j = 0; j < 6; j++) {
+      dv[i][j][0] = v[i][3 * a] - v[i][3 * b];
+      dv[i][j][1] = v[i][3 * a + 1] - v[i][3 * b + 1];
+      dv[i][j][2] = v[i][3 * a + 2] - v[i][3 * b + 2];
+      b++;
+      if (b > 3) {
+        a++;
+        b = a + 1;
+      }
+    }
+  }
+  for (int i = 0; i < 6; i++) {
+    double* row = L + 10 * i;
+    row[0] = pnp_dot(dv[0][i], dv[0][i]);
+    row[1] = 2.0 * pnp_dot(dv[0][i], dv[1][i]);
+    row[2] = pnp_dot(dv[1][i], dv[1][i]);
+    row[3] = 2.0 * pnp_dot(dv[0][i], dv[2][i]);
+    row[4] = 2.0 * pnp_dot(dv[1][i], dv[2][i]);
+    row[5] = pnp_dot(dv[2][i], dv[2][i]);
+    row[6] = 2.0 * pnp_dot(dv[0][i], dv[3][i]);
+    row[7] = 2.0 * pnp_dot(dv[1][i], dv[3][i]);
+    row[8] = 2.0 * pnp_dot(dv[2][i], dv[3][i]);
+    row[9] = pnp_dot(dv[3][i], dv[3][i]);
+  }
+  auto d2 = [](const double* p, const double* q) {
+    return (p[0] - q[0]) * (p[0] - q[0]) + (p[1] - q[1]) * (p[1] - q[1]) + (p[2] - q[2]) * (p[2] - q[2]);
+  };
+  rho[0] = d2(w.cws[0], w.cws[1]);
+  rho[1] = d2(w.cws[0], w.cws[2]);
+  rho[2] = d2(w.cws[0], w.cws[3]);
+  rho[3] = d2(w.cws[1], w.cws[2]);
+  rho[4] = d2(w.cws[1], w.cws[3]);
+  rho[5] = d2(w.cws[2], w.cws[3]);
+}
+
+// find_betas_approx_1 / 2 / 3 (s = 0, 1, 2): the columns of L each approximation keeps, its SVD solve and its sign rules
+LLD_HD void pnp_betas_approx(int s, const double* L, const double* rho, double* betas) {
+  const int cols[3][5] = {{0, 1, 3, 6, -1}, {0, 1, 2, -1, -1}, {0, 1, 2, 3, 4}};
+  const int k = s == 0 ? 4 : (s == 1 ? 3 : 5);
+  double A[30], b[5];
+  for (int r = 0; r < 6; r++)
+    for (int c = 0; c < k; c++) A[r * k + c] = L[10 * r + cols[s][c]];
+  pnp_svd_solve(A, 6, k, rho, b);
+  if (s == 0) {
+    if (b[0] < 0) {
+      betas[0] = sqrt(-b[0]);
+      betas[1] = -b[1] / betas[0];
+      betas[2] = -b[2] / betas[0];
+      betas[3] = -b[3] / betas[0];
+    } else {
+      betas[0] = sqrt(b[0]);
+      betas[1] = b[1] / betas[0];
+      betas[2] = b[2] / betas[0];
+      betas[3] = b[3] / betas[0];
+    }
+    return;
+  }
+  if (b[0] < 0) {
+    betas[0] = sqrt(-b[0]);
+    betas[1] = (b[2] < 0) ? sqrt(-b[2]) : 0.0;
+  } else {
+    betas[0] = sqrt(b[0]);
+    betas[1] = (b[2] > 0) ? sqrt(b[2]) : 0.0;
+  }
+  if (b[1] < 0) betas[0] = -betas[0];
+  betas[2] = s == 2 ? b[3] / betas[0] : 0.0;
+  betas[3] = 0.0;
+}
+
+// gauss_newton: 5 iterations of compute_A_and_b_gauss_newton + qr_solve
+LLD_HD void pnp_gauss_newton(const double* L, const double* rho, double* betas) {
+  for (int it = 0; it < 5; it++) {
+    double A[24], b[6], x[4];
+    for (int i = 0; i < 6; i++) {
+      const double* l = L + 10 * i;
+      double* a = A + 4 * i;
+      a[0] = 2 * l[0] * betas[0] + l[1] * betas[1] + l[3] * betas[2] + l[6] * betas[3];
+      a[1] = l[1] * betas[0] + 2 * l[2] * betas[1] + l[4] * betas[2] + l[7] * betas[3];
+      a[2] = l[3] * betas[0] + l[4] * betas[1] + 2 * l[5] * betas[2] + l[8] * betas[3];
+      a[3] = l[6] * betas[0] + l[7] * betas[1] + l[8] * betas[2] + 2 * l[9] * betas[3];
+      b[i] = rho[i] - (l[0] * betas[0] * betas[0] + l[1] * betas[0] * betas[1] + l[2] * betas[1] * betas[1] +
+                       l[3] * betas[0] * betas[2] + l[4] * betas[1] * betas[2] + l[5] * betas[2] * betas[2] +
+                       l[6] * betas[0] * betas[3] + l[7] * betas[1] * betas[3] + l[8] * betas[2] * betas[3] +
+                       l[9] * betas[3] * betas[3]);
+    }
+    pnp_qr_solve_6x4(A, b, x);
+    for (int i = 0; i < 4; i++) betas[i] += x[i];
+  }
+}
+
+// estimate_R_and_t's SVD part: ABt = U S V^T, R = U V^T (columns by decreasing singular value), row 2 negated if det < 0,
+// t = pc0 - R pw0
+LLD_HD void pnp_R_t(const double* abt_in, const double* pc0, const double* pw0, double* R, double* t) {
+  double U[9], V[9], sig[3];
+  int ord[3];
+  for (int i = 0; i < 9; i++) U[i] = abt_in[i];
+  pnp_svd_jacobi(U, 3, 3, V, sig, ord);
+  double Un[9];   // left singular vectors, columns by decreasing singular value
+  for (int i = 0; i < 3; i++)
+    for (int k = 0; k < 3; k++) Un[3 * i + k] = U[i * 3 + ord[k]] / sig[ord[k]];
+  const double thr = (sig[ord[0]] + sig[ord[1]] + sig[ord[2]]) * (2 * 2.220446049250313e-16);
+  if (sig[ord[2]] <= thr) {   // coplanar world points: complete U to a proper basis (V is a product of rotations)
+    Un[2] = Un[3] * Un[7] - Un[6] * Un[4];
+    Un[5] = Un[6] * Un[1] - Un[0] * Un[7];
+    Un[8] = Un[0] * Un[4] - Un[3] * Un[1];
+  }
+  for (int i = 0; i < 3; i++) {
+    double vr[3];
+    for (int j = 0; j < 3; j++) {
+      for (int k = 0; k < 3; k++) vr[k] = V[j * 3 + ord[k]];
+      R[3 * i + j] = pnp_dot(Un + 3 * i, vr);
+    }
+  }
+  const double det = R[0] * R[4] * R[8] + R[1] * R[5] * R[6] + R[2] * R[3] * R[7] - R[2] * R[4] * R[6] - R[1] * R[3] * R[8] -
+                     R[0] * R[5] * R[7];
+  if (det < 0) {
+    R[6] = -R[6];
+    R[7] = -R[7];
+    R[8] = -R[8];
+  }
+  t[0] = pc0[0] - pnp_dot(R, pw0);
+  t[1] = pc0[1] - pnp_dot(R + 3, pw0);
+  t[2] = pc0[2] - pnp_dot(R + 6, pw0);
+}
+
+// reprojection_error term of one correspondence
+LLD_HD double pnp_reproj(const double* R, const double* t, const float* X, const float* uv, const PnpCam& cam) {
+  const double pw[3] = {X[0], X[1], X[2]};
+  const double Xc = pnp_dot(R, pw) + t[0];
+  const double Yc = pnp_dot(R + 3, pw) + t[1];
+  const double inv_Zc = 1.0 / (pnp_dot(R + 6, pw) + t[2]);
+  const double ue = cam.uc + cam.fu * Xc * inv_Zc;
+  const double ve = cam.vc + cam.fv * Yc * inv_Zc;
+  const double u = uv[0], v = uv[1];
+  return sqrt((u - ue) * (u - ue) + (v - ve) * (v - ve));
+}
+
+// compute_pose over the n correspondences id(0..n-1) (idx == nullptr: 0..n-1) of X3 ([.][3]) / uv ([.][2]).  R (9), t
+// (3) in double, as mRi / mti; valid on every rank after the call.
+template <class P>
+LLD_HD void pnp_epnp(const P& par, PnpWork& w, const float* X3, const float* uv, const int* idx, int n, const PnpCam& cam) {
+  const int rk = par.rank(), sz = par.size();
+  const double dn = (double)n;
+#define LLD_PNP_ID(i) (idx ? idx[i] : (i))
+  // choose_control_points: centroid, then PW0^T PW0
+  for (int j = rk; j < 3; j += sz) {
+    double s = 0;
+    for (int i = 0; i < n; i++) s += (double)X3[3 * (size_t)LLD_PNP_ID(i) + j];
+    w.c0[j] = s / dn;
+  }
+  par.sync();
+  for (int e = rk; e < 6; e += sz) {
+    const int a = e < 3 ? 0 : (e < 5 ? 1 : 2), b = e < 3 ? e : (e < 5 ? e - 2 : 2);
+    double s = 0;
+    for (int i = 0; i < n; i++) {
+      const float* X = X3 + 3 * (size_t)LLD_PNP_ID(i);
+      s += ((double)X[a] - w.c0[a]) * ((double)X[b] - w.c0[b]);
+    }
+    w.a[3 * a + b] = s;
+    w.a[3 * b + a] = s;
+  }
+  par.sync();
+  pnp_sym_jacobi(par, w.a, w.v, 3, w.ord);
+  if (rk == 0) {
+    for (int j = 0; j < 3; j++) w.cws[0][j] = w.c0[j];
+    for (int i = 1; i < 4; i++) {
+      const int e = w.ord[i - 1];
+      const double d = w.a[4 * e];
+      const double k = sqrt((d > 0.0 ? d : 0.0) / dn);
+      for (int j = 0; j < 3; j++) w.cws[i][j] = w.cws[0][j] + k * w.v[3 * j + e];
+    }
+    // compute_barycentric_coordinates: CC^-1 through the SVD, V diag(1 / s) U^T
+    double CC[9], V[9], sig[3];
+    int ord[3];
+    for (int i = 0; i < 3; i++)
+      for (int j = 1; j < 4; j++) CC[3 * i + j - 1] = w.cws[j][i] - w.cws[0][i];
+    pnp_svd_jacobi(CC, 3, 3, V, sig, ord);
+    double thr = 0;   // cvInvert(CV_SVD): singular values <= 2 DBL_EPSILON sum(sig) are skipped (a pseudo-inverse)
+    for (int kk = 0; kk < 3; kk++) thr += sig[ord[kk]];
+    thr *= 2 * 2.220446049250313e-16;
+    for (int i = 0; i < 3; i++)
+      for (int r = 0; r < 3; r++) {
+        double s = 0;
+        for (int kk = 0; kk < 3; kk++) {
+          const int c = ord[kk];
+          if (fabs(sig[c]) <= thr) continue;
+          s += V[3 * i + c] * ((CC[3 * r + c] / sig[c]) / sig[c]);
+        }
+        w.cci[3 * i + r] = s;
+      }
+  }
+  par.sync();
+  // fill_M, M^T M: entry (a, b), rows in correspondence order (u row, then v row)
+  for (int e = rk; e < 78; e += sz) {
+    int a = 0, rem = e;
+    while (rem >= 12 - a) {
+      rem -= 12 - a;
+      a++;
+    }
+    const int b = a + rem;
+    double s = 0;
+    for (int i = 0; i < n; i++) {
+      const int id = LLD_PNP_ID(i);
+      double al[4];
+      pnp_alphas(w, X3 + 3 * (size_t)id, al);
+      const double u = uv[2 * (size_t)id], v = uv[2 * (size_t)id + 1];
+      const double m1a = (a % 3 == 0) ? al[a / 3] * cam.fu : (a % 3 == 1 ? 0.0 : al[a / 3] * (cam.uc - u));
+      const double m1b = (b % 3 == 0) ? al[b / 3] * cam.fu : (b % 3 == 1 ? 0.0 : al[b / 3] * (cam.uc - u));
+      const double m2a = (a % 3 == 0) ? 0.0 : (a % 3 == 1 ? al[a / 3] * cam.fv : al[a / 3] * (cam.vc - v));
+      const double m2b = (b % 3 == 0) ? 0.0 : (b % 3 == 1 ? al[b / 3] * cam.fv : al[b / 3] * (cam.vc - v));
+      s += m1a * m1b;
+      s += m2a * m2b;
+    }
+    w.a[12 * a + b] = s;
+    w.a[12 * b + a] = s;
+  }
+  par.sync();
+  pnp_sym_jacobi(par, w.a, w.v, 12, w.ord);
+  // L, rho, the three beta approximations with Gauss-Newton, ccs and solve_for_sign (the first point's depth)
+  if (rk == 0) {
+    double L[60], rho[6];
+    pnp_L_rho(w, L, rho);
+    for (int s = 0; s < 3; s++) {
+      double betas[4];
+      pnp_betas_approx(s, L, rho, betas);
+      pnp_gauss_newton(L, rho, betas);
+      double* ccs = w.ccs[s];
+      for (int k = 0; k < 12; k++) ccs[k] = 0.0;
+      for (int i = 0; i < 4; i++)
+        for (int k = 0; k < 12; k++) ccs[k] += betas[i] * w.v[k * 12 + w.ord[11 - i]];
+      double al[4];
+      pnp_alphas(w, X3 + 3 * (size_t)LLD_PNP_ID(0), al);
+      if (pnp_pc(al, ccs, 2) < 0)
+        for (int k = 0; k < 12; k++) ccs[k] = -ccs[k];
+    }
+  }
+  par.sync();
+  // estimate_R_and_t: centroids of the camera points of each solution and of the world points
+  for (int e = rk; e < 12; e += sz) {
+    const int s = e / 3, j = e % 3;
+    double acc = 0;
+    for (int i = 0; i < n; i++) {
+      const int id = LLD_PNP_ID(i);
+      if (s == 3) {
+        acc += (double)X3[3 * (size_t)id + j];
+      } else {
+        double al[4];
+        pnp_alphas(w, X3 + 3 * (size_t)id, al);
+        acc += pnp_pc(al, w.ccs[s], j);
+      }
+    }
+    if (s == 3)
+      w.pw0[j] = acc / dn;
+    else
+      w.pc0[s][j] = acc / dn;
+  }
+  par.sync();
+  for (int e = rk; e < 27; e += sz) {
+    const int s = e / 9, j = (e % 9) / 3, c = e % 3;
+    double acc = 0;
+    for (int i = 0; i < n; i++) {
+      const int id = LLD_PNP_ID(i);
+      double al[4];
+      pnp_alphas(w, X3 + 3 * (size_t)id, al);
+      acc += (pnp_pc(al, w.ccs[s], j) - w.pc0[s][j]) * ((double)X3[3 * (size_t)id + c] - w.pw0[c]);
+    }
+    w.abt[s][3 * j + c] = acc;
+  }
+  par.sync();
+  for (int s = rk; s < 3; s += sz) pnp_R_t(w.abt[s], w.pc0[s], w.pw0, w.R[s], w.t[s]);
+  par.sync();
+  for (int s = rk; s < 3; s += sz) {
+    double acc = 0;
+    for (int i = 0; i < n; i++) {
+      const int id = LLD_PNP_ID(i);
+      acc += pnp_reproj(w.R[s], w.t[s], X3 + 3 * (size_t)id, uv + 2 * (size_t)id, cam);
+    }
+    w.err[s] = acc / dn;
+  }
+  par.sync();
+#undef LLD_PNP_ID
+}
+
+// the solution compute_pose keeps: 1, replaced by 2 if its error is smaller, then by 3 if smaller than the kept one
+LLD_HD int pnp_pick(const PnpWork& w) {
+  int b = 0;
+  if (w.err[1] < w.err[0]) b = 1;
+  if (w.err[2] < w.err[b]) b = 2;
+  return b;
+}
+
+// PnPsolver::CheckInliers for one correspondence: Xc, Yc, invZc stored to float, ue / ve in double, distX / distY and
+// error2 in float; inlier iff error2 < mvMaxError (a NaN is an outlier, no depth test)
+LLD_HD bool pnp_inlier(const double* R, const double* t, const float* X, const float* uv, float max_err, const PnpCam& cam) {
+  const float Xc = (float)(R[0] * X[0] + R[1] * X[1] + R[2] * X[2] + t[0]);
+  const float Yc = (float)(R[3] * X[0] + R[4] * X[1] + R[5] * X[2] + t[1]);
+  const float invZc = (float)(1 / (R[6] * X[0] + R[7] * X[1] + R[8] * X[2] + t[2]));
+  const double ue = cam.uc + cam.fu * Xc * invZc;
+  const double ve = cam.vc + cam.fv * Yc * invZc;
+  const float distX = (float)(uv[0] - ue);
+  const float distY = (float)(uv[1] - ve);
+  const float error2 = distX * distX + distY * distY;
+  return error2 < max_err;
+}
+
 // ---- tiny dense helpers --------------------------------------------------------------------------
 // symmetric 3x3 / 4x4 inverse via cofactors / blockwise (general inverse, like MatrixXd::inverse()).
 LLD_HD void inv3_sym(const double* A /*full 9*/, double* I) {

@@ -125,6 +125,7 @@ struct Frame {
   std::vector<KeyPoint> mvKeys, mvKeysUn;
   std::vector<float> mvuRight;
   std::vector<uint8_t> mDescriptors;                  // N x 32
+  std::vector<float> mvLevelSigma2;                   // per pyramid level (read by PnPsolver)
   std::vector<MapPoint*> mvpMapPoints;
   std::vector<uint8_t> mvpMapPointDesc;               // descriptor of mvpMapPoints[i] (pMP->GetDescriptor()), N x 32
   std::vector<uint8_t> mvpMapPointHasObs;             // pMP->Observations() > 0
@@ -787,6 +788,149 @@ class Sim3Solver {
   std::vector<bool> mvbInliers;
   int mnInliers = 0, mLastError = 0;
   float mBestRotation[9] = {0}, mBestTranslation[3] = {0}, mBestScale = 1.f;
+};
+
+// PnPsolver (ORB-SLAM2 include/PnPsolver.h, src/PnPsolver.cc) over lld_pnp_ransac.  The constructor keeps the
+// correspondences the reference keeps (map point present and not bad, in index order) with mvP2D = mvKeysUn[i].pt,
+// mvP3Dw = GetWorldPos() and mvSigma2 = mvLevelSigma2[octave]; SetRansacParameters is lld_pnp_ransac_params plus
+// mvMaxError = mvSigma2 * th2 in float; iterate() draws its minimal sets of 4 on the host through RandomInt (the DUtils
+// formula on rand(), Sim3Solver::DefaultRandomInt, by default) and evaluates them on the device.  The solver state the
+// reference keeps between calls (mnIterations, mnBestInliers, mvbBestInliers, mBestTcw) lives here and is passed through
+// every call.  IterateBatch runs one Tracking::Relocalization round (iterate(nIterations) for every live candidate) in one
+// call; each solver's whole budget is drawn up front, so draws after an early success are consumed from the stream where
+// the reference would not consume them (include/lldba.h).
+class PnPsolver {
+ public:
+  std::function<int(int, int)> RandomInt = Sim3Solver::DefaultRandomInt;
+
+  PnPsolver(const Frame& F, const std::vector<MapPoint*>& vpMapPointMatches) : mN1((int)vpMapPointMatches.size()) {
+    for (size_t i = 0; i < vpMapPointMatches.size(); i++) {
+      MapPoint* pMP = vpMapPointMatches[i];
+      if (!pMP || pMP->isBad()) continue;
+      const KeyPoint& kp = F.mvKeysUn[i];
+      mvP2D.push_back(kp.x);
+      mvP2D.push_back(kp.y);
+      mvSigma2.push_back(F.mvLevelSigma2[(size_t)kp.octave]);
+      mvP3Dw.insert(mvP3Dw.end(), pMP->pos, pMP->pos + 3);
+      mvKeyPointIndices.push_back((int)i);
+    }
+    mCam[0] = F.fx; mCam[1] = F.fy; mCam[2] = F.cx; mCam[3] = F.cy;
+    N = (int)mvKeyPointIndices.size();
+    mvbBestInliers.assign((size_t)N, 0);
+    SetRansacParameters();
+  }
+
+  void SetRansacParameters(double probability = 0.99, int minInliers = 8, int maxIterations = 300, int minSet = 4,
+                           float epsilon = 0.4f, float th2 = 5.991f) {
+    int32_t o[2] = {minInliers, 1};
+    mLastError = lld_pnp_ransac_params(N, probability, minInliers, maxIterations, minSet, epsilon, o);
+    mRansacMinInliers = o[0];
+    mRansacMaxIts = o[1];
+    mvMaxError.resize(mvSigma2.size());
+    for (size_t i = 0; i < mvSigma2.size(); i++) mvMaxError[i] = mvSigma2[i] * th2;
+  }
+
+  // cv::Mat iterate(int nIterations, bool& bNoMore, vector<bool>& vbInliers, int& nInliers): true where the reference returns
+  // a pose (written to Tcw: R row-major, t).  A failed library call returns false with LastError() != 0.
+  bool iterate(void* ctx, int nIterations, bool& bNoMore, std::vector<bool>& vbInliers, int& nInliers, float Tcw[12]) {
+    std::vector<PnPsolver*> one{this};
+    mLastError = IterateBatch(ctx, one, nIterations);
+    bNoMore = mbNoMore;
+    vbInliers = mbFound ? mvbInliers : std::vector<bool>();
+    nInliers = mnInliers;
+    if (mbFound) std::memcpy(Tcw, mTcw, sizeof(mTcw));
+    return mbFound && mLastError == 0;
+  }
+
+  // One relocalisation round (iterate(nIterations) for every solver) in one lld_pnp_ransac call; each solver's outputs are
+  // read with Found() / NoMore() / Inliers() / NumInliers() / GetTcw().  Returns the library's status.
+  static int IterateBatch(void* ctx, const std::vector<PnPsolver*>& solvers, int nIterations) {
+    const int n = (int)solvers.size();
+    if (n == 0) return 0;
+    std::vector<float> cam, p2d, p3d, merr, bT;
+    std::vector<int32_t> mi, mx, its, best, off{0}, hoff{0}, hidx;
+    std::vector<uint8_t> bmask;
+    for (PnPsolver* S : solvers) {
+      cam.insert(cam.end(), S->mCam, S->mCam + 4);
+      mi.push_back(S->mRansacMinInliers);
+      mx.push_back(S->mRansacMaxIts);
+      its.push_back(S->mnIterations);
+      best.push_back(S->mnBestInliers);
+      p2d.insert(p2d.end(), S->mvP2D.begin(), S->mvP2D.end());
+      p3d.insert(p3d.end(), S->mvP3Dw.begin(), S->mvP3Dw.end());
+      merr.insert(merr.end(), S->mvMaxError.begin(), S->mvMaxError.end());
+      bmask.insert(bmask.end(), S->mvbBestInliers.begin(), S->mvbBestInliers.end());
+      bT.insert(bT.end(), S->mBestTcw, S->mBestTcw + 12);
+      off.push_back(off.back() + S->N);
+      const int B = S->N < S->mRansacMinInliers ? 0 : std::max(nIterations, S->mRansacMaxIts - S->mnIterations);
+      for (int h = 0; h < B; h++) {   // the minimal set of iterate(): swap-with-back from a fresh copy of mvAllIndices
+        std::vector<int> vAvailableIndices((size_t)S->N);
+        for (int i = 0; i < S->N; i++) vAvailableIndices[(size_t)i] = i;
+        for (int i = 0; i < 4; ++i) {
+          const int randi = S->RandomInt(0, (int)vAvailableIndices.size() - 1);
+          hidx.push_back(vAvailableIndices[(size_t)randi]);
+          vAvailableIndices[(size_t)randi] = vAvailableIndices.back();
+          vAvailableIndices.pop_back();
+        }
+      }
+      hoff.push_back(hoff.back() + B);
+    }
+    lld_pnp_ransac_problem p;
+    std::memset(&p, 0, sizeof(p));
+    p.n_problems = n; p.cam = cam.data(); p.min_inliers = mi.data(); p.max_its = mx.data(); p.its_done = its.data();
+    p.best_inliers = best.data(); p.off = off.data(); p.p2d = p2d.data(); p.p3dw = p3d.data(); p.max_err = merr.data();
+    p.best_mask = bmask.data(); p.best_Tcw = bT.data(); p.n_iterations = nIterations; p.hyp_off = hoff.data();
+    p.hyp_idx = hidx.data();
+    std::vector<uint8_t> found((size_t)n), no_more((size_t)n), inl((size_t)off.back() + 1);
+    std::vector<int32_t> n_in((size_t)n);
+    std::vector<float> T(12 * (size_t)n);
+    lld_pnp_ransac_result r;
+    std::memset(&r, 0, sizeof(r));
+    r.found = found.data(); r.no_more = no_more.data(); r.n_inliers = n_in.data(); r.Tcw = T.data(); r.inlier = inl.data();
+    r.its_done = its.data(); r.best_inliers = best.data(); r.best_mask = bmask.data(); r.best_Tcw = bT.data();
+    const int rc = lld_pnp_ransac(ctx, &p, &r);
+    if (rc) return rc;
+    for (int k = 0; k < n; k++) {
+      PnPsolver* S = solvers[(size_t)k];
+      const size_t e0 = (size_t)off[(size_t)k];
+      S->mnIterations = its[(size_t)k];
+      S->mnBestInliers = best[(size_t)k];
+      std::memcpy(S->mvbBestInliers.data(), bmask.data() + e0, (size_t)S->N);
+      std::memcpy(S->mBestTcw, &bT[12 * (size_t)k], sizeof(S->mBestTcw));
+      S->mbFound = found[(size_t)k] != 0;
+      S->mbNoMore = no_more[(size_t)k] != 0;
+      S->mnInliers = n_in[(size_t)k];
+      std::memcpy(S->mTcw, &T[12 * (size_t)k], sizeof(S->mTcw));
+      S->mvbInliers.assign((size_t)S->mN1, false);   // vbInliers over vpMapPointMatches (mvKeyPointIndices)
+      for (int i = 0; i < S->N; i++)
+        if (inl[e0 + (size_t)i]) S->mvbInliers[(size_t)S->mvKeyPointIndices[(size_t)i]] = true;
+    }
+    return 0;
+  }
+
+  bool Found() const { return mbFound; }
+  bool NoMore() const { return mbNoMore; }
+  const std::vector<bool>& Inliers() const { return mvbInliers; }
+  int NumInliers() const { return mnInliers; }
+  void GetTcw(float T[12]) const { std::memcpy(T, mTcw, sizeof(mTcw)); }
+  int LastError() const { return mLastError; }
+  int NumCorrespondences() const { return N; }
+  int MinInliers() const { return mRansacMinInliers; }
+  int MaxIterations() const { return mRansacMaxIts; }
+  int Iterations() const { return mnIterations; }
+
+ private:
+  int mN1, N = 0;
+  float mCam[4];
+  std::vector<float> mvP2D, mvP3Dw, mvSigma2, mvMaxError;
+  std::vector<int> mvKeyPointIndices;
+  int mRansacMinInliers = 8, mRansacMaxIts = 300, mnIterations = 0, mnBestInliers = 0;
+  std::vector<uint8_t> mvbBestInliers;
+  float mBestTcw[12] = {0};
+  bool mbFound = false, mbNoMore = false;
+  std::vector<bool> mvbInliers;
+  int mnInliers = 0, mLastError = 0;
+  float mTcw[12] = {0};
 };
 
 class ORBmatcher {

@@ -814,11 +814,12 @@ def rand_stream(seed):
             yield int(r)
 
 
-def draw_minimal_set(n, stream):
-    """Sim3Solver::iterate's draw: three indices by swap-with-back from a fresh copy of 0..n-1"""
+def draw_minimal_set(n, stream, size=3):
+    """the minimal-set draw of Sim3Solver::iterate (size 3) and PnPsolver::iterate (size 4): indices by swap-with-back from a
+    fresh copy of 0..n-1"""
     avail = list(range(n))
     out = []
-    for _ in range(3):
+    for _ in range(size):
         k = random_int(next(stream), 0, len(avail) - 1)
         out.append(avail[k])
         avail[k] = avail[-1]
@@ -879,6 +880,95 @@ def make_sim3_ransac_batch(n_problems, n_corr, seed, fix_scale=1, outlier_range=
              max_its=np.asarray([sim3_ransac_max_its_py(int(k), 0.99, min_inliers, 300) for k in N], np.int32),
              its_done=np.zeros(n_problems, np.int32), best_inliers=np.zeros(n_problems, np.int32), n_iterations=n_iterations)
     return draw_sim3_ransac_sets(p, rand_stream(seed))
+
+
+def pnp_ransac_params_py(n, probability=0.99, min_inliers=8, max_iterations=300, min_set=4, epsilon=0.4):
+    """PnPsolver::SetRansacParameters in Python: (mRansacMinInliers, mRansacMaxIts)"""
+    eps = np.float32(epsilon)
+    n_min = int(np.float32(np.float32(n) * eps))
+    n_min = max(n_min, min_inliers, min_set)
+    with np.errstate(all="ignore"):
+        ratio = np.float32(np.float32(n_min) / np.float32(n))
+    if eps < ratio:
+        eps = ratio
+    if n_min == n:
+        it = 1
+    else:
+        with np.errstate(all="ignore"):
+            x = np.float64(1 - probability)
+            v = np.log(x) / np.log(np.float64(1) - np.float64(eps) ** 3)
+            c = np.ceil(v)
+        it = -2**31 if not np.isfinite(c) and not c > 0 else (2**31 - 1 if c >= 2**31 - 1 else int(c))
+    return n_min, max(1, min(it, max_iterations))
+
+
+def pnp_ransac_budget(p):
+    """minimal sets lld_pnp_ransac expects per problem: N < min_inliers ? 0 : max(n_iterations, max_its - its_done)"""
+    N = np.diff(p["off"])
+    return np.where(N < p["min_inliers"], 0, np.maximum(p["n_iterations"], p["max_its"] - p["its_done"])).astype(np.int32)
+
+
+def draw_pnp_ransac_sets(p, stream):
+    """fills hyp_off / hyp_idx of p with each problem's budget of minimal sets of 4, drawn in problem order from stream"""
+    B = pnp_ransac_budget(p)
+    N = np.diff(p["off"])
+    idx = [draw_minimal_set(int(N[i]), stream, 4) for i in range(len(B)) for _ in range(int(B[i]))]
+    p["hyp_off"] = np.concatenate([[0], np.cumsum(B)]).astype(np.int32)
+    p["hyp_idx"] = np.ascontiguousarray(np.asarray(idx, np.int32).reshape(-1, 4))
+    return p
+
+
+def make_pnp_ransac_batch(n_problems, n_corr, seed, outlier_range=(0.05, 0.9), n_iterations=5, params=(0.99, 10, 300, 4, 0.5),
+                          th2=5.991, noise=1.0):
+    """PnPsolver as Tracking::Relocalization uses it (SetRansacParameters(0.99, 10, 300, 4, 0.5, 5.991)): per candidate a
+    camera pose among the first 100 keyframes of the KITTI trajectory (trajectory(), KITTI04-12 camera), world points from the §8(d) box (x in [-15, 15],
+    y in [-2, 3], z in [4, 60] m ahead of the camera) that project into the 1241 x 376 image, keypoints at their projections
+    with N(0, (noise 1.2^octave)^2) px noise (noise = 1 by default) rounded to float32, outliers as 2-D/3-D mismatches (p3dw swapped among a share of the
+    correspondences drawn per candidate from outlier_range), fresh solvers and each candidate's budget of minimal sets drawn
+    with DUtils' RandomInt from a seeded stream.  n_corr may be a list.  truth_Tcw holds the poses."""
+    rng = np.random.default_rng(seed)
+    ns = [int(n_corr)] * n_problems if np.isscalar(n_corr) else [int(k) for k in n_corr]
+    assert len(ns) == n_problems
+    sig2 = level_sigma2()
+    th2 = np.float32(th2)
+    starts = rng.integers(0, 100, n_problems)   # keyframe positions within the first 100 m of the trajectory
+    Rwc, twc = trajectory(100, rng)
+    Rwc, twc = Rwc[starts], twc[starts]
+    Rcw, tcw = _tcw(Rwc, twc)
+    p2d, p3dw, me, tru, off = [], [], [], [], [0]
+    for pb in range(n_problems):
+        m = ns[pb]
+        X = np.zeros((0, 3))
+        while len(X) < m:
+            Xl = np.stack([rng.uniform(-15, 15, 2 * m + 8), rng.uniform(-2, 3, 2 * m + 8), rng.uniform(4, 60, 2 * m + 8)], 1)
+            u = FX * Xl[:, 0] / Xl[:, 2] + CX
+            v = FY * Xl[:, 1] / Xl[:, 2] + CY
+            X = np.concatenate([X, Xl[(u >= 0) & (u < IMG_W) & (v >= 0) & (v < IMG_H)]])
+        Xc = X[:m]
+        Xw = f32((Rwc[pb] @ Xc.T).T + twc[pb])
+        Rf, tf = f32(Rcw[pb]), f32(tcw[pb])
+        Xc2 = Xw.astype(np.float64) @ Rf.astype(np.float64).T + tf
+        octv = rng.integers(0, N_LEVELS, m)
+        s = SCALE ** octv
+        uv = np.stack([FX * Xc2[:, 0] / Xc2[:, 2] + CX + rng.normal(0, noise, m) * s,
+                       FY * Xc2[:, 1] / Xc2[:, 2] + CY + rng.normal(0, noise, m) * s], 1)
+        bad = np.where(rng.random(m) < rng.uniform(*outlier_range))[0]
+        if len(bad) >= 2:
+            Xw[bad] = Xw[np.roll(bad, 1)]
+        p2d.append(f32(uv)); p3dw.append(Xw); me.append(f32(sig2[octv] * th2))
+        tru.append(np.concatenate([Rf.reshape(-1), tf]))
+        off.append(off[-1] + m)
+    N = np.diff(off)
+    prm = [pnp_ransac_params_py(int(k), *params) for k in N]
+    cat = lambda a, w: np.ascontiguousarray(f32(np.concatenate(a)).reshape(-1, w) if a else np.zeros((0, w), np.float32))  # noqa: E731
+    p = dict(n_problems=n_problems,
+             cam=np.ascontiguousarray(np.tile(f32([FX, FY, CX, CY]), (n_problems, 1))),
+             min_inliers=np.asarray([a for a, _ in prm], np.int32), max_its=np.asarray([b for _, b in prm], np.int32),
+             its_done=np.zeros(n_problems, np.int32), best_inliers=np.zeros(n_problems, np.int32), off=np.asarray(off, np.int32),
+             p2d=cat(p2d, 2), p3dw=cat(p3dw, 3), max_err=np.ascontiguousarray(cat(me, 1).reshape(-1)),
+             best_mask=np.zeros(max(off[-1], 0), np.uint8), best_Tcw=np.zeros((n_problems, 12), np.float32),
+             n_iterations=n_iterations, truth_Tcw=np.asarray(tru, np.float32).reshape(-1, 12))
+    return draw_pnp_ransac_sets(p, rand_stream(seed))
 
 
 def make_line_match_batch(n_pairs, n_lines, desc_dim, seed, tau=2.0, min_len=10, ragged=False):

@@ -1,6 +1,6 @@
 #!/usr/bin/env python
 """Timing of the SURVEY §8(f) kernels (ComputeStereoMatches, relocalisation / map-point SearchByProjection, temporal line
-association, distinctive descriptors, SearchForInitialization, OptimizeSim3, Sim3Solver): device compute time from the library's own CUDA events (host buffers in, results
+association, distinctive descriptors, SearchForInitialization, OptimizeSim3, Sim3Solver, PnPsolver): device compute time from the library's own CUDA events (host buffers in, results
 out through the public call), wall clock of the same call, and the CPU oracle on the same or a smaller sample.
 Prints one JSON object; results are compared with the oracle where the sample is the same.
 Usage: aux_kernels.py [section ...]   (default: every section)"""
@@ -206,4 +206,46 @@ if want("sim3_ransac"):
     res["nvidia_smi_name_power_limit"] = smi.strip()
     res["cpu"] = next((l.split(":", 1)[1].strip() for l in open("/proc/cpuinfo") if l.startswith("model name")), "")
     out["sim3_ransac"] = res
+# ---- PnPsolver (Tracking::Relocalization: SetRansacParameters(0.99, 10, 300, 4, 0.5, 5.991), iterate(5) per round)
+if want("pnp_ransac"):
+    import subprocess
+    import torch
+    from test_pnp_ransac import run_rounds
+    res = {}
+    ps = synth.make_pnp_ransac_batch(4096, 200, 801)
+    g, ms, wall = timed(lambda: api.pnp_ransac(ps, impl="gpu", ctx=ctx))
+    _, prof = ctx.profile(lambda: api.pnp_ransac(ps, impl="gpu", ctx=ctx))   # separate, profiled run: per-launch CUDA events
+    # relocalisation rounds of 5 over the same candidates (each round one call; draws on the host are not timed)
+    dev, calls = [], []
+    def gpu_round(q):
+        t0 = time.perf_counter(); o = api.pnp_ransac(q, impl="gpu", ctx=ctx); calls.append((time.perf_counter() - t0) * 1e3)
+        dev.append(ctx.last_timing()[1]); return o
+    fin, n_rounds = run_rounds(ps, gpu_round)
+    # the batch-of-one round (iterate(5) on one candidate) a caller without batching makes
+    p1 = synth.make_pnp_ransac_batch(1, 200, 811, outlier_range=(0.9, 0.9))
+    one = []
+    api.pnp_ransac(p1, impl="gpu", ctx=ctx)
+    for _ in range(50):
+        t0 = time.perf_counter(); api.pnp_ransac(p1, impl="gpu", ctx=ctx); one.append((time.perf_counter() - t0) * 1e3)
+    one_dev = ctx.last_timing()[1]
+    o1, t1 = cpu(lambda: [api.pnp_ransac(p1, impl="oracle") for _ in range(50)])
+    sub = synth.make_pnp_ransac_batch(4096, 200, 801)
+    o, tc = cpu(lambda: api.pnp_ransac(sub, impl="oracle"))
+    same = all(np.array_equal(g[k], o[k], equal_nan=True) for k in g)
+    fo, _ = run_rounds(ps, lambda q: api.pnp_ransac(q, impl="oracle"))
+    same_rounds = all(np.array_equal(fin[k], fo[k]) for k in fin)
+    res["reloc"] = {
+        "problems": 4096, "correspondences": 200, "minimal_sets_in_call": int(ps["hyp_off"][-1]),
+        "sets_evaluated": int((g["hyp_inliers"] >= 0).sum()), "found": int(g["found"].sum()),
+        "full_budget_one_call": {"device_ms": ms, "call_ms_from_host_buffers": wall, "problems_per_s_device": 4096 / ms * 1e3,
+                                 "kernel_profile_ms": {k: v["ms"] for k, v in prof.items()}, "cpu_oracle_ms": tc,
+                                 "identical_to_oracle": bool(same)},
+        "rounds_of_5": {"rounds": n_rounds, "device_ms_total": float(np.sum(dev)), "call_ms_total": float(np.sum(calls)),
+                        "first_round_call_ms": calls[0], "last_round_call_ms": calls[-1], "identical_to_oracle": bool(same_rounds)},
+        "batch_of_one_round_of_5": {"call_ms_median": float(np.median(one)), "device_ms": one_dev, "cpu_oracle_ms": t1 / 50}}
+    smi = subprocess.run(["nvidia-smi", "--query-gpu=name,power.limit", "--format=csv,noheader"], stdout=subprocess.PIPE, text=True).stdout
+    res["gpu"] = torch.cuda.get_device_name(0)
+    res["nvidia_smi_name_power_limit"] = smi.strip()
+    res["cpu"] = next((l.split(":", 1)[1].strip() for l in open("/proc/cpuinfo") if l.startswith("model name")), "")
+    out["pnp_ransac"] = res
 print(json.dumps(out))
